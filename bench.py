@@ -10,6 +10,10 @@ histogram + occurrence lists) and run mergeUntil to the configured number of mer
 with the corpus ids already resident in HBM; `e2e` runs the same step from pinned HOST buffers through
 bpe_add_documents / bpe_merge_until (H2D copy and log read-back inside the timed region).  The encode leg
 (bpe_encode_batch*) is timed the same way and reported under "encode".
+
+--dump-outputs DIR writes what the last timed steps returned, so that two builds can be compared output for output
+on the same seeded inputs: merge_log.npy (float64 [merges, 4]: a, b, c, weight of bpe_merge_until) and, on one GPU, a
+seeded sample of the device-resident encode (encode_docs.npy, encode_doc_lengths.npy: float64; encode_tokens.npy: float32).
 """
 from __future__ import annotations
 
@@ -28,6 +32,7 @@ _OUT = sys.stdout
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 WORKLOADS = {
     # name: (train bytes, merges, encode bytes)
@@ -40,6 +45,9 @@ WORKLOADS = {
     "tinyw": (200_000, 200, 200_000),
 }
 WORD_SEED, TRAIN_SEED, ENCODE_SEED, VOCAB = 42, 43, 44, 50000
+# --dump-outputs: documents of the encode text drawn with DUMP_SEED, as many as fit in DUMP_CHARS characters (a character
+# encodes to at most one token, so the sample stays under 32 MB of float32 and is the same set of documents for every build)
+DUMP_SEED, DUMP_CHARS = 45, 8_000_000
 
 
 def measured_peak():
@@ -266,6 +274,9 @@ def run_b200(args):
     l1 = stats().kernel_launches
     done = n_done.value
     weights = log["weight"][:done].copy()
+    dumps = {}
+    if args.dump_outputs:  # (the later steps overwrite `log`)
+        dumps["merge_log"] = np.stack([log[f][:done].astype(np.float64) for f in ("a", "b", "c", "weight")], axis=1)
     k1_ms = None
     s_before = stats()
     # K1 alone (ingest + histogram + lists), for its own roofline line
@@ -346,6 +357,8 @@ def run_b200(args):
     ms_enc = timed(encode_step_dev, args.steps)
     le1 = stats().kernel_launches
     k_out = n_out.value
+    if args.dump_outputs and world == 1:  # (at N > 1 every rank holds only its shard of the vectors)
+        dumps.update(encode_sample(out_dev[:k_out].cpu().numpy(), ooff_dev.cpu().numpy(), off2))
     enc_kernel_ms = stats().ms_encode
     encode_step_host()
     ms_enc_e2e = timed(encode_step_host, e2e_steps)
@@ -508,10 +521,30 @@ def run_b200(args):
             line["encode"]["full_output"] = enc_full
         if enc_cpu is not None:
             line["encode"]["cpu_baseline"] = enc_cpu
+        if args.dump_outputs:
+            write_dumps(args.dump_outputs, dumps)
         print(json.dumps(line), file=_OUT, flush=True)
     lib.bpe_destroy(h)
     if world > 1:
         dist.destroy_process_group()
+
+
+def encode_sample(values, offsets, in_offsets):
+    """The encoded vectors of a seeded sample of documents: values / offsets = the encode output, in_offsets = its input's."""
+    order = np.random.default_rng(DUMP_SEED).permutation(len(in_offsets) - 1)
+    keep = int(np.searchsorted(np.cumsum(np.diff(in_offsets)[order]), DUMP_CHARS, side="right"))
+    docs = np.sort(order[:keep])
+    lo, lens = offsets[docs], offsets[docs + 1] - offsets[docs]
+    idx = np.repeat(lo - (np.cumsum(lens) - lens), lens) + np.arange(int(lens.sum()))
+    return {"encode_docs": docs.astype(np.float64), "encode_doc_lengths": lens.astype(np.float64), "encode_tokens": values[idx].astype(np.float32)}
+
+
+def write_dumps(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "outputs larger than 64 MB"
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -703,7 +736,12 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=os.environ.get("BPE_BENCH_WORKLOAD", "cfg3"), choices=sorted(WORKLOADS))
     ap.add_argument("--merges", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the outputs of the last timed steps to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA engine (--impl b200)")
     # stdout carries ONE JSON line: anything native code writes to descriptor 1 on the way (NCCL's version banner) goes to stderr
     global _OUT
     sys.stdout.flush()

@@ -39,6 +39,52 @@ def test_reference_arm_prints_one_json_line_and_never_loads_the_product_library(
     assert "PRODUCT_LIB_MAPPED=0" in r.stderr, r.stderr[-500:]
 
 
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step_and_steps_sets_the_timed_steps(tmp_path):
+    """`--dump-outputs DIR`: the merge log of the last timed step (the CPU oracle's) and a seeded sample of the encode output (the
+    oracle's encoding of those documents), float .npy files, identical for any --steps; the timed launches scale with --steps."""
+    import numpy as np
+
+    from bpe_tokenizer_b200.synth import first_appearance_ids, synth_corpus
+    from oracle.fast_oracle import FastOracle
+    from oracle.int_oracle import IntOracle
+
+    lines, dumps = {}, {}
+    for steps in (1, 2):
+        out = tmp_path / ("steps%d" % steps)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--workload", "tiny", "--steps", str(steps), "--warmup", "1",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines[steps] = json.loads(r.stdout)
+        dumps[steps] = {f[:-4]: np.load(out / f) for f in sorted(os.listdir(out))}
+    assert lines[1]["steps"] == 1 and lines[2]["steps"] == 2
+    assert lines[2]["gpu_launches"] == 2 * lines[1]["gpu_launches"] > 0
+    d = dumps[2]
+    assert sorted(d) == ["encode_doc_lengths", "encode_docs", "encode_tokens", "merge_log"] and sorted(dumps[1]) == sorted(d)
+    assert all(np.array_equal(d[k], dumps[1][k]) for k in d)
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values()) and sum(a.nbytes for a in d.values()) <= 64 << 20
+
+    text, off = synth_corpus(200_000, seed=43)
+    ids, alphabet = first_appearance_ids(text)
+    o = FastOracle()
+    o.set_len16(np.ones(len(alphabet), dtype=np.int32))
+    o.add_documents(ids, off)
+    la, lb, lw = o.merge_until(2, 0, 200, len(alphabet), 200)
+    want = np.stack([la, lb, len(alphabet) + np.arange(len(la)), lw], axis=1).astype(np.float64)
+    assert len(la) == 200 and np.array_equal(d["merge_log"], want)
+
+    text2, off2 = synth_corpus(200_000, seed=44)
+    lut = np.full(256, -1, dtype=np.int32)
+    lut[alphabet] = np.arange(len(alphabet), dtype=np.int32)
+    enc = IntOracle()
+    enc.load_merges(want[:, :3].astype(np.int32))
+    docs, lens = d["encode_docs"].astype(np.int64), d["encode_doc_lengths"].astype(np.int64)
+    assert docs.size == len(off2) - 1  # 200 kB of text: the sample is every document
+    got = np.split(d["encode_tokens"].astype(np.int32), np.cumsum(lens)[:-1])
+    for doc, vec in zip(docs, got):
+        assert np.array_equal(vec, enc.encode(lut[text2[off2[doc]:off2[doc + 1]]])), doc
+
+
 @pytest.mark.parametrize("n", [1, 2, 4, 8])
 def test_committed_bench_lines_of_this_round(n):
     with open(os.path.join(ROOT, "profiles", "r02_bench_n%d.json" % n)) as f:
