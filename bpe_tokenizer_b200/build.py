@@ -41,7 +41,7 @@ def build(force: bool = False, verbose: bool = False, out: str = LIB) -> str:
         extra.append("-DBPE_ML_THREADS=" + os.environ["BPE_ML_THREADS"])  # tuning: threads per block of the loop kernels
     if os.environ.get("BPE_TBL_STRIDE"):
         extra.append("-DBPE_TBL_STRIDE=" + os.environ["BPE_TBL_STRIDE"])  # tuning: 8 = one 32-byte entry per pair-table slot
-    for knob in ("BPE_R_SMALL_LOG", "BPE_R_BATCH_LOG", "BPE_K1B_CHUNK_LOG"):  # tuning: size limits of a round's batch (round_kernels.cuh)
+    for knob in ("BPE_R_SMALL_LOG", "BPE_R_BATCH_LOG", "BPE_K1B_CHUNK_LOG", "BPE_STAGE_T"):  # tuning: size limits of a round's batch, staged neighbours (round_kernels.cuh)
         if os.environ.get(knob):
             extra.append("-D%s=%s" % (knob, os.environ[knob]))
     if os.environ.get("BPE_RD_THREADS"):

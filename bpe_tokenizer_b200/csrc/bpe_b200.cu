@@ -1041,7 +1041,8 @@ int append_docs_dev(bpe_engine* e, const int32_t* dev_ids, const int64_t* host_o
 int ensure_round_buffers(bpe_engine* e) {
   if (!e->round_blocks) {
     int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_merge_rounds, RD_THREADS, 0));
+    CK(cudaFuncSetAttribute(k_merge_rounds, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R_STAGE_BYTES));  // the staged cells
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_merge_rounds, RD_THREADS, R_STAGE_BYTES));
     if (per_sm < 1) return fail(e, BPE_E_CUDA, "k_merge_rounds does not fit on an SM");
     // (a decision folds RT partial entries per block with one thread each)
     const int most = std::min({e->sm_count * per_sm, (int)(R_QCAP / RT), RD_THREADS / RT});
@@ -1079,6 +1080,8 @@ RoundArgs round_args(bpe_engine* e, const LoopArgs& L, int round_k) {
   RA.gk = e->r_gk.p;
   RA.rs = e->r_state.p;
   RA.kmax = (uint32_t)round_k;
+  RA.stage_min = R_STAGE_MIN_DEFAULT;
+  if (const char* v = getenv("BPE_BLOCK_CELLS_MIN_SITES")) RA.stage_min = (uint32_t)std::max(0ll, std::min(atoll(v), 0xFFFFFFFFll));  // tuning / tests
   RA.bar_mode = 1;
   if (const char* v = getenv("BPE_LOOP_BAR")) RA.bar_mode = atoi(v) ? 1 : 0;
   RA.mg_on = 0;
@@ -1210,7 +1213,7 @@ int merge_until_device(bpe_engine* e, int64_t min_weight, int32_t max_length, in
       k_rounds_prepare<<<1, 32, 0, e->stream>>>(e->r_state.p);
       e->stats.kernel_launches++;
       void* rargs[] = {&RA};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), rargs, 0, e->stream);
+      ce = cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), rargs, R_STAGE_BYTES, e->stream);
     } else {
       void* args[] = {&L};
       ce = cudaLaunchCooperativeKernel((void*)k_merge_loop, dim3(e->loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
@@ -1490,7 +1493,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
       k_rounds_prepare<<<1, 32, 0, e->stream>>>(e->r_state.p);
       e->stats.kernel_launches++;
       void* rargs[] = {&RA};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), rargs, 0, e->stream);
+      ce = cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), rargs, R_STAGE_BYTES, e->stream);
     } else {
       // (rounds: the winner has more sites than the packed delta cells can count -- k_merge_loop_mg takes the merges above
       // R_HUGE, it stops, "done", at the first winner at or below it)

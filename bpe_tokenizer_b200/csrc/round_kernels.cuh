@@ -73,6 +73,18 @@ static_assert(BPE_R_SMALL_LOG <= 20, "a batched merge must fit the 21-bit fields
 constexpr uint32_t R_HUGE = 1u << 20;    // merges with more counted occurrences overflow the fields: they run through k_merge_loop
 constexpr uint32_t R_POOL_CHUNK = 1u << 16;  // occurrence-pool cells a block reserves at a time
 constexpr uint32_t R_LISTCAP = 32768;    // touched cells a block can list per round (more: the round falls back to scanning the rows)
+// Per-block staging of the cells of frequent neighbours: in P1 of a merge whose occurrence list is longer than
+// RoundArgs::stage_min, the cells of neighbour tokens below R_STAGE_T -- on Zipf text the characters and the earliest merges,
+// the neighbours of nearly every site of a big merge -- are summed in shared memory and added to the global cells ONCE per
+// block before P1's barrier (round_flush_stage), instead of by one returning ATOM per warp-iteration on a few hot L2 lines.
+#ifndef BPE_STAGE_T
+#define BPE_STAGE_T 256
+#endif
+constexpr uint32_t R_STAGE_T = BPE_STAGE_T;
+constexpr uint32_t R_STAGE_CELLS = RB * 2u * R_STAGE_T;  // [RB][2][R_STAGE_T] u64 cells, then as many u16 list entries
+constexpr size_t R_STAGE_BYTES = (size_t)R_STAGE_CELLS * (sizeof(unsigned long long) + sizeof(uint16_t));
+static_assert(R_STAGE_CELLS <= 65536u, "a staged cell's index must fit the 16-bit entries of the block's list");
+constexpr uint32_t R_STAGE_MIN_DEFAULT = 16384;  // list entries above which a merge stages its cells (measured: profiles/r03a)
 __host__ __device__ __forceinline__ uint32_t cell_dec(unsigned long long v) { return (uint32_t)(v & R_FMASK); }
 __host__ __device__ __forceinline__ uint32_t cell_len(unsigned long long v) { return (uint32_t)((v >> R_FIELD) & R_FMASK); }
 __host__ __device__ __forceinline__ uint32_t cell_cnt(unsigned long long v) { return (uint32_t)((v >> (2 * R_FIELD)) & R_FMASK); }
@@ -119,6 +131,7 @@ struct RoundArgs {
   uint32_t* gk;      // [RT * blocks] ... and the pair key of that slot
   RoundState* rs;
   uint32_t kmax;     // merges per round (1 .. RB)
+  uint32_t stage_min;  // a merge whose occurrence list is longer stages its frequent neighbours' cells per block (R_STAGE_T)
   // corpus sharded by document over several GPUs (mg_kernels.cuh): the counts of the pair table are global and replicated, the
   // cells above hold THIS shard's deltas; once per round every rank stores its non-empty cells as records into every rank's
   // inbox over NVLink, and every rank sums all records into gcells -- the global deltas P2 then works from
@@ -273,6 +286,7 @@ struct RoundSm {
   uint32_t g_n_keys, g_pool_cursor, g_snap_err, g_abort;
   uint32_t gv[8];  // sharded: the folded header values (OR of the ranks' error flags, minima of their capacities)
   uint32_t ncell[2];  // cells this block touched first in the round of either parity (entries of its list)
+  uint32_t nstage;    // staged cells this block touched in the current P1 (entries of r_stage_list)
   uint32_t gncell[2]; // sharded: global cells this block touched first while summing the ranks' records
   uint32_t rec_base, rec_cnt;  // sharded: where this block's records go in the inboxes, how many they are
   uint32_t mg_mask, mg_cnt[MG_MAX_WORLD];  // sharded: senders whose message is complete and not summed yet, their records
@@ -314,12 +328,44 @@ __device__ __forceinline__ Top2 top2_block_reduce(Top2 v, Top2* s_t2) {
   return top2_warp_reduce(u);
 }
 
+// the block's staged cells (dynamic shared memory of k_merge_rounds, R_STAGE_BYTES): [RB][2][R_STAGE_T] packed cells, then the
+// list of those the block touched in the current P1 (index (merge * 2 + side) * R_STAGE_T + token)
+extern __shared__ __align__(16) unsigned long long r_stage[];
+__device__ __forceinline__ uint16_t* r_stage_list() { return reinterpret_cast<uint16_t*>(r_stage + R_STAGE_CELLS); }
+
+// All 32 lanes call; each `first` lane found the global cell of (js = merge * 2 + side, tok) empty: it lists the cell for P2
+// (one shared-memory counter bump per warp).  c is the merge's new token, partner its a (side 0) or b (side 1).
+__device__ __forceinline__ void cell_list_first(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t js, uint32_t tok, bool first, uint32_t c,
+                                                uint32_t partner) {
+  const uint32_t lane = lane_id();
+  const uint32_t fm = __ballot_sync(0xFFFFFFFFu, first);
+  if (!fm) return;
+  uint32_t base = 0;
+  const int src = __ffs(fm) - 1;
+  if ((int)lane == src) base = atomicAdd(&S.ncell[par], (uint32_t)__popc(fm));
+  base = __shfl_sync(0xFFFFFFFFu, base, src);
+  if (first) {
+    const uint32_t k = base + __popc(fm & ((1u << lane) - 1u));
+    if (k < R_LISTCAP) round_list(R, par)[k] = (js << 16) | tok;
+    else R.rs->overflow[par] = 1;
+    // P2 will probe the pair table for the born pair (tok, c) / (c, tok) and for the old pair (tok, a) / (b, tok): ask for
+    // their home slots now, so that they sit in L2 by then (hints only)
+    const PairTable& t = R.L.A.t;
+    const uint32_t side = js & 1u;
+    prefetch_l2(t.keys + tbl_hash(t, side ? pair_key(c, tok) : pair_key(tok, c)));
+    const uint32_t h2 = tbl_hash(t, side ? pair_key(partner, tok) : pair_key(tok, partner));
+    prefetch_l2(t.keys + h2);
+    prefetch_l2(t.cnt + h2);
+  }
+}
+
 // All 32 lanes call; `has` lanes contribute to the cell of `tok`: a decrement (dec), an occurrence of the born pair (newp),
-// a counted occurrence (counted).  Lanes that agree on tok elect a leader which issues ONE 64-bit atomic for all of them; the
-// lane that finds the cell empty lists it for P2 (one shared-memory counter bump per warp).  Returns the leader's counted
-// occurrences (0 elsewhere): the ingredient of the born-pair bound.
+// a counted occurrence (counted).  Lanes that agree on tok elect a leader which issues ONE 64-bit atomic for all of them: into
+// the block's staged cell when the merge stages (`staged`, warp-uniform) and tok < R_STAGE_T -- the first toucher appends it
+// to the block's list, round_flush_stage lists it globally --, else into the global cell, whose first toucher lists it.
+// Returns the leader's counted occurrences (0 elsewhere): the ingredient of the born-pair bound.
 __device__ __forceinline__ uint32_t cell_add_warp(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t js, unsigned long long* cells, uint32_t tok, bool has,
-                                                  bool dec, bool newp, bool counted, uint32_t c, uint32_t partner, uint32_t epar) {
+                                                  bool dec, bool newp, bool counted, uint32_t c, uint32_t partner, bool staged) {
   const uint32_t lane = lane_id();
   const uint32_t peers = __match_any_sync(0xFFFFFFFFu, has ? tok : (0xFFFFFF00u + lane));
   const uint32_t dmask = __ballot_sync(0xFFFFFFFFu, has && dec);
@@ -332,29 +378,38 @@ __device__ __forceinline__ uint32_t cell_add_warp(const RoundArgs& R, RoundSm& S
     nc = (uint32_t)__popc(peers & cmask);
     nd = (uint32_t)__popc(peers & dmask);
     const unsigned long long add = (unsigned long long)nd | ((unsigned long long)__popc(peers & nmask) << R_FIELD) | ((unsigned long long)nc << (2 * R_FIELD));
-    first = atomicAdd(cells + tok, add) == 0ull;
-  }
-  const uint32_t fm = __ballot_sync(0xFFFFFFFFu, first);
-  if (fm) {
-    uint32_t base = 0;
-    const int src = __ffs(fm) - 1;
-    if ((int)lane == src) base = atomicAdd(&S.ncell[par], (uint32_t)__popc(fm));
-    base = __shfl_sync(0xFFFFFFFFu, base, src);
-    if (first) {
-      const uint32_t k = base + __popc(fm & ((1u << lane) - 1u));
-      if (k < R_LISTCAP) round_list(R, par)[k] = (js << 16) | tok;
-      else R.rs->overflow[par] = 1;
-      // P2 will probe the pair table for the born pair (tok, c) / (c, tok) and for the old pair (tok, a) / (b, tok): ask for
-      // their home slots now, so that they sit in L2 by then (hints only)
-      const PairTable& t = R.L.A.t;
-      const uint32_t side = js & 1u;
-      prefetch_l2(t.keys + tbl_hash(t, side ? pair_key(c, tok) : pair_key(tok, c)));
-      const uint32_t h2 = tbl_hash(t, side ? pair_key(partner, tok) : pair_key(tok, partner));
-      prefetch_l2(t.keys + h2);
-      prefetch_l2(t.cnt + h2);
+    if (staged && tok < R_STAGE_T) {
+      const uint32_t e = js * R_STAGE_T + tok;
+      if (atomicAdd(&r_stage[e], add) == 0ull) r_stage_list()[atomicAdd(&S.nstage, 1u)] = (uint16_t)e;
+    } else {
+      first = atomicAdd(cells + tok, add) == 0ull;
     }
   }
+  cell_list_first(R, S, par, js, tok, first, c, partner);
   return nc;
+}
+
+// End of P1 in this block (all its threads call): every staged cell the block touched goes into its global cell with one
+// atomic, and is zeroed for the next round; the block that finds a global cell empty lists it, as cell_add_warp does -- so
+// P2 and the exchange of the sharded engine see the same cells and lists as without staging.  (Per-block sums of a merge's
+// counts fit the 21-bit fields: its totals do, R_HUGE.)
+__device__ __forceinline__ void round_flush_stage(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t c_first) {
+  __syncthreads();
+  const uint32_t ns = S.nstage;
+  const uint16_t* list = r_stage_list();
+  for (uint32_t i0 = threadIdx.x & ~31u; i0 < ns; i0 += blockDim.x) {
+    const uint32_t i = i0 + lane_id();
+    const bool has = i < ns;
+    const uint32_t e = has ? list[i] : 0u;
+    const uint32_t js = e / R_STAGE_T, tok = e - js * R_STAGE_T, j = js >> 1;
+    bool first = false;
+    if (has) {
+      const unsigned long long v = r_stage[e];
+      r_stage[e] = 0ull;
+      first = atomicAdd(round_cells(R, par, j, js & 1u) + tok, v) == 0ull;
+    }
+    cell_list_first(R, S, par, js, tok, first, c_first + j, (js & 1u) ? S.b[j] : S.a[j]);
+  }
 }
 
 // ---- sharded corpus: the message of a round ----
@@ -641,13 +696,14 @@ __device__ __forceinline__ void mgr_collect(const RoundArgs& R, RoundSm& S, uint
 // The logic of the neighbourhoods is phase_sites' (train_kernels.cuh); what differs is where the deltas go (the merge's
 // dense rows) and the virtual neighbours c_i of the earlier merges of the batch.
 __device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t j, uint32_t c_first,
-                                                 uint32_t i, SiteRec* site_out, uint32_t sites_cap, uint32_t epar) {
+                                                 uint32_t i, SiteRec* site_out, uint32_t sites_cap) {
   const ApplyArgs& A = R.L.A;
   const uint32_t* slots = A.slots;
   const uint32_t n = A.n;
   DevState* st = A.st;
   const uint32_t a = S.a[j], b = S.b[j], c = c_first + j;
   const uint32_t total = S.llen[j];
+  const bool staged = total > R.stage_min;
   const uint32_t lane = lane_id();
   unsigned long long* const cells_l = round_cells(R, par, j, 0);
   unsigned long long* const cells_r = round_cells(R, par, j, 1);
@@ -748,8 +804,8 @@ __device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S,
   // one atomic per distinct left neighbour: the born pair (new1_tok, c), with the decrement when it concerns the same token
   // (it does unless the site is chained to the one on its left: then the decrement is (b,a)'s and goes out on its own)
   const bool dec1_same = dec1 && dec1_tok == new1_tok;
-  const uint32_t nc1 = cell_add_warp(R, S, par, j * 2u, cells_l, new1_tok, new1, dec1_same, true, new1_counted, c, a, epar);
-  if (__any_sync(0xFFFFFFFFu, dec1 && !dec1_same)) cell_add_warp(R, S, par, j * 2u, cells_l, dec1_tok, dec1 && !dec1_same, true, false, false, c, a, epar);
+  const uint32_t nc1 = cell_add_warp(R, S, par, j * 2u, cells_l, new1_tok, new1, dec1_same, true, new1_counted, c, a, staged);
+  if (__any_sync(0xFFFFFFFFu, dec1 && !dec1_same)) cell_add_warp(R, S, par, j * 2u, cells_l, dec1_tok, dec1 && !dec1_same, true, false, false, c, a, staged);
   rec.lslot = new1 ? new1_tok : R_NOTOK;
 
   // ---- adjacency on the right of the new token (left to the next site when that one is chained) ----
@@ -794,8 +850,8 @@ __device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S,
     }
   }
   const bool dec2_same = dec2 && new2 && dec2_tok == new2_tok;  // (always, when there is a decrement: kept general)
-  const uint32_t nc2 = cell_add_warp(R, S, par, j * 2u + 1u, cells_r, new2_tok, new2, dec2_same, true, true, c, b, epar);
-  if (__any_sync(0xFFFFFFFFu, dec2 && !dec2_same)) cell_add_warp(R, S, par, j * 2u + 1u, cells_r, dec2_tok, dec2 && !dec2_same, true, false, false, c, b, epar);
+  const uint32_t nc2 = cell_add_warp(R, S, par, j * 2u + 1u, cells_r, new2_tok, new2, dec2_same, true, true, c, b, staged);
+  if (__any_sync(0xFFFFFFFFu, dec2 && !dec2_same)) cell_add_warp(R, S, par, j * 2u + 1u, cells_r, dec2_tok, dec2 && !dec2_same, true, false, false, c, b, staged);
   rec.rslot = new2 ? new2_tok : R_NOTOK;
   // upper bounds of the born pairs' counts: the largest group of lanes that share a neighbour, summed over the warps
   const uint32_t u1 = __reduce_max_sync(0xFFFFFFFFu, nc1), u2 = __reduce_max_sync(0xFFFFFFFFu, nc2);
@@ -954,7 +1010,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
     }
     if (tid < RB) S.fill_n[tid] = 0;
     if (tid < 2) S.ncell[tid] = S.gncell[tid] = 0;
-    if (tid == 0) S.pool_next = S.pool_end = S.keys_ins = 0;
+    if (tid == 0) S.pool_next = S.pool_end = S.keys_ins = S.nstage = 0;
+    for (uint32_t i = tid; i < R_STAGE_CELLS; i += blockDim.x) r_stage[i] = 0ull;  // (each flush zeroes what it adds)
   }
   // sharded: exchanges completed so far (the peers' flags keep counting across launches), what the previous round may have
   // taken from the pool since the headers were written
@@ -1313,7 +1370,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         for (uint32_t wi = bid * ws + warp; wi < iters; wi += nblk * ws) {
           uint32_t j = 0;
           while (j + 1 < k && wi >= S.iter0[j + 1]) j++;
-          round_sites_iter(R, S, par, j, c_first, (wi - S.iter0[j]) * 32u + lane, round_sites_buf(R, par, j), j == 0 ? A.sites_cap : R_SMALL, (uint32_t)((mg_epoch + 1) & 1u));
+          round_sites_iter(R, S, par, j, c_first, (wi - S.iter0[j]) * 32u + lane, round_sites_buf(R, par, j), j == 0 ? A.sites_cap : R_SMALL);
         }
         if (!split) {
           if (F.v) round_fill_all(R, S, F, gt, gn);
@@ -1343,9 +1400,13 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           }
         }
       }
+      bool staging = false;
+      for (uint32_t j = 0; j < k; j++) staging |= S.llen[j] > R.stage_min;
+      if (staging) round_flush_stage(R, S, par, c_first);
     }
     RPROF(1)
     RBARRIER();
+    if (tid == 0) S.nstage = 0;  // (every thread of the block has read it: RBARRIER ends with __syncthreads)
     RPROF(2)
     if (R.mg_on) {
       // ================= sharded: one exchange per round =================
