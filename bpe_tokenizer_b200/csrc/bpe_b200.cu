@@ -434,9 +434,11 @@ int build_index(bpe_engine* e) {
   if (n) {
     k_alloc_lists<<<e->grid(4), 256, 0, e->stream>>>(e->table(), e->d_st.p, (uint32_t)e->pool.cap);
     CKL();
-    int k1b_per_sm = 8;
-    if (const char* v = getenv("BPE_K1B_PER_SM")) k1b_per_sm = std::max(1, std::min(atoi(v), 8));  // tuning knob
-    k_scatter<<<e->grid(k1b_per_sm), K1_THREADS, 0, e->stream>>>(e->slots.p, (uint32_t)n, e->table(), e->pool.p, e->d_st.p);
+    int k1b_per_sm = 0;
+    CK(cudaFuncSetAttribute(k_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1B_SMEM_BYTES));  // the staging buffer
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k1b_per_sm, k_scatter, K1B_THREADS, K1B_SMEM_BYTES));
+    if (k1b_per_sm < 1) return fail(e, BPE_E_CUDA, "k_scatter does not fit on an SM");
+    k_scatter<<<e->grid(k1b_per_sm), K1B_THREADS, K1B_SMEM_BYTES, e->stream>>>(e->slots.p, (uint32_t)n, e->table(), e->pool.p, e->d_st.p);
     CKL();
   }
   CK(cudaEventRecord(e->ev1, e->stream));

@@ -146,16 +146,31 @@ __global__ void k_mark_docstarts(uint32_t* __restrict__ slots, const int64_t* __
 constexpr int K1_THREADS = 256;
 constexpr int K1_SMEM_SLOTS = 2048;  // 24 KB
 constexpr int K1_MAX_PROBE = 8;
+// 2^15 positions: 96 KB of shared memory per block, two 1024-thread blocks per SM (9.1 ms for K1 on cfg3 against 10.1 ms
+// with 2^16 and one block per SM; profiles/r04a_k1b_staged.md)
 #ifndef BPE_K1B_CHUNK_LOG
-#define BPE_K1B_CHUNK_LOG 16
+#define BPE_K1B_CHUNK_LOG 15
 #endif
+static_assert(BPE_K1B_CHUNK_LOG >= 10 && BPE_K1B_CHUNK_LOG <= 16, "k_scatter stages 16-bit offsets within a chunk");
 constexpr uint32_t K1B_CHUNK = 1u << BPE_K1B_CHUNK_LOG;  // positions per block iteration of the scatter
+constexpr int K1B_THREADS = 1024;
+static_assert(K1_SMEM_SLOTS % K1B_THREADS == 0 && K1B_THREADS % 32 == 0, "the prefix gives every thread whole slots");
 
 struct SmemHist {
   uint32_t key[K1_SMEM_SLOTS];
-  uint32_t a[K1_SMEM_SLOTS];  // k_hist: adjacencies seen        k_scatter: ticket counter
+  uint32_t a[K1_SMEM_SLOTS];  // k_hist: adjacencies seen        k_scatter: count, then staging cursor
   uint32_t b[K1_SMEM_SLOTS];  // k_hist: of which NOT counted    k_scatter: base cell in the pool
 };
+
+// k_scatter's dynamic shared memory: the block-local table, where each slot's run starts in the staging buffer, and the
+// staging buffer itself (the chunk's adjacencies as 16-bit offsets, grouped by slot)
+struct SmemScatter {
+  SmemHist h;
+  uint32_t start[K1_SMEM_SLOTS + 1];
+  uint32_t warp_sum[K1B_THREADS / 32];
+  uint16_t stage[K1B_CHUNK];
+};
+constexpr size_t K1B_SMEM_BYTES = sizeof(SmemScatter);
 
 // slot of `key` in the block-local table (inserting it), or -1 when the neighbourhood is crowded
 __device__ __forceinline__ int sh_slot(SmemHist& sh, uint32_t key, bool insert) {
@@ -281,22 +296,35 @@ __global__ void k_alloc_lists(PairTable t, DevState* st, uint32_t pool_cap) {
   }
 }
 
-// K1b: scatter every adjacency's position into its pair's list.  Per 64 Ki-position chunk a block counts its
-// adjacencies per pair in shared memory, reserves one contiguous range per pair with a single global atomic,
-// then hands out cells with shared-memory tickets (the chunk is re-read from L2).
-__global__ void __launch_bounds__(K1_THREADS) k_scatter(const uint32_t* __restrict__ slots, uint32_t n, PairTable t,
-                                                         uint32_t* __restrict__ pool, DevState* st) {
-  __shared__ SmemHist sh;
-  uint32_t n_chunks = (n + K1B_CHUNK - 1) / K1B_CHUNK;
+// K1b: scatter every adjacency's position into its pair's list.  Per chunk of K1B_CHUNK positions a block
+//  1. counts the chunk's adjacencies per pair in its shared table;
+//  2. lays the pairs' runs out back to back in a shared staging buffer (an exclusive prefix of the counts) and reserves
+//     one range per pair in the pool with a single global atomic;
+//  3. re-reads the chunk (from L2) and puts each adjacency's 16-bit offset into its pair's run with a shared ticket;
+//  4. copies the staging buffer out with consecutive threads on consecutive cells of one range, so that a range leaves
+//     as whole sectors plus at most two partial edges.  Stored one adjacency at a time, the cells of a range reach the
+//     L2 spread over the whole time the block spends on the chunk, and partly written sectors go back to HBM as
+//     read-modify-writes.
+// A pair that found no room in the shared table takes one global cursor atomic per adjacency and stores directly.
+// The order of the cells inside a range follows the tickets and is not deterministic; no reader of the lists depends on it.
+__global__ void __launch_bounds__(K1B_THREADS) k_scatter(const uint32_t* __restrict__ slots, uint32_t n, PairTable t,
+                                                          uint32_t* __restrict__ pool, DevState* st) {
+  extern __shared__ __align__(16) unsigned char k1b_smem[];
+  SmemScatter& sh = *reinterpret_cast<SmemScatter*>(k1b_smem);
+  constexpr int PER = K1_SMEM_SLOTS / K1B_THREADS;  // slots per thread in the prefix
+  constexpr int WARPS = K1B_THREADS / 32;
+  const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
+  const uint32_t n_chunks = (n + K1B_CHUNK - 1) / K1B_CHUNK;
   for (uint32_t chunk = blockIdx.x; chunk < n_chunks; chunk += gridDim.x) {
-    for (int i = threadIdx.x; i < K1_SMEM_SLOTS; i += K1_THREADS) {
-      sh.key[i] = EMPTY_KEY;
-      sh.a[i] = 0;
+    for (int i = threadIdx.x; i < K1_SMEM_SLOTS; i += K1B_THREADS) {
+      sh.h.key[i] = EMPTY_KEY;
+      sh.h.a[i] = 0;
     }
     __syncthreads();
-    uint32_t g_begin = chunk * (K1B_CHUNK >> 2);
-    uint32_t g_end = min((n + 3) >> 2, g_begin + (K1B_CHUNK >> 2));
-    for (uint32_t g = g_begin + threadIdx.x; g < g_end; g += K1_THREADS) {
+    const uint32_t c0 = chunk * K1B_CHUNK;
+    const uint32_t g_begin = c0 >> 2;
+    const uint32_t g_end = min((n + 3) >> 2, g_begin + (K1B_CHUNK >> 2));
+    for (uint32_t g = g_begin + threadIdx.x; g < g_end; g += K1B_THREADS) {
       uint32_t p0 = g << 2;
       uint32_t v[5];
       load_group(slots, n, g, v);
@@ -304,26 +332,58 @@ __global__ void __launch_bounds__(K1_THREADS) k_scatter(const uint32_t* __restri
       for (int j = 0; j < 4; j++) {
         uint32_t key;
         if (p0 + j < n && edge_at(slots, n, p0 + j, v[j], v[j + 1], &key, nullptr)) {
-          int h = sh_slot(sh, key, true);
-          if (h >= 0) atomicAdd(&sh.a[h], 1u);
+          int h = sh_slot(sh.h, key, true);
+          if (h >= 0) atomicAdd(&sh.h.a[h], 1u);
         }
       }
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < K1_SMEM_SLOTS; i += K1_THREADS) {
-      uint32_t key = sh.key[i];
-      if (key == EMPTY_KEY) continue;
-      uint32_t gs = tbl_find(t, key);
-      if (gs == NOSLOT) {
-        atomicOr(&st->err, ERR_MISSING_KEY);
-        sh.b[i] = NOPOS;
-      } else {
-        sh.b[i] = t.occ_start[gs] + atomicAdd(t.occ_fill + gs, sh.a[i]);
+    // exclusive prefix of the counts: thread i owns slots PER*i .. PER*i + PER-1
+    const int i0 = threadIdx.x * PER;
+    uint32_t cnt[PER], sum = 0;
+#pragma unroll
+    for (int e = 0; e < PER; e++) {
+      cnt[e] = sh.h.a[i0 + e];
+      sum += cnt[e];
+    }
+    uint32_t inc = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      uint32_t y = __shfl_up_sync(0xFFFFFFFFu, inc, o);
+      if (lane >= (uint32_t)o) inc += y;
+    }
+    if (lane == 31) sh.warp_sum[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+      uint32_t w = lane < (uint32_t)WARPS ? sh.warp_sum[lane] : 0u, wi = w;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        uint32_t y = __shfl_up_sync(0xFFFFFFFFu, wi, o);
+        if (lane >= (uint32_t)o) wi += y;
       }
-      sh.a[i] = 0;
+      if (lane < (uint32_t)WARPS) sh.warp_sum[lane] = wi - w;
     }
     __syncthreads();
-    for (uint32_t g = g_begin + threadIdx.x; g < g_end; g += K1_THREADS) {
+    uint32_t run = sh.warp_sum[warp] + inc - sum;
+#pragma unroll
+    for (int e = 0; e < PER; e++) {
+      const int i = i0 + e;
+      sh.start[i] = run;
+      if (cnt[e]) {  // (every key in the table has a count)
+        uint32_t gs = tbl_find(t, sh.h.key[i]);
+        if (gs == NOSLOT) {
+          atomicOr(&st->err, ERR_MISSING_KEY);
+          sh.h.b[i] = NOPOS;
+        } else {
+          sh.h.b[i] = t.occ_start[gs] + atomicAdd(t.occ_fill + gs, cnt[e]);
+        }
+      }
+      sh.h.a[i] = run;  // staging cursor
+      run += cnt[e];
+    }
+    if (threadIdx.x == K1B_THREADS - 1) sh.start[K1_SMEM_SLOTS] = run;
+    __syncthreads();
+    for (uint32_t g = g_begin + threadIdx.x; g < g_end; g += K1B_THREADS) {
       uint32_t p0 = g << 2;
       uint32_t v[5];
       load_group(slots, n, g, v);
@@ -331,10 +391,9 @@ __global__ void __launch_bounds__(K1_THREADS) k_scatter(const uint32_t* __restri
       for (int j = 0; j < 4; j++) {
         uint32_t key;
         if (p0 + j < n && edge_at(slots, n, p0 + j, v[j], v[j + 1], &key, nullptr)) {
-          int h = sh_slot(sh, key, false);
+          int h = sh_slot(sh.h, key, false);
           if (h >= 0) {
-            uint32_t base = sh.b[h];
-            if (base != NOPOS) pool[base + atomicAdd(&sh.a[h], 1u)] = p0 + j;
+            sh.stage[atomicAdd(&sh.h.a[h], 1u)] = (uint16_t)(p0 + j - c0);
           } else {  // pair did not fit the block-local table: one global cursor atomic
             uint32_t gs = tbl_find(t, key);
             if (gs == NOSLOT) atomicOr(&st->err, ERR_MISSING_KEY);
@@ -342,6 +401,16 @@ __global__ void __launch_bounds__(K1_THREADS) k_scatter(const uint32_t* __restri
           }
         }
       }
+    }
+    __syncthreads();
+    const uint32_t total = sh.start[K1_SMEM_SLOTS];
+    for (uint32_t k = threadIdx.x; k < total; k += K1B_THREADS) {
+      uint32_t s = 0;  // the last slot whose run starts at or before k: the slot whose run holds k
+#pragma unroll
+      for (uint32_t half = K1_SMEM_SLOTS / 2; half; half >>= 1)
+        if (sh.start[s + half] <= k) s += half;
+      const uint32_t base = sh.h.b[s];
+      if (base != NOPOS) pool[base + (k - sh.start[s])] = c0 + sh.stage[k];
     }
     __syncthreads();
   }
