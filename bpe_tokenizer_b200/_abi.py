@@ -20,6 +20,7 @@ class BpeError(RuntimeError):
     def __init__(self, code: int, message: str):
         super().__init__(f"{_CODE_NAMES.get(code, code)}: {message}")
         self.code = code
+        self.message = message
 
 
 class bpe_merge(C.Structure):
@@ -68,6 +69,8 @@ SYMBOLS = {
     "bpe_decode_batch": (C.c_int, [vp, i32p, i64p, C.c_int64, i32p, C.c_int32, u8p, i64p, C.c_int32, u8p, C.c_int64, i64p, i64p, i64p]),
     "bpe_set_chars": (C.c_int, [vp, i32p, i32p, C.c_int32]),
     "bpe_add_text": (C.c_int, [vp, u8p, i64p, C.c_int64, i32p, C.c_int32, i32p, i64p, C.c_int64]),
+    "bpe_add_text_stage": (C.c_int, [vp, u8p, i64p, C.c_int64, i32p, i64p, C.c_int32, i32p]),
+    "bpe_add_text_commit": (C.c_int, [vp, i32p, C.c_int32, i64p, C.c_int64]),
     "bpe_debug_lane_table": (C.c_int, [i32p, C.c_int64, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, C.c_int64, i64p]),
     "bpe_debug_plan_chunks": (C.c_int, [i64p, C.c_int64, C.c_int64, i64p, C.c_int64, i64p, i64p]),
     "bpe_encode_text_batch": (C.c_int, [vp, u8p, i64p, C.c_int64, i32p, C.c_int32, i32p, C.c_int64, i64p, i64p, i64p, i64p, i32p]),

@@ -229,6 +229,11 @@ struct bpe_engine {
   DevBuf<unsigned long long> x_counts;
   DevBuf<uint32_t> x_doccnt;
   DevBuf<uint64_t> x_docoff;
+  // bpe_add_text_stage -> bpe_add_text_commit: the decoded batch waits in x_ids (placeholders for its new code points) with its
+  // document boundaries in h_rel.  Every other call that reuses those buffers, or replaces the character table, drops it.
+  bool txt_staged = false;
+  int64_t txt_chars = 0, txt_docs = 0;
+  std::vector<int32_t> txt_new;  // the staged batch's new code points, ascending
 
   // staging of the host-buffer encode / restore calls (grow-only, reused across calls)
   DevBuf<int32_t> x_ids, x_out, x_tvi;
@@ -2182,6 +2187,7 @@ int bpe_encode_batch_dev(bpe_engine* e, const int32_t* dev_ids, const int64_t* d
 
 // host buffers in, host buffers out: stage through grow-only device buffers owned by the engine
 int stage_encode_inputs(bpe_engine* e, const int32_t* ids, const int64_t* doc_offsets, int64_t n_docs, int64_t* total_out, int64_t* max_len_out) {
+  e->txt_staged = false;  // x_ids / h_rel are about to be reused
   int64_t base = n_docs ? doc_offsets[0] : 0, total = n_docs ? doc_offsets[n_docs] - base : 0;
   if (total > 0 && !ids) return fail(e, BPE_E_INVALID, "null ids");
   int64_t max_len = 0;
@@ -2299,6 +2305,7 @@ int text_decode_dev(bpe_engine* e, const uint8_t* d_text, int64_t nbytes, const 
 // and e->h_rel (host)
 int text_to_ids(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs, bool track_new, int64_t* n_chars,
                 unsigned long long* unknown) {
+  e->txt_staged = false;
   TRY(check_offsets(e, doc_byte_offsets, n_docs));
   TRY(ensure_cpmap(e));
   int64_t base = n_docs ? doc_byte_offsets[0] : 0, nbytes = n_docs ? doc_byte_offsets[n_docs] - base : 0;
@@ -2388,6 +2395,7 @@ int64_t pipe_want(const PipePlan& P, int64_t index, int64_t remaining) {
 int encode_pipeline(bpe_engine* e, const bool is_text, const int32_t* ids, const uint8_t* utf8, const int64_t* off, int64_t n_docs,
                     const int32_t* to_vector_index, int32_t n_tvi, int32_t* out, int64_t out_cap, int64_t* out_offsets, int64_t* first_bad,
                     int64_t* n_out, int64_t* unknown_pos, int32_t* unknown_code_point) {
+  e->txt_staged = false;
   const int64_t base = off[0];
   if (off[n_docs] < base) return fail(e, BPE_E_INVALID, "document offsets must be non-decreasing");
   const int64_t total = off[n_docs] - base;
@@ -2552,6 +2560,7 @@ int bpe_decode_batch(bpe_engine* e, const int32_t* values, const int64_t* doc_of
                      int32_t n_fvi, const uint8_t* token_bytes, const int64_t* token_byte_offsets, int32_t n_tokens, uint8_t* out,
                      int64_t out_cap, int64_t* out_offsets, int64_t* first_bad, int64_t* n_out) {
   if (!e || !n_out || !out_offsets || n_tokens < 0 || (n_tokens > 0 && (!token_byte_offsets))) return fail(e, BPE_E_INVALID, "bad decode arguments");
+  e->txt_staged = false;
   TRY(check_offsets(e, doc_offsets, n_docs));
   CK(cudaSetDevice(e->device));
   int64_t base = n_docs ? doc_offsets[0] : 0, total = n_docs ? doc_offsets[n_docs] - base : 0;
@@ -2621,6 +2630,7 @@ int bpe_decode_batch(bpe_engine* e, const int32_t* values, const int64_t* doc_of
 // ---- text in, tokens out ---------------------------------------------------------------------------------------------
 int bpe_set_chars(bpe_engine* e, const int32_t* code_points, const int32_t* indices, int32_t n) {
   if (!e || n < 0 || (n > 0 && (!code_points || !indices))) return fail(e, BPE_E_INVALID, "bad character table");
+  e->txt_staged = false;  // its ids were resolved against the table being replaced
   CK(cudaSetDevice(e->device));
   TRY(ensure_cpmap(e));
   CK(cudaMemsetAsync(e->d_cpmap.p, 0xFF, (size_t)CP_LIMIT * 4, e->stream));
@@ -2637,19 +2647,14 @@ int bpe_set_chars(bpe_engine* e, const int32_t* code_points, const int32_t* indi
   return BPE_OK;
 }
 
-int bpe_add_text(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs, int32_t* new_code_points, int32_t new_cap,
-                 int32_t* n_new, int64_t* counts, int64_t counts_cap) {
-  if (!e || !n_new) return fail(e, BPE_E_INVALID, "bad arguments");
+int bpe_add_text_stage(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs, int32_t* new_code_points,
+                       int64_t* first_pos, int32_t new_cap, int32_t* n_new) {
+  if (!e || !n_new || new_cap < 0 || (new_cap > 0 && (!new_code_points || !first_pos))) return fail(e, BPE_E_INVALID, "bad arguments");
   *n_new = 0;
   CK(cudaSetDevice(e->device));
   int64_t n_chars = 0;
-  const bool trace_t = getenv("BPE_TRACE") != nullptr;
-  auto clk = [] { return std::chrono::steady_clock::now(); };
-  auto since = [&](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(clk() - t).count(); };
-  auto tt0 = clk();
   TRY(text_to_ids(e, utf8, doc_byte_offsets, n_docs, true, &n_chars, nullptr));
-  const double ms_ids = since(tt0);
-  // unknown code points become tokens in first-appearance order (core.ts:186-199)
+  // the unknown code points with their first positions; k_collect_new_cps resets d_firstpos as it reads it
   DevBuf<uint32_t> d_cp, d_pos, d_n;
   const uint32_t cap = 1u << 16;
   CK(d_cp.reserve(cap));
@@ -2666,50 +2671,114 @@ int bpe_add_text(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_off
     *n_new = (int32_t)nn;
     return fail(e, BPE_E_CAPACITY, "%u new characters, room for %d", nn, new_cap);
   }
-  std::vector<uint32_t> cps(nn), pos(nn);
+  std::vector<uint32_t> cps(nn), pos(nn), order(nn);
   if (nn) {
     CK(cudaMemcpy(cps.data(), d_cp.p, (size_t)nn * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(pos.data(), d_pos.p, (size_t)nn * 4, cudaMemcpyDeviceToHost));
-    std::vector<uint32_t> order(nn);
-    for (uint32_t i = 0; i < nn; i++) order[i] = i;
-    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return pos[a] < pos[b]; });
-    std::vector<int32_t> h_cp(nn), h_idx(nn);
-    for (uint32_t k = 0; k < nn; k++) {
-      h_cp[k] = (int32_t)cps[order[k]];
-      h_idx[k] = e->n_tokens + (int32_t)k;
-      new_code_points[k] = h_cp[k];
-      e->h_len16.push_back(h_cp[k] >= 0x10000 ? 2 : 1);  // `chars.length` in UTF-16 units (core.ts:272)
+  }
+  // reported in first-appearance order (the collection order is arbitrary)
+  for (uint32_t i = 0; i < nn; i++) order[i] = i;
+  std::sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return pos[x] < pos[y]; });
+  e->txt_new.resize(nn);
+  for (uint32_t k = 0; k < nn; k++) {
+    new_code_points[k] = (int32_t)cps[order[k]];
+    first_pos[k] = (int64_t)pos[order[k]];
+    e->txt_new[k] = (int32_t)cps[k];
+  }
+  std::sort(e->txt_new.begin(), e->txt_new.end());
+  *n_new = (int32_t)nn;
+  e->txt_chars = n_chars;
+  e->txt_docs = n_docs;
+  e->txt_staged = true;
+  return BPE_OK;
+}
+
+int bpe_add_text_commit(bpe_engine* e, const int32_t* code_points, int32_t n, int64_t* counts, int64_t counts_cap) {
+  if (!e) return BPE_E_INVALID;
+  if (!e->txt_staged) return fail(e, BPE_E_INVALID, "no staged text batch: bpe_add_text_stage first (another call since then reused its buffers)");
+  if (n < 0 || (n > 0 && !code_points)) return fail(e, BPE_E_INVALID, "bad code point list");
+  CK(cudaSetDevice(e->device));
+  // the list comes from outside the library (another rank's exchange): check it before anything changes
+  std::vector<int32_t> sorted(code_points, code_points + n);
+  std::sort(sorted.begin(), sorted.end());
+  for (int32_t i = 0; i < n; i++) {
+    if ((uint32_t)sorted[i] >= CP_LIMIT) return fail(e, BPE_E_INVALID, "code point %d is not a Unicode code point", sorted[i]);
+    if (i && sorted[i] == sorted[i - 1]) return fail(e, BPE_E_INVALID, "code point U+%04X is listed twice", sorted[i]);
+  }
+  for (int32_t cp : e->txt_new)
+    if (!std::binary_search(sorted.begin(), sorted.end(), cp)) return fail(e, BPE_E_INVALID, "the list misses U+%04X, a new character of the staged batch", cp);
+  DevBuf<int32_t> a, b;
+  if (n) {
+    std::vector<int32_t> known((size_t)n);
+    CK(a.reserve((size_t)n));
+    CK(b.reserve((size_t)n));
+    CK(cudaMemcpyAsync(a.p, code_points, (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+    k_get_cpmap<<<(n + 255) / 256, 256, 0, e->stream>>>(e->d_cpmap.p, a.p, b.p, (uint32_t)n);
+    CKL();
+    CK(cudaMemcpyAsync(known.data(), b.p, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    for (int32_t k = 0; k < n; k++)
+      if (known[k] >= 0) return fail(e, BPE_E_INVALID, "code point U+%04X already is token %d", code_points[k], known[k]);
+  }
+  if ((int64_t)e->n_tokens + n > BPE_MAX_TOKENS) return fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
+  if (counts && counts_cap < (int64_t)e->n_tokens + n)
+    return fail(e, BPE_E_CAPACITY, "counts holds %lld entries, need %d", (long long)counts_cap, e->n_tokens + n);
+  e->txt_staged = false;
+  if (n) {
+    // code_points[k] becomes token n_tokens + k (core.ts:186-199)
+    std::vector<int32_t> h_idx((size_t)n);
+    for (int32_t k = 0; k < n; k++) {
+      h_idx[k] = e->n_tokens + k;
+      e->h_len16.push_back(code_points[k] >= 0x10000 ? 2 : 1);  // `chars.length` in UTF-16 units (core.ts:272)
     }
-    e->n_tokens += (int32_t)nn;
+    e->n_tokens += n;
     e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
     TRY(sync_len16(e));
-    DevBuf<int32_t> a, b;
-    CK(a.reserve(nn));
-    CK(b.reserve(nn));
-    CK(cudaMemcpyAsync(a.p, h_cp.data(), (size_t)nn * 4, cudaMemcpyHostToDevice, e->stream));
-    CK(cudaMemcpyAsync(b.p, h_idx.data(), (size_t)nn * 4, cudaMemcpyHostToDevice, e->stream));
-    k_set_cpmap<<<(nn + 255) / 256, 256, 0, e->stream>>>(e->d_cpmap.p, a.p, b.p, nn);
+    CK(cudaMemcpyAsync(b.p, h_idx.data(), (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
+    k_set_cpmap<<<(n + 255) / 256, 256, 0, e->stream>>>(e->d_cpmap.p, a.p, b.p, (uint32_t)n);
     CKL();
     CK(cudaStreamSynchronize(e->stream));
   }
-  *n_new = (int32_t)nn;
-  if (counts_cap < e->n_tokens && counts) return fail(e, BPE_E_CAPACITY, "counts holds %lld entries, need %d", (long long)counts_cap, e->n_tokens);
   CK(e->x_counts.reserve((size_t)std::max(e->n_tokens, 1)));
   CK(cudaMemsetAsync(e->x_counts.p, 0, (size_t)std::max(e->n_tokens, 1) * 8, e->stream));
-  if (n_chars) {
-    k_fix_and_count<<<e->grid(8), 256, 0, e->stream>>>(e->x_ids.p, (uint64_t)n_chars, e->d_cpmap.p, e->x_counts.p, (uint32_t)e->n_tokens);
+  if (e->txt_chars) {
+    k_fix_and_count<<<e->grid(8), 256, 0, e->stream>>>(e->x_ids.p, (uint64_t)e->txt_chars, e->d_cpmap.p, e->x_counts.p, (uint32_t)e->n_tokens);
     CKL();
   }
   if (counts) CK(cudaMemcpyAsync(counts, e->x_counts.p, (size_t)e->n_tokens * 8, cudaMemcpyDeviceToHost, e->stream));
   CK(cudaStreamSynchronize(e->stream));
-  const double ms_fix = since(tt0) - ms_ids;
-  int rc_app = append_docs_dev(e, e->x_ids.p, e->h_rel.data(), n_docs);
+  return append_docs_dev(e, e->x_ids.p, e->h_rel.data(), e->txt_docs);
+}
+
+int bpe_add_text(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs, int32_t* new_code_points, int32_t new_cap,
+                 int32_t* n_new, int64_t* counts, int64_t counts_cap) {
+  if (!e || !n_new) return fail(e, BPE_E_INVALID, "bad arguments");
+  *n_new = 0;
+  const bool trace_t = getenv("BPE_TRACE") != nullptr;
+  auto clk = [] { return std::chrono::steady_clock::now(); };
+  auto since = [&](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(clk() - t).count(); };
+  auto tt0 = clk();
+  // one engine holds the whole batch: its own first-appearance order is the global one
+  std::vector<int32_t> cps(1u << 16);
+  std::vector<int64_t> pos(1u << 16);
+  int32_t nn = 0;
+  TRY(bpe_add_text_stage(e, utf8, doc_byte_offsets, n_docs, cps.data(), pos.data(), (int32_t)cps.size(), &nn));
+  const double ms_stage = since(tt0);
+  if (nn > new_cap) {
+    e->txt_staged = false;
+    *n_new = nn;
+    return fail(e, BPE_E_CAPACITY, "%d new characters, room for %d", nn, new_cap);
+  }
+  std::copy(cps.begin(), cps.begin() + nn, new_code_points);  // (stage reports them in first-appearance order)
+  const int64_t n_chars = e->txt_chars;
+  int rc = bpe_add_text_commit(e, cps.data(), nn, counts, counts_cap);
+  if (rc == BPE_OK) *n_new = nn;
   if (trace_t) {
     cudaStreamSynchronize(e->stream);
-    fprintf(stderr, "[bpe] add_text: %lld chars: copy in + decode %.1f ms, new characters + counts %.1f ms, append %.1f ms\n", (long long)n_chars, ms_ids, ms_fix,
-            since(tt0) - ms_ids - ms_fix);
+    fprintf(stderr, "[bpe] add_text: %lld chars: copy in + decode + new characters %.1f ms, commit (table, counts, append) %.1f ms\n", (long long)n_chars,
+            ms_stage, since(tt0) - ms_stage);
   }
-  return rc_app;
+  return rc;
 }
 
 int bpe_encode_text_batch(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs, const int32_t* to_vector_index,

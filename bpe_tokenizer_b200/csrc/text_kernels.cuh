@@ -148,6 +148,11 @@ __global__ void k_set_cpmap(int32_t* __restrict__ cpmap, const int32_t* __restri
     if ((uint32_t)cps[i] < CP_LIMIT) cpmap[cps[i]] = idx[i];
 }
 
+// the table's current entries for n code points (all < CP_LIMIT): bpe_add_text_commit refuses to reassign a known one
+__global__ void k_get_cpmap(const int32_t* __restrict__ cpmap, const int32_t* __restrict__ cps, int32_t* __restrict__ out, uint32_t n) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[i] = cpmap[cps[i]];
+}
+
 constexpr uint32_t FIX_SMEM_TOKENS = 2048;
 // resolve the -(cp + 1) placeholders after the new tokens got their indices; count every token (weights, core.ts:201-202)
 __global__ void k_fix_and_count(int32_t* __restrict__ ids, uint64_t n, const int32_t* __restrict__ cpmap, unsigned long long* __restrict__ counts,

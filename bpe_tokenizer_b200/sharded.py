@@ -10,6 +10,9 @@ constructs the tokenizer on its own device and calls the same methods in the sam
   (rank, local position) -- what the reference's position tie-break needs (core.ts:294-305).
 * ``addDocuments(ids, offsets, local_shard=True)`` is the bulk form for corpora too large to replicate: each rank
   passes only its own documents (rank order = document order); character weights are summed over the group.
+* ``addTextBatch(utf8, offsets, local_shard=True)`` is the same from raw UTF-8 text: each rank decodes its shard on its
+  device (bpe_add_text_stage), the ranks exchange their new characters with their first positions and order them by
+  (rank, position), and every rank appends its shard with that one global order (bpe_add_text_commit).
 * ``mergeUntil`` first sums the pair histograms of all shards (one all-gather of (pair, count) lists over NCCL), then
   runs the persistent sharded kernel (csrc/mg_kernels.cuh): count deltas travel GPU to GPU over NVLink inside the
   kernel, the arg-max is replicated, every rank returns the same merge log and replays it on its host table.
@@ -18,7 +21,7 @@ constructs the tokenizer on its own device and calls the same methods in the sam
 from __future__ import annotations
 
 import ctypes as C
-from typing import List, Optional, Sequence, Tuple
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -83,6 +86,79 @@ def exchange_pair_counts(lib, handle, rank: int, world: int, device, group=None)
     for q in peers:
         g = gathered[q]
         check(lib.bpe_mg_import_counts(handle, C.c_void_p(g[0].data_ptr()), C.c_void_p(g[1].data_ptr()), sizes[q], int(q == peers[-1])))
+
+
+def order_new_chars(per_rank: Sequence[Tuple[Sequence[int], Sequence[int]]]) -> List[int]:
+    """The new characters of a sharded text batch in the global first-appearance order of core.ts:186-199.
+    per_rank[r] = (code_points, first_pos) as rank r's engine reported them, positions local to its shard.  Ranks hold
+    contiguous document ranges in rank order, so the order key is (rank, first_pos) and a character that several ranks
+    report belongs to the first of them, whatever its local positions."""
+    seen, out = set(), []
+    for cps, pos in per_rank:
+        cps = np.asarray(cps, dtype=np.int64).reshape(-1)
+        pos = np.asarray(pos, dtype=np.int64).reshape(-1)
+        for k in np.argsort(pos, kind="stable").tolist():
+            cp = int(cps[k])
+            if cp not in seen:
+                seen.add(cp)
+                out.append(cp)
+    return out
+
+
+def _error_of(ex: Exception) -> Tuple[int, str]:
+    if isinstance(ex, BpeError):
+        return ex.code, ex.message
+    return _abi.BPE_E_INTERNAL, repr(ex)
+
+
+def text_ingest_collective(stage: Callable[[], Tuple[Sequence[int], Sequence[int]]], commit: Callable[[List[int]], np.ndarray],
+                           n_tokens: int, world: int, group=None, device=None) -> Tuple[List[int], np.ndarray]:
+    """The rank-side protocol of a sharded text ingest.  stage() decodes this rank's shard and returns its new
+    characters with their local first positions; commit(code_points) appends the shard with the agreed characters and
+    returns its counts (int64, n_tokens + len(code_points)).  -> (new characters in global order, counts summed over
+    the ranks).  Two collectives on success: a gather of every rank's status and list, an all-reduce of the counts.
+    A failure on any rank raises the same BpeError on every rank, and no rank is left waiting in a collective: a stage
+    failure travels with the lists, a commit failure as a flag after the counts (then one more gather names it)."""
+    import torch
+    import torch.distributed as dist
+
+    err: Optional[Tuple[int, str]] = None
+    cps: Sequence[int] = []
+    pos: Sequence[int] = []
+    try:
+        cps, pos = stage()
+    except Exception as ex:  # (every rank must reach the gather below)
+        err = _error_of(ex)
+    mine = (err, [int(c) for c in cps], [int(p) for p in pos])
+    parts = [mine]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, mine, group=group)
+    for e in parts:
+        if e[0] is not None:
+            raise BpeError(*e[0])  # the first failing rank's error, on every rank
+    new = order_new_chars([(p[1], p[2]) for p in parts])
+    if n_tokens + len(new) > _abi.BPE_MAX_TOKENS:  # judged on the global count, identically everywhere
+        raise BpeError(_abi.BPE_E_DOMAIN, "token table would exceed %d entries (%d new characters over %d ranks)" % (_abi.BPE_MAX_TOKENS, len(new), world))
+    counts = np.zeros(n_tokens + len(new) + 1, dtype=np.int64)  # [-1]: ranks whose commit failed
+    try:
+        counts[:-1] = np.asarray(commit(new), dtype=np.int64)[: n_tokens + len(new)]
+    except Exception as ex:
+        err = _error_of(ex)
+        counts[:] = 0
+        counts[-1] = 1
+    if world > 1:
+        nccl = dist.get_backend(group) == "nccl"
+        t = torch.from_numpy(counts).to(device if nccl else "cpu")
+        dist.all_reduce(t, group=group)
+        counts = t.cpu().numpy()
+    if counts[-1]:
+        errs = [err]
+        if world > 1:
+            errs = [None] * world
+            dist.all_gather_object(errs, err, group=group)
+        raise BpeError(*next(e for e in errs if e is not None))
+    return new, counts[:-1]
 
 
 class ShardedBPETokenizer(BPETokenizer):
@@ -163,10 +239,40 @@ class ShardedBPETokenizer(BPETokenizer):
         self._check(self._lib.bpe_restore_documents(self._h, p32(ids), p64(off), hi - lo))
         self._uploaded = True
 
-    def addTextBatch(self, utf8: bytes, doc_byte_offsets: np.ndarray) -> None:
-        # the device-side ingest assigns first-appearance indices over the documents it is given; a rank that only sees
-        # its shard cannot reproduce the global order of core.ts:186-199
-        raise BpeError(_abi.BPE_E_INVALID, "addTextBatch is not available on a sharded corpus; use addToCorpus or addDocuments")
+    def addTextBatch(self, utf8: bytes, doc_byte_offsets: np.ndarray, local_shard: bool = False) -> None:
+        """Bulk addToCorpus from UTF-8 text (core.ts:182-207), bit-exact with one engine holding the whole batch.
+        local_shard=False: every rank passes ALL documents and keeps a contiguous range balanced by bytes;
+        local_shard=True: the arguments hold only this rank's documents (ranks in document order).  Each rank decodes
+        its own shard on its device; the ranks then agree on the new characters' global first-appearance order (a list
+        of at most 65 536 entries per rank, whatever the corpus size) and each appends its shard with it."""
+        def stage():
+            self._flush()
+            if self._uploaded:
+                raise BpeError(_abi.BPE_E_INVALID, self._ONCE)
+            self._sync_chars()
+            off = np.ascontiguousarray(doc_byte_offsets, dtype=np.int64)
+            self._check_offsets(off, len(utf8))
+            lo, hi = 0, len(off) - 1
+            if not local_shard:
+                b = shard_bounds(np.diff(off), self.world)
+                lo, hi = b[self.rank], b[self.rank + 1]
+            mine = np.ascontiguousarray(off[lo:hi + 1])
+            buf = np.frombuffer(utf8, dtype=np.uint8) if len(utf8) else np.zeros(1, dtype=np.uint8)
+            cps = np.empty(1 << 16, dtype=np.int32)
+            pos = np.empty(1 << 16, dtype=np.int64)
+            n = C.c_int32()
+            self._check(self._lib.bpe_add_text_stage(self._h, buf.ctypes.data_as(_abi.u8p), p64(mine), hi - lo, p32(cps), p64(pos), cps.size, C.byref(n)))
+            return cps[: n.value], pos[: n.value]
+
+        def commit(new: List[int]) -> np.ndarray:
+            cps = np.asarray(new, dtype=np.int32)
+            counts = np.zeros(len(self.token_table) + cps.size, dtype=np.int64)
+            self._check(self._lib.bpe_add_text_commit(self._h, p32(cps), cps.size, p64(counts), counts.size))
+            return counts
+
+        new, counts = text_ingest_collective(stage, commit, len(self.token_table), self.world, self._group, self._torch_device)
+        self._uploaded = True
+        self._add_text_tokens(new, counts)
 
     @property
     def corpus_in_code(self) -> List[str]:  # this rank's shard (corpusIdsAllRanks gathers every shard)

@@ -289,6 +289,21 @@ class BPETokenizer:
         self._check(self._lib.bpe_set_chars(self._h, p32(cps), p32(idx), len(cps)))
         self._chars_synced = len(self.char_to_token)
 
+    def _add_text_tokens(self, new_code_points: Sequence[int], counts: np.ndarray) -> None:
+        """Host half of a text ingest: the tokens the engine just appended for the new characters, in its order
+        (core.ts:188-199), then the batch's occurrence counts of every token (core.ts:201-202)."""
+        for cp in new_code_points:
+            index = len(self.token_table)
+            token = Token(chr(cp), 0, 0, chr(index + 1), index)
+            self.char_to_token[token.chars] = token
+            self.code_to_token[token.code] = token
+            self.token_table.append(token)
+        self._chars_synced = len(self.char_to_token)
+        for i in np.nonzero(counts[: len(self.token_table)])[0]:
+            t = self.token_table[i]
+            t.weight += int(counts[i])
+            t.original_weight += int(counts[i])
+
     def addTextBatch(self, utf8: bytes, doc_byte_offsets: np.ndarray) -> None:
         """addToCorpus (core.ts:182-207) for many documents given as UTF-8 bytes, with the code-point loop, the
         first-appearance token creation and the weight counts done on the device.  Equivalent to calling
@@ -303,17 +318,7 @@ class BPETokenizer:
         n_new = C.c_int32()
         self._check(self._lib.bpe_add_text(self._h, buf.ctypes.data_as(_abi.u8p), p64(doc_byte_offsets), len(doc_byte_offsets) - 1,
                                            p32(new_cps), new_cps.size, C.byref(n_new), p64(counts), counts.size))
-        for cp in new_cps[: n_new.value].tolist():  # the same tokens the engine just appended (core.ts:188-199)
-            index = len(self.token_table)
-            token = Token(chr(cp), 0, 0, chr(index + 1), index)
-            self.char_to_token[token.chars] = token
-            self.code_to_token[token.code] = token
-            self.token_table.append(token)
-        self._chars_synced = len(self.char_to_token)
-        for i in np.nonzero(counts[: len(self.token_table)])[0]:
-            t = self.token_table[i]
-            t.weight += int(counts[i])
-            t.original_weight += int(counts[i])
+        self._add_text_tokens(new_cps[: n_new.value].tolist(), counts)
         # like addToCorpus (core.ts:182-207) this does NOT invalidate the vector index: a following encodeToVector with a
         # stale index throws `unknown token index` for the new characters, exactly as the reference does
 

@@ -240,6 +240,21 @@ int bpe_set_chars(bpe_engine* e, const int32_t* code_points, const int32_t* indi
  * (the `weight++ / original_weight++` of core.ts:201-202). */
 int bpe_add_text(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs,
                  int32_t* new_code_points, int32_t new_cap, int32_t* n_new, int64_t* counts, int64_t counts_cap);
+/* bpe_add_text in two steps, for a corpus sharded over engines whose ranks must agree on ONE first-appearance order
+ * (bpe_add_text is exactly stage, then commit of the list stage reported).
+ * Step 1 on one rank: decode the batch into the engine's staging buffers and report the code points the character
+ * table does not know, each with its first position (code-point index within the batch), in first-appearance order.
+ * Nothing is added to the corpus or the vocabulary yet.  BPE_E_CAPACITY stores the required new_cap in *n_new;
+ * BPE_E_DOMAIN when the new characters alone would take the table past BPE_MAX_TOKENS. */
+int bpe_add_text_stage(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs,
+                       int32_t* new_code_points, int64_t* first_pos, int32_t new_cap, int32_t* n_new);
+/* Step 2: code_points[i] becomes token n_tokens + i.  The list must hold every code point the staged batch reported and
+ * may hold others (those only other ranks saw).  Appends the staged documents; counts as in bpe_add_text (this batch only,
+ * counts_cap >= n_tokens + n).  Changes nothing and returns BPE_E_INVALID when no batch is staged, or when the list misses a
+ * code point the batch reported, repeats one, or names one the table already knows; BPE_E_DOMAIN when n_tokens + n would
+ * exceed BPE_MAX_TOKENS.  Every other call that reuses the staging buffers (encode, decode, restore, another stage) or
+ * replaces the character table (bpe_set_chars) discards the staged batch. */
+int bpe_add_text_commit(bpe_engine* e, const int32_t* code_points, int32_t n, int64_t* counts, int64_t counts_cap);
 /* bpe_encode_batch with the char -> index step on the device.  An unknown character fails the call with
  * BPE_E_INVALID (the reference throws `unknown token, char: ...`, core.ts:398-400); *unknown_pos / *unknown_code_point
  * (optional) identify the first one (code-point index within the batch). */
