@@ -1076,6 +1076,13 @@ int ensure_round_buffers(bpe_engine* e) {
   return BPE_OK;
 }
 
+// a merge whose occurrence list is longer than this stages its frequent neighbours' deltas and list cells per block
+// (LoopArgs::stage_min, read where each LoopArgs is built)
+uint32_t stage_min_knob() {
+  if (const char* v = getenv("BPE_BLOCK_CELLS_MIN_SITES")) return (uint32_t)std::max(0ll, std::min(atoll(v), 0xFFFFFFFFll));  // tuning / tests
+  return R_STAGE_MIN_DEFAULT;
+}
+
 RoundArgs round_args(bpe_engine* e, const LoopArgs& L, int round_k) {
   RoundArgs RA{};
   RA.L = L;
@@ -1087,8 +1094,6 @@ RoundArgs round_args(bpe_engine* e, const LoopArgs& L, int round_k) {
   RA.gk = e->r_gk.p;
   RA.rs = e->r_state.p;
   RA.kmax = (uint32_t)round_k;
-  RA.stage_min = R_STAGE_MIN_DEFAULT;
-  if (const char* v = getenv("BPE_BLOCK_CELLS_MIN_SITES")) RA.stage_min = (uint32_t)std::max(0ll, std::min(atoll(v), 0xFFFFFFFFll));  // tuning / tests
   RA.bar_mode = 1;
   if (const char* v = getenv("BPE_LOOP_BAR")) RA.bar_mode = atoi(v) ? 1 : 0;
   RA.mg_on = 0;
@@ -1203,6 +1208,7 @@ int merge_until_device(bpe_engine* e, int64_t min_weight, int32_t max_length, in
     }
     const char* pf = getenv("BPE_LOOP_PREFETCH");  // read per launch: a tuning knob
     L.prefetch = pf ? std::max(0, std::min(atoi(pf), 2)) : (use_rounds ? 0 : 1);  // (k_merge_rounds: measured, the helper warps become the tail)
+    L.stage_min = stage_min_knob();
     L.replay = dev_replay ? dev_replay + 2 * done : nullptr;
     if (dev_replay) e->hot_valid = false;  // replayed merges do not feed the hot list
     static const bool trace = getenv("BPE_TRACE") != nullptr;
@@ -1481,6 +1487,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
     L.max_tokens = BPE_MAX_TOKENS;
     L.tbl_cap = e->tbl_cap;
     L.replay = nullptr;
+    L.stage_min = stage_min_knob();
     P.M = mg_args(e);
     static const bool trace = getenv("BPE_TRACE") != nullptr;
     auto tw0 = std::chrono::steady_clock::now();

@@ -73,18 +73,12 @@ static_assert(BPE_R_SMALL_LOG <= 20, "a batched merge must fit the 21-bit fields
 constexpr uint32_t R_HUGE = 1u << 20;    // merges with more counted occurrences overflow the fields: they run through k_merge_loop
 constexpr uint32_t R_POOL_CHUNK = 1u << 16;  // occurrence-pool cells a block reserves at a time
 constexpr uint32_t R_LISTCAP = 32768;    // touched cells a block can list per round (more: the round falls back to scanning the rows)
-// Per-block staging of the cells of frequent neighbours: in P1 of a merge whose occurrence list is longer than
-// RoundArgs::stage_min, the cells of neighbour tokens below R_STAGE_T -- on Zipf text the characters and the earliest merges,
-// the neighbours of nearly every site of a big merge -- are summed in shared memory and added to the global cells ONCE per
-// block before P1's barrier (round_flush_stage), instead of by one returning ATOM per warp-iteration on a few hot L2 lines.
-#ifndef BPE_STAGE_T
-#define BPE_STAGE_T 256
-#endif
-constexpr uint32_t R_STAGE_T = BPE_STAGE_T;
+// Per-block staging of the cells of frequent neighbours (R_STAGE_T, train_kernels.cuh): in P1 of a merge whose occurrence list
+// is longer than LoopArgs::stage_min, their cells are summed in shared memory and added to the global cells ONCE per block
+// before P1's barrier (round_flush_stage), instead of by one returning ATOM per warp-iteration on a few hot L2 lines.
 constexpr uint32_t R_STAGE_CELLS = RB * 2u * R_STAGE_T;  // [RB][2][R_STAGE_T] u64 cells, then as many u16 list entries
 constexpr size_t R_STAGE_BYTES = (size_t)R_STAGE_CELLS * (sizeof(unsigned long long) + sizeof(uint16_t));
 static_assert(R_STAGE_CELLS <= 65536u, "a staged cell's index must fit the 16-bit entries of the block's list");
-constexpr uint32_t R_STAGE_MIN_DEFAULT = 16384;  // list entries above which a merge stages its cells (measured: profiles/r03a)
 __host__ __device__ __forceinline__ uint32_t cell_dec(unsigned long long v) { return (uint32_t)(v & R_FMASK); }
 __host__ __device__ __forceinline__ uint32_t cell_len(unsigned long long v) { return (uint32_t)((v >> R_FIELD) & R_FMASK); }
 __host__ __device__ __forceinline__ uint32_t cell_cnt(unsigned long long v) { return (uint32_t)((v >> (2 * R_FIELD)) & R_FMASK); }
@@ -131,7 +125,6 @@ struct RoundArgs {
   uint32_t* gk;      // [RT * blocks] ... and the pair key of that slot
   RoundState* rs;
   uint32_t kmax;     // merges per round (1 .. RB)
-  uint32_t stage_min;  // a merge whose occurrence list is longer stages its frequent neighbours' cells per block (R_STAGE_T)
   // corpus sharded by document over several GPUs (mg_kernels.cuh): the counts of the pair table are global and replicated, the
   // cells above hold THIS shard's deltas; once per round every rank stores its non-empty cells as records into every rank's
   // inbox over NVLink, and every rank sums all records into gcells -- the global deltas P2 then works from
@@ -703,7 +696,7 @@ __device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S,
   DevState* st = A.st;
   const uint32_t a = S.a[j], b = S.b[j], c = c_first + j;
   const uint32_t total = S.llen[j];
-  const bool staged = total > R.stage_min;
+  const bool staged = total > R.L.stage_min;
   const uint32_t lane = lane_id();
   unsigned long long* const cells_l = round_cells(R, par, j, 0);
   unsigned long long* const cells_r = round_cells(R, par, j, 1);
@@ -1401,7 +1394,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         }
       }
       bool staging = false;
-      for (uint32_t j = 0; j < k; j++) staging |= S.llen[j] > R.stage_min;
+      for (uint32_t j = 0; j < k; j++) staging |= S.llen[j] > R.L.stage_min;
       if (staging) round_flush_stage(R, S, par, c_first);
     }
     RPROF(1)

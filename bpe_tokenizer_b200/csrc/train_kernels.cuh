@@ -706,6 +706,20 @@ constexpr uint32_t ND_STRIDE = 56320;  // >= BPE_MAX_TOKENS + 1
 enum { ND_L_LEN = 0, ND_L_CNT, ND_R_LEN, ND_R_CNT, ND_L_SLOT, ND_R_SLOT, ND_ROWS };
 constexpr uint32_t NOTOKV = 0xFFFFFFFFu;
 
+// Per-block staging of the deltas of frequent neighbours: in the site pass of a merge whose occurrence list is longer than
+// LoopArgs::stage_min, the deltas whose other token is below R_STAGE_T -- on Zipf text the characters and the earliest merges,
+// the neighbours of nearly every site of a big merge -- are summed in shared memory and added to their global word ONCE per
+// block before P1's barrier, instead of by one atomic per warp-iteration on a few hot L2 lines (k_merge_rounds: profiles/r03a,
+// k_merge_loop: profiles/r06a).
+#ifndef BPE_STAGE_T
+#define BPE_STAGE_T 256
+#endif
+constexpr uint32_t R_STAGE_T = BPE_STAGE_T;
+constexpr uint32_t R_STAGE_MIN_DEFAULT = 16384;  // list entries above which a merge stages its deltas (measured: profiles/r03a)
+// k_merge_loop's staged rows, [LS_ROWS][R_STAGE_T] u32 in shared memory: the four born-pair rows of nd (ND_L_LEN .. ND_R_CNT,
+// same order), then the decrements of the old pairs (tok, a) and (b, tok)
+enum { LS_DEC_L = ND_R_CNT + 1, LS_DEC_R, LS_ROWS };
+
 constexpr uint32_t ERR_TOUCH_OVERFLOW = 128u, ERR_PEER_TIMEOUT = 256u, ERR_INBOX_OVERFLOW = 512u, ERR_PEER = 1024u;
 
 __device__ __forceinline__ unsigned long long now_ns();
@@ -774,14 +788,28 @@ __device__ __forceinline__ void agg_dec(const ApplyArgs& A, uint32_t key, bool h
   cnt_delta_warp(A, leader && s != NOSLOT, s, key, -(int32_t)__popc(peers), par);
 }
 
-// Two decrements at once: both first probes are issued before either is consumed (one DRAM round trip instead of two)
-__device__ __forceinline__ void agg_dec2(const ApplyArgs& A, uint32_t key1, bool has1, uint32_t key2, bool has2, uint32_t par) {
+// Two decrements at once: both first probes are issued before either is consumed (one DRAM round trip instead of two).
+// key1 is always (x, a) and key2 always (b, y) of the merge (a, b): with `stage` (single GPU, k_merge_loop), a decrement whose
+// x / y is below R_STAGE_T goes into the block's staged row of that token instead, and loop_flush_stage applies it (single GPU
+// only: see phase_sites).
+__device__ __forceinline__ void agg_dec2(const ApplyArgs& A, uint32_t key1, bool has1, uint32_t key2, bool has2, uint32_t par,
+                                         uint32_t* stage = nullptr) {
   const PairTable& t = A.t;
   uint32_t lane = lane_id();
   uint32_t peers1 = __match_any_sync(0xFFFFFFFFu, has1 ? key1 : (EMPTY_KEY - 1 - lane));
   uint32_t peers2 = __match_any_sync(0xFFFFFFFFu, has2 ? key2 : (EMPTY_KEY - 1 - lane));
   bool lead1 = has1 && lane == (uint32_t)(__ffs(peers1) - 1);
   bool lead2 = has2 && lane == (uint32_t)(__ffs(peers2) - 1);
+  if (stage) {
+    if (lead1 && (key1 >> 16) < R_STAGE_T) {
+      atomicAdd(stage + LS_DEC_L * R_STAGE_T + (key1 >> 16), (uint32_t)__popc(peers1));
+      lead1 = false;
+    }
+    if (lead2 && (key2 & 0xFFFFu) < R_STAGE_T) {
+      atomicAdd(stage + LS_DEC_R * R_STAGE_T + (key2 & 0xFFFFu), (uint32_t)__popc(peers2));
+      lead2 = false;
+    }
+  }
   uint32_t h1 = tbl_hash(t, key1), h2 = tbl_hash(t, key2);
   uint32_t k1 = lead1 ? t.keys[h1] : EMPTY_KEY;
   uint32_t k2 = lead2 ? t.keys[h2] : EMPTY_KEY;
@@ -799,9 +827,10 @@ __device__ __forceinline__ void agg_dec2(const ApplyArgs& A, uint32_t key1, bool
 }
 
 // One adjacency of a pair BORN by this merge -- (tok, c) for side 0, (c, tok) for side 1 -- per `has` lane: occurrences
-// and counted occurrences go to the dense rows with fire-and-forget atomics (one per distinct token per warp).
+// and counted occurrences go to the dense rows with fire-and-forget atomics (one per distinct token per warp), or, with
+// `stage` and tok below R_STAGE_T, to the block's staged copy of those rows (single GPU only: see phase_sites).
 __device__ __forceinline__ void agg_new_dense(const ApplyArgs& A, uint32_t side, uint32_t tok, uint32_t c, bool has, bool counted,
-                                              uint32_t par) {
+                                              uint32_t par, uint32_t* stage = nullptr) {
   uint32_t lane = lane_id();
   uint32_t k = has ? tok : (0xFFFFFF00u + lane);
   uint32_t peers = __match_any_sync(0xFFFFFFFFu, k);
@@ -809,10 +838,16 @@ __device__ __forceinline__ void agg_new_dense(const ApplyArgs& A, uint32_t side,
   const bool leader = has && lane == (uint32_t)(__ffs(peers) - 1);
   uint32_t nc = 0;
   if (leader) {
-    uint32_t* row = A.nd + (size_t)(side ? ND_R_LEN : ND_L_LEN) * ND_STRIDE;
-    atomicAdd(row + tok, (uint32_t)__popc(peers));
     nc = __popc(peers & cmask);
-    if (nc && !A.push_world) atomicAdd(row + ND_STRIDE + tok, nc);
+    if (stage && tok < R_STAGE_T) {
+      uint32_t* srow = stage + (side ? ND_R_LEN : ND_L_LEN) * R_STAGE_T;
+      atomicAdd(srow + tok, (uint32_t)__popc(peers));
+      if (nc) atomicAdd(srow + R_STAGE_T + tok, nc);
+    } else {
+      uint32_t* row = A.nd + (size_t)(side ? ND_R_LEN : ND_L_LEN) * ND_STRIDE;
+      atomicAdd(row + tok, (uint32_t)__popc(peers));
+      if (nc && !A.push_world) atomicAdd(row + ND_STRIDE + tok, nc);
+    }
   }
   // sharded, small merges: the count goes straight to every rank's inbox (partial counts per warp add up on arrival)
   if (A.push_world) cnt_delta_warp(A, nc != 0, NOSLOT, side ? pair_key(c, tok) : pair_key(tok, c), (int32_t)nc, par);
@@ -820,8 +855,12 @@ __device__ __forceinline__ void agg_new_dense(const ApplyArgs& A, uint32_t side,
 
 // vt / nvt: virtual thread id and count (whole warps), so that a loop kernel can give the phase a subset of its warps;
 // site_buf: where the site records go (the loop kernel alternates between two buffers), A.sites when null.
+// stage: the block's staged rows ([LS_ROWS][R_STAGE_T] u32 in shared memory, zero) when every thread of the block runs the phase
+// and the merge stages; loop_flush_stage must then follow, with every thread of the block.  Single GPU only (A.push_world == 0,
+// A.dlt == nullptr, as in k_merge_loop): the staged words go to nd and the table counts, not to an inbox or the touched list.
 __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint32_t b, uint32_t c, uint32_t par,
-                                            uint32_t pair_slot, uint32_t vt, uint32_t nvt, SiteRec* site_buf = nullptr) {
+                                            uint32_t pair_slot, uint32_t vt, uint32_t nvt, SiteRec* site_buf = nullptr,
+                                            uint32_t* stage = nullptr) {
   SiteRec* const site_out = site_buf ? site_buf : A.sites;
   const uint32_t* slots = A.slots;
   const uint32_t n = A.n;
@@ -923,7 +962,7 @@ __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint
     }
     FINE(2, (uint32_t)dec1_key + new1_tok)
     FINE(3, 0)
-    agg_new_dense(A, 0, new1_tok, c, new1, new1_counted, par);
+    agg_new_dense(A, 0, new1_tok, c, new1, new1_counted, par, stage);
     rec.lslot = new1 ? new1_tok : NOTOKV;  // resolved to the pair's table slot by phase_apply (ND_L_SLOT)
     FINE(4, rec.lslot)
 
@@ -954,9 +993,9 @@ __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint
       }
     }
     FINE(5, (uint32_t)dec2_key + new2_tok)
-    agg_dec2(A, dec1_key, dec1, dec2_key, dec2, par);
+    agg_dec2(A, dec1_key, dec1, dec2_key, dec2, par, stage);
     FINE(6, 0)
-    agg_new_dense(A, 1, new2_tok, c, new2, true, par);
+    agg_new_dense(A, 1, new2_tok, c, new2, true, par, stage);
     rec.rslot = new2 ? new2_tok : NOTOKV;
     FINE(7, rec.rslot)
 
@@ -970,6 +1009,27 @@ __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint
     FINE(8, base)
   }
 #undef FINE
+}
+
+// End of a staged site pass in this block (all its threads call): every non-zero staged word goes to its global word with one
+// atomic -- the born-pair rows to nd, a decrement to the count of (tok, a) / (b, tok) after one table probe -- and is zeroed for
+// the next merge.  The rows are scanned rather than listed: LS_ROWS x R_STAGE_T words of shared memory (1 536, three per thread
+// at the defaults) take a few hundred cycles, which is nothing next to a pass over more than stage_min sites.
+__device__ __forceinline__ void loop_flush_stage(const ApplyArgs& A, uint32_t* stage, uint32_t a, uint32_t b) {
+  __syncthreads();
+  for (uint32_t i = threadIdx.x; i < LS_ROWS * R_STAGE_T; i += blockDim.x) {
+    const uint32_t v = stage[i];
+    if (!v) continue;
+    stage[i] = 0;
+    const uint32_t row = i / R_STAGE_T, tok = i - row * R_STAGE_T;
+    if (row < LS_DEC_L) {
+      atomicAdd(A.nd + (size_t)row * ND_STRIDE + tok, v);
+    } else {
+      const uint32_t s = tbl_find(A.t, row == LS_DEC_L ? pair_key(tok, a) : pair_key(b, tok));
+      if (s == NOSLOT) atomicOr(&A.st->err, ERR_MISSING_KEY);
+      else atomicAdd(A.t.cnt + s, 0u - v);
+    }
+  }
 }
 
 // K3 phase 2: every pair born in this merge -- the non-empty cells of the dense rows -- enters the pair table ONCE:
@@ -1101,16 +1161,43 @@ __device__ __forceinline__ void phase_rewrite(const ApplyArgs& A, uint32_t c, ui
   }
 }
 
-__device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites, uint32_t vt, uint32_t nvt, const SiteRec* site_buf = nullptr) {
+// All 32 lanes call: lanes that agree on `key` elect a leader which adds their number to the shared-memory word ctr[key] once;
+// returns each `has` lane's ticket (the word's old value plus its rank among its peers).
+__device__ __forceinline__ uint32_t agg_smem_ticket(uint32_t* ctr, uint32_t key, bool has) {
+  const uint32_t lane = lane_id();
+  const uint32_t peers = __match_any_sync(0xFFFFFFFFu, has ? key : (0xFFFFFF00u + lane));
+  const uint32_t leader = __ffs(peers) - 1;
+  uint32_t base = 0;
+  if (has && lane == leader) base = atomicAdd(ctr + key, (uint32_t)__popc(peers));
+  base = __shfl_sync(0xFFFFFFFFu, base, leader);
+  return base + __popc(peers & ((1u << lane) - 1u));
+}
+
+// stage: the block's staged rows (as for phase_sites, zero) when every thread of the block runs the phase (vt / nvt of the whole
+// grid) and the merge whose sites these are had more than stage_min of them.  The adjacencies of born pairs whose other token is
+// below R_STAGE_T then take their list cells in three steps instead of one returning occ_fill atomic per warp on a few words of
+// the whole grid: the block counts them per (side, token) in shared memory, reserves each (pair, block) range with ONE occ_fill
+// atomic, and a second pass over the sites hands out shared-memory tickets inside the ranges.  The rows are zero on return.
+// (The order of the cells inside a list was never fixed; nothing reads it.)
+__device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites, uint32_t vt, uint32_t nvt, const SiteRec* site_buf = nullptr,
+                                           uint32_t* stage = nullptr) {
   const PairTable& t = A.t;
   const SiteRec* const sites = site_buf ? site_buf : A.sites;
+  uint32_t* const scnt = stage;                      // [2][R_STAGE_T]: the block's cells per (side, token), then its tickets
+  uint32_t* const sbase = stage + 2u * R_STAGE_T;    // [2][R_STAGE_T]: start of the block's range in that list (FILL_NONE: no list)
+  constexpr uint32_t FILL_NONE = 0xFFFFFFFFu;
   uint32_t round = (n_sites + 31u) & ~31u;
   for (uint32_t i = vt; i < round; i += nvt) {
     bool has = i < n_sites;
     uint4 rv = has ? ld_cg4(reinterpret_cast<const uint4*>(sites) + i) : make_uint4(0, NOPOS, NOTOKV, NOTOKV);
     uint32_t p = rv.x, lpos = rv.y;
-    uint32_t lslot = (has && rv.z != NOTOKV) ? ld_cg(A.nd + (size_t)ND_L_SLOT * ND_STRIDE + rv.z) : NOSLOT;
-    uint32_t rslot = (has && rv.w != NOTOKV) ? ld_cg(A.nd + (size_t)ND_R_SLOT * ND_STRIDE + rv.w) : NOSLOT;
+    const bool sl = stage && has && rv.z < R_STAGE_T, sr = stage && has && rv.w < R_STAGE_T;  // (NOTOKV is not below it)
+    if (stage) {
+      agg_smem_ticket(scnt, rv.z, sl);
+      agg_smem_ticket(scnt, R_STAGE_T + rv.w, sr);
+    }
+    uint32_t lslot = (has && !sl && rv.z != NOTOKV) ? ld_cg(A.nd + (size_t)ND_L_SLOT * ND_STRIDE + rv.z) : NOSLOT;
+    uint32_t rslot = (has && !sr && rv.w != NOTOKV) ? ld_cg(A.nd + (size_t)ND_R_SLOT * ND_STRIDE + rv.w) : NOSLOT;
     bool hl = has && lslot != NOSLOT && t.occ_len[lslot];
     bool hr = has && rslot != NOSLOT && t.occ_len[rslot];
     uint32_t il = agg_cursor(t, lslot, hl);
@@ -1118,6 +1205,30 @@ __device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites,
     if (hl) A.pool[il] = lpos;
     if (hr) A.pool[ir] = p;
   }
+  if (!stage) return;
+  __syncthreads();
+  for (uint32_t e = threadIdx.x; e < 2u * R_STAGE_T; e += blockDim.x) {
+    const uint32_t v = scnt[e];
+    if (!v) continue;
+    scnt[e] = 0;
+    const uint32_t side = e >= R_STAGE_T ? 1u : 0u, tok = e - side * R_STAGE_T;
+    const uint32_t s = ld_cg(A.nd + (size_t)(side ? ND_R_SLOT : ND_L_SLOT) * ND_STRIDE + tok);
+    sbase[e] = (s != NOSLOT && t.occ_len[s]) ? t.occ_start[s] + atomicAdd(t.occ_fill + s, v) : FILL_NONE;
+  }
+  __syncthreads();
+  for (uint32_t i = vt; i < round; i += nvt) {
+    const bool has = i < n_sites;
+    const uint4 rv = has ? ld_cg4(reinterpret_cast<const uint4*>(sites) + i) : make_uint4(0, NOPOS, NOTOKV, NOTOKV);
+    const bool sl = has && rv.z < R_STAGE_T, sr = has && rv.w < R_STAGE_T;
+    const uint32_t kl = agg_smem_ticket(scnt, rv.z, sl);
+    const uint32_t kr = agg_smem_ticket(scnt, R_STAGE_T + rv.w, sr);
+    const uint32_t bl = sl ? sbase[rv.z] : FILL_NONE, br = sr ? sbase[R_STAGE_T + rv.w] : FILL_NONE;
+    if (bl != FILL_NONE) A.pool[bl + kl] = rv.y;
+    if (br != FILL_NONE) A.pool[br + kr] = rv.x;
+  }
+  __syncthreads();
+  for (uint32_t e = threadIdx.x; e < 4u * R_STAGE_T; e += blockDim.x) stage[e] = 0;
+  __syncthreads();
 }
 
 __device__ __forceinline__ void phase_apply(const ApplyArgs& A, uint32_t a, uint32_t b, uint32_t c, uint32_t n_sites,
@@ -1195,6 +1306,8 @@ struct LoopArgs {
   uint32_t p1_sites, p2_new, p2_rw;
   uint32_t bar_ns;  // longest back-off of a barrier poll
   int prefetch;  // speculative L2 prefetch of the sites of this many runner-ups (prefetch_runner_up); BPE_LOOP_PREFETCH=0..2
+  uint32_t stage_min;  // a merge whose occurrence list is longer stages its frequent neighbours' deltas per block (R_STAGE_T);
+                       // k_merge_loop and k_merge_rounds, BPE_BLOCK_CELLS_MIN_SITES
 };
 
 // Grid barrier for the co-resident (cooperative) launch.  The arrival counter lives in its own 128-byte line, away
@@ -1270,6 +1383,8 @@ __global__ void k_loop_prepare(DevState* st, uint32_t n_tokens, unsigned long lo
 __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopArgs L) {
   __shared__ Best s_best[ML_THREADS / 32];
   __shared__ uint32_t s_max[32];
+  __shared__ uint32_t s_stage[LS_ROWS * R_STAGE_T];  // loop_flush_stage leaves it zero
+  for (uint32_t i = threadIdx.x; i < LS_ROWS * R_STAGE_T; i += blockDim.x) s_stage[i] = 0;
   const ApplyArgs& A = L.A;
   DevState* st = A.st;
   const PairTable& t = A.t;
@@ -1364,7 +1479,7 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopAr
       if (w.mult > L.cand_cap) status = LOOP_NEED_HOST;
       else {
         if (fill_n) {  // the tie-break reads occurrence lists: those of the last merge must be complete
-          phase_fill(A, fill_n, gt, gn, fill_sites);
+          phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);
           fill_n = 0;
           grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
         }
@@ -1395,7 +1510,7 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopAr
       else if (c + 1 > L.len16_cap) status = LOOP_NEED_HOST;
     }
     if (status != LOOP_RUNNING) {
-      if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites);  // the kernel leaves every list complete
+      if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);  // the kernel leaves every list complete
       if (bid == 0 && threadIdx.x == 0) {
         st->status = status;
         st->iters_done = it;
@@ -1414,7 +1529,7 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopAr
     }
     if (fill_n && it && (wa == c - 1u || wb == c - 1u)) {
       // the winner was born by the previous merge: its list is exactly what fill(t-1) still has to write
-      phase_fill(A, fill_n, gt, gn, fill_sites);
+      phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);
       fill_n = 0;
       grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
     }
@@ -1443,8 +1558,11 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopAr
         if (L.prefetch && !replay) prefetch_runner_up(L, w.slot, nblk, (bid * wh + warp - ws) * 32 + lane, nblk * wh * 32);
       }
     } else {
-      if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites);
-      phase_sites(A, wa, wb, c, par, w.slot, gt, gn, my_sites);
+      // (the list length is block-uniform: nothing writes occ_len between P2's barrier and the next P2)
+      const bool staged = w.slot != NOSLOT && t.occ_len[w.slot] > L.stage_min;
+      if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);
+      phase_sites(A, wa, wb, c, par, w.slot, gt, gn, my_sites, staged ? s_stage : nullptr);
+      if (staged) loop_flush_stage(A, s_stage, wa, wb);
     }
     fill_n = 0;
 #ifdef BPE_FINE_PROF
