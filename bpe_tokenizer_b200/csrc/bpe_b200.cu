@@ -175,7 +175,7 @@ struct bpe_engine {
   // pair index
   bool index_valid = false;
   uint32_t tbl_cap = 0;
-  DevBuf<uint32_t> t_ent;  // 5 fields x capacity words (field-major when TBL_STRIDE == 1, common.cuh)
+  DevBuf<uint32_t> t_ent;  // 6 words per slot: 4 u32 fields and the u64 list start (field-major when TBL_STRIDE == 1, common.cuh)
   DevBuf<uint32_t> u_ent;  // second buffer, target of the next rehash (kept at high water)
   DevBuf<uint32_t> pool;
   DevBuf<DevState> d_st;
@@ -262,9 +262,9 @@ struct bpe_engine {
     const size_t fs = (TBL_STRIDE == 1) ? (size_t)tbl_cap : 1;  // distance between fields
     t.keys.p = t_ent.p;
     t.cnt.p = t_ent.p + fs;
-    t.occ_start.p = t_ent.p + 2 * fs;
-    t.occ_len.p = t_ent.p + 3 * fs;
-    t.occ_fill.p = t_ent.p + 4 * fs;
+    t.occ_len.p = t_ent.p + 2 * fs;
+    t.occ_fill.p = t_ent.p + 3 * fs;
+    t.occ_start.p = reinterpret_cast<unsigned long long*>(t_ent.p + (TBL_STRIDE == 1 ? 4 * fs : 6));  // (8-byte aligned)
     t.mask = tbl_cap - 1;
     t.shift = 32 - ilog2(tbl_cap);
     return t;
@@ -316,6 +316,7 @@ int check_dev_err(bpe_engine* e) {
   if (f & ERR_POOL_FULL) return fail(e, BPE_E_INTERNAL, "occurrence pool exhausted (flags 0x%x)", f);
   if (f & ERR_MISSING_KEY) return fail(e, BPE_E_INTERNAL, "pair missing from the table (flags 0x%x)", f);
   if (f & ERR_SPAN_OVERFLOW) return fail(e, BPE_E_DOMAIN, "token span exceeds 2^29 positions");
+  if (f & ERR_COUNT_OVERFLOW) return fail(e, BPE_E_DOMAIN, "a pair's count summed over the shards exceeds 2^32 - 1");
   return fail(e, BPE_E_INTERNAL, "device error flags 0x%x", f);
 }
 
@@ -341,11 +342,11 @@ __global__ void k_init_table(uint4* __restrict__ ent, uint64_t cap) {  // key = 
 
 int alloc_table(bpe_engine* e, uint32_t cap) {
   // buffers only ever grow (cudaFree / cudaMalloc of GBs costs up to seconds); the logical capacity is `cap`
-  CK(e->t_ent.reserve((size_t)cap * (TBL_STRIDE == 1 ? 5 : TBL_STRIDE)));
+  CK(e->t_ent.reserve((size_t)cap * (TBL_STRIDE == 1 ? 6 : TBL_STRIDE)));
   e->tbl_cap = cap;
   if (TBL_STRIDE == 1) {
     CK(cudaMemsetAsync(e->t_ent.p, 0xFF, (size_t)cap * 4, e->stream));
-    CK(cudaMemsetAsync(e->t_ent.p + cap, 0, (size_t)cap * 16, e->stream));
+    CK(cudaMemsetAsync(e->t_ent.p + cap, 0, (size_t)cap * 20, e->stream));
   } else {
     k_init_table<<<e->grid(8), 256, 0, e->stream>>>(reinterpret_cast<uint4*>(e->t_ent.p), (uint64_t)cap);
     CKL();
@@ -369,7 +370,7 @@ __global__ void k_rehash(PairTable src, PairTable dst, DevState* st) {
       h = (h + 1) & dst.mask;
     }
     dst.cnt[h] = src.cnt[i];
-    dst.occ_start[h] = src.occ_start[i];
+    dst.occ_start.set(h, src.occ_start.get(i));
     dst.occ_len[h] = src.occ_len[i];
     dst.occ_fill[h] = src.occ_fill[i];
   }
@@ -387,6 +388,13 @@ int grow_table(bpe_engine* e, uint32_t new_cap) {
 }
 
 // ---- K1: build histogram + occurrence lists from the corpus -------------------------------------
+// BPE_POOL_BASE (cells, default 0): index build starts the occurrence pool's cursor there, with real memory reserved below
+// it, so that a corpus of a few MB puts its lists on both sides of cell 2^32 (tests of the 64-bit cell indices)
+uint64_t pool_base_knob() {
+  if (const char* v = getenv("BPE_POOL_BASE")) return (uint64_t)std::max(0ll, atoll(v));
+  return 0;
+}
+
 int build_index(bpe_engine* e) {
   e->index_valid = false;
   e->hot_valid = false;
@@ -398,8 +406,12 @@ int build_index(bpe_engine* e) {
   TRY(sync_len16(e));
   uint64_t n = e->n_slots;
   if (n >= 0xFFFFFFF0ull) return fail(e, BPE_E_DOMAIN, "corpus of %llu positions exceeds the 2^32 engine limit", (unsigned long long)n);
-  uint64_t pool_need = 3 * n + 1024;
-  if (pool_need > 0xFFFFFFF0ull) pool_need = 0xFFFFFFF0ull;
+  // The pool holds K1's n cells and at most two per merge site, n + 2 * sites <= 3n (DESIGN.md section 1), plus the private
+  // chunks the blocks of k_merge_rounds open and the sharded loop's one-round lag.  It is reserved here, once, so that a run
+  // does not grow it: a growth copies the old pool into the new one and needs both resident.
+  const uint64_t pool_base = pool_base_knob();
+  const uint64_t pool_need = pool_base + 3 * n + 2ull * R_HUGE + 2ull * std::max(R_HUGE, R_BATCH_SITES) + 2ull * e->sm_count * R_POOL_CHUNK;
+  if (e->pool.cap < pool_need) e->pool.release();  // (nothing in it survives the rebuild: never hold the old and the new pool together)
   CK(e->pool.reserve((size_t)pool_need));
   uint64_t t2 = (uint64_t)e->n_tokens * (uint64_t)e->n_tokens;
   uint32_t cap = pow2_at_least(std::min<uint64_t>(std::max<uint64_t>(2 * std::min(n, t2), 1u << 16), 1u << 24));
@@ -413,6 +425,7 @@ int build_index(bpe_engine* e) {
   for (;;) {
     TRY(alloc_table(e, cap));
     DevState init{};
+    init.pool_cursor = pool_base;
     init.live_tokens = e->live_tokens;
     init.tie_pos = ~0ull;
     init.mg_epoch = e->mg_epoch;  // the peers' flags keep counting across index rebuilds
@@ -437,7 +450,7 @@ int build_index(bpe_engine* e) {
     break;
   }
   if (n) {
-    k_alloc_lists<<<e->grid(4), 256, 0, e->stream>>>(e->table(), e->d_st.p, (uint32_t)e->pool.cap);
+    k_alloc_lists<<<e->grid(4), 256, 0, e->stream>>>(e->table(), e->d_st.p, (unsigned long long)e->pool.cap);
     CKL();
     int k1b_per_sm = 0;
     CK(cudaFuncSetAttribute(k_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1B_SMEM_BYTES));  // the staging buffer
@@ -566,10 +579,7 @@ int run_apply(bpe_engine* e, uint32_t a, uint32_t b, uint32_t c, uint32_t bound)
     TRY(grow_table(e, pow2_at_least(want)));
   }
   uint64_t pool_after = (uint64_t)e->h_st->pool_cursor + 2ull * bound;
-  if (pool_after > e->pool.cap) {
-    if (pool_after > 0xFFFFFFF0ull) return fail(e, BPE_E_DOMAIN, "occurrence pool exceeds 2^32 cells");
-    CK(e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5));
-  }
+  if (pool_after > e->pool.cap) CK(e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5));
   CK(e->sites.reserve(std::max<size_t>(bound, 4096), 0, e->stream, 2.0));
   CK(e->newslots.reserve(std::max<size_t>(2ull * bound + 2, 8192), 0, e->stream, 2.0));
   if ((size_t)c + 1 > e->d_len16.cap) CK(e->d_len16.reserve((size_t)c + 1, (size_t)c, e->stream, 2.0));
@@ -580,7 +590,7 @@ int run_apply(bpe_engine* e, uint32_t a, uint32_t b, uint32_t c, uint32_t bound)
   k_sites<<<blocks, 256, 0, e->stream>>>(A, a, b, c);
   CKL();
   int blocks2 = (int)std::min<uint64_t>((uint64_t)e->grid(8), std::max<uint64_t>(1, (2ull * bound + 255) / 256));
-  k_alloc_new<<<blocks2, 256, 0, e->stream>>>(A, c, e->hot_max_length, e->hot_valid ? 1 : 0, e->hot.p, (uint32_t)e->hot.cap, (uint32_t)e->pool.cap);
+  k_alloc_new<<<blocks2, 256, 0, e->stream>>>(A, c, e->hot_max_length, e->hot_valid ? 1 : 0, e->hot.p, (uint32_t)e->hot.cap, (unsigned long long)e->pool.cap);
   CKL();
   int blocks3 = (int)std::min<uint64_t>((uint64_t)e->grid(8), std::max<uint64_t>(1, ((uint64_t)bound + 255) / 256));
   k_apply<<<blocks3, 256, 0, e->stream>>>(A, a, b, c);
@@ -1173,7 +1183,7 @@ int merge_until_device(bpe_engine* e, int64_t min_weight, int32_t max_length, in
     }
     LoopArgs L;
     L.A = apply_args(e);
-    L.pool_cap = (uint32_t)std::min<size_t>(e->pool.cap, 0xFFFFFFF0u);
+    L.pool_cap = e->pool.cap;
     L.len16_cap = (uint32_t)std::min<size_t>(e->d_len16.cap, 0xFFFFFFF0u);
     L.hot = e->hot.p;
     L.hot_cap = (uint32_t)std::min<size_t>(e->hot.cap, 0xFFFFFFF0u);
@@ -1309,10 +1319,6 @@ int merge_until_device(bpe_engine* e, int64_t min_weight, int32_t max_length, in
       }
       uint64_t pool_after = (uint64_t)e->h_st->pool_cursor + 2 * w;
       if (use_rounds) pool_after += (uint64_t)e->round_blocks * R_POOL_CHUNK;  // every block of k_merge_rounds may open a private chunk
-      if (pool_after > 0xFFFFFFF0ull) {
-        rc = fail(e, BPE_E_DOMAIN, "occurrence pool exceeds 2^32 cells");
-        break;
-      }
       if ((ce = e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5)) != cudaSuccess ||
           (ce = e->sites.reserve((size_t)w, 0, e->stream, 1.25)) != cudaSuccess ||
           (ce = e->sites2.reserve(e->sites.cap, 0, e->stream, 1.0)) != cudaSuccess ||
@@ -1471,7 +1477,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
     L.A.dlt = e->mg_dlt.p;
     L.A.touched = e->mg_touched.p;
     L.A.touched_cap = (uint32_t)e->mg_touched.cap;
-    L.pool_cap = (uint32_t)std::min<size_t>(e->pool.cap, 0xFFFFFFF0u);
+    L.pool_cap = e->pool.cap;
     L.len16_cap = (uint32_t)std::min<size_t>(e->d_len16.cap, 0xFFFFFFF0u);
     L.hot = e->hot.p;
     L.hot_cap = (uint32_t)std::min<size_t>(e->hot.cap, 0xFFFFFFF0u);
@@ -1607,10 +1613,6 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
       // the previous round's batch -- whose allocation the figure in the header does not show yet -- at most as many
       if (use_rounds) pool_after += 2ull * R_HUGE + 2ull * std::max(R_HUGE, R_BATCH_SITES) + 2ull * e->round_blocks * R_POOL_CHUNK;
       auto tp = clk();
-      if (pool_after > 0xFFFFFFF0ull) {
-        rc = fail(e, BPE_E_DOMAIN, "occurrence pool exceeds 2^32 cells");
-        break;
-      }
       if ((ce = e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5)) != cudaSuccess ||
           (ce = e->sites.reserve((size_t)w, 0, e->stream, 1.25)) != cudaSuccess ||
           (use_rounds && (ce = e->sites2.reserve(e->sites.cap, 0, e->stream, 1.0)) != cudaSuccess) ||

@@ -130,10 +130,20 @@ struct TblField {
   __host__ __device__ __forceinline__ uint32_t& operator[](uint32_t i) const { return p[(size_t)i * TBL_STRIDE]; }
   __host__ __device__ __forceinline__ uint32_t* operator+(uint32_t i) const { return p + (size_t)i * TBL_STRIDE; }
 };
+// Where a pair's occurrence list starts in the pool.  The pool holds up to 3 cells per corpus position, so on one engine of
+// more than ~1.4 G positions its cell indices pass 2^32: the start is 64-bit, one 8-byte word per slot (the words 6..7 of a
+// 32-byte entry when TBL_STRIDE = 8).  Kernels read and write it through get / set only and never see the layout.
+struct TblStart {
+  unsigned long long* p;
+  static constexpr uint32_t STRIDE = TBL_STRIDE == 1 ? 1u : TBL_STRIDE / 2u;  // u64 words between consecutive slots
+  __host__ __device__ __forceinline__ unsigned long long get(uint32_t i) const { return p[(size_t)i * STRIDE]; }
+  __host__ __device__ __forceinline__ void set(uint32_t i, unsigned long long v) const { p[(size_t)i * STRIDE] = v; }
+  __host__ __device__ __forceinline__ const void* addr(uint32_t i) const { return p + (size_t)i * STRIDE; }  // (prefetch)
+};
 struct PairTable {
   TblField keys;       // pair_key(a,b) or EMPTY_KEY
   TblField cnt;        // counted occurrences (run-parity rule of core.ts:285-290 applied)
-  TblField occ_start;  // occurrence list = pool[occ_start .. occ_start+occ_len)
+  TblStart occ_start;  // occurrence list = pool[occ_start .. occ_start+occ_len)
   TblField occ_len;    //   every adjacency (a,b) born in the iteration that created the pair
   TblField occ_fill;   //   scatter cursor
   uint32_t mask;       // capacity - 1
@@ -194,6 +204,6 @@ __device__ __forceinline__ uint32_t tbl_find_or_insert_ex(const PairTable& t, ui
 
 // error flags raised by kernels (checked by the host after each phase)
 constexpr uint32_t ERR_TABLE_FULL = 1u, ERR_MISSING_KEY = 2u, ERR_POOL_FULL = 4u, ERR_SITE_OVERFLOW = 8u,
-                   ERR_SPAN_OVERFLOW = 16u, ERR_CAND_OVERFLOW = 32u, ERR_HOT_OVERFLOW = 64u;
+                   ERR_SPAN_OVERFLOW = 16u, ERR_CAND_OVERFLOW = 32u, ERR_HOT_OVERFLOW = 64u, ERR_COUNT_OVERFLOW = 4096u;
 
 }  // namespace bpe

@@ -100,8 +100,12 @@ __global__ void k_mg_import_counts(PairTable t, const uint32_t* __restrict__ key
                                    DevState* st) {
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     uint32_t s = tbl_find_or_insert(t, keys[i], &st->n_keys);
-    if (s == NOSLOT) atomicOr(&st->err, ERR_TABLE_FULL);
-    else atomicAdd(t.cnt + s, cnts[i]);
+    if (s == NOSLOT) {
+      atomicOr(&st->err, ERR_TABLE_FULL);
+    } else {
+      const uint32_t old = atomicAdd(t.cnt + s, cnts[i]);
+      if (old + cnts[i] < old) atomicOr(&st->err, ERR_COUNT_OVERFLOW);  // the global count does not fit 32 bits
+    }
   }
 }
 
@@ -120,13 +124,13 @@ __device__ __forceinline__ void mg_send_warp(const LoopArgsMg& P, DevState* st, 
   const int q = (int)(threadIdx.x & 31u);
   const bool peer = q < M.world && q != M.rank;
   if (q < M.world) {
-    uint32_t cur = ld_cg(&st->pool_cursor);
+    const unsigned long long cur = ld_cg(&st->pool_cursor);
     uint32_t h[12];
 #pragma unroll
     for (int i = 0; i < 12; i++) h[i] = 0;
     h[H_N] = n_rec;
     h[H_ERR] = ld_cg(&st->err);
-    h[H_POOL_FREE] = L.pool_cap > cur ? L.pool_cap - cur : 0;
+    h[H_POOL_FREE] = (uint32_t)min(L.pool_cap > cur ? L.pool_cap - cur : 0ull, 0xFFFFFFFFull);  // (only gates the next merge)
     h[H_SITES_CAP] = L.A.sites_cap;
     h[H_NEW_CAP] = L.A.new_cap;
     h[H_HOT_CAP] = min(L.hot_cap, L.hot_limit);
@@ -291,7 +295,8 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
         uint32_t s = ld_cg(&M.tie_sorted[cnd]);
         uint32_t key = t.keys[s];
         uint32_t a = key >> 16, b = key & 0xFFFFu;
-        uint32_t start = t.occ_start[s], len = t.occ_len[s];
+        const unsigned long long start = t.occ_start.get(s);
+        uint32_t len = t.occ_len[s];
         uint32_t v = 0;
         for (uint32_t i = threadIdx.x; i < len; i += blockDim.x) {
           uint32_t p = A.pool[start + i];

@@ -267,7 +267,8 @@ __device__ __forceinline__ void top2_publish(const Top2& v, uint4* gp, uint32_t*
 struct RoundSm {
   // the batch of the current round (same in every block)
   uint32_t k, status, mult0, pad0;
-  uint32_t a[RB], b[RB], w[RB], slot[RB], lstart[RB], llen[RB], lenc[RB];
+  uint32_t a[RB], b[RB], w[RB], slot[RB], llen[RB], lenc[RB];
+  unsigned long long lstart[RB];  // where each merge's occurrence list starts in the pool
   uint32_t iter0[RB + 1];  // warp-iterations of P1: merge j owns [iter0[j], iter0[j+1])
   uint32_t fill_n[RB];     // sites of the previous round's merges whose born adjacencies are not in their lists yet
   // decision scratch
@@ -275,15 +276,18 @@ struct RoundSm {
   unsigned long long qp[R_QCAP];
   uint32_t qs[R_QCAP], qm[R_QCAP], qk[R_QCAP];
   unsigned long long cp[RB];
-  uint32_t cs[RB], cm[RB], ck[RB], cls[RB], cll[RB], clen[RB];
-  uint32_t g_n_keys, g_pool_cursor, g_snap_err, g_abort;
+  uint32_t cs[RB], cm[RB], ck[RB], cll[RB], clen[RB];
+  unsigned long long cls[RB];
+  unsigned long long g_pool_cursor;
+  uint32_t g_n_keys, g_snap_err, g_abort;
   uint32_t gv[8];  // sharded: the folded header values (OR of the ranks' error flags, minima of their capacities)
   uint32_t ncell[2];  // cells this block touched first in the round of either parity (entries of its list)
   uint32_t nstage;    // staged cells this block touched in the current P1 (entries of r_stage_list)
   uint32_t gncell[2]; // sharded: global cells this block touched first while summing the ranks' records
   uint32_t rec_base, rec_cnt;  // sharded: where this block's records go in the inboxes, how many they are
   uint32_t mg_mask, mg_cnt[MG_MAX_WORLD];  // sharded: senders whose message is complete and not summed yet, their records
-  uint32_t pool_next, pool_end;  // this block's private chunk of the occurrence pool (list space without a grid-wide atomic)
+  unsigned long long pool_base;  // this block's private chunk of the occurrence pool (list space without a grid-wide atomic) ...
+  uint32_t pool_next, pool_end;  // ... and the bump cursor / end inside it (32-bit offsets: a 64-bit shared atomic is a CAS loop)
   uint32_t keys_ins;             // keys this block inserted in the current P2 (one n_keys atomic per block and round)
   uint32_t filt_a[8], filt_b[8]; // role_maybe filters: the a's / the b's of the batch
   Top2 t2[32];
@@ -495,13 +499,13 @@ __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, 
   const unsigned long long ub_lane = ((uint32_t)q < k) ? ld_cg(&R.rs->ub[par][q].v) : 0ull;
   const uint32_t ns_lane = ((uint32_t)q < k) ? ld_cg(&R.rs->n_sites[par][q].v) : 0u;
   if (q < M.world) {
-    const uint32_t cur = ld_cg(&st->pool_cursor);
+    const unsigned long long cur = ld_cg(&st->pool_cursor);
     uint32_t h[12];
 #pragma unroll
     for (int i = 0; i < 12; i++) h[i] = 0;
     h[H_N] = min(ld_cg(&st->n_out), M.inbox_stride - MGR_HDR);
     h[H_ERR] = ld_cg(&st->err);
-    h[H_POOL_FREE] = L.pool_cap > cur ? L.pool_cap - cur : 0;
+    h[H_POOL_FREE] = (uint32_t)min(L.pool_cap > cur ? L.pool_cap - cur : 0ull, 0xFFFFFFFFull);  // (only gates the next batch)
     h[H_SITES_CAP] = L.A.sites_cap;
     h[H_NEW_CAP] = 0xFFFFFFFFu;
     h[H_HOT_CAP] = min(L.hot_cap, L.hot_limit);
@@ -892,8 +896,8 @@ __device__ __forceinline__ void round_fill_all(const RoundArgs& R, const RoundSm
     const uint32_t rslot = (has && rtok != R_NOTOK) ? ld_cg(round_slotrow(R, F.par, j, 1) + rtok) : NOSLOT;
     const bool hl = has && lslot != NOSLOT && t.occ_len[lslot];
     const bool hr = has && rslot != NOSLOT && t.occ_len[rslot];
-    const uint32_t il = agg_cursor(t, lslot, hl);
-    const uint32_t ir = agg_cursor(t, rslot, hr);
+    const unsigned long long il = agg_cursor(t, lslot, hl);
+    const unsigned long long ir = agg_cursor(t, rslot, hr);
     if (hl) A.pool[il] = rv.y;
     if (hr) A.pool[ir] = rv.x;
   }
@@ -1093,7 +1097,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           S.cm[rank] = mult;
           S.ck[rank] = key;
           // what the batch builder needs of this candidate, loaded side by side by the candidates' own threads
-          S.cls[rank] = t.occ_start[slot];
+          S.cls[rank] = t.occ_start.get(slot);
           S.cll[rank] = t.occ_len[slot];
           S.clen[rank] = A.len16[key >> 16] + A.len16[key & 0xFFFFu];
         }
@@ -1104,7 +1108,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         const uint32_t j = lane;
         const unsigned long long p0 = S.cp[0];
         const uint32_t w0 = (uint32_t)(p0 >> 20);
-        const uint32_t n_keys = S.g_n_keys, pool_cursor = S.g_pool_cursor;
+        const uint32_t n_keys = S.g_n_keys;
+        const unsigned long long pool_cursor = S.g_pool_cursor;
         uint32_t status = LOOP_RUNNING;
         if (S.g_snap_err || (R.mg_on && (S.g_abort || S.gv[0]))) status = LOOP_ERROR;
         else if (!p0) status = (thresh <= 1) ? LOOP_EMPTY : LOOP_NEED_REBUILD;
@@ -1139,7 +1144,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           else if (cj + 1 > S.gv[5]) cap_fail = LOOP_NEED_HOST;
         } else
         if ((unsigned long long)n_keys + keys_incl > (unsigned long long)(L.tbl_cap >> 1)) cap_fail = LOOP_NEED_HOST;
-        else if ((unsigned long long)pool_cursor + 2ull * w_incl + (unsigned long long)nblk * R_POOL_CHUNK > L.pool_cap) cap_fail = LOOP_NEED_HOST;
+        else if (pool_cursor + 2ull * w_incl + (unsigned long long)nblk * R_POOL_CHUNK > L.pool_cap) cap_fail = LOOP_NEED_HOST;
         else if (j == 0 && wj > A.sites_cap) cap_fail = LOOP_NEED_HOST;
         else if ((unsigned long long)hot_pre + keys_incl > min(L.hot_cap, L.hot_limit)) cap_fail = LOOP_NEED_REBUILD;
         else if (cj + 1 > L.len16_cap) cap_fail = LOOP_NEED_HOST;
@@ -1252,7 +1257,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           const uint32_t sc = ld_cg(&M.tie_sorted[cnd]);
           const uint32_t key = t.keys[sc];
           const uint32_t ca = key >> 16, cb = key & 0xFFFFu;
-          const uint32_t start = t.occ_start[sc], len = t.occ_len[sc];
+          const unsigned long long start = t.occ_start.get(sc);
+          const uint32_t len = t.occ_len[sc];
           uint32_t vmax = 0;
           for (uint32_t i = tid; i < len; i += blockDim.x) {
             const uint32_t pp = A.pool[start + i];
@@ -1306,7 +1312,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         for (int i = 0; i < 8; i++) S.filt_a[i] = S.filt_b[i] = 0;
         S.filt_a[((key >> 16) >> 5) & 7u] = 1u << ((key >> 16) & 31u);
         S.filt_b[((key & 0xFFFFu) >> 5) & 7u] = 1u << (key & 31u);
-        S.lstart[0] = t.occ_start[s];
+        S.lstart[0] = t.occ_start.get(s);
         S.llen[0] = t.occ_len[s];
         S.lenc[0] = A.len16[key >> 16] + A.len16[key & 0xFFFFu];
         S.iter0[1] = (S.llen[0] + 31u) >> 5;
@@ -1380,7 +1386,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           uint32_t budget = 32768u;
           for (uint32_t j = k; j < RB && budget; j++) {
             if (!S.cp[j]) break;
-            const uint32_t len = min(S.cll[j], budget), start = S.cls[j];
+            const uint32_t len = min(S.cll[j], budget);
+            const unsigned long long start = S.cls[j];
             for (uint32_t i = hvt; i < len; i += hnvt) {
               const uint32_t pp = ld_cg(A.pool + start + i);
               if (pp >= A.n) continue;
@@ -1493,10 +1500,11 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
     if (tid == 0) {
       S.keys_ins = 0;
       if (S.pool_next + R_POOL_CHUNK / 4u > S.pool_end || S.pool_next > S.pool_end) {  // the chunk is (nearly) used up: take a fresh one
-        const uint32_t at = atomicAdd(&st->pool_cursor, R_POOL_CHUNK);
+        const unsigned long long at = atomicAdd(&st->pool_cursor, (unsigned long long)R_POOL_CHUNK);
         if (at <= L.pool_cap && R_POOL_CHUNK <= L.pool_cap - at) {
-          S.pool_next = at;
-          S.pool_end = at + R_POOL_CHUNK;
+          S.pool_base = at;
+          S.pool_next = 0;
+          S.pool_end = R_POOL_CHUNK;
         } else {
           S.pool_next = S.pool_end = 0;  // (the decision keeps this from happening; lists then come from the cursor and fail its check)
         }
@@ -1547,20 +1555,20 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
             const uint32_t wtotal = __shfl_sync(0xFFFFFFFFu, inc, 31);
             // the warp's list cells come out of the block's private chunk of the pool (a shared-memory bump); only a warp that
             // needs more than a chunk holds, or finds the chunk used up, goes to the grid-wide cursor
-            uint32_t wbase = 0;
+            unsigned long long wbase = 0;
             if (lane == 31 && wtotal) {
               bool got = false;
               if (wtotal <= R_POOL_CHUNK / 4u) {
                 const uint32_t at = atomicAdd(&S.pool_next, wtotal);
                 if (at + wtotal <= S.pool_end) {
-                  wbase = at;
+                  wbase = S.pool_base + at;
                   got = true;
                 }
               }
               if (!got) {
                 // (a failed bump leaves pool_next past pool_end: every later warp of the round takes this path too, and the
                 // block fetches a fresh chunk at the start of its next P2)
-                wbase = atomicAdd(&st->pool_cursor, wtotal);
+                wbase = atomicAdd(&st->pool_cursor, (unsigned long long)wtotal);
               }
             }
             uint32_t s = NOSLOT, hot_s = NOSLOT, hot_key = 0;
@@ -1593,13 +1601,13 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
             if (im && lane == (uint32_t)(__ffs(im) - 1)) atomicAdd(&S.keys_ins, (uint32_t)__popc(im));
             wbase = __shfl_sync(0xFFFFFFFFu, wbase, 31);
             if (born && s != NOSLOT) {
-              uint32_t start = wbase + (inc - mylen);
+              unsigned long long start = wbase + (inc - mylen);
               if (start > L.pool_cap || mylen > L.pool_cap - start) {
                 atomicOr(&st->err, ERR_POOL_FULL);
                 start = 0;
                 mylen = 0;
               }
-              t.occ_start[s] = start;
+              t.occ_start.set(s, start);
               t.occ_len[s] = mylen;
               t.occ_fill[s] = 0;
               round_slotrow(R, par, jj, side)[tok] = s;
@@ -1760,7 +1768,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       if (tid < 2 && tv.p[0]) {  // the next decision reads the list fields of its candidates: ask for them now
         const uint32_t ps = tid == 0 ? tv.s[0] : tv.s[RT - 1];
         if (ps != NOSLOT) {
-          prefetch_l2(t.occ_start + ps);
+          prefetch_l2(t.occ_start.addr(ps));
           prefetch_l2(t.occ_len + ps);
         }
       }

@@ -25,7 +25,7 @@ namespace bpe {
 struct DevState {
   // persistent
   uint32_t n_keys;
-  uint32_t pool_cursor;
+  unsigned long long pool_cursor;  // next free cell of the occurrence pool (64-bit: the pool may pass 2^32 cells)
   uint32_t err;
   uint32_t hot_n;
   uint32_t hot_thresh;
@@ -51,7 +51,8 @@ struct DevState {
   unsigned long long sites_total;
   // snapshot taken by block 0 while nothing changes these (start of P3), read by every block for its exit decision:
   // the decision must not depend on values a faster block may already be changing in the next phase
-  uint32_t snap_n_keys, snap_pool_cursor, snap_hot_n, snap_err;
+  uint32_t snap_n_keys, snap_hot_n, snap_err;
+  unsigned long long snap_pool_cursor;
   unsigned long long prof_ns[8];  // block 0's view: decide, P1 work, P1 wait, P2 work, P2 wait, P3 work, P3 wait, tie path
   uint32_t bins[36];  // histogram of bit lengths of counts (hot-list threshold selection)
   // ---- sharded (multi-GPU) training, mg_kernels.cuh ----
@@ -159,13 +160,14 @@ static_assert(K1_SMEM_SLOTS % K1B_THREADS == 0 && K1B_THREADS % 32 == 0, "the pr
 struct SmemHist {
   uint32_t key[K1_SMEM_SLOTS];
   uint32_t a[K1_SMEM_SLOTS];  // k_hist: adjacencies seen        k_scatter: count, then staging cursor
-  uint32_t b[K1_SMEM_SLOTS];  // k_hist: of which NOT counted    k_scatter: base cell in the pool
+  uint32_t b[K1_SMEM_SLOTS];  // k_hist: of which NOT counted    k_scatter: base cell in the pool, low word
 };
 
 // k_scatter's dynamic shared memory: the block-local table, where each slot's run starts in the staging buffer, and the
 // staging buffer itself (the chunk's adjacencies as 16-bit offsets, grouped by slot)
 struct SmemScatter {
   SmemHist h;
+  uint32_t bhi[K1_SMEM_SLOTS];  // high word of the base cell (NOPOS: the pair is missing from the table)
   uint32_t start[K1_SMEM_SLOTS + 1];
   uint32_t warp_sum[K1B_THREADS / 32];
   uint16_t stage[K1B_CHUNK];
@@ -283,16 +285,16 @@ __global__ void __launch_bounds__(K1_THREADS) k_hist(const uint32_t* __restrict_
 }
 
 // carve every pair's occurrence list out of the pool
-__global__ void k_alloc_lists(PairTable t, DevState* st, uint32_t pool_cap) {
+__global__ void k_alloc_lists(PairTable t, DevState* st, unsigned long long pool_cap) {
   uint32_t cap = t.mask + 1;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < cap; i += gridDim.x * blockDim.x) {
     if (t.keys[i] == EMPTY_KEY) continue;
     uint32_t len = t.occ_len[i];
     t.occ_fill[i] = 0;
     if (len == 0) continue;
-    uint32_t start = atomicAdd(&st->pool_cursor, len);
+    const unsigned long long start = atomicAdd(&st->pool_cursor, (unsigned long long)len);
     if (start > pool_cap || len > pool_cap - start) atomicOr(&st->err, ERR_POOL_FULL);
-    t.occ_start[i] = start;
+    t.occ_start.set(i, start);
   }
 }
 
@@ -373,9 +375,11 @@ __global__ void __launch_bounds__(K1B_THREADS) k_scatter(const uint32_t* __restr
         uint32_t gs = tbl_find(t, sh.h.key[i]);
         if (gs == NOSLOT) {
           atomicOr(&st->err, ERR_MISSING_KEY);
-          sh.h.b[i] = NOPOS;
+          sh.bhi[i] = NOPOS;
         } else {
-          sh.h.b[i] = t.occ_start[gs] + atomicAdd(t.occ_fill + gs, cnt[e]);
+          const unsigned long long base = t.occ_start.get(gs) + atomicAdd(t.occ_fill + gs, cnt[e]);
+          sh.h.b[i] = (uint32_t)base;
+          sh.bhi[i] = (uint32_t)(base >> 32);  // (< 4: the pool holds at most 3 * 2^32 cells)
         }
       }
       sh.h.a[i] = run;  // staging cursor
@@ -397,7 +401,7 @@ __global__ void __launch_bounds__(K1B_THREADS) k_scatter(const uint32_t* __restr
           } else {  // pair did not fit the block-local table: one global cursor atomic
             uint32_t gs = tbl_find(t, key);
             if (gs == NOSLOT) atomicOr(&st->err, ERR_MISSING_KEY);
-            else pool[t.occ_start[gs] + atomicAdd(t.occ_fill + gs, 1u)] = p0 + j;
+            else pool[t.occ_start.get(gs) + atomicAdd(t.occ_fill + gs, 1u)] = p0 + j;
           }
         }
       }
@@ -409,8 +413,8 @@ __global__ void __launch_bounds__(K1B_THREADS) k_scatter(const uint32_t* __restr
 #pragma unroll
       for (uint32_t half = K1_SMEM_SLOTS / 2; half; half >>= 1)
         if (sh.start[s + half] <= k) s += half;
-      const uint32_t base = sh.h.b[s];
-      if (base != NOPOS) pool[base + (k - sh.start[s])] = c0 + sh.stage[k];
+      const uint32_t hi = sh.bhi[s];
+      if (hi != NOPOS) pool[(((unsigned long long)hi << 32) | sh.h.b[s]) + (k - sh.start[s])] = c0 + sh.stage[k];
     }
     __syncthreads();
   }
@@ -582,7 +586,8 @@ __device__ __forceinline__ void phase_tie(const uint32_t* slots, uint32_t n, con
     uint32_t s = cands[c];
     uint32_t key = t.keys[s];
     uint32_t a = key >> 16, b = key & 0xFFFFu;
-    uint32_t start = t.occ_start[s], len = t.occ_len[s];
+    const unsigned long long start = t.occ_start.get(s);
+    uint32_t len = t.occ_len[s];
     uint32_t v = 0;  // 1 + max position, 0 = none
     for (uint32_t i = threadIdx.x; i < len; i += blockDim.x) {
       uint32_t p = pool[start + i];
@@ -866,11 +871,12 @@ __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint
   const uint32_t n = A.n;
   const PairTable& t = A.t;
   DevState* st = A.st;
-  uint32_t list_start = 0, total = n;
+  unsigned long long list_start = 0;
+  uint32_t total = n;
   if (!A.scan_mode) {
     uint32_t s = pair_slot;
     total = (s == NOSLOT) ? 0 : t.occ_len[s];
-    list_start = (s == NOSLOT) ? 0 : t.occ_start[s];
+    list_start = (s == NOSLOT) ? 0 : t.occ_start.get(s);
   }
   uint32_t lane = lane_id();
   uint32_t total_round = (total + 31u) & ~31u;
@@ -1037,7 +1043,7 @@ __device__ __forceinline__ void loop_flush_stage(const ApplyArgs& A, uint32_t* s
 // through the sharded exchange), hot list.  The cells are cleared for the next merge; ND_*_SLOT keeps the table slot for
 // phase_apply.
 __device__ __forceinline__ void phase_new_pairs(const ApplyArgs& A, uint32_t c, const uint32_t* len16, uint32_t max_length,
-                                                int hot_valid, uint32_t* hot, uint32_t hot_cap, uint32_t pool_cap, bool counts_elsewhere,
+                                                int hot_valid, uint32_t* hot, uint32_t hot_cap, unsigned long long pool_cap, bool counts_elsewhere,
                                                 uint32_t vt, uint32_t nvt,  // virtual thread id / count (whole warps)
                                                 Best* mine = nullptr,       // arg-max candidate of the caller: pairs that go onto the hot list join it
                                                 uint32_t* mine_key = nullptr) {  // ... and the key of that candidate
@@ -1077,17 +1083,17 @@ __device__ __forceinline__ void phase_new_pairs(const ApplyArgs& A, uint32_t c, 
       if ((int)lane >= o) inc += v;
     }
     uint32_t wtotal = __shfl_sync(0xFFFFFFFFu, inc, 31);
-    uint32_t wbase = 0;
-    if (lane == 31 && wtotal) wbase = atomicAdd(&st->pool_cursor, wtotal);
+    unsigned long long wbase = 0;
+    if (lane == 31 && wtotal) wbase = atomicAdd(&st->pool_cursor, (unsigned long long)wtotal);
     wbase = __shfl_sync(0xFFFFFFFFu, wbase, 31);
     if (!act || s == NOSLOT) continue;
-    uint32_t start = wbase + (inc - mylen);
+    unsigned long long start = wbase + (inc - mylen);
     if (start > pool_cap || len > pool_cap - start) {
       atomicOr(&st->err, ERR_POOL_FULL);
       start = 0;
       len = 0;
     }
-    t.occ_start[s] = start;
+    t.occ_start.set(s, start);
     t.occ_len[s] = len;
     t.occ_fill[s] = 0;
     A.nd[(size_t)(side ? ND_R_SLOT : ND_L_SLOT) * ND_STRIDE + tok] = s;
@@ -1119,13 +1125,13 @@ __device__ __forceinline__ void phase_new_pairs(const ApplyArgs& A, uint32_t c, 
 }
 
 // K3 phase 3: rewrite the corpus in place and fill the new pairs' occurrence lists.
-__device__ __forceinline__ uint32_t agg_cursor(const PairTable& t, uint32_t slot, bool has) {
+__device__ __forceinline__ unsigned long long agg_cursor(const PairTable& t, uint32_t slot, bool has) {
   uint32_t lane = lane_id();
   uint32_t k = has ? slot : (0xFFFFFF00u + lane);
   uint32_t peers = __match_any_sync(0xFFFFFFFFu, k);
   uint32_t leader = __ffs(peers) - 1;
-  uint32_t base = 0;
-  if (has && lane == leader) base = t.occ_start[slot] + atomicAdd(t.occ_fill + slot, (uint32_t)__popc(peers));
+  unsigned long long base = 0;
+  if (has && lane == leader) base = t.occ_start.get(slot) + atomicAdd(t.occ_fill + slot, (uint32_t)__popc(peers));
   base = __shfl_sync(0xFFFFFFFFu, base, leader);
   return base + __popc(peers & ((1u << lane) - 1u));
 }
@@ -1184,8 +1190,9 @@ __device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites,
   const PairTable& t = A.t;
   const SiteRec* const sites = site_buf ? site_buf : A.sites;
   uint32_t* const scnt = stage;                      // [2][R_STAGE_T]: the block's cells per (side, token), then its tickets
-  uint32_t* const sbase = stage + 2u * R_STAGE_T;    // [2][R_STAGE_T]: start of the block's range in that list (FILL_NONE: no list)
-  constexpr uint32_t FILL_NONE = 0xFFFFFFFFu;
+  // [2][R_STAGE_T] u64 over the other four rows: start of the block's range in that list (FILL_NONE: no list)
+  unsigned long long* const sbase = reinterpret_cast<unsigned long long*>(stage + 2u * R_STAGE_T);
+  constexpr unsigned long long FILL_NONE = ~0ull;
   uint32_t round = (n_sites + 31u) & ~31u;
   for (uint32_t i = vt; i < round; i += nvt) {
     bool has = i < n_sites;
@@ -1200,8 +1207,8 @@ __device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites,
     uint32_t rslot = (has && !sr && rv.w != NOTOKV) ? ld_cg(A.nd + (size_t)ND_R_SLOT * ND_STRIDE + rv.w) : NOSLOT;
     bool hl = has && lslot != NOSLOT && t.occ_len[lslot];
     bool hr = has && rslot != NOSLOT && t.occ_len[rslot];
-    uint32_t il = agg_cursor(t, lslot, hl);
-    uint32_t ir = agg_cursor(t, rslot, hr);
+    const unsigned long long il = agg_cursor(t, lslot, hl);
+    const unsigned long long ir = agg_cursor(t, rslot, hr);
     if (hl) A.pool[il] = lpos;
     if (hr) A.pool[ir] = p;
   }
@@ -1213,7 +1220,7 @@ __device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites,
     scnt[e] = 0;
     const uint32_t side = e >= R_STAGE_T ? 1u : 0u, tok = e - side * R_STAGE_T;
     const uint32_t s = ld_cg(A.nd + (size_t)(side ? ND_R_SLOT : ND_L_SLOT) * ND_STRIDE + tok);
-    sbase[e] = (s != NOSLOT && t.occ_len[s]) ? t.occ_start[s] + atomicAdd(t.occ_fill + s, v) : FILL_NONE;
+    sbase[e] = (s != NOSLOT && t.occ_len[s]) ? t.occ_start.get(s) + atomicAdd(t.occ_fill + s, v) : FILL_NONE;
   }
   __syncthreads();
   for (uint32_t i = vt; i < round; i += nvt) {
@@ -1222,12 +1229,12 @@ __device__ __forceinline__ void phase_fill(const ApplyArgs& A, uint32_t n_sites,
     const bool sl = has && rv.z < R_STAGE_T, sr = has && rv.w < R_STAGE_T;
     const uint32_t kl = agg_smem_ticket(scnt, rv.z, sl);
     const uint32_t kr = agg_smem_ticket(scnt, R_STAGE_T + rv.w, sr);
-    const uint32_t bl = sl ? sbase[rv.z] : FILL_NONE, br = sr ? sbase[R_STAGE_T + rv.w] : FILL_NONE;
+    const unsigned long long bl = sl ? sbase[rv.z] : FILL_NONE, br = sr ? sbase[R_STAGE_T + rv.w] : FILL_NONE;
     if (bl != FILL_NONE) A.pool[bl + kl] = rv.y;
     if (br != FILL_NONE) A.pool[br + kr] = rv.x;
   }
   __syncthreads();
-  for (uint32_t e = threadIdx.x; e < 4u * R_STAGE_T; e += blockDim.x) stage[e] = 0;
+  for (uint32_t e = threadIdx.x; e < 6u * R_STAGE_T; e += blockDim.x) stage[e] = 0;
   __syncthreads();
 }
 
@@ -1248,7 +1255,7 @@ __global__ void __launch_bounds__(256) k_sites(ApplyArgs A, uint32_t a, uint32_t
 }
 
 __global__ void __launch_bounds__(256) k_alloc_new(ApplyArgs A, uint32_t c, uint32_t max_length, int hot_valid, uint32_t* __restrict__ hot,
-                                                    uint32_t hot_cap, uint32_t pool_cap) {
+                                                    uint32_t hot_cap, unsigned long long pool_cap) {
   phase_new_pairs(A, c, A.len16, max_length, hot_valid, hot, hot_cap, pool_cap, false, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
 }
 
@@ -1279,7 +1286,7 @@ constexpr int ML_MIN_BLOCKS = ML_THREADS >= 1024 ? 1 : 2;
 
 struct LoopArgs {
   ApplyArgs A;
-  uint32_t pool_cap;
+  unsigned long long pool_cap;  // cells of the occurrence pool
   uint32_t len16_cap;
   uint32_t* hot;
   uint32_t hot_cap;
@@ -1350,7 +1357,8 @@ __device__ __forceinline__ void prefetch_runner_up(const LoopArgs& L, uint32_t w
     r = best_warp_reduce(r);
     if (!r.primary || r.slot == NOSLOT) return;
     skip = r.slot;
-    const uint32_t start = t.occ_start[r.slot], len = t.occ_len[r.slot];
+    const unsigned long long start = t.occ_start.get(r.slot);
+    const uint32_t len = t.occ_len[r.slot];
     if (len > 32768u) continue;  // a merge of that size is throughput bound
     for (uint32_t i = vt; i < len; i += nvt) {
       const uint32_t p = ld_cg(L.A.pool + start + i);
@@ -1383,7 +1391,7 @@ __global__ void k_loop_prepare(DevState* st, uint32_t n_tokens, unsigned long lo
 __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopArgs L) {
   __shared__ Best s_best[ML_THREADS / 32];
   __shared__ uint32_t s_max[32];
-  __shared__ uint32_t s_stage[LS_ROWS * R_STAGE_T];  // loop_flush_stage leaves it zero
+  __shared__ __align__(8) uint32_t s_stage[LS_ROWS * R_STAGE_T];  // loop_flush_stage leaves it zero (phase_fill: u64 rows)
   for (uint32_t i = threadIdx.x; i < LS_ROWS * R_STAGE_T; i += blockDim.x) s_stage[i] = 0;
   const ApplyArgs& A = L.A;
   DevState* st = A.st;
