@@ -24,6 +24,7 @@
 #include <node_api.h>
 #include <stddef.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <string.h>
 
 #include "bpe_b200.h"
@@ -138,6 +139,31 @@ static napi_value Create(napi_env env, napi_callback_info info) { /* create(devi
   if (napi_get_cb_info(env, info, &argc, argv, NULL, NULL) == napi_ok && argc >= 1) napi_get_value_int32(env, argv[0], &device);
   bpe_engine* e = NULL;
   int rc = bpe_create(device, &e);
+  if (rc != BPE_OK) return throw_rc(env, NULL, rc);
+  if (napi_create_external(env, e, finalize_engine, NULL, &out) != napi_ok) {
+    bpe_destroy(e);
+    return NULL;
+  }
+  return out;
+}
+
+static napi_value CreateGroup(napi_env env, napi_callback_info info) { /* createGroup(Int32Array devices) -> engine over those GPUs */
+  size_t argc = 1;
+  napi_value argv[1], out;
+  napi_typedarray_type t;
+  size_t n = 0;
+  void* p = NULL;
+  if (napi_get_cb_info(env, info, &argc, argv, NULL, NULL) != napi_ok || argc < 1 ||
+      napi_get_typedarray_info(env, argv[0], &t, &n, &p, NULL, NULL) != napi_ok || t != napi_int32_array)
+    return throw_type(env, "expected (Int32Array devices)");
+  bpe_engine* e = NULL;
+  int rc = bpe_create_group((const int*)p, (int)n, &e);
+  if (rc == BPE_E_INVALID) {
+    char msg[64];
+    snprintf(msg, sizeof msg, "devices must list 1 to %d distinct GPUs", BPE_MG_MAX_WORLD);
+    napi_throw_error(env, code_name(rc), msg);
+    return NULL;
+  }
   if (rc != BPE_OK) return throw_rc(env, NULL, rc);
   if (napi_create_external(env, e, finalize_engine, NULL, &out) != napi_ok) {
     bpe_destroy(e);
@@ -387,7 +413,7 @@ static napi_value Init(napi_env env, napi_value exports) {
     const char* name;
     napi_callback fn;
   } table[] = {
-      {"create", Create},           {"setTokens", SetTokens},       {"numTokens", NumTokens},       {"loadMerges", LoadMerges},
+      {"create", Create},           {"createGroup", CreateGroup},   {"setTokens", SetTokens},       {"numTokens", NumTokens},       {"loadMerges", LoadMerges},
       {"setChars", SetChars},       {"addDocuments", AddDocuments}, {"restoreDocuments", RestoreDocuments},
       {"addText", AddText},         {"clearCorpus", ClearCorpus},   {"corpusSize", CorpusSize},     {"getCorpus", GetCorpus},
       {"findNextMerge", FindNextMerge}, {"applyMerge", ApplyMerge}, {"applyMerges", ApplyMerges},   {"mergeUntil", MergeUntil},

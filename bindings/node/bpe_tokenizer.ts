@@ -24,6 +24,7 @@ interface Native {
   MAX_TOKENS: number
   ABI_VERSION: number
   create(device?: number): Engine
+  createGroup(devices: Int32Array): Engine
   setTokens(e: Engine, utf16_len: Int32Array): void
   numTokens(e: Engine): number
   loadMerges(e: Engine, abc: Int32Array): void
@@ -124,8 +125,9 @@ export class BPETokenizer {
   private tvi: Int32Array | null = null
   private chars_synced = -1
 
-  constructor(options?: { device?: number }) {
-    this.engine = native.create(options?.device ?? 0)
+  /** `devices`: one engine over those GPUs of this process (bpe_create_group), the corpus sharded by document across them */
+  constructor(options?: { device?: number; devices?: number[] }) {
+    this.engine = options?.devices ? native.createGroup(Int32Array.from(options.devices)) : native.create(options?.device ?? 0)
   }
 
   // ---- plumbing ---------------------------------------------------------------------------------------------------

@@ -44,6 +44,7 @@ i32p, i64p, u8p, vp = C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_
 SYMBOLS = {
     "bpe_abi_version": (C.c_int, []),
     "bpe_create": (C.c_int, [C.c_int, C.POINTER(vp)]),
+    "bpe_create_group": (C.c_int, [C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]),
     "bpe_destroy": (None, [vp]),
     "bpe_last_error": (C.c_char_p, [vp]),
     "bpe_set_stream": (C.c_int, [vp, vp]),

@@ -10,7 +10,11 @@
 #include <cstring>
 #include <functional>
 #include <string>
+#include <condition_variable>
+#include <mutex>
+#include <thread>
 #include <unordered_map>
+#include <unordered_set>
 #include <vector>
 
 #include "encode_kernels.cuh"
@@ -114,6 +118,34 @@ int ilog2(uint32_t p) {
 }
 
 }  // namespace
+
+// Host rendezvous of a group's members before every launch of the sharded mergeUntil loop: no member starts a kernel that waits for
+// its peers while another member still does host work between launches (buffer growth frees memory, and cudaFree waits for the
+// device's kernels).  A member that leaves the loop drops out, so the others never wait for it here.
+struct LaunchGate {
+  std::mutex mu;
+  std::condition_variable cv;
+  int expected;
+  int arrived = 0;
+  uint64_t generation = 0;
+  explicit LaunchGate(int n) : expected(n) {}
+  void release() {
+    arrived = 0;
+    generation++;
+    cv.notify_all();
+  }
+  void arrive() {
+    std::unique_lock<std::mutex> lk(mu);
+    const uint64_t g = generation;
+    if (++arrived >= expected) release();
+    else cv.wait(lk, [&] { return generation != g; });
+  }
+  void drop() {
+    std::lock_guard<std::mutex> lk(mu);
+    expected--;
+    if (arrived > 0 && arrived >= expected) release();
+  }
+};
 
 struct EncodeScratch {
   DevBuf<int32_t> out_tmp;
@@ -219,6 +251,16 @@ struct bpe_engine {
   DevBuf<uint32_t> mg_mark, mg_touched, mg_tie_sorted, mg_export_n, mg_newpair;
   int mg_loop_blocks = 0;
   unsigned long long mg_epoch = 0, mg_tie_epoch = 0;
+  bool mg_timed_out = false;             // the last sharded mergeUntil stopped because a peer did not answer
+  LaunchGate* mg_gate = nullptr;         // group member inside the group's bpe_merge_until: the members' launch rendezvous
+
+  // device group (bpe_create_group): the handle holds one member engine per device, member r initialised as rank r of the group
+  // with its mailbox connected to the others' by pointer.  The handle itself owns no device state; the entry points forward to
+  // the members (group_* below).
+  std::vector<bpe_engine*> members;
+  bool grp_uploaded = false;              // the corpus got its first, partitioned upload: later uploads go to the last member
+  DevBuf<uint32_t> grp_keys, grp_counts;  // member: its pair histogram, exported for the other members to import over NVLink
+  int64_t grp_n = 0;
 
   // text front end (text_kernels.cuh): code point -> single-character token index, -1 = unknown
   DevBuf<int32_t> d_cpmap;
@@ -250,6 +292,8 @@ struct bpe_engine {
   unsigned long long* h_pipe = nullptr;  // pinned: 3 slots x 4 words of per-chunk flags, [12..13] flags of the lane kernel
   PinBuf<int64_t> h_in_off, h_out_off, h_bad;  // pinned staging of document offsets in, output offsets and first offenders out
   int64_t enc_chunk = 128ll << 20;       // input units (ids or bytes) per full-size chunk; BPE_ENC_CHUNK overrides
+  std::vector<int64_t> enc_parts;        // the last host-buffer encode, per chunk: where its vectors wait in x_out, how many
+  int64_t enc_bad_id_pos = -1;           // the last host-buffer encode: input position of an id outside the token table
 
   // scratch
   DevBuf<int32_t> stage_ids;
@@ -1403,6 +1447,13 @@ MgArgs mg_args(bpe_engine* e) {
 int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log, int64_t log_cap,
                    int64_t* n_done) {
   *n_done = 0;
+  e->mg_timed_out = false;
+  struct LeaveGate {
+    LaunchGate* gate;
+    ~LeaveGate() {
+      if (gate) gate->drop();
+    }
+  } leave_gate{e->mg_gate};
   CK(cudaSetDevice(e->device));
   if (!e->mg_connected) return fail(e, BPE_E_INVALID, "sharded engine: call bpe_mg_connect first");
   TRY(ensure_index(e));
@@ -1497,6 +1548,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
     P.M = mg_args(e);
     static const bool trace = getenv("BPE_TRACE") != nullptr;
     auto tw0 = std::chrono::steady_clock::now();
+    if (e->mg_gate) e->mg_gate->arrive();
     k_loop_prepare<<<1, 32, 0, e->stream>>>(e->d_st.p, (uint32_t)e->n_tokens, e->barrier.p);
     e->stats.kernel_launches++;
     if (use_rounds && !legacy_above) {
@@ -1581,8 +1633,10 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
     }
     if (status == LOOP_ERROR) {
       uint32_t f = e->h_st->err | e->h_st->g_vals[0];
-      if (f & ERR_PEER_TIMEOUT) rc = fail(e, BPE_E_INTERNAL, "a peer GPU did not answer within %.0f s (flags 0x%x)", MG_TIMEOUT_NS / 1e9, f);
-      else {
+      if (f & ERR_PEER_TIMEOUT) {
+        e->mg_timed_out = true;
+        rc = fail(e, BPE_E_INTERNAL, "a peer GPU did not answer within %.0f s (flags 0x%x)", MG_TIMEOUT_NS / 1e9, f);
+      } else {
         rc = check_dev_err(e);
         if (rc == BPE_OK) rc = fail(e, BPE_E_INTERNAL, "sharded merge loop stopped: local flags 0x%x, all ranks 0x%x", e->h_st->err, e->h_st->g_vals[0]);
       }
@@ -1739,6 +1793,443 @@ int merge_until_host(bpe_engine* e, int64_t min_weight, int32_t max_length, int6
 }
 
 
+// mailbox of rank `rank` in a sharded corpus of `world` engines: the peers store their count deltas into it (mg_kernels.cuh)
+int mg_alloc_mailbox(bpe_engine* e, int rank, int world) {
+  e->mg_rank = rank;
+  e->mg_world = world;
+  // records one rank can send per exchange (k_merge_rounds: the cells of up to 16 merges a round; k_merge_loop_mg: of one merge)
+  e->mg_inbox_stride = 1u << 20;
+  e->mg_tie_cap = 4096;
+  size_t bytes = (size_t)2 * MG_MAX_WORLD * 128 + (size_t)2 * world * e->mg_inbox_stride * 8 + (size_t)2 * world * e->mg_tie_cap * 4;
+  CK(cudaMalloc(&e->mg_mailbox, bytes));
+  CK(cudaMemset(e->mg_mailbox, 0, bytes));
+  e->mg_mailbox_bytes = bytes;
+  e->mg_peer[rank] = e->mg_mailbox;
+  e->index_valid = false;  // per-slot side arrays are allocated with the table
+  return BPE_OK;
+}
+
+// a batch of restoreMerge lines (a_i, b_i) -> n_tokens + i: every operand must exist when its merge comes
+int check_merge_list(bpe_engine* e, const int32_t* ab, int64_t n) {
+  if ((int64_t)e->n_tokens + n > BPE_MAX_TOKENS) return fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
+  for (int64_t i = 0; i < n; i++)
+    if (ab[2 * i] < 0 || ab[2 * i + 1] < 0 || ab[2 * i] >= e->n_tokens + i || ab[2 * i + 1] >= e->n_tokens + i)
+      return fail(e, BPE_E_INVALID, "merge %lld refers to a token that does not exist yet", (long long)i);
+  return BPE_OK;
+}
+
+// ---- device groups (bpe_create_group): the GPUs of one process hold one corpus, sharded by document ----------------------------
+// Member r is an ordinary engine on devices[r], rank r of the group as bpe_mg_init makes it, so the sharded kernels run unchanged;
+// the mailboxes are connected by pointer under peer access (cudaIpcOpenMemHandle cannot open a handle its own process exported).
+// Every call that runs device work on several members runs each member on a host thread of its own: the sharded mergeUntil waits
+// on the host after every launch, so one thread driving the members in turn would leave member 0's cooperative kernel waiting for
+// peers that were never launched.
+bool is_group(const bpe_engine* e) { return e && !e->members.empty(); }
+
+#define GROUP_REFUSES(e, what)                                                                                                  \
+  do {                                                                                                                          \
+    if (is_group(e)) return fail(e, BPE_E_INVALID, "%s is not available on a device group (a corpus sharded over its GPUs)", what); \
+  } while (0)
+
+// the group's answer for a call that one member ran on the caller's thread
+int member_rc(bpe_engine* g, const bpe_engine* m, int rc) {
+  return rc == BPE_OK ? rc : fail(g, rc, "device %d: %s", m->device, m->err.c_str());
+}
+
+// Runs fn(r) for every member on its own host thread and joins them all.  A member that fails inside the sharded mergeUntil leaves
+// its peers waiting until the peer timeout (MG_TIMEOUT_NS), so the group reports the first member's error that is not such a
+// timeout, and the timeout only when there is nothing else.
+int run_members(bpe_engine* g, const std::function<int(int)>& fn) {
+  const int n = (int)g->members.size();
+  std::vector<int> rc((size_t)n, BPE_OK);
+  std::vector<std::thread> threads;
+  threads.reserve((size_t)n);
+  for (bpe_engine* m : g->members) m->mg_timed_out = false;  // (a timeout is a verdict about this call only)
+  for (int r = 0; r < n; r++) {
+    try {
+      threads.emplace_back([&rc, &fn, r] { rc[(size_t)r] = fn(r); });
+    } catch (...) {
+      rc[(size_t)r] = fail(g->members[(size_t)r], BPE_E_NOMEM, "cannot start a host thread for this member");
+      if (g->members[(size_t)r]->mg_gate) g->members[(size_t)r]->mg_gate->drop();  // (the others must not wait for it)
+    }
+  }
+  for (std::thread& t : threads) t.join();
+  int pick = -1;
+  for (int r = 0; r < n && pick < 0; r++)
+    if (rc[(size_t)r] != BPE_OK && !g->members[(size_t)r]->mg_timed_out) pick = r;
+  for (int r = 0; r < n && pick < 0; r++)
+    if (rc[(size_t)r] != BPE_OK) pick = r;
+  return pick < 0 ? BPE_OK : member_rc(g, g->members[(size_t)pick], rc[(size_t)pick]);
+}
+
+// Document boundaries of a contiguous partition of documents [0, n_docs) over n parts, balanced by units (ids or bytes): part r owns
+// [b[r], b[r+1]), the documents whose first unit lies in [r*T/n, (r+1)*T/n) of the T units; empty trailing documents go to the
+// last part.  (bpe_tokenizer_b200/sharded.py, shard_bounds, states the same rule for one process per GPU.)
+std::vector<int64_t> shard_bounds(const int64_t* off, int64_t n_docs, int n) {
+  std::vector<int64_t> b((size_t)n + 1, 0);
+  if (n_docs == 0) return b;
+  const int64_t total = off[n_docs] - off[0];
+  int64_t d = 0;
+  for (int r = 1; r < n; r++) {
+    const int64_t cut = (total * r + n - 1) / n;
+    while (d < n_docs && off[d] - off[0] < cut) d++;
+    b[(size_t)r] = d;
+  }
+  b[(size_t)n] = n_docs;
+  return b;
+}
+
+// Where an upload's documents go.  The first upload of a corpus is partitioned; a later one (the reference allows addToCorpus at any
+// time, also after merges) goes to the last member whole, so that the global scan order (member, position) stays the document order
+// the reference's tie-break needs (core.ts:294-305).
+std::vector<int64_t> upload_bounds(const bpe_engine* g, const int64_t* off, int64_t n_docs) {
+  const int n = (int)g->members.size();
+  if (!g->grp_uploaded) return shard_bounds(off, n_docs, n);
+  std::vector<int64_t> b((size_t)n + 1, 0);
+  b[(size_t)n] = n_docs;
+  return b;
+}
+
+// pair counts are global only while no member's corpus changed: an upload anywhere sends every member back to a fresh index
+void after_upload(bpe_engine* g) {
+  g->grp_uploaded = true;
+  for (bpe_engine* m : g->members) {
+    m->index_valid = false;
+    m->hot_valid = false;
+  }
+}
+
+uint64_t group_slots(const bpe_engine* g) {
+  uint64_t s = 0;
+  for (const bpe_engine* m : g->members) s += m->n_slots;
+  return s;
+}
+
+// The new characters of a text batch split over parts that hold contiguous document ranges in order, in the batch's first-appearance
+// order (core.ts:186-199): per part (code points, first positions within the part), the key is (part, first position), and a
+// character that several parts report belongs to the first of them.  (sharded.py, order_new_chars, for one process per GPU.)
+std::vector<int32_t> order_new_chars(const std::vector<std::vector<int32_t>>& cps, const std::vector<std::vector<int64_t>>& pos) {
+  std::unordered_set<int32_t> seen;
+  std::vector<int32_t> out;
+  for (size_t r = 0; r < cps.size(); r++) {
+    std::vector<size_t> order(cps[r].size());
+    for (size_t k = 0; k < order.size(); k++) order[k] = k;
+    std::stable_sort(order.begin(), order.end(), [&](size_t x, size_t y) { return pos[r][x] < pos[r][y]; });
+    for (size_t k : order)
+      if (seen.insert(cps[r][k]).second) out.push_back(cps[r][k]);
+  }
+  return out;
+}
+
+int group_add_documents(bpe_engine* g, const int32_t* ids, const int64_t* off, int64_t n_docs, bool restore) {
+  TRY(check_offsets(g, off, n_docs));
+  if (n_docs == 0) return BPE_OK;
+  const std::vector<int64_t> b = upload_bounds(g, off, n_docs);
+  // as on one engine, a refused upload adds nothing: the members that appended their range drop it again
+  struct Mark {
+    uint64_t n_slots, live_tokens;
+    size_t n_docs;
+  };
+  std::vector<Mark> marks;
+  for (const bpe_engine* m : g->members) marks.push_back({m->n_slots, m->live_tokens, m->doc_off.size()});
+  const int rc = run_members(g, [&](int r) {
+    const int64_t nd = b[(size_t)r + 1] - b[(size_t)r];
+    if (nd == 0) return BPE_OK;
+    bpe_engine* m = g->members[(size_t)r];
+    return restore ? bpe_restore_documents(m, ids, off + b[(size_t)r], nd) : bpe_add_documents(m, ids, off + b[(size_t)r], nd);
+  });
+  if (rc != BPE_OK) {
+    for (size_t r = 0; r < g->members.size(); r++) {
+      bpe_engine* m = g->members[r];
+      if (m->doc_off.size() == marks[r].n_docs) continue;
+      m->n_slots = marks[r].n_slots;  // (slots past n_slots are unused storage)
+      m->live_tokens = marks[r].live_tokens;
+      m->doc_off.resize(marks[r].n_docs);
+      m->index_valid = false;
+      m->hot_valid = false;
+    }
+    return rc;
+  }
+  after_upload(g);
+  return BPE_OK;
+}
+
+// bpe_add_text: stage on every member, agree on one order of the new characters, commit that list everywhere, sum the counts
+int group_add_text(bpe_engine* g, const uint8_t* utf8, const int64_t* off, int64_t n_docs, int32_t* new_code_points, int32_t new_cap,
+                   int32_t* n_new, int64_t* counts, int64_t counts_cap) {
+  TRY(check_offsets(g, off, n_docs));
+  const size_t n = g->members.size();
+  const std::vector<int64_t> b = upload_bounds(g, off, n_docs);
+  const int32_t list_cap = 1 << 16;  // bpe_add_text_stage reports at most this many
+  std::vector<std::vector<int32_t>> cps(n, std::vector<int32_t>((size_t)list_cap));
+  std::vector<std::vector<int64_t>> pos(n, std::vector<int64_t>((size_t)list_cap));
+  std::vector<int32_t> nn(n, 0);
+  auto drop_staged = [&] {
+    for (bpe_engine* m : g->members) m->txt_staged = false;
+  };
+  int rc = run_members(g, [&](int r) {
+    return bpe_add_text_stage(g->members[(size_t)r], utf8, off + b[(size_t)r], b[(size_t)r + 1] - b[(size_t)r], cps[(size_t)r].data(),
+                              pos[(size_t)r].data(), list_cap, &nn[(size_t)r]);
+  });
+  if (rc != BPE_OK) {
+    drop_staged();
+    return rc;
+  }
+  for (size_t r = 0; r < n; r++) {
+    cps[r].resize((size_t)nn[r]);
+    pos[r].resize((size_t)nn[r]);
+  }
+  const std::vector<int32_t> fresh = order_new_chars(cps, pos);
+  const int32_t nt = g->members[0]->n_tokens, nf = (int32_t)fresh.size();
+  // judged on the global list, before any member changes
+  if ((int64_t)nt + nf > BPE_MAX_TOKENS) {
+    drop_staged();
+    return fail(g, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
+  }
+  if (nf > new_cap) {
+    drop_staged();
+    *n_new = nf;
+    return fail(g, BPE_E_CAPACITY, "%d new characters, room for %d", nf, new_cap);
+  }
+  if (counts && counts_cap < (int64_t)nt + nf) {
+    drop_staged();
+    return fail(g, BPE_E_CAPACITY, "counts holds %lld entries, need %d", (long long)counts_cap, nt + nf);
+  }
+  std::vector<std::vector<int64_t>> cnt(n, std::vector<int64_t>((size_t)nt + nf + 1));
+  rc = run_members(g, [&](int r) { return bpe_add_text_commit(g->members[(size_t)r], fresh.data(), nf, cnt[(size_t)r].data(), (int64_t)nt + nf); });
+  if (n_docs) after_upload(g);
+  if (rc != BPE_OK) return rc;
+  std::copy(fresh.begin(), fresh.end(), new_code_points);
+  *n_new = nf;
+  if (counts)
+    for (int64_t i = 0; i < (int64_t)nt + nf; i++) {
+      counts[i] = 0;
+      for (size_t r = 0; r < n; r++) counts[i] += cnt[r][(size_t)i];
+    }
+  return BPE_OK;
+}
+
+// Sums the members' pair histograms into every member's table, once per index build: each member exports its (pair, count) list into
+// device buffers it owns, then every member imports every peer's list straight from the peer's memory (no host copy).
+int group_exchange_counts(bpe_engine* g) {
+  bool global = true;
+  for (const bpe_engine* m : g->members) global = global && m->index_valid && m->mg_counts_global;
+  if (global) return BPE_OK;
+  for (bpe_engine* m : g->members) m->index_valid = false;  // (no member may import into counts that are already summed)
+  TRY(run_members(g, [&](int r) {
+    bpe_engine* e = g->members[(size_t)r];
+    int64_t n = 0;
+    TRY(bpe_mg_export_counts(e, nullptr, nullptr, 0, &n));  // builds the index; n = its number of pairs
+    const size_t cap = (size_t)std::max<int64_t>(n, 1);
+    CK(e->grp_keys.reserve(cap));
+    CK(e->grp_counts.reserve(cap));
+    TRY(bpe_mg_export_counts(e, e->grp_keys.p, e->grp_counts.p, (int64_t)cap, &n));
+    e->grp_n = n;
+    return BPE_OK;
+  }));
+  const int n = (int)g->members.size();
+  return run_members(g, [&](int r) {
+    bpe_engine* e = g->members[(size_t)r];
+    const int last = (r == n - 1) ? n - 2 : n - 1;
+    for (int q = 0; q < n; q++) {
+      if (q == r) continue;
+      const bpe_engine* p = g->members[(size_t)q];
+      TRY(bpe_mg_import_counts(e, p->grp_keys.p, p->grp_counts.p, p->grp_n, q == last));
+    }
+    return BPE_OK;
+  });
+}
+
+int group_merge_until(bpe_engine* g, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log, int64_t log_cap,
+                      int64_t* n_done) {
+  *n_done = 0;
+  if (group_slots(g) == 0) return BPE_OK;  // (as one engine: an empty corpus has no pair)
+  TRY(group_exchange_counts(g));
+  const size_t n = g->members.size();
+  const int64_t cap = std::min<int64_t>(log_cap, BPE_MAX_TOKENS);  // (no run can log more merges than there are free token indices)
+  std::vector<std::vector<bpe_merge>> logs(n, std::vector<bpe_merge>((size_t)cap));
+  std::vector<int64_t> done(n, 0);
+  LaunchGate gate((int)n);
+  for (bpe_engine* m : g->members) m->mg_gate = &gate;
+  const int rc = run_members(g, [&](int r) {
+    return bpe_merge_until(g->members[(size_t)r], min_weight, max_length, max_iterations, logs[(size_t)r].data(), cap, &done[(size_t)r]);
+  });
+  for (bpe_engine* m : g->members) m->mg_gate = nullptr;
+  for (size_t r = 1; r < n; r++)
+    if (done[r] != done[0] || (done[0] && memcmp(logs[r].data(), logs[0].data(), (size_t)done[0] * sizeof(bpe_merge)) != 0))
+      return rc != BPE_OK ? rc : fail(g, BPE_E_INTERNAL, "device %d and device %d returned different merge logs", g->members[0]->device, g->members[r]->device);
+  if (done[0]) memcpy(log, logs[0].data(), (size_t)done[0] * sizeof(bpe_merge));
+  *n_done = done[0];
+  return rc;
+}
+
+// bpe_encode_batch / bpe_encode_text_batch.  The documents are split into contiguous ranges balanced by input units, one per member,
+// and the members' pipelines run in parallel, without copying their vectors out: they stay in each member's staging buffer on its
+// device, and each member reports its size.  Once every size is known, each member copies its vectors from its device straight to
+// their place in the caller's `out`, all members at once.  Cost beside the members' pipelines: the device-to-host copy of the output
+// runs after the encode instead of overlapping it.
+int group_encode(bpe_engine* g, bool is_text, const int32_t* ids, const uint8_t* utf8, const int64_t* off, int64_t n_docs,
+                 const int32_t* to_vector_index, int32_t n_tvi, int32_t* out, int64_t out_cap, int64_t* out_offsets, int64_t* first_bad,
+                 int64_t* n_out, int64_t* unknown_pos, int32_t* unknown_code_point) {
+  *n_out = 0;
+  if (n_docs == 0) {
+    out_offsets[0] = 0;
+    return BPE_OK;
+  }
+  TRY(check_offsets(g, off, n_docs));
+  const size_t n = g->members.size();
+  const std::vector<int64_t> b = shard_bounds(off, n_docs, (int)n);
+  std::vector<std::vector<int64_t>> moff(n);
+  std::vector<int64_t> k(n, 0), upos(n, -1), cum(n + 1, 0);
+  std::vector<int32_t> ucp(n, 0);
+  std::vector<int> mrc(n, BPE_OK);
+  for (size_t r = 0; r < n; r++) moff[r].assign((size_t)(b[r + 1] - b[r]) + 1, 0);
+  const int rc = run_members(g, [&](int r) {
+    const size_t i = (size_t)r;
+    const int64_t nd = b[i + 1] - b[i];
+    if (nd == 0) return BPE_OK;
+    bpe_engine* m = g->members[i];
+    int64_t* fb = first_bad ? first_bad + b[i] : nullptr;
+    const int got = is_text ? bpe_encode_text_batch(m, utf8, off + b[i], nd, to_vector_index, n_tvi, nullptr, 0, moff[i].data(), fb, &k[i], &upos[i], &ucp[i])
+                            : bpe_encode_batch(m, ids, off + b[i], nd, to_vector_index, n_tvi, nullptr, 0, moff[i].data(), fb, &k[i]);
+    mrc[i] = got == BPE_E_CAPACITY ? BPE_OK : got;  // (no output buffer: the member reports its size, offsets and first_bad complete)
+    return mrc[i];
+  });
+  if (rc != BPE_OK) {
+    // the error the first failing member met is the first in batch order; its positions are relative to the member's range
+    size_t r = 0;
+    while (r < n && mrc[r] == BPE_OK) r++;
+    if (r < n && upos[r] >= 0) {  // an unknown character: the members before r held this many code points (lead bytes, as text_kernels.cuh counts)
+      int64_t before = 0;
+      for (int64_t p = off[0]; p < off[b[r]]; p++) before += (utf8[p] & 0xC0) != 0x80;
+      if (unknown_pos) *unknown_pos = before + upos[r];
+      if (unknown_code_point) *unknown_code_point = ucp[r];
+    }
+    if (r < n && !is_text && g->members[r]->enc_bad_id_pos >= 0) {
+      const int64_t pos = off[b[r]] - off[0] + g->members[r]->enc_bad_id_pos;
+      return fail(g, BPE_E_INVALID, "id %d at %lld outside the token table", ids[off[0] + pos], (long long)pos);
+    }
+    return rc;
+  }
+  for (size_t r = 0; r < n; r++) cum[r + 1] = cum[r] + k[r];
+  for (size_t r = 0; r < n; r++)
+    for (int64_t d = 0; d < b[r + 1] - b[r]; d++) out_offsets[b[r] + d] = moff[r][(size_t)d] + cum[r];
+  out_offsets[n_docs] = cum[n];
+  *n_out = cum[n];
+  if (cum[n] > out_cap || (cum[n] && !out)) return fail(g, BPE_E_CAPACITY, "output buffer holds %lld values, need %lld", (long long)out_cap, (long long)cum[n]);
+  return run_members(g, [&](int r) {
+    bpe_engine* e = g->members[(size_t)r];
+    if (k[(size_t)r] == 0) return BPE_OK;
+    CK(cudaSetDevice(e->device));
+    int32_t* dst = out + cum[(size_t)r];
+    for (size_t c = 0; c + 1 < e->enc_parts.size(); c += 2) {
+      const int64_t reg = e->enc_parts[c], len = e->enc_parts[c + 1];
+      if (len) CK(cudaMemcpyAsync(dst, e->x_out.p + reg, (size_t)len * sizeof(int32_t), cudaMemcpyDeviceToHost, e->s_out));
+      dst += len;
+    }
+    CK(cudaStreamSynchronize(e->s_out));
+    return BPE_OK;
+  });
+}
+
+// bpe_decode_batch.  Decoded bytes have no bound the caller's buffer must meet, so the members first report their sizes (the values
+// and the token bytes go up, the lengths are scanned), then decode straight into the caller's `out` at their place: the upload and
+// the length pass run twice, the gather and the copy out once.
+int group_decode(bpe_engine* g, const int32_t* values, const int64_t* off, int64_t n_docs, const int32_t* from_vector_index, int32_t n_fvi,
+                 const uint8_t* token_bytes, const int64_t* token_byte_offsets, int32_t n_tokens, uint8_t* out, int64_t out_cap,
+                 int64_t* out_offsets, int64_t* first_bad, int64_t* n_out) {
+  *n_out = 0;
+  TRY(check_offsets(g, off, n_docs));
+  if (n_docs == 0) {
+    bpe_engine* m = g->members[0];
+    return member_rc(g, m, bpe_decode_batch(m, values, off, 0, from_vector_index, n_fvi, token_bytes, token_byte_offsets, n_tokens, out, out_cap,
+                                            out_offsets, first_bad, n_out));
+  }
+  const size_t n = g->members.size();
+  const std::vector<int64_t> b = shard_bounds(off, n_docs, (int)n);
+  std::vector<std::vector<int64_t>> moff(n);
+  std::vector<int64_t> k(n, 0), cum(n + 1, 0);
+  for (size_t r = 0; r < n; r++) moff[r].assign((size_t)(b[r + 1] - b[r]) + 1, 0);
+  auto pass = [&](bool sizes) {
+    return run_members(g, [&](int r) {
+      const size_t i = (size_t)r;
+      const int64_t nd = b[i + 1] - b[i];
+      if (nd == 0 || (!sizes && k[i] == 0)) return BPE_OK;
+      uint8_t* dst = sizes ? nullptr : out + cum[i];
+      const int got = bpe_decode_batch(g->members[i], values, off + b[i], nd, from_vector_index, n_fvi, token_bytes, token_byte_offsets, n_tokens, dst,
+                                       sizes ? 0 : k[i], moff[i].data(), first_bad ? first_bad + b[i] : nullptr, &k[i]);
+      return (sizes && got == BPE_E_CAPACITY) ? BPE_OK : got;
+    });
+  };
+  TRY(pass(true));
+  for (size_t r = 0; r < n; r++) cum[r + 1] = cum[r] + k[r];
+  for (size_t r = 0; r < n; r++)
+    for (int64_t d = 0; d < b[r + 1] - b[r]; d++) out_offsets[b[r] + d] = moff[r][(size_t)d] + cum[r];
+  out_offsets[n_docs] = cum[n];
+  *n_out = cum[n];
+  if (cum[n] > out_cap || (cum[n] && !out)) return fail(g, BPE_E_CAPACITY, "output buffer holds %lld bytes, need %lld", (long long)out_cap, (long long)cum[n]);
+  return pass(false);
+}
+
+// bpe_get_corpus: the members' document ranges back to back; sizes first, then every member copies into its place
+int group_get_corpus(bpe_engine* g, int64_t doc_begin, int64_t doc_end, int32_t* out, int64_t out_cap, int64_t* out_offsets, int64_t* n_out) {
+  const size_t n = g->members.size();
+  std::vector<int64_t> lo(n), hi(n), k(n, 0), cum(n + 1, 0);
+  int64_t nd = 0;
+  for (size_t r = 0; r < n; r++) {
+    const int64_t first = nd, count = (int64_t)g->members[r]->doc_off.size() - 1;
+    nd += count;
+    lo[r] = std::min(std::max<int64_t>(doc_begin - first, 0), count);
+    hi[r] = std::min(std::max<int64_t>(doc_end - first, 0), count);
+  }
+  if (doc_begin < 0 || doc_end < doc_begin || doc_end > nd)
+    return fail(g, BPE_E_INVALID, "document range [%lld,%lld) outside [0,%lld)", (long long)doc_begin, (long long)doc_end, (long long)nd);
+  std::vector<std::vector<int64_t>> moff(n);
+  for (size_t r = 0; r < n; r++) moff[r].assign((size_t)(hi[r] - lo[r]) + 1, 0);
+  TRY(run_members(g, [&](int r) {
+    const size_t i = (size_t)r;
+    if (hi[i] == lo[i]) return BPE_OK;
+    const int got = bpe_get_corpus(g->members[i], lo[i], hi[i], nullptr, 0, moff[i].data(), &k[i]);
+    return got == BPE_E_CAPACITY ? BPE_OK : got;
+  }));
+  for (size_t r = 0; r < n; r++) cum[r + 1] = cum[r] + k[r];
+  *n_out = cum[n];
+  if (cum[n] > out_cap || (!out && cum[n]) || !out_offsets) return fail(g, BPE_E_CAPACITY, "output buffer holds %lld values, need %lld", (long long)out_cap, (long long)cum[n]);
+  TRY(run_members(g, [&](int r) {
+    const size_t i = (size_t)r;
+    if (hi[i] == lo[i]) return BPE_OK;
+    int64_t got = 0;
+    return bpe_get_corpus(g->members[i], lo[i], hi[i], out ? out + cum[i] : nullptr, k[i], moff[i].data(), &got);
+  }));
+  int64_t at = 0;
+  out_offsets[0] = 0;
+  for (size_t r = 0; r < n; r++)
+    for (int64_t d = 1; d <= hi[r] - lo[r]; d++) out_offsets[++at] = moff[r][(size_t)d] + cum[r];
+  return BPE_OK;
+}
+
+int group_get_stats(bpe_engine* g, bpe_stats* out) {
+  std::vector<bpe_stats> s(g->members.size());
+  TRY(run_members(g, [&](int r) { return bpe_get_stats(g->members[(size_t)r], &s[(size_t)r]); }));
+  *out = s[0];
+  for (size_t r = 1; r < s.size(); r++) {
+    out->kernel_launches += s[r].kernel_launches;
+    out->sites_merged += s[r].sites_merged;
+    out->corpus_positions += s[r].corpus_positions;
+    out->corpus_tokens += s[r].corpus_tokens;
+    out->pool_used += s[r].pool_used;
+  }
+  return BPE_OK;
+}
+
+void destroy_group(bpe_engine* g) {
+  for (bpe_engine* m : g->members)  // the peers' mailboxes are the other members' allocations, not cudaIpc mappings to close
+    for (int q = 0; q < m->mg_world; q++)
+      if (q != m->mg_rank) m->mg_peer[q] = nullptr;
+  for (bpe_engine* m : g->members) bpe_destroy(m);
+  delete g;
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -1770,7 +2261,65 @@ int bpe_create(int device, bpe_engine** out) {
   return BPE_OK;
 }
 
+int bpe_create_group(const int* devices, int n, bpe_engine** out) {
+  if (!out) return BPE_E_INVALID;
+  *out = nullptr;
+  if (!devices || n < 1 || n > BPE_MG_MAX_WORLD) return BPE_E_INVALID;
+  // BPE_GROUP_SHARE_DEVICE=1 (tests on a host with fewer GPUs than members): members may share a device, each with its share of
+  // the SMs, so that the group's cooperative kernels stay co-resident.  It exercises the group, not its speed.
+  const char* share_env = getenv("BPE_GROUP_SHARE_DEVICE");
+  const bool share = share_env && atoi(share_env) != 0;
+  for (int r = 0; r < n; r++)
+    for (int q = 0; q < r; q++)
+      if (devices[q] == devices[r] && !share) return BPE_E_INVALID;
+  if (n == 1) return bpe_create(devices[0], out);
+  int count = 0;
+  if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0) return BPE_E_CUDA;
+  for (int r = 0; r < n; r++) {
+    if (devices[r] < 0 || devices[r] >= count) return BPE_E_CUDA;
+    for (int q = 0; q < n; q++) {
+      int ok = 0;
+      if (devices[q] != devices[r] && (cudaDeviceCanAccessPeer(&ok, devices[r], devices[q]) != cudaSuccess || !ok)) return BPE_E_CUDA;
+    }
+  }
+  bpe_engine* g = new bpe_engine();
+  g->device = devices[0];
+  int rc = BPE_OK;
+  for (int r = 0; r < n && rc == BPE_OK; r++) {
+    bpe_engine* m = nullptr;
+    rc = bpe_create(devices[r], &m);
+    if (rc != BPE_OK) break;
+    g->members.push_back(m);
+    rc = mg_alloc_mailbox(m, r, n);
+  }
+  for (int r = 0; r < n && rc == BPE_OK; r++) {
+    if (cudaSetDevice(devices[r]) != cudaSuccess) rc = BPE_E_CUDA;
+    for (int q = 0; q < n && rc == BPE_OK; q++) {
+      if (devices[q] == devices[r]) continue;
+      cudaError_t err = cudaDeviceEnablePeerAccess(devices[q], 0);
+      if (err == cudaErrorPeerAccessAlreadyEnabled) (void)cudaGetLastError();  // (torch, or an earlier group, enabled it)
+      else if (err != cudaSuccess) rc = BPE_E_CUDA;
+    }
+  }
+  if (rc != BPE_OK) {
+    destroy_group(g);
+    return rc;
+  }
+  for (bpe_engine* m : g->members) {
+    for (int q = 0; q < n; q++) m->mg_peer[q] = g->members[(size_t)q]->mg_mailbox;
+    m->mg_connected = true;
+    const int sharing = (int)std::count(devices, devices + n, m->device);
+    m->sm_count = std::max(1, m->sm_count / sharing);
+  }
+  *out = g;
+  return BPE_OK;
+}
+
 void bpe_destroy(bpe_engine* e) {
+  if (is_group(e)) {
+    destroy_group(e);
+    return;
+  }
   if (e && e->mg_mailbox) {
     cudaSetDevice(e->device);
     for (int q = 0; q < e->mg_world; q++)
@@ -1797,6 +2346,7 @@ const char* bpe_last_error(bpe_engine* e) { return e ? e->err.c_str() : "null en
 
 int bpe_set_stream(bpe_engine* e, void* cuda_stream) {
   if (!e) return BPE_E_INVALID;
+  GROUP_REFUSES(e, "bpe_set_stream (a stream belongs to one device)");
   cudaSetDevice(e->device);
   cudaStreamSynchronize(e->stream);
   e->stream = cuda_stream ? (cudaStream_t)cuda_stream : e->own_stream;
@@ -1805,6 +2355,7 @@ int bpe_set_stream(bpe_engine* e, void* cuda_stream) {
 
 int bpe_synchronize(bpe_engine* e) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) return run_members(e, [&](int r) { return bpe_synchronize(e->members[(size_t)r]); });
   CK(cudaSetDevice(e->device));
   CK(cudaStreamSynchronize(e->stream));
   return BPE_OK;
@@ -1812,6 +2363,7 @@ int bpe_synchronize(bpe_engine* e) {
 
 int bpe_set_profiling(bpe_engine* e, int enabled) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) return run_members(e, [&](int r) { return bpe_set_profiling(e->members[(size_t)r], enabled); });
   e->profiling = enabled != 0;
   e->scan_mode = (enabled & 2) ? 1 : 0;  // bit 1: debug full-scan site discovery
   e->host_loop = (enabled & 4) ? 1 : 0;  // bit 2: debug host-driven mergeUntil (one launch per phase)
@@ -1820,6 +2372,7 @@ int bpe_set_profiling(bpe_engine* e, int enabled) {
 
 int bpe_get_stats(bpe_engine* e, bpe_stats* out) {
   if (!e || !out) return BPE_E_INVALID;
+  if (is_group(e)) return group_get_stats(e, out);
   CK(cudaSetDevice(e->device));
   if (e->index_valid && e->d_st.p) {
     TRY(fetch_state(e));
@@ -1849,6 +2402,7 @@ int bpe_set_tokens(bpe_engine* e, const int32_t* utf16_len, int32_t n_tokens) {
   if (n_tokens > BPE_MAX_TOKENS) return fail(e, BPE_E_DOMAIN, "token table of %d exceeds %d", n_tokens, BPE_MAX_TOKENS);
   for (int32_t i = 0; i < n_tokens; i++)
     if (utf16_len[i] < 0) return fail(e, BPE_E_INVALID, "negative token length");
+  if (is_group(e)) return run_members(e, [&](int r) { return bpe_set_tokens(e->members[(size_t)r], utf16_len, n_tokens); });
   CK(cudaSetDevice(e->device));
   e->h_len16.assign(utf16_len, utf16_len + n_tokens);
   e->n_tokens = n_tokens;
@@ -1860,7 +2414,7 @@ int bpe_set_tokens(bpe_engine* e, const int32_t* utf16_len, int32_t n_tokens) {
 
 int bpe_num_tokens(bpe_engine* e, int32_t* n_tokens) {
   if (!e || !n_tokens) return BPE_E_INVALID;
-  *n_tokens = e->n_tokens;
+  *n_tokens = is_group(e) ? e->members[0]->n_tokens : e->n_tokens;
   return BPE_OK;
 }
 
@@ -1868,6 +2422,7 @@ int bpe_load_merges(bpe_engine* e, const int32_t* abc, int64_t n_merges) {
   if (!e || n_merges < 0 || (!abc && n_merges > 0)) return fail(e, BPE_E_INVALID, "bad merge list");
   for (int64_t i = 0; i < 3 * n_merges; i++)
     if (abc[i] < 0 || abc[i] >= BPE_MAX_TOKENS) return fail(e, BPE_E_INVALID, "merge %lld holds index %d", (long long)(i / 3), abc[i]);
+  if (is_group(e)) return run_members(e, [&](int r) { return bpe_load_merges(e->members[(size_t)r], abc, n_merges); });
   e->h_merges.assign(abc, abc + 3 * n_merges);
   e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
   return BPE_OK;
@@ -1875,6 +2430,7 @@ int bpe_load_merges(bpe_engine* e, const int32_t* abc, int64_t n_merges) {
 
 int bpe_add_documents_dev(bpe_engine* e, const int32_t* dev_ids, const int64_t* host_doc_offsets, int64_t n_docs) {
   if (!e) return BPE_E_INVALID;
+  GROUP_REFUSES(e, "bpe_add_documents_dev (device pointers belong to one device)");
   TRY(check_offsets(e, host_doc_offsets, n_docs));
   if (n_docs == 0) return BPE_OK;
   if (!dev_ids && host_doc_offsets[n_docs] > host_doc_offsets[0]) return fail(e, BPE_E_INVALID, "null ids");
@@ -1884,6 +2440,7 @@ int bpe_add_documents_dev(bpe_engine* e, const int32_t* dev_ids, const int64_t* 
 
 int bpe_add_documents(bpe_engine* e, const int32_t* ids, const int64_t* doc_offsets, int64_t n_docs) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) return group_add_documents(e, ids, doc_offsets, n_docs, false);
   TRY(check_offsets(e, doc_offsets, n_docs));
   if (n_docs == 0) return BPE_OK;
   int64_t base = doc_offsets[0], total = doc_offsets[n_docs] - base;
@@ -1902,6 +2459,10 @@ int bpe_add_documents(bpe_engine* e, const int32_t* ids, const int64_t* doc_offs
 
 int bpe_clear_corpus(bpe_engine* e) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) {
+    e->grp_uploaded = false;
+    return run_members(e, [&](int r) { return bpe_clear_corpus(e->members[(size_t)r]); });
+  }
   e->n_slots = 0;
   e->doc_off.assign(1, 0);
   e->live_tokens = 0;
@@ -1912,6 +2473,18 @@ int bpe_clear_corpus(bpe_engine* e) {
 
 int bpe_corpus_size(bpe_engine* e, int64_t* n_docs, int64_t* n_tokens) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) {
+    std::vector<int64_t> d(e->members.size(), 0), t(e->members.size(), 0);
+    TRY(run_members(e, [&](int r) { return bpe_corpus_size(e->members[(size_t)r], &d[(size_t)r], &t[(size_t)r]); }));
+    int64_t sd = 0, st = 0;
+    for (size_t r = 0; r < d.size(); r++) {
+      sd += d[r];
+      st += t[r];
+    }
+    if (n_docs) *n_docs = sd;
+    if (n_tokens) *n_tokens = st;
+    return BPE_OK;
+  }
   CK(cudaSetDevice(e->device));
   if (e->index_valid && e->d_st.p) {
     TRY(fetch_state(e));
@@ -1925,6 +2498,7 @@ int bpe_corpus_size(bpe_engine* e, int64_t* n_docs, int64_t* n_tokens) {
 int bpe_get_corpus(bpe_engine* e, int64_t doc_begin, int64_t doc_end, int32_t* out, int64_t out_cap, int64_t* out_offsets,
                    int64_t* n_out) {
   if (!e || !n_out) return BPE_E_INVALID;
+  if (is_group(e)) return group_get_corpus(e, doc_begin, doc_end, out, out_cap, out_offsets, n_out);
   int64_t nd = (int64_t)e->doc_off.size() - 1;
   if (doc_begin < 0 || doc_end < doc_begin || doc_end > nd) return fail(e, BPE_E_INVALID, "document range [%lld,%lld) outside [0,%lld)", (long long)doc_begin, (long long)doc_end, (long long)nd);
   CK(cudaSetDevice(e->device));
@@ -1972,6 +2546,7 @@ int bpe_find_next_merge(bpe_engine* e, int64_t min_weight, int32_t max_length, b
   if (!e || !out || !found) return BPE_E_INVALID;
   *found = 0;
   // a shard alone would answer with ITS best pair, not the corpus's (core.ts:265-310 counts over all documents)
+  GROUP_REFUSES(e, "bpe_find_next_merge (use bpe_merge_until(max_iterations = 1))");
   if (e->mg_world > 1) return fail(e, BPE_E_INVALID, "bpe_find_next_merge is not available on a sharded engine; use bpe_merge_until(max_iterations = 1)");
   CK(cudaSetDevice(e->device));
   if (e->n_slots == 0) return BPE_OK;
@@ -1992,6 +2567,11 @@ int bpe_find_next_merge(bpe_engine* e, int64_t min_weight, int32_t max_length, b
 
 int bpe_apply_merge(bpe_engine* e, int32_t a, int32_t b, int32_t c, int64_t* n_replaced) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) {  // on an empty corpus only the vocabulary grows, on every member
+    if (group_slots(e)) return fail(e, BPE_E_INVALID, "bpe_apply_merge on a corpus is not available on a device group; use bpe_merge_until");
+    if (n_replaced) *n_replaced = 0;
+    return run_members(e, [&](int r) { return bpe_apply_merge(e->members[(size_t)r], a, b, c, nullptr); });
+  }
   if (a < 0 || b < 0 || a >= e->n_tokens || b >= e->n_tokens) return fail(e, BPE_E_INVALID, "merge operands (%d,%d) outside the token table (%d)", a, b, e->n_tokens);
   if (c != e->n_tokens) return fail(e, BPE_E_INVALID, "new token index must be %d, got %d", e->n_tokens, c);
   if (c >= BPE_MAX_TOKENS) return fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
@@ -2027,12 +2607,20 @@ int bpe_apply_merge(bpe_engine* e, int32_t a, int32_t b, int32_t c, int64_t* n_r
 int bpe_apply_merges(bpe_engine* e, const int32_t* ab, int64_t n, int64_t* n_replaced) {
   if (!e || n < 0 || (n > 0 && !ab)) return fail(e, BPE_E_INVALID, "bad merge list");
   if (n == 0) return BPE_OK;
+  if (is_group(e)) {  // on an empty corpus only the vocabulary grows, on every member (one bpe_apply_merge per line: no device work)
+    if (group_slots(e)) return fail(e, BPE_E_INVALID, "bpe_apply_merges on a corpus is not available on a device group; use bpe_merge_until");
+    bpe_engine* m0 = e->members[0];
+    TRY(member_rc(e, m0, check_merge_list(m0, ab, n)));
+    if (n_replaced) std::fill(n_replaced, n_replaced + n, (int64_t)0);
+    return run_members(e, [&](int r) {
+      bpe_engine* m = e->members[(size_t)r];
+      for (int64_t i = 0; i < n; i++) TRY(bpe_apply_merge(m, ab[2 * i], ab[2 * i + 1], m->n_tokens, nullptr));
+      return BPE_OK;
+    });
+  }
   CK(cudaSetDevice(e->device));
   if (e->mg_world > 1) return fail(e, BPE_E_INVALID, "bpe_apply_merges is not available on a sharded engine");
-  if ((int64_t)e->n_tokens + n > BPE_MAX_TOKENS) return fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
-  for (int64_t i = 0; i < n; i++)
-    if (ab[2 * i] < 0 || ab[2 * i + 1] < 0 || ab[2 * i] >= e->n_tokens + i || ab[2 * i + 1] >= e->n_tokens + i)
-      return fail(e, BPE_E_INVALID, "merge %lld refers to a token that does not exist yet", (long long)i);
+  TRY(check_merge_list(e, ab, n));
   if (e->n_slots == 0) {  // no corpus: only the vocabulary / merge list grow (import-merge-log-to-ram.ts:22 empties the corpus first)
     for (int64_t i = 0; i < n; i++) {
       e->h_len16.push_back(e->h_len16[ab[2 * i]] + e->h_len16[ab[2 * i + 1]]);
@@ -2061,6 +2649,7 @@ int bpe_apply_merges(bpe_engine* e, const int32_t* ab, int64_t n, int64_t* n_rep
 int bpe_merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log,
                     int64_t log_cap, int64_t* n_done) {
   if (!e || !n_done || (log_cap > 0 && !log) || log_cap < 0) return BPE_E_INVALID;
+  if (is_group(e)) return group_merge_until(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
   if (e->mg_world > 1) return merge_until_mg(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
   if (e->host_loop) return merge_until_host(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
   return merge_until_device(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
@@ -2070,28 +2659,20 @@ int bpe_merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64
 // ---- sharded training: mailbox set-up and the initial pair-count exchange ------------------------------------------
 int bpe_mg_init(bpe_engine* e, int rank, int world, void* handle_out64) {
   if (!e || !handle_out64 || world < 1 || world > MG_MAX_WORLD || rank < 0 || rank >= world) return fail(e, BPE_E_INVALID, "bad rank/world");
+  GROUP_REFUSES(e, "bpe_mg_init (the group's members are connected already)");
   CK(cudaSetDevice(e->device));
   if (e->mg_mailbox) return fail(e, BPE_E_INVALID, "bpe_mg_init called twice");
-  e->mg_rank = rank;
-  e->mg_world = world;
-  // records one rank can send per exchange (k_merge_rounds: the cells of up to 16 merges a round; k_merge_loop_mg: of one merge)
-  e->mg_inbox_stride = 1u << 20;
-  e->mg_tie_cap = 4096;
-  size_t bytes = (size_t)2 * MG_MAX_WORLD * 128 + (size_t)2 * world * e->mg_inbox_stride * 8 + (size_t)2 * world * e->mg_tie_cap * 4;
-  CK(cudaMalloc(&e->mg_mailbox, bytes));
-  CK(cudaMemset(e->mg_mailbox, 0, bytes));
-  e->mg_mailbox_bytes = bytes;
-  e->mg_peer[rank] = e->mg_mailbox;
+  TRY(mg_alloc_mailbox(e, rank, world));
   cudaIpcMemHandle_t h;
   static_assert(sizeof(h) == 64, "cudaIpcMemHandle_t is 64 bytes");
   CK(cudaIpcGetMemHandle(&h, e->mg_mailbox));
   memcpy(handle_out64, &h, sizeof h);
-  e->index_valid = false;  // per-slot side arrays are allocated with the table
   e->mg_connected = (world == 1);
   return BPE_OK;
 }
 
 int bpe_mg_connect(bpe_engine* e, const char* handles /* world x 64 bytes, by rank */) {
+  GROUP_REFUSES(e, "bpe_mg_connect (the group's members are connected already)");
   if (!e || !handles || !e->mg_mailbox) return fail(e, BPE_E_INVALID, "call bpe_mg_init first");
   CK(cudaSetDevice(e->device));
   for (int q = 0; q < e->mg_world; q++) {
@@ -2106,12 +2687,14 @@ int bpe_mg_connect(bpe_engine* e, const char* handles /* world x 64 bytes, by ra
 
 int bpe_mg_state(bpe_engine* e, int* counts_global) {
   if (!e || !counts_global) return BPE_E_INVALID;
+  GROUP_REFUSES(e, "bpe_mg_state (the group exchanges its pair counts itself)");
   *counts_global = (e->index_valid && e->mg_counts_global) ? 1 : 0;
   return BPE_OK;
 }
 
 int bpe_mg_export_counts(bpe_engine* e, uint32_t* dev_keys, uint32_t* dev_counts, int64_t cap, int64_t* n) {
   if (!e || !n || cap < 0 || (cap > 0 && (!dev_keys || !dev_counts))) return fail(e, BPE_E_INVALID, "bad export arguments");
+  GROUP_REFUSES(e, "bpe_mg_export_counts (the group exchanges its pair counts itself)");
   CK(cudaSetDevice(e->device));
   TRY(ensure_index(e));
   if (e->mg_counts_global) return fail(e, BPE_E_INVALID, "pair counts of this index were already exchanged");
@@ -2132,6 +2715,7 @@ int bpe_mg_export_counts(bpe_engine* e, uint32_t* dev_keys, uint32_t* dev_counts
 
 int bpe_mg_import_counts(bpe_engine* e, const uint32_t* dev_keys, const uint32_t* dev_counts, int64_t n, int last) {
   if (!e || n < 0 || (n > 0 && (!dev_keys || !dev_counts))) return fail(e, BPE_E_INVALID, "bad import arguments");
+  GROUP_REFUSES(e, "bpe_mg_import_counts (the group exchanges its pair counts itself)");
   CK(cudaSetDevice(e->device));
   if (!e->index_valid) return fail(e, BPE_E_INVALID, "no pair index to import into");
   TRY(fetch_state(e));
@@ -2155,6 +2739,14 @@ int bpe_mg_import_counts(bpe_engine* e, const uint32_t* dev_keys, const uint32_t
 int bpe_pair_counts(bpe_engine* e, int32_t* a, int32_t* b, int64_t* count, int64_t cap, int64_t* n) {
   if (!e || !n || cap < 0) return BPE_E_INVALID;
   *n = 0;
+  if (is_group(e)) {  // after the exchange every member's table holds the corpus-wide counts: read one that has a corpus
+    for (bpe_engine* m : e->members) {
+      if (m->n_slots == 0) continue;
+      TRY(group_exchange_counts(e));
+      return member_rc(e, m, bpe_pair_counts(m, a, b, count, cap, n));
+    }
+    return BPE_OK;
+  }
   CK(cudaSetDevice(e->device));
   if (e->n_slots == 0) return BPE_OK;
   TRY(ensure_index(e));
@@ -2187,6 +2779,7 @@ int bpe_encode_batch_dev(bpe_engine* e, const int32_t* dev_ids, const int64_t* d
                          int64_t* dev_out_offsets, int64_t* dev_first_bad, int64_t* n_out) {
   if (!e || !n_out || n_docs < 0 || n_ids < 0 || !dev_doc_offsets || !dev_out_offsets || (n_ids > 0 && (!dev_ids || !dev_out)))
     return fail(e, BPE_E_INVALID, "bad encode arguments");
+  GROUP_REFUSES(e, "bpe_encode_batch_dev (device pointers belong to one device)");
   CK(cudaSetDevice(e->device));
   // scratch owned by the engine (freed by bpe_destroy, on the engine's device): reused across calls so that steady-state
   // encode does not allocate
@@ -2236,6 +2829,8 @@ int bpe_encode_batch(bpe_engine* e, const int32_t* ids, const int64_t* doc_offse
   if (!e || !n_out || !out_offsets) return fail(e, BPE_E_INVALID, "bad encode arguments");
   if (n_docs < 0 || (!doc_offsets && n_docs > 0)) return fail(e, BPE_E_INVALID, "bad document offsets");
   if (n_docs > 0 && doc_offsets[n_docs] > doc_offsets[0] && !ids) return fail(e, BPE_E_INVALID, "null ids");
+  if (is_group(e))
+    return group_encode(e, false, ids, nullptr, doc_offsets, n_docs, to_vector_index, n_tvi, out, out_cap, out_offsets, first_bad, n_out, nullptr, nullptr);
   CK(cudaSetDevice(e->device));
   return encode_host(e, false, ids, nullptr, doc_offsets, n_docs, to_vector_index, n_tvi, out, out_cap, out_offsets, first_bad, n_out, nullptr, nullptr);
 }
@@ -2405,6 +3000,8 @@ int encode_pipeline(bpe_engine* e, const bool is_text, const int32_t* ids, const
                     const int32_t* to_vector_index, int32_t n_tvi, int32_t* out, int64_t out_cap, int64_t* out_offsets, int64_t* first_bad,
                     int64_t* n_out, int64_t* unknown_pos, int32_t* unknown_code_point) {
   e->txt_staged = false;
+  e->enc_parts.clear();
+  e->enc_bad_id_pos = -1;
   const int64_t base = off[0];
   if (off[n_docs] < base) return fail(e, BPE_E_INVALID, "document offsets must be non-decreasing");
   const int64_t total = off[n_docs] - base;
@@ -2488,8 +3085,10 @@ int encode_pipeline(bpe_engine* e, const bool is_text, const int32_t* ids, const
     if (!is_text) {
       CK(cudaEventSynchronize(e->ev_in[slot]));
       unsigned long long fb = *static_cast<volatile unsigned long long*>(e->h_pipe + slot * 4);
-      if (fb != ~0ull)
-        return fail(e, BPE_E_INVALID, "id %d at %lld outside the token table", ids[base + cur.in0 + (int64_t)fb], (long long)(cur.in0 + (int64_t)fb));
+      if (fb != ~0ull) {
+        e->enc_bad_id_pos = cur.in0 + (int64_t)fb;
+        return fail(e, BPE_E_INVALID, "id %d at %lld outside the token table", ids[base + e->enc_bad_id_pos], (long long)e->enc_bad_id_pos);
+      }
     } else {
       CK(cudaStreamWaitEvent(e->stream, e->ev_in[slot], 0));
       TRY(text_decode_dev(e, e->x_text.p + cur.reg, len, d_in_off + cur.oreg, nd, e->x_ids.p + cur.reg, e->x_off.p + cur.oreg, false,
@@ -2533,6 +3132,8 @@ int encode_pipeline(bpe_engine* e, const bool is_text, const int32_t* ids, const
     CK(cudaEventRecord(e->ev_res[c & 1], e->s_out));
     if (cum + k > out_cap || (k && !out)) overflow = true;  // keep going: the caller learns the size it needs
     if (!overflow && k) CK(cudaMemcpyAsync(out + cum, e->x_out.p + cur.reg, (size_t)k * 4, cudaMemcpyDeviceToHost, e->s_out));
+    e->enc_parts.push_back(cur.reg);
+    e->enc_parts.push_back(k);
     cum += k;
     char_cum += n_units;
     done = cur;
@@ -2569,6 +3170,9 @@ int bpe_decode_batch(bpe_engine* e, const int32_t* values, const int64_t* doc_of
                      int32_t n_fvi, const uint8_t* token_bytes, const int64_t* token_byte_offsets, int32_t n_tokens, uint8_t* out,
                      int64_t out_cap, int64_t* out_offsets, int64_t* first_bad, int64_t* n_out) {
   if (!e || !n_out || !out_offsets || n_tokens < 0 || (n_tokens > 0 && (!token_byte_offsets))) return fail(e, BPE_E_INVALID, "bad decode arguments");
+  if (is_group(e))
+    return group_decode(e, values, doc_offsets, n_docs, from_vector_index, n_fvi, token_bytes, token_byte_offsets, n_tokens, out, out_cap, out_offsets,
+                        first_bad, n_out);
   e->txt_staged = false;
   TRY(check_offsets(e, doc_offsets, n_docs));
   CK(cudaSetDevice(e->device));
@@ -2639,6 +3243,7 @@ int bpe_decode_batch(bpe_engine* e, const int32_t* values, const int64_t* doc_of
 // ---- text in, tokens out ---------------------------------------------------------------------------------------------
 int bpe_set_chars(bpe_engine* e, const int32_t* code_points, const int32_t* indices, int32_t n) {
   if (!e || n < 0 || (n > 0 && (!code_points || !indices))) return fail(e, BPE_E_INVALID, "bad character table");
+  if (is_group(e)) return run_members(e, [&](int r) { return bpe_set_chars(e->members[(size_t)r], code_points, indices, n); });
   e->txt_staged = false;  // its ids were resolved against the table being replaced
   CK(cudaSetDevice(e->device));
   TRY(ensure_cpmap(e));
@@ -2659,6 +3264,7 @@ int bpe_set_chars(bpe_engine* e, const int32_t* code_points, const int32_t* indi
 int bpe_add_text_stage(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_offsets, int64_t n_docs, int32_t* new_code_points,
                        int64_t* first_pos, int32_t new_cap, int32_t* n_new) {
   if (!e || !n_new || new_cap < 0 || (new_cap > 0 && (!new_code_points || !first_pos))) return fail(e, BPE_E_INVALID, "bad arguments");
+  GROUP_REFUSES(e, "bpe_add_text_stage (bpe_add_text orders the new characters over the group itself)");
   *n_new = 0;
   CK(cudaSetDevice(e->device));
   int64_t n_chars = 0;
@@ -2704,6 +3310,7 @@ int bpe_add_text_stage(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_by
 
 int bpe_add_text_commit(bpe_engine* e, const int32_t* code_points, int32_t n, int64_t* counts, int64_t counts_cap) {
   if (!e) return BPE_E_INVALID;
+  GROUP_REFUSES(e, "bpe_add_text_commit (bpe_add_text orders the new characters over the group itself)");
   if (!e->txt_staged) return fail(e, BPE_E_INVALID, "no staged text batch: bpe_add_text_stage first (another call since then reused its buffers)");
   if (n < 0 || (n > 0 && !code_points)) return fail(e, BPE_E_INVALID, "bad code point list");
   CK(cudaSetDevice(e->device));
@@ -2763,6 +3370,7 @@ int bpe_add_text(bpe_engine* e, const uint8_t* utf8, const int64_t* doc_byte_off
                  int32_t* n_new, int64_t* counts, int64_t counts_cap) {
   if (!e || !n_new) return fail(e, BPE_E_INVALID, "bad arguments");
   *n_new = 0;
+  if (is_group(e)) return group_add_text(e, utf8, doc_byte_offsets, n_docs, new_code_points, new_cap, n_new, counts, counts_cap);
   const bool trace_t = getenv("BPE_TRACE") != nullptr;
   auto clk = [] { return std::chrono::steady_clock::now(); };
   auto since = [&](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(clk() - t).count(); };
@@ -2797,6 +3405,9 @@ int bpe_encode_text_batch(bpe_engine* e, const uint8_t* utf8, const int64_t* doc
   if (n_docs < 0 || (!doc_byte_offsets && n_docs > 0)) return fail(e, BPE_E_INVALID, "bad document offsets");
   if (unknown_pos) *unknown_pos = -1;
   if (!utf8 && n_docs > 0 && doc_byte_offsets[n_docs] > doc_byte_offsets[0]) return fail(e, BPE_E_INVALID, "null text");
+  if (is_group(e))
+    return group_encode(e, true, nullptr, utf8, doc_byte_offsets, n_docs, to_vector_index, n_tvi, out, out_cap, out_offsets, first_bad, n_out, unknown_pos,
+                        unknown_code_point);
   CK(cudaSetDevice(e->device));
   return encode_host(e, true, nullptr, utf8, doc_byte_offsets, n_docs, to_vector_index, n_tvi, out, out_cap, out_offsets, first_bad, n_out, unknown_pos,
                      unknown_code_point);
@@ -2854,6 +3465,7 @@ int bpe_debug_plan_chunks(const int64_t* doc_offsets, int64_t n_docs, int64_t ch
 
 int bpe_restore_documents(bpe_engine* e, const int32_t* ids, const int64_t* doc_offsets, int64_t n_docs) {
   if (!e) return BPE_E_INVALID;
+  if (is_group(e)) return group_add_documents(e, ids, doc_offsets, n_docs, true);
   TRY(check_offsets(e, doc_offsets, n_docs));
   if (n_docs == 0) return BPE_OK;
   CK(cudaSetDevice(e->device));

@@ -113,12 +113,21 @@ def _min_weight(o) -> int:
 
 
 class BPETokenizer:
-    def __init__(self, device: int = 0):
+    def __init__(self, device: int = 0, devices: Optional[Sequence[int]] = None):
+        """One engine on `device`, or, with `devices`, one engine over those GPUs of this process (bpe_create_group): the corpus is
+        sharded by document across them and every method keeps the single-engine results."""
         self._lib = _abi.load_library()
         h = C.c_void_p()
-        rc = self._lib.bpe_create(device, C.byref(h))
+        if devices is None:
+            rc = self._lib.bpe_create(device, C.byref(h))
+        else:
+            devices = [int(d) for d in devices]
+            rc = self._lib.bpe_create_group((C.c_int * max(len(devices), 1))(*devices), len(devices), C.byref(h))
+            if rc == _abi.BPE_E_INVALID:
+                raise BpeError(rc, "devices must list 1 to %d distinct GPUs, got %r" % (_abi.MG_MAX_WORLD, devices))
+            device = devices[0]
         if rc != _abi.BPE_OK:
-            raise BpeError(rc, "cannot create the CUDA engine (no usable device? there is no CPU fallback)")
+            raise BpeError(rc, "cannot create the CUDA engine (no usable device, or GPUs without peer access? there is no CPU fallback)")
         self._h = h
         self._device = device
         self._reset_host()

@@ -163,6 +163,38 @@ int bpe_pair_counts(bpe_engine* e, int32_t* a, int32_t* b, int64_t* count, int64
  * an engine initialised with world > 1: a shard alone cannot answer for the whole corpus; bpe_merge_until(max_iterations
  * = 1) is the exact single step. */
 #define BPE_MG_MAX_WORLD 8
+/* One engine over the GPUs devices[0..n) of this process: a corpus sharded by document, as bpe_mg_* does across processes.
+ * n == 1 gives a plain engine.  Fails with BPE_E_INVALID on n < 1, n > BPE_MG_MAX_WORLD, or a repeated device;
+ * with BPE_E_CUDA when a pair of the devices has no peer access.
+ * The handle is an ordinary bpe_engine* that every entry point accepts.  It holds one member engine per device, member r on
+ * devices[r] as rank r of n; their mailboxes are connected by pointer (peer access is enabled for every ordered pair, and stays
+ * enabled after bpe_destroy).  A call that runs device work on several members runs each on a host thread of its own and joins
+ * them all before it returns; when a member fails, the call returns the first member's error that is not a peer timeout, else the
+ * timeout, and bpe_last_error names the device.
+ *   - bpe_set_tokens, bpe_load_merges, bpe_set_chars, bpe_clear_corpus, bpe_set_profiling, bpe_synchronize: every member.
+ *   - bpe_add_documents, bpe_restore_documents, bpe_add_text: the first upload after creation or bpe_clear_corpus is split into
+ *     contiguous ranges of documents balanced by ids (bytes for text), one per member; a later upload goes to the last member
+ *     whole, so that (member, position) stays the document order.  A document upload that any member refuses adds nothing on
+ *     any member, as on one engine.  bpe_add_text gives the new characters one first-appearance order over the whole batch and
+ *     returns the counts summed over the members; its checks all come before any member changes, so only a CUDA or memory
+ *     failure in the final step can leave some members with the batch.
+ *   - bpe_merge_until sums the members' pair histograms first when an upload made them stale (device to device, no host
+ *     copy), then runs on every member; all of them return the same log (BPE_E_INTERNAL otherwise).  The members meet on the
+ *     host before every launch of the loop kernel, so that none waits in a kernel for a peer still doing host work.
+ *   - bpe_encode_batch, bpe_encode_text_batch, bpe_decode_batch: contiguous ranges of documents balanced by input units, one
+ *     per member, encoded in parallel; the results are exactly one engine's, BPE_E_CAPACITY, the sizes and the positions in
+ *     error messages included.  Encode copies each member's vectors from its device to their place in `out` once every
+ *     member's size is known (that copy follows the encode instead of overlapping it); decode sizes first, then decodes into
+ *     place (the values go up twice).
+ *   - bpe_get_corpus, bpe_corpus_size, bpe_pair_counts: the whole corpus (members' ranges in order; corpus-wide counts).
+ *   - bpe_get_stats: kernel_launches, sites_merged, corpus_positions, corpus_tokens and pool_used summed over the members;
+ *     every other field (the times included) is member 0's.
+ *   - BPE_E_INVALID, as on a sharded engine: bpe_find_next_merge, bpe_apply_merge and bpe_apply_merges on a non-empty corpus
+ *     (on an empty one they grow the vocabulary of every member), bpe_set_stream, bpe_add_documents_dev,
+ *     bpe_encode_batch_dev, bpe_add_text_stage / _commit and bpe_mg_*.
+ * With BPE_GROUP_SHARE_DEVICE=1 in the environment, devices may repeat: the members on one device share its SMs.  It lets the
+ * group run on a host with fewer GPUs than members (tests); it gives no speed-up. */
+int bpe_create_group(const int* devices, int n, bpe_engine** out);
 /* Allocates this rank's mailbox (peers store count deltas into it over NVLink) and writes its
  * cudaIpcMemHandle_t (64 bytes) to handle_out. */
 int bpe_mg_init(bpe_engine* e, int rank, int world, void* handle_out);
