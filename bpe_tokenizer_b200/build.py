@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbpe_b200.so")
 SOURCES = ["bpe_b200.cu", "synth.cpp"]
-DEPS = ["common.cuh", "train_kernels.cuh", "encode_kernels.cuh", "encode_lanes.cuh", "encode_dp.cuh", "mg_kernels.cuh", "round_kernels.cuh", "text_kernels.cuh", os.path.join("..", "..", "include", "bpe_b200.h")]
+DEPS = ["common.cuh", "train_kernels.cuh", "encode_kernels.cuh", "encode_lanes.cuh", "mg_kernels.cuh", "round_kernels.cuh", "text_kernels.cuh", os.path.join("..", "..", "include", "bpe_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17", "-shared",

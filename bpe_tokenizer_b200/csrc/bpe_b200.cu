@@ -19,7 +19,6 @@
 
 #include "encode_kernels.cuh"
 #include "encode_lanes.cuh"
-#include "encode_dp.cuh"
 #include "train_kernels.cuh"
 #include "mg_kernels.cuh"
 #include "round_kernels.cuh"
@@ -155,8 +154,6 @@ struct EncodeScratch {
   DevBuf<uint32_t> range_first, tile_sums;
   DevBuf<uint64_t> tile_off;
   DevBuf<uint32_t> flags;  // [0] long documents left for the per-document kernel, [1] error, [2] next range to claim
-  DevBuf<uint16_t> dp_last;              // forward path (encode_dp.cuh): last[] of every document, per warp [position][lane]
-  DevBuf<unsigned long long> dp_cursor;  // ... and where the next warp's rows start
 };
 
 struct bpe_engine {
@@ -191,15 +188,6 @@ struct bpe_engine {
   DevBuf<uint16_t> d_rule_c;
   uint32_t lt_cap = 0;
   int32_t lt_c_affine = -1;
-  // forward path (encode_dp.cuh): Aho-Corasick automaton over the tokens' characters + merge trees
-  bool dp_dirty = true, dp_ok = false;
-  DevBuf<unsigned long long> d_dfa;
-  DevBuf<uint32_t> d_split;
-  DevBuf<uint16_t> d_tok_len, d_shorter;
-  bool dp_attr_set = false;
-  uint32_t dp_alpha = 0;
-  int enc_dp = 0;        // BPE_ENC_DP=1: forward path (exact, measured slower than the lane path: 8.5 vs 26.9 GB/s -- thread-per-document
-                         // keeps 5 of 32 lanes busy; kept as an independent second implementation, see DESIGN.md)
   int enc_lmax = 32;     // rows per lane of the lane path (32 or 48); BPE_ENC_LMAX overrides
   int enc_lmax_forced = 0;
   int enc_force_old = 0; // debug: BPE_ENC_OLD=1 routes every document through the per-document kernel
@@ -220,7 +208,6 @@ struct bpe_engine {
   DevBuf<uint32_t> hot;
   bool hot_valid = false;
   uint32_t hot_max_length = 0;
-  uint32_t hot_thresh = 0;
   uint32_t hot_limit = 0;
   DevBuf<uint32_t> cands;
   DevBuf<MergeRec> dev_log;
@@ -236,7 +223,6 @@ struct bpe_engine {
   DevBuf<unsigned long long> r_gcells;  // sharded rounds: the deltas summed over the ranks
   DevBuf<uint32_t> r_glists;
   int round_blocks = 0;  // co-resident grid of k_merge_rounds
-  int host_loop = 0;     // debug: drive mergeUntil from the host, one launch per phase
   int scan_mode = 0;     // debug: walk all slots instead of occurrence lists
 
   // sharded training (mg_kernels.cuh): this rank's mailbox + the peers' mailboxes mapped through cudaIpc
@@ -553,7 +539,6 @@ int rebuild_hot(bpe_engine* e, uint32_t max_length, bool* any) {
   CK(cudaMemcpyAsync(&e->d_st.p->hot_n, two, sizeof two, cudaMemcpyHostToDevice, e->stream));
   k_build_hot<<<e->grid(4), 256, 0, e->stream>>>(t, e->d_len16.p, max_length, e->hot.p, (uint32_t)e->hot.cap, e->d_st.p);
   CKL();
-  e->hot_thresh = thresh;
   e->hot_limit = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(4ull * HOT_TARGET, 2 * acc + 4096), 0xFFFFFFF0u);
   e->hot_max_length = max_length;
   e->hot_valid = true;
@@ -562,18 +547,18 @@ int rebuild_hot(bpe_engine* e, uint32_t max_length, bool* any) {
 }
 
 // ---- K2 driver: leaves the winner in h_st (best_primary == 0: none) -------------------------------
-int run_argmax(bpe_engine* e, uint32_t max_length, int use_hot) {
+int run_argmax(bpe_engine* e, uint32_t max_length) {
   PairTable t = e->table();
-  int blocks = use_hot ? e->sm_count : e->grid(4);
-  k_argmax<<<blocks, AM_THREADS, 0, e->stream>>>(t, e->d_len16.p, max_length, use_hot, e->hot.p, e->partials.p, e->d_st.p);
+  int blocks = e->grid(4);
+  k_argmax<<<blocks, AM_THREADS, 0, e->stream>>>(t, e->d_len16.p, max_length, e->partials.p, e->d_st.p);
   CKL();
   TRY(fetch_state(e));
   TRY(check_dev_err(e));
-  if (e->h_st->best_primary && e->h_st->best_mult > 1 && !(use_hot && e->h_st->best_cnt < e->hot_thresh)) {
+  if (e->h_st->best_primary && e->h_st->best_mult > 1) {
     // tie on (weight, a.index + b.index): the pair whose last counted occurrence comes first wins (core.ts:294-305)
     uint32_t mult = e->h_st->best_mult;
     CK(e->cands.reserve(std::max<size_t>(mult, 1024), 0, e->stream, 2.0));
-    k_collect_cands<<<blocks, 256, 0, e->stream>>>(t, e->d_len16.p, max_length, use_hot, e->hot.p, e->cands.p, (uint32_t)e->cands.cap, e->d_st.p);
+    k_collect_cands<<<blocks, 256, 0, e->stream>>>(t, e->d_len16.p, max_length, e->cands.p, (uint32_t)e->cands.cap, e->d_st.p);
     CKL();
     k_tie_break<<<std::min<uint32_t>(mult, (uint32_t)e->grid(4)), 256, 0, e->stream>>>(e->slots.p, (uint32_t)e->n_slots, t, e->pool.p, e->cands.p, e->d_st.p);
     CKL();
@@ -643,7 +628,7 @@ int run_apply(bpe_engine* e, uint32_t a, uint32_t b, uint32_t c, uint32_t bound)
   e->h_merges.push_back((int32_t)a);
   e->h_merges.push_back((int32_t)b);
   e->h_merges.push_back((int32_t)c);
-  e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+  e->mt_dirty = e->lt_dirty = true;
   e->n_tokens++;
   e->stats.merges_applied++;
   return BPE_OK;
@@ -778,114 +763,6 @@ int ensure_lane_tables(bpe_engine* e) {
   return BPE_OK;
 }
 
-// ---- tables of the forward encode path (encode_dp.cuh): tokens ending at a position, longest first, and merge trees ----
-// Supported when the table is what mergeUntil / fromJSON produce: the single characters are the tokens 0 .. n_alpha-1, merge r
-// creates token n_alpha + r out of older tokens, no two tokens spell the same string, and the dense automaton fits.
-int ensure_dp_tables(bpe_engine* e) {
-  if (!e->dp_dirty) return BPE_OK;
-  e->dp_dirty = false;
-  e->dp_ok = false;
-  const size_t m = e->h_merges.size() / 3;
-  const int64_t n_tok = e->n_tokens;
-  const int64_t A = n_tok - (int64_t)m;
-  if (A <= 0 || A > 4096 || n_tok > 0xFFF0) return BPE_OK;
-  std::vector<uint32_t> split((size_t)n_tok), off((size_t)n_tok + 1, 0);
-  std::vector<uint16_t> tok_len((size_t)n_tok, 1);
-  for (int64_t t = 0; t < A; t++) split[(size_t)t] = (uint32_t)t | ((uint32_t)t << 16);
-  for (size_t r = 0; r < m; r++) {
-    const int64_t a = e->h_merges[3 * r], b = e->h_merges[3 * r + 1], c = e->h_merges[3 * r + 2];
-    if (c != A + (int64_t)r || a < 0 || b < 0 || a >= c || b >= c) return BPE_OK;  // (characters added after merges: lane path)
-    const uint32_t L = (uint32_t)tok_len[(size_t)a] + tok_len[(size_t)b];
-    if (L > 0xFFF0u) return BPE_OK;
-    tok_len[(size_t)c] = (uint16_t)L;
-    split[(size_t)c] = (uint32_t)a | ((uint32_t)b << 16);
-  }
-  // the tokens' characters, then the trie
-  for (int64_t t = 0; t < n_tok; t++) off[(size_t)t + 1] = off[(size_t)t] + tok_len[(size_t)t];
-  if (off[(size_t)n_tok] > (64u << 20)) return BPE_OK;
-  std::vector<uint16_t> text(off[(size_t)n_tok]);
-  for (int64_t t = 0; t < A; t++) text[off[(size_t)t]] = (uint16_t)t;
-  for (size_t r = 0; r < m; r++) {
-    const size_t a = (size_t)e->h_merges[3 * r], b = (size_t)e->h_merges[3 * r + 1], c = (size_t)e->h_merges[3 * r + 2];
-    std::copy(text.begin() + off[a], text.begin() + off[a + 1], text.begin() + off[c]);
-    std::copy(text.begin() + off[b], text.begin() + off[b + 1], text.begin() + off[c] + tok_len[a]);
-  }
-  std::unordered_map<uint64_t, uint32_t> child;  // (node << 16 | char) -> node
-  child.reserve(text.size() * 2);
-  std::vector<uint16_t> node_tok(1, (uint16_t)DP_NONE);
-  std::vector<uint32_t> node_of((size_t)n_tok), parent(1, 0);
-  std::vector<uint16_t> pch(1, 0);
-  for (int64_t t = 0; t < n_tok; t++) {
-    uint32_t v = 0;
-    for (uint32_t i = off[(size_t)t]; i < off[(size_t)t + 1]; i++) {
-      const uint64_t key = ((uint64_t)v << 16) | text[i];
-      auto it = child.find(key);
-      if (it == child.end()) {
-        const uint32_t nv = (uint32_t)node_tok.size();
-        child.emplace(key, nv);
-        node_tok.push_back((uint16_t)DP_NONE);
-        parent.push_back(v);
-        pch.push_back(text[i]);
-        v = nv;
-      } else {
-        v = it->second;
-      }
-    }
-    if (node_tok[v] != DP_NONE) return BPE_OK;  // two tokens spell the same string: the string does not identify the token
-    node_tok[v] = (uint16_t)t;
-    node_of[(size_t)t] = v;
-  }
-  const size_t S = node_tok.size();
-  if (S * (size_t)A > (64u << 20)) return BPE_OK;  // dense automaton too large (huge alphabets): lane path
-  // Aho-Corasick as a dense automaton, nodes in order of depth: the row of a node is the row of its failure node (shallower,
-  // hence complete) with its own children written over it; the failure node of a child u = (v, ch) is row[fail(v)][ch]
-  std::vector<uint32_t> depth(S, 0), order(S);
-  for (size_t v = 1; v < S; v++) depth[v] = depth[parent[v]] + 1;  // (a parent's index is smaller than its children's)
-  for (size_t v = 0; v < S; v++) order[v] = (uint32_t)v;
-  std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return depth[x] < depth[y]; });
-  std::vector<uint32_t> kid_begin(S + 1, 0), kids(S > 0 ? S - 1 : 0);
-  for (size_t v = 1; v < S; v++) kid_begin[parent[v] + 1]++;
-  for (size_t v = 0; v < S; v++) kid_begin[v + 1] += kid_begin[v];
-  {
-    std::vector<uint32_t> fill(kid_begin.begin(), kid_begin.end() - 1);
-    for (size_t v = 1; v < S; v++) kids[fill[parent[v]]++] = (uint32_t)v;
-  }
-  std::vector<uint32_t> dfa(S * (size_t)A, 0), fail_(S, 0);
-  std::vector<uint16_t> out_tok(S, (uint16_t)DP_NONE);
-  for (uint32_t v : order) {
-    if (v != 0) {
-      out_tok[v] = node_tok[v] != DP_NONE ? node_tok[v] : out_tok[fail_[v]];
-      std::copy(dfa.begin() + (size_t)fail_[v] * A, dfa.begin() + (size_t)(fail_[v] + 1) * A, dfa.begin() + (size_t)v * A);
-    }
-    for (uint32_t i = kid_begin[v]; i < kid_begin[v + 1]; i++) {
-      const uint32_t u = kids[i];
-      fail_[u] = v == 0 ? 0u : dfa[(size_t)fail_[v] * A + pch[u]];
-      dfa[(size_t)v * A + pch[u]] = u;
-    }
-  }
-  std::vector<uint16_t> shorter((size_t)n_tok, (uint16_t)DP_NONE);
-  for (int64_t t = 0; t < n_tok; t++) shorter[(size_t)t] = out_tok[fail_[node_of[(size_t)t]]];
-  // one 8-byte entry per transition: next state | longest token ending there << 32 | its length << 48
-  std::vector<unsigned long long> dfa64(dfa.size());
-  for (size_t i = 0; i < dfa.size(); i++) {
-    const uint32_t nx = dfa[i];
-    const uint16_t ot = out_tok[nx];
-    dfa64[i] = (unsigned long long)nx | ((unsigned long long)ot << 32) | ((unsigned long long)(ot == DP_NONE ? 0 : tok_len[ot]) << 48);
-  }
-  CK(e->d_dfa.reserve(dfa64.size()));
-  CK(cudaMemcpyAsync(e->d_dfa.p, dfa64.data(), dfa64.size() * 8, cudaMemcpyHostToDevice, e->stream));
-  CK(e->d_tok_len.reserve((size_t)n_tok));
-  CK(cudaMemcpyAsync(e->d_tok_len.p, tok_len.data(), (size_t)n_tok * 2, cudaMemcpyHostToDevice, e->stream));
-  CK(e->d_shorter.reserve((size_t)n_tok));
-  CK(cudaMemcpyAsync(e->d_shorter.p, shorter.data(), (size_t)n_tok * 2, cudaMemcpyHostToDevice, e->stream));
-  CK(e->d_split.reserve((size_t)n_tok));
-  CK(cudaMemcpyAsync(e->d_split.p, split.data(), (size_t)n_tok * 4, cudaMemcpyHostToDevice, e->stream));
-  CK(cudaStreamSynchronize(e->stream));
-  e->dp_alpha = (uint32_t)A;
-  e->dp_ok = true;
-  return BPE_OK;
-}
-
 template <int LMAX, int WARPS>
 int launch_encode_lanes(bpe_engine* e, const int32_t* dev_ids, const int64_t* dev_doc_off, int64_t n_docs, const uint32_t* range_first,
                         uint32_t n_ranges, const LaneTables& lt, int32_t* out_tmp, uint32_t* out_len, uint32_t* n_long, uint32_t* err,
@@ -929,7 +806,6 @@ int encode_dev(bpe_engine* e, EncodeScratch& sc, const int32_t* dev_ids, const i
   int overlap_rc = BPE_OK;
   if (e->h_merges.size() / 3 > EL_MAX_RANK + 1) return fail(e, BPE_E_DOMAIN, "merge list too long");
   TRY(ensure_lane_tables(e));
-  TRY(ensure_dp_tables(e));
   TRY(ensure_pipe(e));
   CK(sc.out_tmp.reserve((size_t)std::max<int64_t>(n_ids, 1)));
   CK(sc.out_len.reserve((size_t)n_docs + 1));
@@ -959,28 +835,8 @@ int encode_dev(bpe_engine* e, EncodeScratch& sc, const int32_t* dev_ids, const i
                                                                                                              sc.range_first.p);
     CKL();
     LaneTables lt{e->d_lt.p, e->lt_cap - 1, (uint32_t)(32 - ilog2(e->lt_cap)), e->d_lt_dense.p, e->d_rule_c.p, e->lt_c_affine};
-    e->stats.encode_path = (e->enc_dp && e->dp_ok) ? 1 : 2;
-    if (e->enc_dp && e->dp_ok) {
-      // forward path: one left-to-right pass per document (encode_dp.cuh), one thread per document
-      constexpr int DPW = 16;
-      const size_t dp_smem_bytes = (size_t)DP_CACHE * 8 + (size_t)EL_DENSE * EL_DENSE * sizeof(uint2);
-      if (!e->dp_attr_set) {
-        CK(cudaFuncSetAttribute(k_encode_dp<DPW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dp_smem_bytes));
-        e->dp_attr_set = true;
-      }
-      const unsigned long long cap_entries = 3ull * (unsigned long long)n_ids + (1ull << 20);  // (a warp of 32 documents needs 32 x its longest)
-      CK(sc.dp_last.reserve((size_t)cap_entries));
-      CK(sc.dp_cursor.reserve(1));
-      CK(cudaMemsetAsync(sc.dp_cursor.p, 0, 8, e->stream));
-      DpTables dt{e->d_dfa.p, e->d_tok_len.p, e->d_shorter.p, e->d_split.p, e->dp_alpha};
-      int per_sm = 1;
-      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_encode_dp<DPW>, DPW * 32, dp_smem_bytes));
-      const int64_t want = (n_docs + DPW * 32 - 1) / (DPW * 32);
-      const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)e->sm_count * std::max(per_sm, 1)));
-      k_encode_dp<DPW><<<blocks, DPW * 32, dp_smem_bytes, e->stream>>>(dev_ids, dev_doc_off, n_docs, lt, dt, sc.dp_last.p, cap_entries, sc.dp_cursor.p, sc.out_tmp.p,
-                                                          sc.out_len.p, sc.flags.p, sc.flags.p + 1);
-      CKL();
-    } else if (lmax == 16)
+    e->stats.encode_path = 2;
+    if (lmax == 16)
       TRY((launch_encode_lanes<16, 20>(e, dev_ids, dev_doc_off, n_docs, sc.range_first.p, n_ranges, lt, sc.out_tmp.p, sc.out_len.p, sc.flags.p, sc.flags.p + 1, sc.flags.p + 2)));
     else if (lmax == 20)
       TRY((launch_encode_lanes<20, 16>(e, dev_ids, dev_doc_off, n_docs, sc.range_first.p, n_ranges, lt, sc.out_tmp.p, sc.out_len.p, sc.flags.p, sc.flags.p + 1, sc.flags.p + 2)));
@@ -1319,7 +1175,7 @@ int merge_until_device(bpe_engine* e, int64_t min_weight, int32_t max_length, in
         e->h_merges.push_back(r.c);
       }
       e->n_tokens += (int32_t)iters;
-      e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+      e->mt_dirty = e->lt_dirty = true;
       e->stats.merges_applied += iters;
     }
     uint32_t status = e->h_st->status;
@@ -1612,7 +1468,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
         e->h_merges.push_back(r.c);
       }
       e->n_tokens += (int32_t)iters;
-      e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+      e->mt_dirty = e->lt_dirty = true;
       e->stats.merges_applied += iters;
     }
     host_ms[3] += since(tl);
@@ -1724,74 +1580,6 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
   cudaEventDestroy(t1);
   return rc;
 }
-
-int merge_until_host(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log,
-                            int64_t log_cap, int64_t* n_done) {
-  if (!e || !n_done || (log_cap > 0 && !log) || log_cap < 0) return BPE_E_INVALID;
-  *n_done = 0;
-  CK(cudaSetDevice(e->device));
-  if (e->n_slots == 0) return BPE_OK;
-  TRY(ensure_index(e));
-  uint32_t ml = max_length > 0 ? (uint32_t)max_length : 0;
-  int64_t mw = min_weight > 0 ? min_weight : 2;
-  if (!e->ev0) {
-    CK(cudaEventCreate(&e->ev0));
-    CK(cudaEventCreate(&e->ev1));
-  }
-  cudaEvent_t t0, t1;
-  CK(cudaEventCreate(&t0));
-  CK(cudaEventCreate(&t1));
-  CK(cudaEventRecord(t0, e->stream));
-  int rc = BPE_OK;
-  int64_t done = 0;
-  // core.ts:374-382: for (iteration = 1; !max_iterations || iteration <= max_iterations; iteration++)
-  while ((max_iterations <= 0 || done < max_iterations) && done < log_cap) {
-    if (!e->hot_valid || e->hot_max_length != ml) {
-      bool any = false;
-      if ((rc = rebuild_hot(e, ml, &any)) != BPE_OK) break;
-      if (!any) break;  // nothing countable left (core.ts:312)
-    }
-    if ((rc = run_argmax(e, ml, 1)) != BPE_OK) break;
-    if ((e->h_st->err & ERR_HOT_OVERFLOW) || e->h_st->hot_n > e->hot_limit) {
-      e->hot_valid = false;
-      CK(cudaMemsetAsync(&e->d_st.p->err, 0, sizeof(uint32_t), e->stream));
-      continue;
-    }
-    if (!e->h_st->best_primary || e->h_st->best_cnt < e->hot_thresh) {
-      if (e->hot_thresh <= 1 && !e->h_st->best_primary) break;
-      e->hot_valid = false;  // the maximum fell below the list's threshold: rebuild lower
-      continue;
-    }
-    uint32_t a = e->h_st->best_a, b = e->h_st->best_b, w = e->h_st->best_cnt;
-    if ((int64_t)w < mw) break;  // core.ts:313
-    int32_t c = e->n_tokens;
-    if (c >= BPE_MAX_TOKENS) {
-      rc = fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
-      break;
-    }
-    if ((rc = run_apply(e, a, b, (uint32_t)c, e->scan_mode ? w : e->h_st->list_len)) != BPE_OK) break;
-    log[done].a = (int32_t)a;
-    log[done].b = (int32_t)b;
-    log[done].c = c;
-    log[done].reserved = 0;
-    log[done].weight = (int64_t)w;
-    e->stats.sites_merged += w;
-    done++;
-  }
-  *n_done = done;
-  if (rc != BPE_OK) return rc;
-  CK(cudaEventRecord(t1, e->stream));
-  TRY(fetch_state(e));
-  TRY(check_dev_err(e));
-  float ms = 0;
-  CK(cudaEventElapsedTime(&ms, t0, t1));
-  cudaEventDestroy(t0);
-  cudaEventDestroy(t1);
-  e->stats.ms_last_merge_until = ms;
-  e->live_tokens = e->h_st->live_tokens;
-  return BPE_OK;
-}
-
 
 // mailbox of rank `rank` in a sharded corpus of `world` engines: the peers store their count deltas into it (mg_kernels.cuh)
 int mg_alloc_mailbox(bpe_engine* e, int rank, int world) {
@@ -2252,9 +2040,7 @@ int bpe_create(int device, bpe_engine** out) {
     return BPE_E_CUDA;
   }
   e->stream = e->own_stream;
-  if (getenv("BPE_HOST_LOOP")) e->host_loop = 1;
   if (getenv("BPE_ENC_OLD")) e->enc_force_old = 1;
-  if (const char* v = getenv("BPE_ENC_DP")) e->enc_dp = atoi(v) != 0;
   if (getenv("BPE_ENC_LMAX")) e->enc_lmax_forced = 1;
   if (const char* v = getenv("BPE_ENC_LMAX")) e->enc_lmax = (atoi(v) == 48 || atoi(v) == 24 || atoi(v) == 20 || atoi(v) == 16) ? atoi(v) : 32;
   *out = e;
@@ -2366,7 +2152,6 @@ int bpe_set_profiling(bpe_engine* e, int enabled) {
   if (is_group(e)) return run_members(e, [&](int r) { return bpe_set_profiling(e->members[(size_t)r], enabled); });
   e->profiling = enabled != 0;
   e->scan_mode = (enabled & 2) ? 1 : 0;  // bit 1: debug full-scan site discovery
-  e->host_loop = (enabled & 4) ? 1 : 0;  // bit 2: debug host-driven mergeUntil (one launch per phase)
   return BPE_OK;
 }
 
@@ -2406,7 +2191,7 @@ int bpe_set_tokens(bpe_engine* e, const int32_t* utf16_len, int32_t n_tokens) {
   CK(cudaSetDevice(e->device));
   e->h_len16.assign(utf16_len, utf16_len + n_tokens);
   e->n_tokens = n_tokens;
-  e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+  e->mt_dirty = e->lt_dirty = true;
   TRY(sync_len16(e));
   e->hot_valid = false;
   return BPE_OK;
@@ -2424,7 +2209,7 @@ int bpe_load_merges(bpe_engine* e, const int32_t* abc, int64_t n_merges) {
     if (abc[i] < 0 || abc[i] >= BPE_MAX_TOKENS) return fail(e, BPE_E_INVALID, "merge %lld holds index %d", (long long)(i / 3), abc[i]);
   if (is_group(e)) return run_members(e, [&](int r) { return bpe_load_merges(e->members[(size_t)r], abc, n_merges); });
   e->h_merges.assign(abc, abc + 3 * n_merges);
-  e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+  e->mt_dirty = e->lt_dirty = true;
   return BPE_OK;
 }
 
@@ -2553,7 +2338,7 @@ int bpe_find_next_merge(bpe_engine* e, int64_t min_weight, int32_t max_length, b
   TRY(ensure_index(e));
   uint32_t ml = max_length > 0 ? (uint32_t)max_length : 0;
   int64_t mw = min_weight > 0 ? min_weight : 2;  // core.ts:256
-  TRY(run_argmax(e, ml, 0));
+  TRY(run_argmax(e, ml));
   if (!e->h_st->best_primary) return BPE_OK;            // core.ts:312
   if ((int64_t)e->h_st->best_cnt < mw) return BPE_OK;   // core.ts:313
   out->a = (int32_t)e->h_st->best_a;
@@ -2582,7 +2367,7 @@ int bpe_apply_merge(bpe_engine* e, int32_t a, int32_t b, int32_t c, int64_t* n_r
     e->h_merges.push_back(a);
     e->h_merges.push_back(b);
     e->h_merges.push_back(c);
-    e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+    e->mt_dirty = e->lt_dirty = true;
     e->n_tokens++;
     e->index_valid = false;
     return BPE_OK;
@@ -2630,7 +2415,7 @@ int bpe_apply_merges(bpe_engine* e, const int32_t* ab, int64_t n, int64_t* n_rep
       e->n_tokens++;
       if (n_replaced) n_replaced[i] = 0;
     }
-    e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+    e->mt_dirty = e->lt_dirty = true;
     TRY(sync_len16(e));
     return BPE_OK;
   }
@@ -2651,7 +2436,6 @@ int bpe_merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64
   if (!e || !n_done || (log_cap > 0 && !log) || log_cap < 0) return BPE_E_INVALID;
   if (is_group(e)) return group_merge_until(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
   if (e->mg_world > 1) return merge_until_mg(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
-  if (e->host_loop) return merge_until_host(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
   return merge_until_device(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
 }
 
@@ -3348,7 +3132,7 @@ int bpe_add_text_commit(bpe_engine* e, const int32_t* code_points, int32_t n, in
       e->h_len16.push_back(code_points[k] >= 0x10000 ? 2 : 1);  // `chars.length` in UTF-16 units (core.ts:272)
     }
     e->n_tokens += n;
-    e->mt_dirty = e->lt_dirty = e->dp_dirty = true;
+    e->mt_dirty = e->lt_dirty = true;
     TRY(sync_len16(e));
     CK(cudaMemcpyAsync(b.p, h_idx.data(), (size_t)n * 4, cudaMemcpyHostToDevice, e->stream));
     k_set_cpmap<<<(n + 255) / 256, 256, 0, e->stream>>>(e->d_cpmap.p, a.p, b.p, (uint32_t)n);

@@ -516,15 +516,12 @@ __device__ __forceinline__ void publish_best(const PairTable& t, DevState* st, B
 
 constexpr int AM_THREADS = 256;
 
-// Stand-alone K2.  The last block to finish folds the per-block partials and resets the per-iteration counters.
+// Stand-alone K2 over the whole table.  The last block to finish folds the per-block partials and resets the per-iteration counters.
 __global__ void __launch_bounds__(AM_THREADS) k_argmax(PairTable t, const uint32_t* __restrict__ len16,
-                                                        uint32_t max_length, int use_hot,
-                                                        const uint32_t* __restrict__ hot, Best* __restrict__ partials,
-                                                        DevState* st) {
+                                                        uint32_t max_length, Best* __restrict__ partials, DevState* st) {
   __shared__ Best s_best[AM_THREADS / 32];
   __shared__ bool s_last;
-  uint32_t n = use_hot ? st->hot_n : (t.mask + 1);
-  Best v = best_block_reduce(argmax_stripe(t, len16, max_length, use_hot, hot, n, blockIdx.x, gridDim.x), s_best);
+  Best v = best_block_reduce(argmax_stripe(t, len16, max_length, 0, nullptr, t.mask + 1, blockIdx.x, gridDim.x), s_best);
   if (threadIdx.x == 0) {
     partials[blockIdx.x] = v;
     __threadfence();
@@ -561,11 +558,9 @@ __device__ __forceinline__ void phase_collect(const PairTable& t, const uint32_t
   }
 }
 
-__global__ void k_collect_cands(PairTable t, const uint32_t* __restrict__ len16, uint32_t max_length, int use_hot,
-                                const uint32_t* __restrict__ hot, uint32_t* __restrict__ cands, uint32_t cand_cap,
-                                DevState* st) {
-  uint32_t n = use_hot ? st->hot_n : (t.mask + 1);
-  phase_collect(t, len16, max_length, use_hot, hot, n, st->best_primary, cands, cand_cap, st, blockIdx.x, gridDim.x);
+__global__ void k_collect_cands(PairTable t, const uint32_t* __restrict__ len16, uint32_t max_length, uint32_t* __restrict__ cands,
+                                uint32_t cand_cap, DevState* st) {
+  phase_collect(t, len16, max_length, 0, nullptr, t.mask + 1, st->best_primary, cands, cand_cap, st, blockIdx.x, gridDim.x);
 }
 
 // Is position p a *counted* occurrence of (a,b) right now?
@@ -1248,7 +1243,7 @@ __device__ __forceinline__ void phase_apply(const ApplyArgs& A, uint32_t a, uint
   phase_rewrite(A, c, n_sites, bid * blockDim.x + threadIdx.x, nblk * blockDim.x);
 }
 
-// ---- stand-alone K3 kernels (applyMerge / restoreMerge one at a time, and the host-driven loop) ----
+// ---- stand-alone K3 kernels (applyMerge / restoreMerge one at a time) ----
 __global__ void __launch_bounds__(256) k_sites(ApplyArgs A, uint32_t a, uint32_t b, uint32_t c) {
   if (blockIdx.x == 0 && threadIdx.x == 0) A.len16[c] = A.len16[a] + A.len16[b];  // chars = a.chars + b.chars (:318)
   phase_sites(A, a, b, c, 0, tbl_find(A.t, pair_key(a, b)), blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);

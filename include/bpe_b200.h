@@ -82,8 +82,8 @@ typedef struct bpe_stats {
   int64_t loop_round_merges;   /* merges those rounds committed (/ loop_rounds = merges per round) */
   int64_t loop_round_tried;    /* merges whose site pass ran (committed + dropped by the born-pair bound) */
   int64_t loop_rounds_cut;     /* rounds that dropped a tail of their batch                       */
-  int64_t encode_path;         /* kernel the last encode call ran: 1 forward pass per document (csrc/encode_dp.cuh),
-                                  2 lane rounds (csrc/encode_lanes.cuh), 3 per-document kernel only                */
+  int64_t encode_path;         /* kernel the last encode call ran: 2 lane rounds (csrc/encode_lanes.cuh), 3 per-document
+                                  kernel only; 1 (a forward pass per document, since removed) is no longer produced */
 } bpe_stats;
 
 int bpe_abi_version(void);
@@ -97,7 +97,8 @@ const char* bpe_last_error(bpe_engine* e);
 int bpe_set_stream(bpe_engine* e, void* cuda_stream);
 int bpe_synchronize(bpe_engine* e);
 int bpe_get_stats(bpe_engine* e, bpe_stats* out);
-/* Enable per-phase CUDA-event timing inside bpe_merge_until (adds host syncs; default off). */
+/* Enable per-phase CUDA-event timing inside bpe_merge_until (adds host syncs; default off).  Bit 1 (debug): site discovery
+ * scans every slot instead of the occurrence lists.  Other bits are ignored. */
 int bpe_set_profiling(bpe_engine* e, int enabled);
 
 /* ---- vocabulary --------------------------------------------------------------------------- */
