@@ -1019,266 +1019,11 @@ void round_stats(bpe_engine* e, const RoundState& hrs) {
   e->stats.loop_rounds_cut = (int64_t)hrs.rounds_cut_born;
 }
 
-// ---- mergeUntil: persistent cooperative kernel, the host only grows buffers / rebuilds the hot list -----------
-int merge_until_device(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log,
-                       int64_t log_cap, int64_t* n_done, const int32_t* dev_replay = nullptr) {
-  *n_done = 0;
-  CK(cudaSetDevice(e->device));
-  if (e->n_slots == 0) return BPE_OK;
-  TRY(ensure_index(e));
-  uint32_t ml = max_length > 0 ? (uint32_t)max_length : 0;
-  int64_t mw = min_weight > 0 ? min_weight : 2;
-  if (!e->loop_blocks) {
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_merge_loop, ML_THREADS, 0));
-    if (per_sm < 1) return fail(e, BPE_E_CUDA, "k_merge_loop does not fit on an SM");
-    // one 512-thread block per SM: measured best on cfg3 (1.28 s vs 1.41 s with two per SM, 1.33 s with half an SM count,
-    // 1.55 s with 1024-thread blocks) -- a merge is latency bound, fewer arrivals per grid barrier and fewer partials win
-    int want = 1;
-    if (const char* v = getenv("BPE_LOOP_PER_SM")) want = std::max(1, atoi(v));  // tuning knob: co-resident blocks per SM
-    e->loop_blocks = e->sm_count * std::min(per_sm, want);
-    if (const char* v = getenv("BPE_LOOP_BLOCKS")) e->loop_blocks = std::max(1, std::min(atoi(v), e->sm_count * per_sm));
-  }
-  // several exact merges per barrier round (round_kernels.cuh) unless a merge list is replayed; BPE_LOOP_ROUNDS=0 keeps k_merge_loop
-  bool use_rounds = !dev_replay;
-  int round_k = RB;
-  if (const char* v = getenv("BPE_LOOP_ROUNDS")) use_rounds = use_rounds && atoi(v) != 0;
-  if (const char* v = getenv("BPE_LOOP_K")) round_k = std::max(1, std::min(atoi(v), (int)RB));
-  if (use_rounds) TRY(ensure_round_buffers(e));
-  CK(e->partials.reserve((size_t)std::max(e->loop_blocks, e->grid(8))));
-  CK(e->partial_keys.reserve((size_t)std::max(e->loop_blocks, e->grid(8))));
-  CK(e->sites.reserve(1u << 16, 0, e->stream, 1.0));
-  CK(e->sites2.reserve(std::max<size_t>(e->sites.cap, 1u << 16), 0, e->stream, 1.0));
-  CK(e->newslots.reserve(1u << 16, 0, e->stream, 1.0));
-  CK(e->cands.reserve(4096, 0, e->stream, 1.0));
-  CK(e->barrier.reserve(64));
-  cudaEvent_t t0, t1;
-  CK(cudaEventCreate(&t0));
-  CK(cudaEventCreate(&t1));
-  CK(cudaEventRecord(t0, e->stream));
-  int rc = BPE_OK;
-  int64_t done = 0;
-  bool legacy_above = false;
-  std::vector<MergeRec> tmp;
-  for (;;) {
-    int64_t remaining = log_cap - done;
-    if (max_iterations > 0) remaining = std::min(remaining, max_iterations - done);  // core.ts:374-377
-    if (remaining <= 0) break;
-    if (!dev_replay && (!e->hot_valid || e->hot_max_length != ml)) {
-      bool any = false;
-      if ((rc = rebuild_hot(e, ml, &any)) != BPE_OK) break;
-      if (!any) break;  // nothing countable left (core.ts:312)
-    }
-    uint32_t chunk = (uint32_t)std::min<int64_t>(remaining, 1 << 16);
-    if (e->n_tokens + (int64_t)chunk > BPE_MAX_TOKENS) chunk = (uint32_t)std::max<int64_t>(0, BPE_MAX_TOKENS - e->n_tokens);
-    if (chunk == 0) {
-      rc = fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
-      break;
-    }
-    cudaError_t ce;
-    if ((ce = e->dev_log.reserve(chunk)) != cudaSuccess ||
-        (ce = e->d_len16.reserve((size_t)e->n_tokens + chunk + 1, (size_t)e->n_tokens, e->stream, 1.5)) != cudaSuccess) {
-      rc = fail(e, BPE_E_NOMEM, "%s", cudaGetErrorString(ce));
-      break;
-    }
-    LoopArgs L;
-    L.A = apply_args(e);
-    L.pool_cap = e->pool.cap;
-    L.len16_cap = (uint32_t)std::min<size_t>(e->d_len16.cap, 0xFFFFFFF0u);
-    L.hot = e->hot.p;
-    L.hot_cap = (uint32_t)std::min<size_t>(e->hot.cap, 0xFFFFFFF0u);
-    L.hot_limit = e->hot_limit;
-    L.cands = e->cands.p;
-    L.cand_cap = (uint32_t)std::min<size_t>(e->cands.cap, 0xFFFFFFF0u);
-    L.partials = e->partials.p;
-    L.partial_keys = e->partial_keys.p;
-    L.barrier = e->barrier.p;
-    L.log = e->dev_log.p;
-    L.log_cap = chunk;
-    L.max_length = ml;
-    L.min_weight = (uint32_t)std::min<int64_t>(mw, 0xFFFFFFFFll);
-    L.max_tokens = BPE_MAX_TOKENS;
-    L.tbl_cap = e->tbl_cap;
-    L.sites2 = e->sites2.p;
-    L.A.sites_cap = (uint32_t)std::min<size_t>(L.A.sites_cap, e->sites2.cap);  // (only this kernel alternates between the two)
-    {  // warp split of the latency-bound phases and barrier back-off (tuning knobs, read per launch)
-      // measured on cfg3 (profiles/r01i): born pairs / rewrite / old-hot arg-max = 10/2/4 warps beats 8/4/4 by 1 %, 6/x loses 1-2 %;
-      // 10..14 site warps and 64..512 ns of back-off are all within noise
-      int a = 12, b = 10, c = 2, ns = 256;
-      if (const char* v = getenv("BPE_LOOP_P1_SITES")) a = atoi(v);
-      if (const char* v = getenv("BPE_LOOP_P2_NEW")) b = atoi(v);
-      if (const char* v = getenv("BPE_LOOP_P2_RW")) c = atoi(v);
-      if (const char* v = getenv("BPE_LOOP_BAR_NS")) ns = atoi(v);
-      if (a < 1 || a > 15) a = 12;
-      if (b < 1 || c < 1 || b + c > 15) b = 10, c = 2;
-      L.p1_sites = (uint32_t)a;
-      L.p2_new = (uint32_t)b;
-      L.p2_rw = (uint32_t)c;
-      L.bar_ns = (uint32_t)std::max(32, std::min(ns, 4096));
-    }
-    const char* pf = getenv("BPE_LOOP_PREFETCH");  // read per launch: a tuning knob
-    L.prefetch = pf ? std::max(0, std::min(atoi(pf), 2)) : (use_rounds ? 0 : 1);  // (k_merge_rounds: measured, the helper warps become the tail)
-    L.stage_min = stage_min_knob();
-    L.replay = dev_replay ? dev_replay + 2 * done : nullptr;
-    if (dev_replay) e->hot_valid = false;  // replayed merges do not feed the hot list
-    static const bool trace = getenv("BPE_TRACE") != nullptr;
-    auto tw0 = std::chrono::steady_clock::now();
-    k_loop_prepare<<<1, 32, 0, e->stream>>>(e->d_st.p, (uint32_t)e->n_tokens, e->barrier.p);
-    e->stats.kernel_launches++;
-    if (use_rounds && legacy_above) {
-      // the winner has more sites than the packed delta cells of a round can count: k_merge_loop takes the merges above
-      // R_HUGE (it stops, "done", at the first winner at or below it) and the rounds continue from there
-      L.min_weight = (uint32_t)std::max<int64_t>(mw, (int64_t)R_HUGE + 1);
-      void* args[] = {&L};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_loop, dim3(e->loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
-    } else if (use_rounds) {
-      RoundArgs RA = round_args(e, L, round_k);
-      k_rounds_prepare<<<1, 32, 0, e->stream>>>(e->r_state.p);
-      e->stats.kernel_launches++;
-      void* rargs[] = {&RA};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), rargs, R_STAGE_BYTES, e->stream);
-    } else {
-      void* args[] = {&L};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_loop, dim3(e->loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
-    }
-    if (ce != cudaSuccess) {
-      rc = fail(e, BPE_E_CUDA, "cooperative launch of the mergeUntil kernel: %s", cudaGetErrorString(ce));
-      break;
-    }
-    e->stats.kernel_launches++;
-    if ((rc = fetch_state(e)) != BPE_OK) break;
-    uint32_t iters = e->h_st->iters_done;
-    if (trace) {
-      double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tw0).count();
-      fprintf(stderr, "[bpe] k_merge_loop: %u merges in %.2f ms, status %u, best_cnt %u, hot_n %u thresh %u, keys %u/%u\n", iters, ms,
-              e->h_st->status, e->h_st->best_cnt, e->h_st->hot_n, e->h_st->hot_thresh, e->h_st->n_keys, e->tbl_cap);
-    }
-    if (iters) {
-      tmp.resize(iters);
-      ce = cudaMemcpyAsync(tmp.data(), e->dev_log.p, (size_t)iters * sizeof(MergeRec), cudaMemcpyDeviceToHost, e->stream);
-      if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-      if (ce != cudaSuccess) {
-        rc = fail(e, BPE_E_CUDA, "merge log read-back: %s", cudaGetErrorString(ce));
-        break;
-      }
-      for (uint32_t i = 0; i < iters; i++) {
-        const MergeRec& r = tmp[i];
-        log[done].a = r.a;
-        log[done].b = r.b;
-        log[done].c = r.c;
-        log[done].reserved = 0;
-        log[done].weight = r.weight;
-        done++;
-        e->h_len16.push_back(e->h_len16[r.a] + e->h_len16[r.b]);
-        e->h_merges.push_back(r.a);
-        e->h_merges.push_back(r.b);
-        e->h_merges.push_back(r.c);
-      }
-      e->n_tokens += (int32_t)iters;
-      e->mt_dirty = e->lt_dirty = true;
-      e->stats.merges_applied += iters;
-    }
-    uint32_t status = e->h_st->status;
-    if (use_rounds && legacy_above && status == LOOP_DONE && (int64_t)e->h_st->best_cnt >= mw) {
-      legacy_above = false;  // below R_HUGE now: back to the rounds
-      continue;
-    }
-    if (status == LOOP_NEED_LEGACY) {
-      legacy_above = true;
-      continue;
-    }
-    if (status == LOOP_DONE || status == LOOP_EMPTY) break;
-    if (status == LOOP_LIMIT) continue;
-    if (status == LOOP_NEED_REBUILD) {
-      e->hot_valid = false;
-      continue;
-    }
-    if (status == LOOP_ERROR) {
-      rc = check_dev_err(e);
-      if (rc == BPE_OK) rc = fail(e, BPE_E_INTERNAL, "merge loop stopped with an unexplained error (flags 0x%x)", e->h_st->err);
-      break;
-    }
-    if (status == LOOP_NEED_HOST) {
-      if (e->n_tokens >= BPE_MAX_TOKENS) {
-        rc = fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
-        break;
-      }
-      uint64_t w = e->h_st->best_cnt;
-      uint64_t new_keys = std::min<uint64_t>(2 * w + 2, 2 * ((uint64_t)e->n_tokens + 1) + 2);
-      uint64_t keys_after = (uint64_t)e->h_st->n_keys + new_keys;
-      if (keys_after * 2 > e->tbl_cap) {
-        uint64_t want = std::min<uint64_t>(keys_after * 5 / 2, 0x80000000ull);  // next power of two: load 0.2 .. 0.4
-        // a run over a big corpus ends with distinct pairs ~ 5 % of its positions (48 M for the 1 GB Zipf corpus): the first
-        // growth goes most of the way instead of doubling eleven times (a relaunch + rehash each)
-        want = std::max<uint64_t>(want, std::min<uint64_t>(e->n_slots / 16, 1ull << 27));
-        if (keys_after * 2 > pow2_at_least(want)) {
-          rc = fail(e, BPE_E_NOMEM, "pair table cannot grow further");
-          break;
-        }
-        if ((rc = grow_table(e, pow2_at_least(want))) != BPE_OK) break;
-      }
-      uint64_t pool_after = (uint64_t)e->h_st->pool_cursor + 2 * w;
-      if (use_rounds) pool_after += (uint64_t)e->round_blocks * R_POOL_CHUNK;  // every block of k_merge_rounds may open a private chunk
-      if ((ce = e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5)) != cudaSuccess ||
-          (ce = e->sites.reserve((size_t)w, 0, e->stream, 1.25)) != cudaSuccess ||
-          (ce = e->sites2.reserve(e->sites.cap, 0, e->stream, 1.0)) != cudaSuccess ||
-          (ce = e->newslots.reserve((size_t)new_keys, 0, e->stream, 1.25)) != cudaSuccess ||
-          (ce = e->hot.reserve((size_t)e->h_st->hot_n + new_keys, e->h_st->hot_n, e->stream, 1.5)) != cudaSuccess ||
-          (ce = e->cands.reserve((size_t)e->h_st->best_mult, 0, e->stream, 1.5)) != cudaSuccess) {
-        rc = fail(e, BPE_E_NOMEM, "growing merge buffers: %s", cudaGetErrorString(ce));
-        break;
-      }
-      continue;
-    }
-    rc = fail(e, BPE_E_INTERNAL, "merge loop returned status %u", status);
-    break;
-  }
-  *n_done = done;
-  if (rc == BPE_OK) {
-    CK(cudaEventRecord(t1, e->stream));
-    TRY(fetch_state(e));
-    TRY(check_dev_err(e));
-    float ms = 0;
-    CK(cudaEventElapsedTime(&ms, t0, t1));
-    e->stats.ms_last_merge_until = ms;
-    e->live_tokens = e->h_st->live_tokens;
-    e->stats.sites_merged = (int64_t)e->h_st->sites_total;
-    e->stats.tie_breaks = e->h_st->tie_breaks;
-    if (use_rounds) {
-      RoundState hrs;
-      CK(cudaMemcpyAsync(&hrs, e->r_state.p, sizeof(RoundState), cudaMemcpyDeviceToHost, e->stream));
-      CK(cudaStreamSynchronize(e->stream));
-      round_stats(e, hrs);
-      static const bool trace_r = getenv("BPE_TRACE") != nullptr;
-      if (trace_r)
-        fprintf(stderr, "[bpe] rounds %llu, merges %llu (tried %llu), cut by the born-pair bound %llu, single %llu; batch ends: cap %llu, no-candidate %llu, tie %llu, big %llu, "
-                        "token %llu, fresh-token %llu, limits %llu\n", hrs.rounds, hrs.round_merges, hrs.tried, hrs.rounds_cut_born, hrs.rounds_single, hrs.stop_reason[0],
-                hrs.stop_reason[1], hrs.stop_reason[2], hrs.stop_reason[3], hrs.stop_reason[4], hrs.stop_reason[5], hrs.stop_reason[6]);
-      if (trace_r)
-        fprintf(stderr, "[bpe] P1 warp-iterations small %llu big %llu; touched cells small %llu big %llu; sites small %llu big %llu\n", hrs.iters_small, hrs.iters_big,
-                hrs.cells_small, hrs.cells_big, hrs.sites_small, hrs.sites_big);
-      if (trace_r) {
-        const unsigned long long* m = e->h_st->mg_prof_ns;
-        const double n = std::max(1.0, (double)m[4]);
-        fprintf(stderr, "[bpe] P2 of rounds of small merges, block 0, us after the barrier: cells done %.1f, rewrite done %.1f, arg-max done %.1f, partials out %.1f\n",
-                m[0] / n * 1e-3, m[1] / n * 1e-3, m[2] / n * 1e-3, m[3] / n * 1e-3);
-      }
-      if (trace_r) {
-        const unsigned long long* f = e->h_st->fine_ns;
-        const double ns = std::max(1.0, (double)f[5]), nb = std::max(1.0, (double)f[11]);
-        fprintf(stderr, "[bpe] block 0, us per round whose first merge has <= 16384 sites (%.0f rounds): decide %.1f, P1 %.1f, wait %.1f, P2 %.1f, wait %.1f; per round whose first merge has more (%.0f): "
-                        "decide %.1f, P1 %.1f, wait %.1f, P2 %.1f, wait %.1f\n", (double)f[5], f[0] / ns * 1e-3, f[1] / ns * 1e-3, f[2] / ns * 1e-3, f[3] / ns * 1e-3, f[4] / ns * 1e-3,
-                (double)f[11], f[6] / nb * 1e-3, f[7] / nb * 1e-3, f[8] / nb * 1e-3, f[9] / nb * 1e-3, f[10] / nb * 1e-3);
-      }
-    }
-  }
-  cudaEventDestroy(t0);
-  cudaEventDestroy(t1);
-  return rc;
-}
+// ---- mergeUntil: persistent cooperative kernels, the host only grows buffers / rebuilds the hot list ----------------------------
+// One driver serves one GPU, the batched replay (the winners are given) and every rank of a sharded corpus (mg), where the ranks run
+// it in step: their kernels leave at the same merge with the same status.
 
-
-// ---- mergeUntil on a sharded corpus: k_merge_loop_mg, same host protocol as merge_until_device ---------------------
+// the sharded kernels' view of the mailboxes: this rank's place, every peer's flags, inbox and tie mailbox
 MgArgs mg_args(bpe_engine* e) {
   MgArgs M{};
   M.rank = e->mg_rank;
@@ -1300,69 +1045,230 @@ MgArgs mg_args(bpe_engine* e) {
   return M;
 }
 
-int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log, int64_t log_cap,
-                   int64_t* n_done) {
+double ms_since(std::chrono::steady_clock::time_point t) {
+  return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count();
+}
+
+// the arguments of one launch; a sharded engine stages its count deltas (dlt, touched) and lists the pairs born on any rank
+LoopArgs loop_args(bpe_engine* e, bool mg, bool use_rounds, uint32_t chunk, uint32_t ml, int64_t mw) {
+  LoopArgs L{};
+  L.A = apply_args(e);
+  if (mg) {
+    L.A.newpair = e->mg_newpair.p;
+    L.A.newpair_cap = (uint32_t)e->mg_newpair.cap;
+    L.A.dlt = e->mg_dlt.p;
+    L.A.touched = e->mg_touched.p;
+    L.A.touched_cap = (uint32_t)e->mg_touched.cap;
+  }
+  L.pool_cap = e->pool.cap;
+  L.len16_cap = (uint32_t)std::min<size_t>(e->d_len16.cap, 0xFFFFFFF0u);
+  L.hot = e->hot.p;
+  L.hot_cap = (uint32_t)std::min<size_t>(e->hot.cap, 0xFFFFFFF0u);
+  L.hot_limit = e->hot_limit;
+  L.cands = e->cands.p;
+  L.cand_cap = (uint32_t)std::min<size_t>(e->cands.cap, 0xFFFFFFF0u);
+  L.partials = e->partials.p;
+  L.partial_keys = e->partial_keys.p;
+  L.barrier = e->barrier.p;
+  L.log = e->dev_log.p;
+  L.log_cap = chunk;
+  L.max_length = ml;
+  L.min_weight = (uint32_t)std::min<int64_t>(mw, 0xFFFFFFFFll);
+  L.max_tokens = BPE_MAX_TOKENS;
+  L.tbl_cap = e->tbl_cap;
+  L.stage_min = stage_min_knob();
+  // warp split of the latency-bound phases, barrier back-off and prefetch depth (tuning knobs, read per launch).
+  // measured on cfg3 (profiles/r01i): born pairs / rewrite / old-hot arg-max = 10/2/4 warps beats 8/4/4 by 1 %, 6/x loses 1-2 %;
+  // 10..14 site warps and 64..512 ns of back-off are all within noise
+  int a = 12, b = 10, c = 2, ns = 256, pf = 0;
+  if (!mg) {  // (the sweeps that set these ran on one GPU: the sharded loop keeps the defaults of the rounds)
+    if (const char* v = getenv("BPE_LOOP_P1_SITES")) a = atoi(v);
+    if (const char* v = getenv("BPE_LOOP_P2_NEW")) b = atoi(v);
+    if (const char* v = getenv("BPE_LOOP_P2_RW")) c = atoi(v);
+    if (const char* v = getenv("BPE_LOOP_BAR_NS")) ns = atoi(v);
+    const char* v = getenv("BPE_LOOP_PREFETCH");
+    pf = v ? std::max(0, std::min(atoi(v), 2)) : (use_rounds ? 0 : 1);  // (k_merge_rounds: measured, the helper warps become the tail)
+  }
+  if (a < 1 || a > 15) a = 12;
+  if (b < 1 || c < 1 || b + c > 15) b = 10, c = 2;
+  L.p1_sites = (uint32_t)a;
+  L.p2_new = (uint32_t)b;
+  L.p2_rw = (uint32_t)c;
+  L.bar_ns = (uint32_t)std::max(32, std::min(ns, 4096));
+  L.prefetch = pf;
+  return L;
+}
+
+// one launch: k_merge_rounds, or the one-merge kernel (k_merge_loop, k_merge_loop_mg).  `above`: the winner has more sites than the
+// packed delta cells of a round can count, so the one-merge kernel takes the merges above R_HUGE -- it stops, "done", at the first
+// winner at or below it -- and the rounds continue from there
+cudaError_t launch_merge_loop(bpe_engine* e, bool mg, LoopArgs L, bool rounds, bool above, int64_t mw, int round_k) {
+  if (!mg || rounds) {  // the second site buffer, which k_merge_loop_mg does not use
+    L.sites2 = e->sites2.p;
+    L.A.sites_cap = (uint32_t)std::min<size_t>(L.A.sites_cap, e->sites2.cap);
+  }
+  if (rounds) {
+    RoundArgs RA = round_args(e, L, round_k);
+    if (mg) {
+      RA.mg_on = 1;
+      RA.mg = mg_args(e);
+    }
+    k_rounds_prepare<<<1, 32, 0, e->stream>>>(e->r_state.p);
+    e->stats.kernel_launches++;
+    void* args[] = {&RA};
+    return cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), args, R_STAGE_BYTES, e->stream);
+  }
+  if (above) L.min_weight = (uint32_t)std::max<int64_t>(mw, (int64_t)R_HUGE + 1);
+  if (mg) {
+    LoopArgsMg P{L, mg_args(e)};
+    void* args[] = {&P};
+    return cudaLaunchCooperativeKernel((void*)k_merge_loop_mg, dim3(e->mg_loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
+  }
+  void* args[] = {&L};
+  return cudaLaunchCooperativeKernel((void*)k_merge_loop, dim3(e->loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
+}
+
+// appends the `iters` merges of the last launch to the caller's log and to the host's token lengths and merge list
+int read_merge_log(bpe_engine* e, uint32_t iters, bpe_merge* log, int64_t* done, std::vector<MergeRec>& tmp) {
+  tmp.resize(iters);
+  cudaError_t ce = cudaMemcpyAsync(tmp.data(), e->dev_log.p, (size_t)iters * sizeof(MergeRec), cudaMemcpyDeviceToHost, e->stream);
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+  if (ce != cudaSuccess) return fail(e, BPE_E_CUDA, "merge log read-back: %s", cudaGetErrorString(ce));
+  for (const MergeRec& r : tmp) {
+    bpe_merge& m = log[(*done)++];
+    m.a = r.a;
+    m.b = r.b;
+    m.c = r.c;
+    m.reserved = 0;
+    m.weight = r.weight;
+    e->h_len16.push_back(e->h_len16[r.a] + e->h_len16[r.b]);
+    e->h_merges.push_back(r.a);
+    e->h_merges.push_back(r.b);
+    e->h_merges.push_back(r.c);
+  }
+  e->n_tokens += (int32_t)iters;
+  e->mt_dirty = e->lt_dirty = true;
+  e->stats.merges_applied += iters;
+  return BPE_OK;
+}
+
+// LOOP_NEED_HOST: grow the pair table, the occurrence pool and the merge buffers for the winner the kernel stopped at.  On a sharded
+// corpus every rank is here with the same winner, and each one grows what IT lacks.
+int grow_merge_buffers(bpe_engine* e, bool mg, bool use_rounds, bool trace) {
+  if (e->n_tokens >= BPE_MAX_TOKENS) return fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
+  const uint64_t w = e->h_st->best_cnt;
+  const uint64_t new_keys = std::min<uint64_t>(2 * w + 2, 2 * ((uint64_t)e->n_tokens + 1) + 2);
+  const uint64_t keys_after = (uint64_t)e->h_st->n_keys + new_keys;
+  if (keys_after * 2 > e->tbl_cap) {
+    uint64_t want = std::min<uint64_t>(keys_after * 5 / 2, 0x80000000ull);  // next power of two: load 0.2 .. 0.4
+    // a run over a big corpus ends with distinct pairs ~ 5 % of its positions (48 M for the 1 GB Zipf corpus): the first
+    // growth goes most of the way instead of doubling eleven times (a relaunch + rehash each).  (A sharded table holds the
+    // pairs of every shard.)
+    want = std::max<uint64_t>(want, std::min<uint64_t>(e->n_slots * e->mg_world / 16, 1ull << 27));
+    if (keys_after * 2 > pow2_at_least(want)) return fail(e, BPE_E_NOMEM, "pair table cannot grow further");
+    const auto tt = std::chrono::steady_clock::now();
+    TRY(grow_table(e, pow2_at_least(want)));
+    if (mg && trace) fprintf(stderr, "[bpe r%d] grow_table -> %u slots: %.1f ms\n", e->mg_rank, e->tbl_cap, ms_since(tt));
+  }
+  // the in-kernel test is one merge conservative: one GPU reserves 2w cells past the cursor.  A sharded rank reserves 4w, and with
+  // rounds one ROUND conservative there: the first merge of a round has at most R_HUGE sites (larger ones take the other kernel),
+  // the previous round's batch -- whose allocation the figure in the header does not show yet -- at most as many.
+  uint64_t pool_after = (uint64_t)e->h_st->pool_cursor + (mg ? 4 : 2) * w;
+  if (use_rounds)  // every block of k_merge_rounds may open a private chunk
+    pool_after += mg ? 2ull * R_HUGE + 2ull * std::max(R_HUGE, R_BATCH_SITES) + 2ull * e->round_blocks * R_POOL_CHUNK
+                     : (uint64_t)e->round_blocks * R_POOL_CHUNK;
+  // (the hot list of a sharded rank takes both the pairs born on its shard and those that only the peers' records bring)
+  const auto tp = std::chrono::steady_clock::now();
+  cudaError_t ce;
+  if ((ce = e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5)) != cudaSuccess ||
+      (ce = e->sites.reserve((size_t)w, 0, e->stream, 1.25)) != cudaSuccess ||
+      ((!mg || use_rounds) && (ce = e->sites2.reserve(e->sites.cap, 0, e->stream, 1.0)) != cudaSuccess) ||
+      (ce = e->newslots.reserve((size_t)new_keys, 0, e->stream, 1.25)) != cudaSuccess ||
+      (ce = e->hot.reserve((size_t)e->h_st->hot_n + (mg ? 2 : 1) * new_keys, e->h_st->hot_n, e->stream, 1.5)) != cudaSuccess ||
+      (ce = e->cands.reserve((size_t)e->h_st->best_mult, 0, e->stream, 1.5)) != cudaSuccess)
+    return fail(e, BPE_E_NOMEM, "growing merge buffers: %s", cudaGetErrorString(ce));
+  if (mg && trace && ms_since(tp) > 1.0) fprintf(stderr, "[bpe r%d] buffer growth (pool %zu cells): %.1f ms\n", e->mg_rank, e->pool.cap, ms_since(tp));
+  if (mg && e->h_st->best_mult > e->mg_tie_cap)  // (the ranks settle a tie through the tie mailbox)
+    return fail(e, BPE_E_DOMAIN, "%u pairs tie on (weight, index sum): more than the tie mailbox holds (%u)", e->h_st->best_mult, e->mg_tie_cap);
+  return BPE_OK;
+}
+
+int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t max_iterations, bpe_merge* log, int64_t log_cap,
+                int64_t* n_done, const int32_t* dev_replay = nullptr) {
+  const bool mg = e->mg_world > 1;
   *n_done = 0;
-  e->mg_timed_out = false;
-  struct LeaveGate {
+  e->mg_timed_out = false;  // (a verdict about this call only)
+  struct LeaveGate {  // a group member leaves the launch gate on every exit, so that its peers never wait for it there
     LaunchGate* gate;
     ~LeaveGate() {
       if (gate) gate->drop();
     }
   } leave_gate{e->mg_gate};
   CK(cudaSetDevice(e->device));
-  if (!e->mg_connected) return fail(e, BPE_E_INVALID, "sharded engine: call bpe_mg_connect first");
-  TRY(ensure_index(e));
-  if (!e->mg_counts_global) return fail(e, BPE_E_INVALID, "sharded engine: exchange the pair counts first (bpe_mg_export_counts / bpe_mg_import_counts)");
-  uint32_t ml = max_length > 0 ? (uint32_t)max_length : 0;
-  int64_t mw = min_weight > 0 ? min_weight : 2;
-  if (!e->mg_loop_blocks) {
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_merge_loop_mg, ML_THREADS, 0));
-    if (per_sm < 1) return fail(e, BPE_E_CUDA, "k_merge_loop_mg does not fit on an SM");
-    int want = 1;
-    if (const char* v = getenv("BPE_LOOP_PER_SM")) want = std::max(1, atoi(v));
-    e->mg_loop_blocks = e->sm_count * std::min(per_sm, want);
+  if (mg) {  // (no early return on an empty shard: its peers wait for it in every exchange)
+    if (!e->mg_connected) return fail(e, BPE_E_INVALID, "sharded engine: call bpe_mg_connect first");
+  } else if (e->n_slots == 0) {
+    return BPE_OK;
   }
-  CK(e->partials.reserve((size_t)std::max(e->mg_loop_blocks, e->grid(8))));
+  TRY(ensure_index(e));
+  if (mg && !e->mg_counts_global)
+    return fail(e, BPE_E_INVALID, "sharded engine: exchange the pair counts first (bpe_mg_export_counts / bpe_mg_import_counts)");
+  const uint32_t ml = max_length > 0 ? (uint32_t)max_length : 0;
+  const int64_t mw = min_weight > 0 ? min_weight : 2;
+  int& loop_blocks = mg ? e->mg_loop_blocks : e->loop_blocks;
+  if (!loop_blocks) {
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mg ? (const void*)k_merge_loop_mg : (const void*)k_merge_loop, ML_THREADS, 0));
+    if (per_sm < 1) return fail(e, BPE_E_CUDA, "%s does not fit on an SM", mg ? "k_merge_loop_mg" : "k_merge_loop");
+    // one 512-thread block per SM: measured best on cfg3 (1.28 s vs 1.41 s with two per SM, 1.33 s with half an SM count,
+    // 1.55 s with 1024-thread blocks) -- a merge is latency bound, fewer arrivals per grid barrier and fewer partials win
+    int want = 1;
+    if (const char* v = getenv("BPE_LOOP_PER_SM")) want = std::max(1, atoi(v));  // tuning knob: co-resident blocks per SM
+    loop_blocks = e->sm_count * std::min(per_sm, want);
+    const char* v = getenv("BPE_LOOP_BLOCKS");  // (a single-GPU knob: it has never sized k_merge_loop_mg's grid)
+    if (v && !mg) loop_blocks = std::max(1, std::min(atoi(v), e->sm_count * per_sm));
+  }
+  // several exact merges per barrier round (round_kernels.cuh; on a sharded corpus ONE exchange per round) unless a merge list is
+  // replayed; BPE_LOOP_ROUNDS=0 keeps the one-merge kernel
+  bool use_rounds = !dev_replay;
+  int round_k = RB;
+  if (const char* v = getenv("BPE_LOOP_ROUNDS")) use_rounds = use_rounds && atoi(v) != 0;
+  if (const char* v = getenv("BPE_LOOP_K")) round_k = std::max(1, std::min(atoi(v), (int)RB));
+  if (use_rounds) TRY(ensure_round_buffers(e));
+  CK(e->partials.reserve((size_t)std::max(loop_blocks, e->grid(8))));
   CK(e->sites.reserve(1u << 16, 0, e->stream, 1.0));
-  CK(e->newslots.reserve(1u << 17, 0, e->stream, 1.0));
+  if (!mg || use_rounds) CK(e->sites2.reserve(std::max<size_t>(e->sites.cap, 1u << 16), 0, e->stream, 1.0));  // (not read by k_merge_loop_mg)
+  CK(e->newslots.reserve(mg ? 1u << 17 : 1u << 16, 0, e->stream, 1.0));
   CK(e->cands.reserve(4096, 0, e->stream, 1.0));
   CK(e->barrier.reserve(64));
-  CK(e->mg_touched.reserve((size_t)4 * BPE_MAX_TOKENS + 64));
-  CK(e->mg_tie_sorted.reserve(e->mg_tie_cap));
-  CK(e->mg_newpair.reserve((size_t)2 * BPE_MAX_TOKENS + 64));
-  // several exact merges per barrier round and ONE exchange per round (round_kernels.cuh); BPE_LOOP_ROUNDS=0 keeps k_merge_loop_mg
-  bool use_rounds = true;
-  int round_k = RB;
-  if (const char* v = getenv("BPE_LOOP_ROUNDS")) use_rounds = atoi(v) != 0;
-  if (const char* v = getenv("BPE_LOOP_K")) round_k = std::max(1, std::min(atoi(v), (int)RB));
-  if (use_rounds) {
-    TRY(ensure_round_buffers(e));
-    CK(e->sites2.reserve(std::max<size_t>(e->sites.cap, 1u << 16), 0, e->stream, 1.0));
+  if (mg) {  // the staged deltas' cell list, the sorted tie mailbox, the pairs born on any rank
+    CK(e->mg_touched.reserve((size_t)4 * BPE_MAX_TOKENS + 64));
+    CK(e->mg_tie_sorted.reserve(e->mg_tie_cap));
+    CK(e->mg_newpair.reserve((size_t)2 * BPE_MAX_TOKENS + 64));
+  } else {
+    CK(e->partial_keys.reserve((size_t)std::max(loop_blocks, e->grid(8))));  // (read by k_merge_loop only)
   }
-  bool legacy_above = false;
+  static const bool trace = getenv("BPE_TRACE") != nullptr;
   cudaEvent_t t0, t1;
   CK(cudaEventCreate(&t0));
   CK(cudaEventCreate(&t1));
   CK(cudaEventRecord(t0, e->stream));
   int rc = BPE_OK;
   int64_t done = 0;
+  bool legacy_above = false;
   std::vector<MergeRec> tmp;
   double host_ms[4] = {0, 0, 0, 0};  // hot rebuilds, growth (NEED_HOST), launch+state fetch, log read-back
-  auto clk = [] { return std::chrono::steady_clock::now(); };
-  auto since = [](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count(); };
   for (;;) {
     int64_t remaining = log_cap - done;
     if (max_iterations > 0) remaining = std::min(remaining, max_iterations - done);  // core.ts:374-377
     if (remaining <= 0) break;
-    if (!e->hot_valid || e->hot_max_length != ml) {
+    if (!dev_replay && (!e->hot_valid || e->hot_max_length != ml)) {
       bool any = false;
-      auto th = clk();
+      const auto th = std::chrono::steady_clock::now();
       rc = rebuild_hot(e, ml, &any);
-      host_ms[0] += since(th);
+      host_ms[0] += ms_since(th);
       if (rc != BPE_OK) break;
-      if (!any) break;  // nothing countable left on ANY rank: the counts are global (core.ts:312)
+      if (!any) break;  // nothing countable left, on ANY rank of a sharded corpus: the counts are global (core.ts:312)
     }
     uint32_t chunk = (uint32_t)std::min<int64_t>(remaining, 1 << 16);
     if (e->n_tokens + (int64_t)chunk > BPE_MAX_TOKENS) chunk = (uint32_t)std::max<int64_t>(0, BPE_MAX_TOKENS - e->n_tokens);
@@ -1376,103 +1282,37 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
       rc = fail(e, BPE_E_NOMEM, "%s", cudaGetErrorString(ce));
       break;
     }
-    LoopArgsMg P;
-    LoopArgs& L = P.L;
-    L.A = apply_args(e);
-    L.A.newpair = e->mg_newpair.p;
-    L.A.newpair_cap = (uint32_t)e->mg_newpair.cap;
-    L.A.dlt = e->mg_dlt.p;
-    L.A.touched = e->mg_touched.p;
-    L.A.touched_cap = (uint32_t)e->mg_touched.cap;
-    L.pool_cap = e->pool.cap;
-    L.len16_cap = (uint32_t)std::min<size_t>(e->d_len16.cap, 0xFFFFFFF0u);
-    L.hot = e->hot.p;
-    L.hot_cap = (uint32_t)std::min<size_t>(e->hot.cap, 0xFFFFFFF0u);
-    L.hot_limit = e->hot_limit;
-    L.cands = e->cands.p;
-    L.cand_cap = (uint32_t)std::min<size_t>(e->cands.cap, 0xFFFFFFF0u);
-    L.partials = e->partials.p;
-    L.barrier = e->barrier.p;
-    L.log = e->dev_log.p;
-    L.log_cap = chunk;
-    L.max_length = ml;
-    L.min_weight = (uint32_t)std::min<int64_t>(mw, 0xFFFFFFFFll);
-    L.max_tokens = BPE_MAX_TOKENS;
-    L.tbl_cap = e->tbl_cap;
-    L.replay = nullptr;
-    L.stage_min = stage_min_knob();
-    P.M = mg_args(e);
-    static const bool trace = getenv("BPE_TRACE") != nullptr;
-    auto tw0 = std::chrono::steady_clock::now();
+    LoopArgs L = loop_args(e, mg, use_rounds, chunk, ml, mw);
+    L.replay = dev_replay ? dev_replay + 2 * done : nullptr;
+    if (dev_replay) e->hot_valid = false;  // replayed merges do not feed the hot list
+    const auto tw0 = std::chrono::steady_clock::now();
     if (e->mg_gate) e->mg_gate->arrive();
     k_loop_prepare<<<1, 32, 0, e->stream>>>(e->d_st.p, (uint32_t)e->n_tokens, e->barrier.p);
     e->stats.kernel_launches++;
-    if (use_rounds && !legacy_above) {
-      L.sites2 = e->sites2.p;
-      L.A.sites_cap = (uint32_t)std::min<size_t>(L.A.sites_cap, e->sites2.cap);
-      L.p1_sites = 12;
-      L.p2_new = 10;
-      L.p2_rw = 2;
-      L.bar_ns = 256;
-      L.prefetch = 0;
-      RoundArgs RA = round_args(e, L, round_k);
-      RA.mg_on = 1;
-      RA.mg = P.M;
-      k_rounds_prepare<<<1, 32, 0, e->stream>>>(e->r_state.p);
-      e->stats.kernel_launches++;
-      void* rargs[] = {&RA};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), rargs, R_STAGE_BYTES, e->stream);
-    } else {
-      // (rounds: the winner has more sites than the packed delta cells can count -- k_merge_loop_mg takes the merges above
-      // R_HUGE, it stops, "done", at the first winner at or below it)
-      if (use_rounds) L.min_weight = (uint32_t)std::max<int64_t>(mw, (int64_t)R_HUGE + 1);
-      void* args[] = {&P};
-      ce = cudaLaunchCooperativeKernel((void*)k_merge_loop_mg, dim3(e->mg_loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
-    }
+    ce = launch_merge_loop(e, mg, L, use_rounds && !legacy_above, use_rounds && legacy_above, mw, round_k);
     if (ce != cudaSuccess) {
-      rc = fail(e, BPE_E_CUDA, "cooperative launch of the sharded mergeUntil kernel: %s", cudaGetErrorString(ce));
+      rc = fail(e, BPE_E_CUDA, "cooperative launch of the %smergeUntil kernel: %s", mg ? "sharded " : "", cudaGetErrorString(ce));
       break;
     }
     e->stats.kernel_launches++;
     if ((rc = fetch_state(e)) != BPE_OK) break;
-    host_ms[2] += since(tw0);
-    e->mg_epoch = e->h_st->mg_epoch;
-    e->mg_tie_epoch = e->h_st->mg_tie_epoch;
-    uint32_t iters = e->h_st->iters_done;
-    if (trace) {
-      double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tw0).count();
+    host_ms[2] += ms_since(tw0);
+    if (mg) {  // the exchange epochs the next launch continues from
+      e->mg_epoch = e->h_st->mg_epoch;
+      e->mg_tie_epoch = e->h_st->mg_tie_epoch;
+    }
+    const uint32_t iters = e->h_st->iters_done;
+    if (trace && !mg)
+      fprintf(stderr, "[bpe] k_merge_loop: %u merges in %.2f ms, status %u, best_cnt %u, hot_n %u thresh %u, keys %u/%u\n", iters, ms_since(tw0),
+              e->h_st->status, e->h_st->best_cnt, e->h_st->hot_n, e->h_st->hot_thresh, e->h_st->n_keys, e->tbl_cap);
+    if (trace && mg)
       fprintf(stderr, "[bpe r%d] k_merge_loop_mg: %u merges in %.2f ms, status %u, best_cnt %u, hot_n %u thresh %u, keys %u/%u err 0x%x gerr 0x%x\n",
-              e->mg_rank, iters, ms, e->h_st->status, e->h_st->best_cnt, e->h_st->hot_n, e->h_st->hot_thresh, e->h_st->n_keys, e->tbl_cap,
+              e->mg_rank, iters, ms_since(tw0), e->h_st->status, e->h_st->best_cnt, e->h_st->hot_n, e->h_st->hot_thresh, e->h_st->n_keys, e->tbl_cap,
               e->h_st->err, e->h_st->g_vals[0]);
-    }
-    auto tl = clk();
-    if (iters) {
-      tmp.resize(iters);
-      ce = cudaMemcpyAsync(tmp.data(), e->dev_log.p, (size_t)iters * sizeof(MergeRec), cudaMemcpyDeviceToHost, e->stream);
-      if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
-      if (ce != cudaSuccess) {
-        rc = fail(e, BPE_E_CUDA, "merge log read-back: %s", cudaGetErrorString(ce));
-        break;
-      }
-      for (uint32_t i = 0; i < iters; i++) {
-        const MergeRec& r = tmp[i];
-        log[done].a = r.a;
-        log[done].b = r.b;
-        log[done].c = r.c;
-        log[done].reserved = 0;
-        log[done].weight = r.weight;
-        done++;
-        e->h_len16.push_back(e->h_len16[r.a] + e->h_len16[r.b]);
-        e->h_merges.push_back(r.a);
-        e->h_merges.push_back(r.b);
-        e->h_merges.push_back(r.c);
-      }
-      e->n_tokens += (int32_t)iters;
-      e->mt_dirty = e->lt_dirty = true;
-      e->stats.merges_applied += iters;
-    }
-    host_ms[3] += since(tl);
-    uint32_t status = e->h_st->status;
+    const auto tl = std::chrono::steady_clock::now();
+    if (iters && (rc = read_merge_log(e, iters, log, &done, tmp)) != BPE_OK) break;
+    host_ms[3] += ms_since(tl);
+    const uint32_t status = e->h_st->status;
     if (use_rounds && legacy_above && status == LOOP_DONE && (int64_t)e->h_st->best_cnt >= mw) {
       legacy_above = false;  // below R_HUGE now: back to the rounds
       continue;
@@ -1488,56 +1328,22 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
       continue;
     }
     if (status == LOOP_ERROR) {
-      uint32_t f = e->h_st->err | e->h_st->g_vals[0];
-      if (f & ERR_PEER_TIMEOUT) {
+      const uint32_t f = e->h_st->err | e->h_st->g_vals[0];
+      if (mg && (f & ERR_PEER_TIMEOUT)) {  // (a group reports a member's own error ahead of the timeouts it causes in the others)
         e->mg_timed_out = true;
         rc = fail(e, BPE_E_INTERNAL, "a peer GPU did not answer within %.0f s (flags 0x%x)", MG_TIMEOUT_NS / 1e9, f);
       } else {
         rc = check_dev_err(e);
-        if (rc == BPE_OK) rc = fail(e, BPE_E_INTERNAL, "sharded merge loop stopped: local flags 0x%x, all ranks 0x%x", e->h_st->err, e->h_st->g_vals[0]);
+        if (rc == BPE_OK && mg)
+          rc = fail(e, BPE_E_INTERNAL, "sharded merge loop stopped: local flags 0x%x, all ranks 0x%x", e->h_st->err, e->h_st->g_vals[0]);
+        if (rc == BPE_OK) rc = fail(e, BPE_E_INTERNAL, "merge loop stopped with an unexplained error (flags 0x%x)", e->h_st->err);
       }
       break;
     }
-    if (status == LOOP_NEED_HOST) {  // every rank is here with the same winner: each one grows what IT lacks
-      auto tg = clk();
-      if (e->n_tokens >= BPE_MAX_TOKENS) {
-        rc = fail(e, BPE_E_DOMAIN, "token table would exceed %d", BPE_MAX_TOKENS);
-        break;
-      }
-      uint64_t w = e->h_st->best_cnt;
-      uint64_t new_keys = std::min<uint64_t>(2 * w + 2, 2 * ((uint64_t)e->n_tokens + 1) + 2);
-      uint64_t keys_after = (uint64_t)e->h_st->n_keys + new_keys;
-      if (keys_after * 2 > e->tbl_cap) {
-        uint64_t want = std::min<uint64_t>(keys_after * 5 / 2, 0x80000000ull);
-        want = std::max<uint64_t>(want, std::min<uint64_t>((uint64_t)e->n_slots * e->mg_world / 16, 1ull << 27));  // (the keys are global)
-        if (keys_after * 2 > pow2_at_least(want)) {
-          rc = fail(e, BPE_E_NOMEM, "pair table cannot grow further");
-          break;
-        }
-        auto tt = clk();
-        if ((rc = grow_table(e, pow2_at_least(want))) != BPE_OK) break;
-        if (trace) fprintf(stderr, "[bpe r%d] grow_table -> %u slots: %.1f ms\n", e->mg_rank, e->tbl_cap, since(tt));
-      }
-      uint64_t pool_after = (uint64_t)e->h_st->pool_cursor + 4 * w;  // the in-kernel test is one merge conservative
-      // ... one ROUND conservative there: the first merge of a round has at most R_HUGE sites (larger ones take the other kernel),
-      // the previous round's batch -- whose allocation the figure in the header does not show yet -- at most as many
-      if (use_rounds) pool_after += 2ull * R_HUGE + 2ull * std::max(R_HUGE, R_BATCH_SITES) + 2ull * e->round_blocks * R_POOL_CHUNK;
-      auto tp = clk();
-      if ((ce = e->pool.reserve((size_t)pool_after, e->h_st->pool_cursor, e->stream, 1.5)) != cudaSuccess ||
-          (ce = e->sites.reserve((size_t)w, 0, e->stream, 1.25)) != cudaSuccess ||
-          (use_rounds && (ce = e->sites2.reserve(e->sites.cap, 0, e->stream, 1.0)) != cudaSuccess) ||
-          (ce = e->newslots.reserve((size_t)new_keys, 0, e->stream, 1.25)) != cudaSuccess ||
-          (ce = e->hot.reserve((size_t)e->h_st->hot_n + 2 * new_keys, e->h_st->hot_n, e->stream, 1.5)) != cudaSuccess ||
-          (ce = e->cands.reserve((size_t)e->h_st->best_mult, 0, e->stream, 1.5)) != cudaSuccess) {
-        rc = fail(e, BPE_E_NOMEM, "growing merge buffers: %s", cudaGetErrorString(ce));
-        break;
-      }
-      if (trace && since(tp) > 1.0) fprintf(stderr, "[bpe r%d] buffer growth (pool %zu cells): %.1f ms\n", e->mg_rank, e->pool.cap, since(tp));
-      if (e->h_st->best_mult > e->mg_tie_cap) {
-        rc = fail(e, BPE_E_DOMAIN, "%u pairs tie on (weight, index sum): more than the tie mailbox holds (%u)", e->h_st->best_mult, e->mg_tie_cap);
-        break;
-      }
-      host_ms[1] += since(tg);
+    if (status == LOOP_NEED_HOST) {
+      const auto tg = std::chrono::steady_clock::now();
+      if ((rc = grow_merge_buffers(e, mg, use_rounds, trace)) != BPE_OK) break;
+      host_ms[1] += ms_since(tg);
       continue;
     }
     rc = fail(e, BPE_E_INTERNAL, "merge loop returned status %u", status);
@@ -1547,6 +1353,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
   if (rc == BPE_OK) {
     CK(cudaEventRecord(t1, e->stream));
     TRY(fetch_state(e));
+    if (!mg) TRY(check_dev_err(e));  // (a sharded run's flags reach every rank at once, through LOOP_ERROR)
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, t0, t1));
     e->stats.ms_last_merge_until = ms;
@@ -1558,9 +1365,23 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
       CK(cudaMemcpyAsync(&hrs, e->r_state.p, sizeof(RoundState), cudaMemcpyDeviceToHost, e->stream));
       CK(cudaStreamSynchronize(e->stream));
       round_stats(e, hrs);
-      if (getenv("BPE_TRACE") && e->mg_rank == 0) {
-        const unsigned long long* f = e->h_st->fine_ns;
-        const double ns = std::max(1.0, (double)f[5]), nb = std::max(1.0, (double)f[11]);
+      const unsigned long long* f = e->h_st->fine_ns;
+      const double ns = std::max(1.0, (double)f[5]), nb = std::max(1.0, (double)f[11]);
+      if (trace && !mg) {
+        fprintf(stderr, "[bpe] rounds %llu, merges %llu (tried %llu), cut by the born-pair bound %llu, single %llu; batch ends: cap %llu, no-candidate %llu, tie %llu, big %llu, "
+                        "token %llu, fresh-token %llu, limits %llu\n", hrs.rounds, hrs.round_merges, hrs.tried, hrs.rounds_cut_born, hrs.rounds_single, hrs.stop_reason[0],
+                hrs.stop_reason[1], hrs.stop_reason[2], hrs.stop_reason[3], hrs.stop_reason[4], hrs.stop_reason[5], hrs.stop_reason[6]);
+        fprintf(stderr, "[bpe] P1 warp-iterations small %llu big %llu; touched cells small %llu big %llu; sites small %llu big %llu\n", hrs.iters_small, hrs.iters_big,
+                hrs.cells_small, hrs.cells_big, hrs.sites_small, hrs.sites_big);
+        const unsigned long long* m = e->h_st->mg_prof_ns;
+        const double n = std::max(1.0, (double)m[4]);
+        fprintf(stderr, "[bpe] P2 of rounds of small merges, block 0, us after the barrier: cells done %.1f, rewrite done %.1f, arg-max done %.1f, partials out %.1f\n",
+                m[0] / n * 1e-3, m[1] / n * 1e-3, m[2] / n * 1e-3, m[3] / n * 1e-3);
+        fprintf(stderr, "[bpe] block 0, us per round whose first merge has <= 16384 sites (%.0f rounds): decide %.1f, P1 %.1f, wait %.1f, P2 %.1f, wait %.1f; per round whose first merge has more (%.0f): "
+                        "decide %.1f, P1 %.1f, wait %.1f, P2 %.1f, wait %.1f\n", (double)f[5], f[0] / ns * 1e-3, f[1] / ns * 1e-3, f[2] / ns * 1e-3, f[3] / ns * 1e-3, f[4] / ns * 1e-3,
+                (double)f[11], f[6] / nb * 1e-3, f[7] / nb * 1e-3, f[8] / nb * 1e-3, f[9] / nb * 1e-3, f[10] / nb * 1e-3);
+      }
+      if (trace && mg && e->mg_rank == 0) {
         fprintf(stderr, "[bpe r0] rounds %llu, merges %llu (tried %llu); block 0, us per round whose first merge has <= 16384 sites (%.0f): decide %.1f, P1 %.1f, wait %.1f, P2 %.1f, wait %.1f; "
                         "whose first merge has more (%.0f): decide %.1f, P1 %.1f, wait %.1f, P2 %.1f, wait %.1f; exchange (emit..summed) ms %.1f\n", hrs.rounds, hrs.round_merges, hrs.tried,
                 (double)f[5], f[0] / ns * 1e-3, f[1] / ns * 1e-3, f[2] / ns * 1e-3, f[3] / ns * 1e-3, f[4] / ns * 1e-3, (double)f[11], f[6] / nb * 1e-3, f[7] / nb * 1e-3,
@@ -1569,7 +1390,7 @@ int merge_until_mg(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_
         fprintf(stderr, "[bpe r0] exchange, block 0, ms: header + records out + report %.1f, wait + sum as they arrive + fold %.1f, barrier %.1f\n", m[5] * 1e-6, m[6] * 1e-6, m[7] * 1e-6);
       }
     }
-    if (getenv("BPE_TRACE") && e->mg_rank == 0) {
+    if (trace && mg && e->mg_rank == 0) {
       fprintf(stderr, "[bpe r0] mg phases ms (decide, P1, wait, M1, wait, send+local P2, barrier+peer wait, apply, wait, P3, wait, tie):");
       for (int i = 0; i < 12; i++) fprintf(stderr, " %.1f", (double)e->h_st->mg_prof_ns[i] * 1e-6);
       fprintf(stderr, "  total %.1f ms, %lld merges; host ms: hot rebuild %.1f, growth %.1f, launch..fetch %.1f, log %.1f\n", ms, (long long)done,
@@ -2424,7 +2245,7 @@ int bpe_apply_merges(bpe_engine* e, const int32_t* ab, int64_t n, int64_t* n_rep
   CK(cudaMemcpyAsync(d_ab.p, ab, (size_t)2 * n * 4, cudaMemcpyHostToDevice, e->stream));
   std::vector<bpe_merge> log((size_t)n);
   int64_t done = 0;
-  TRY(merge_until_device(e, 1, 0, n, log.data(), n, &done, d_ab.p));
+  TRY(merge_until(e, 1, 0, n, log.data(), n, &done, d_ab.p));
   if (done != n) return fail(e, BPE_E_INTERNAL, "replayed %lld of %lld merges", (long long)done, (long long)n);
   if (n_replaced)
     for (int64_t i = 0; i < n; i++) n_replaced[i] = log[(size_t)i].weight;
@@ -2435,8 +2256,7 @@ int bpe_merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64
                     int64_t log_cap, int64_t* n_done) {
   if (!e || !n_done || (log_cap > 0 && !log) || log_cap < 0) return BPE_E_INVALID;
   if (is_group(e)) return group_merge_until(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
-  if (e->mg_world > 1) return merge_until_mg(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
-  return merge_until_device(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
+  return merge_until(e, min_weight, max_length, max_iterations, log, log_cap, n_done);
 }
 
 

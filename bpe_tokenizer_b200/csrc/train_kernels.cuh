@@ -1302,7 +1302,7 @@ struct LoopArgs {
   // replay mode (batched restoreMerge, core.ts:477-494): the winners are GIVEN -- (a,b) of merge i at replay[2i..2i+1]
   // -- instead of found by the arg-max; the hot list is neither read nor fed
   const int32_t* replay;
-  // how the 16 warps of a block share the latency-bound phases of small merges (tuning knobs, defaults in merge_until_device):
+  // how the 16 warps of a block share the latency-bound phases of small merges (tuning knobs, defaults in loop_args, bpe_b200.cu):
   // P1: p1_sites warps walk the sites, the others fill the previous merge's lists and prefetch; P2: p2_new warps enter the
   // born pairs, p2_rw warps rewrite the corpus, the others run the arg-max over the old hot pairs
   uint32_t p1_sites, p2_new, p2_rw;
