@@ -12,11 +12,15 @@
 //     redundantly and identically everywhere;
 //   * only when several pairs tie on (weight, a.index + b.index) a second small exchange carries each rank's last
 //     counted position per candidate (candidates in canonical key order); the highest rank holding a candidate owns its
-//     last occurrence.
-// Everything runs inside ONE persistent cooperative kernel per GPU (k_merge_loop_mg): compute and the exchange are
-// fused, there is no host round trip and no NCCL call per merge.  Every decision that ends or interrupts the loop is
-// taken from replicated values (or minima over ranks carried in the message headers), so all ranks leave the kernel
-// at the same merge with the same status.  Waits on peers are bounded (MG_TIMEOUT_NS) and abort the loop.
+//     last occurrence (mg_tie_winner).
+// Everything runs inside a persistent cooperative kernel per GPU: compute and the exchange are fused, there is no host
+// round trip and no NCCL call per merge.  k_merge_rounds with mg_on (round_kernels.cuh) runs almost every merge, several per
+// exchange; k_merge_loop_mg below runs one merge per exchange: those above R_HUGE global sites, or all of them under
+// BPE_LOOP_ROUNDS=0.  Their record formats differ; the steps every rank must run identically live here once, for both: the
+// header of a message (mg_store_header) and its fold (mg_fold_headers_warp), the wait on a peer's flag (mg_wait_flag) and the
+// tie-break.  Every decision that ends or interrupts the loop is taken from replicated values (or minima over ranks carried in
+// the message headers), so all ranks leave the kernel at the same merge with the same status.  Waits on peers are bounded
+// (MG_TIMEOUT_NS) and abort the loop.
 #pragma once
 #include "train_kernels.cuh"
 
@@ -52,26 +56,30 @@ __device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long
   return v;
 }
 
+// wait until a peer's flag `f` reaches `epoch`, sleeping `ns` ns between looks, doubled up to `ns_max`.  Still waiting
+// MG_TIMEOUT_NS after t0: ERR_PEER_TIMEOUT, mg_abort set (the loop ends at its next check), false.
+__device__ __forceinline__ bool mg_wait_flag(const unsigned long long* f, unsigned long long epoch, unsigned long long t0, uint32_t ns,
+                                             uint32_t ns_max, DevState* st) {
+  while (ld_acquire_sys(f) < epoch) {
+    __nanosleep(ns);
+    if (ns < ns_max) ns <<= 1;
+    if (now_ns() - t0 > MG_TIMEOUT_NS) {
+      atomicOr(&st->err, ERR_PEER_TIMEOUT);
+      st->mg_abort = 1;
+      return false;
+    }
+  }
+  return true;
+}
+
 // thread 0 of block 0: publish `epoch` to every peer and wait until every peer has published it to us
 __device__ __forceinline__ void mg_signal_and_wait(const MgArgs& M, unsigned long long* const* flags, unsigned long long epoch,
                                                    DevState* st) {
   for (int q = 0; q < M.world; q++)
     if (q != M.rank) st_release_sys(flags[q] + 16 * M.rank, epoch);
-  unsigned long long t0 = now_ns();
-  for (int q = 0; q < M.world; q++) {
-    if (q == M.rank) continue;
-    const unsigned long long* f = flags[M.rank] + 16 * q;
-    uint32_t ns = 32;
-    while (ld_acquire_sys(f) < epoch) {
-      __nanosleep(ns);
-      if (ns < 1024) ns <<= 1;
-      if (now_ns() - t0 > MG_TIMEOUT_NS) {
-        atomicOr(&st->err, ERR_PEER_TIMEOUT);
-        st->mg_abort = 1;
-        return;
-      }
-    }
-  }
+  const unsigned long long t0 = now_ns();
+  for (int q = 0; q < M.world; q++)
+    if (q != M.rank && !mg_wait_flag(flags[M.rank] + 16 * q, epoch, t0, 32, 1024, st)) return;
 }
 
 struct LoopArgsMg {
@@ -115,71 +123,46 @@ __device__ __forceinline__ unsigned long long* mg_area(const MgArgs& M, int dst,
   return M.inbox[dst] + ((size_t)par * M.world + sender) * M.inbox_stride;
 }
 
-// ---- exchange, executed by warp 0 of block 0: lane q talks to rank q, so its cost does not grow with the world size ----
-// header of a message: 16 u32 (H_* indices) in the first 64 bytes of the area, moved with 128-bit accesses
-__device__ __forceinline__ void mg_send_warp(const LoopArgsMg& P, DevState* st, uint32_t par, uint32_t n_rec, unsigned long long epoch,
-                                             unsigned long long* const* flags) {
-  const MgArgs& M = P.M;
-  const LoopArgs& L = P.L;
-  const int q = (int)(threadIdx.x & 31u);
-  const bool peer = q < M.world && q != M.rank;
-  if (q < M.world) {
-    const unsigned long long cur = ld_cg(&st->pool_cursor);
-    uint32_t h[12];
+// header of a message: 16 u32 (H_* indices) in the first 64 bytes of the area, moved with 128-bit accesses.  This rank's
+// record count, error flags and capacities (H_N .. H_CAND_CAP) into the header at `dst`; the pool figure only gates the next
+// decision.
+__device__ __forceinline__ void mg_store_header(const LoopArgs& L, const MgArgs& M, unsigned long long* dst, uint32_t n_rec, uint32_t new_cap) {
+  DevState* st = L.A.st;
+  const unsigned long long cur = ld_cg(&st->pool_cursor);
+  uint32_t h[12];
 #pragma unroll
-    for (int i = 0; i < 12; i++) h[i] = 0;
-    h[H_N] = n_rec;
-    h[H_ERR] = ld_cg(&st->err);
-    h[H_POOL_FREE] = (uint32_t)min(L.pool_cap > cur ? L.pool_cap - cur : 0ull, 0xFFFFFFFFull);  // (only gates the next merge)
-    h[H_SITES_CAP] = L.A.sites_cap;
-    h[H_NEW_CAP] = L.A.new_cap;
-    h[H_HOT_CAP] = min(L.hot_cap, L.hot_limit);
-    h[H_LEN16_CAP] = L.len16_cap;
-    h[H_TBL_CAP] = L.tbl_cap;
-    h[H_CAND_CAP] = min(L.cand_cap, M.tie_cap);
-    uint4* dst = reinterpret_cast<uint4*>(mg_area(M, q, par, M.rank));
+  for (int i = 0; i < 12; i++) h[i] = 0;
+  h[H_N] = n_rec;
+  h[H_ERR] = ld_cg(&st->err);
+  h[H_POOL_FREE] = (uint32_t)min(L.pool_cap > cur ? L.pool_cap - cur : 0ull, 0xFFFFFFFFull);
+  h[H_SITES_CAP] = L.A.sites_cap;
+  h[H_NEW_CAP] = new_cap;
+  h[H_HOT_CAP] = min(L.hot_cap, L.hot_limit);
+  h[H_LEN16_CAP] = L.len16_cap;
+  h[H_TBL_CAP] = L.tbl_cap;
+  h[H_CAND_CAP] = min(L.cand_cap, M.tie_cap);
+  uint4* d4 = reinterpret_cast<uint4*>(dst);
 #pragma unroll
-    for (int i = 0; i < 3; i++) dst[i] = make_uint4(h[4 * i], h[4 * i + 1], h[4 * i + 2], h[4 * i + 3]);
-    __threadfence_system();
-  }
-  __syncwarp();
-  if (peer) st_release_sys(flags[q] + 16 * M.rank, epoch);
+  for (int i = 0; i < 3; i++) d4[i] = make_uint4(h[4 * i], h[4 * i + 1], h[4 * i + 2], h[4 * i + 3]);
 }
 
-// second half: wait for every peer's flag, then fold the G headers (OR of the error flags, minima of the capacities)
-__device__ __forceinline__ void mg_wait_fold_warp(const LoopArgsMg& P, DevState* st, uint32_t par, unsigned long long epoch,
-                                                  unsigned long long* const* flags) {
-  const MgArgs& M = P.M;
-  const int q = (int)(threadIdx.x & 31u);
-  const bool peer = q < M.world && q != M.rank;
-  if (peer) {
-    const unsigned long long* f = flags[M.rank] + 16 * q;
-    unsigned long long t0 = now_ns();
-    uint32_t ns = 16;
-    while (ld_acquire_sys(f) < epoch) {
-      __nanosleep(ns);
-      if (ns < 128) ns <<= 1;
-      if (now_ns() - t0 > MG_TIMEOUT_NS) {
-        atomicOr(&st->err, ERR_PEER_TIMEOUT);
-        st->mg_abort = 1;
-        break;
-      }
-    }
-  }
-  __syncwarp();
+// One warp, lane q reads sender q's header in this rank's area `par` (the messages are complete): the G headers fold into
+// st->g_vals (OR of the error flags, minima of the capacities), the same values on every rank.  Returns sender q's H_N.
+__device__ __forceinline__ uint32_t mg_fold_headers_warp(const MgArgs& M, DevState* st, uint32_t par) {
+  const int q = (int)lane_id();
   uint32_t w[12];
 #pragma unroll
   for (int i = 0; i < 12; i++) w[i] = (i == H_ERR) ? 0u : 0xFFFFFFFFu;
   if (q < M.world) {
     const uint4* hq = reinterpret_cast<const uint4*>(mg_area(M, M.rank, par, q));
-    uint4 v0 = ld_cg4(hq), v1 = ld_cg4(hq + 1), v2 = ld_cg4(hq + 2);
+    const uint4 v0 = ld_cg4(hq), v1 = ld_cg4(hq + 1), v2 = ld_cg4(hq + 2);
     w[0] = v0.x; w[1] = v0.y; w[2] = v0.z; w[3] = v0.w; w[4] = v1.x; w[5] = v1.y; w[6] = v1.z; w[7] = v1.w; w[8] = v2.x; w[9] = v2.y; w[10] = v2.z; w[11] = v2.w;
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
     for (int i = H_ERR; i <= H_CAND_CAP; i++) {
-      uint32_t other = __shfl_xor_sync(0xFFFFFFFFu, w[i], o);
+      const uint32_t other = __shfl_xor_sync(0xFFFFFFFFu, w[i], o);
       w[i] = (i == H_ERR) ? (w[i] | other) : min(w[i], other);
     }
   }
@@ -188,6 +171,102 @@ __device__ __forceinline__ void mg_wait_fold_warp(const LoopArgsMg& P, DevState*
     g[0] = make_uint4(w[H_ERR], w[H_POOL_FREE], w[H_SITES_CAP], w[H_NEW_CAP]);
     g[1] = make_uint4(w[H_HOT_CAP], w[H_LEN16_CAP], w[H_TBL_CAP], w[H_CAND_CAP]);
   }
+  return w[H_N];
+}
+
+// Position tie-break on a sharded corpus (core.ts:294-305), shared by k_merge_loop_mg and k_merge_rounds: from the candidates
+// phase_collect listed (the same pairs on every rank) to the winner's table slot.  The last counted occurrence in GLOBAL scan
+// order = (rank, local position) decides.  The candidates go in canonical (pair key) order so that every rank talks about the
+// same one; each block takes one and stores its last counted LOCAL occurrence into every rank's tiebox; after the tie exchange
+// the highest rank holding a candidate owns its last occurrence.  Every thread of the grid calls, after a grid barrier that
+// follows phase_collect; `barrier` is the caller's grid barrier, s_max 32 words of shared scratch.  NOSLOT on a peer abort or
+// when no rank holds a candidate.
+template <class Bar>
+__device__ __forceinline__ uint32_t mg_tie_winner(const LoopArgs& L, const MgArgs& M, uint32_t* s_max, unsigned long long& tie_epoch,
+                                                  Bar barrier) {
+  const ApplyArgs& A = L.A;
+  DevState* st = A.st;
+  const PairTable& t = A.t;
+  const uint32_t bid = blockIdx.x, nblk = gridDim.x;
+  const uint32_t gtid = bid * blockDim.x + threadIdx.x, gthreads = nblk * blockDim.x;
+  const uint32_t tpar = (uint32_t)((tie_epoch + 1) & 1u);
+  const uint32_t nc = ld_cg(&st->n_cand);  // == the winner's multiplicity, on every rank
+  for (uint32_t i = gtid; i < nc; i += gthreads) {  // canonical order: by pair key
+    const uint32_t si = ld_cg(&L.cands[i]);
+    const uint32_t ki = t.keys[si];
+    uint32_t r = 0;
+    for (uint32_t j = 0; j < nc; j++) r += t.keys[ld_cg(&L.cands[j])] < ki;
+    M.tie_sorted[r] = si;
+  }
+  barrier();
+  for (uint32_t cnd = bid; cnd < nc; cnd += nblk) {  // one block per candidate: its last counted local occurrence
+    const uint32_t s = ld_cg(&M.tie_sorted[cnd]);
+    const uint32_t key = t.keys[s];
+    const uint32_t a = key >> 16, b = key & 0xFFFFu;
+    const unsigned long long start = t.occ_start.get(s);
+    const uint32_t len = t.occ_len[s];
+    uint32_t v = 0;
+    for (uint32_t i = threadIdx.x; i < len; i += blockDim.x) {
+      const uint32_t p = A.pool[start + i];
+      if (counted_occurrence(A.slots, A.n, p, a, b)) v = max(v, p + 1);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(0xFFFFFFFFu, v, o));
+    __syncthreads();
+    if (lane_id() == 0) s_max[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      uint32_t m = 0;
+      for (uint32_t i = 0; i < (blockDim.x >> 5); i++) m = max(m, s_max[i]);
+      for (int q = 0; q < M.world; q++) M.tiebox[q][((size_t)tpar * M.world + M.rank) * M.tie_cap + cnd] = m;
+      __threadfence_system();
+    }
+  }
+  barrier();
+  if (bid == 0 && threadIdx.x == 0) {
+    st->tie_pos = ~0ull;
+    mg_signal_and_wait(M, M.flag_tie, tie_epoch + 1, st);
+  }
+  tie_epoch++;
+  barrier();
+  if (bid == 0) {
+    const uint32_t* box = M.tiebox[M.rank] + (size_t)tpar * M.world * M.tie_cap;
+    for (uint32_t i = threadIdx.x; i < nc; i += blockDim.x) {
+      for (int q = M.world - 1; q >= 0; q--) {  // the highest rank holding the pair owns its last occurrence
+        const uint32_t v = ld_cg(box + (size_t)q * M.tie_cap + i);
+        if (v) {
+          atomicMin(&st->tie_pos, ((((unsigned long long)q << 32) | (v - 1)) << 16) | i);
+          break;
+        }
+      }
+    }
+  }
+  barrier();
+  const unsigned long long tp = ld_cg(&st->tie_pos);
+  if (ld_cg(&st->mg_abort) || tp == ~0ull) return NOSLOT;
+  return ld_cg(&M.tie_sorted[(uint32_t)(tp & 0xFFFFu)]);
+}
+
+// ---- exchange, executed by warp 0 of block 0: lane q talks to rank q, so its cost does not grow with the world size ----
+__device__ __forceinline__ void mg_send_warp(const LoopArgsMg& P, uint32_t par, uint32_t n_rec, unsigned long long epoch,
+                                             unsigned long long* const* flags) {
+  const MgArgs& M = P.M;
+  const int q = (int)lane_id();
+  if (q < M.world) {
+    mg_store_header(P.L, M, mg_area(M, q, par, M.rank), n_rec, P.L.A.new_cap);
+    __threadfence_system();
+  }
+  __syncwarp();
+  if (q < M.world && q != M.rank) st_release_sys(flags[q] + 16 * M.rank, epoch);
+}
+
+// second half: wait for every peer's flag, then fold the G headers
+__device__ __forceinline__ void mg_wait_fold_warp(const MgArgs& M, DevState* st, uint32_t par, unsigned long long epoch,
+                                                  unsigned long long* const* flags) {
+  const int q = (int)lane_id();
+  if (q < M.world && q != M.rank) mg_wait_flag(flags[M.rank] + 16 * q, epoch, now_ns(), 16, 128, st);
+  __syncwarp();
+  mg_fold_headers_warp(M, st, par);
 }
 
 __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(LoopArgsMg P) {
@@ -216,8 +295,8 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
     st->n_newpair = 0;
   }
   if (bid == 0 && threadIdx.x < 32) {
-    mg_send_warp(P, st, (uint32_t)((epoch + 1) & 1u), 0, epoch + 1, M.flag_data);
-    mg_wait_fold_warp(P, st, (uint32_t)((epoch + 1) & 1u), epoch + 1, M.flag_data);
+    mg_send_warp(P, (uint32_t)((epoch + 1) & 1u), 0, epoch + 1, M.flag_data);
+    mg_wait_fold_warp(M, st, (uint32_t)((epoch + 1) & 1u), epoch + 1, M.flag_data);
   }
   epoch++;
   {
@@ -280,65 +359,12 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
     MGPROF(0)
     if (status == LOOP_RUNNING && w.mult > 1) {
       // ---- tie on (weight, a.index+b.index): last counted occurrence in GLOBAL scan order decides (core.ts:294-305) ----
-      const uint32_t tpar = (uint32_t)((tie_epoch + 1) & 1u);
       phase_collect(t, A.len16, L.max_length, 1, L.hot, ld_cg(&st->hot_n), w.primary, L.cands, L.cand_cap, st, bid, nblk);
       GRID_BARRIER();
-      const uint32_t nc = ld_cg(&st->n_cand);  // == w.mult on every rank
-      for (uint32_t i = gtid; i < nc; i += gthreads) {  // canonical order: by pair key
-        uint32_t si = ld_cg(&L.cands[i]);
-        uint32_t ki = t.keys[si], r = 0;
-        for (uint32_t j = 0; j < nc; j++) r += t.keys[ld_cg(&L.cands[j])] < ki;
-        M.tie_sorted[r] = si;
-      }
-      GRID_BARRIER();
-      for (uint32_t cnd = bid; cnd < nc; cnd += nblk) {  // one block per candidate: its last counted local occurrence
-        uint32_t s = ld_cg(&M.tie_sorted[cnd]);
-        uint32_t key = t.keys[s];
-        uint32_t a = key >> 16, b = key & 0xFFFFu;
-        const unsigned long long start = t.occ_start.get(s);
-        uint32_t len = t.occ_len[s];
-        uint32_t v = 0;
-        for (uint32_t i = threadIdx.x; i < len; i += blockDim.x) {
-          uint32_t p = A.pool[start + i];
-          if (counted_occurrence(A.slots, A.n, p, a, b)) v = max(v, p + 1);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(0xFFFFFFFFu, v, o));
-        __syncthreads();
-        if (lane_id() == 0) s_max[threadIdx.x >> 5] = v;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-          uint32_t m = 0;
-          for (uint32_t i = 0; i < (blockDim.x >> 5); i++) m = max(m, s_max[i]);
-          for (int q = 0; q < M.world; q++) M.tiebox[q][((size_t)tpar * M.world + M.rank) * M.tie_cap + cnd] = m;
-          __threadfence_system();
-        }
-      }
-      GRID_BARRIER();
-      if (lead) {
-        st->tie_pos = ~0ull;
-        mg_signal_and_wait(M, M.flag_tie, tie_epoch + 1, st);
-      }
-      tie_epoch++;
-      GRID_BARRIER();
-      if (bid == 0) {
-        const uint32_t* box = M.tiebox[M.rank] + (size_t)tpar * M.world * M.tie_cap;
-        for (uint32_t i = threadIdx.x; i < nc; i += blockDim.x) {
-          for (int q = M.world - 1; q >= 0; q--) {  // the highest rank holding the pair owns its last occurrence
-            uint32_t v = ld_cg(box + (size_t)q * M.tie_cap + i);
-            if (v) {
-              atomicMin(&st->tie_pos, ((((unsigned long long)q << 32) | (v - 1)) << 16) | i);
-              break;
-            }
-          }
-        }
-      }
-      GRID_BARRIER();
-      unsigned long long tp = ld_cg(&st->tie_pos);
-      if (ld_cg(&st->mg_abort) || tp == ~0ull) status = LOOP_ERROR;
+      const uint32_t s = mg_tie_winner(L, M, s_max, tie_epoch, [&] { GRID_BARRIER(); });
+      if (s == NOSLOT) status = LOOP_ERROR;
       else {
-        uint32_t s = ld_cg(&M.tie_sorted[(uint32_t)(tp & 0xFFFFu)]);
-        uint32_t key = t.keys[s];
+        const uint32_t key = t.keys[s];
         w.slot = s;
         wa = key >> 16;
         wb = key & 0xFFFFu;
@@ -443,13 +469,13 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
     }
     // ---- send, then do the LOCAL half of P2 while the peers' messages travel: the pairs born on this shard enter the table
     // (their counts come with the records), the shard is rewritten.  The wait for the peers sits behind that work. ----
-    if (bid == 0 && threadIdx.x < 32) mg_send_warp(P, st, epar, min(ld_cg(&st->n_out), M.inbox_stride - MG_HDR), epoch + 1, M.flag_data);
+    if (bid == 0 && threadIdx.x < 32) mg_send_warp(P, epar, min(ld_cg(&st->n_out), M.inbox_stride - MG_HDR), epoch + 1, M.flag_data);
     const uint32_t n_sites_now = ld_cg(&st->n_sites[par]);
     phase_new_pairs(A, c, A.len16, L.max_length, 0, L.hot, L.hot_cap, L.pool_cap, true, gtid, gthreads);
     phase_rewrite(A, c, n_sites_now, gtid, gthreads);
     MGPROF(5)
     GRID_BARRIER();
-    if (bid == 0 && threadIdx.x < 32) mg_wait_fold_warp(P, st, epar, epoch + 1, M.flag_data);
+    if (bid == 0 && threadIdx.x < 32) mg_wait_fold_warp(M, st, epar, epoch + 1, M.flag_data);
     if (lead) {
       st->n_out = 0;  // nobody appends before the next merge's P1
       st->n_cand = 0;

@@ -38,10 +38,12 @@
 // listed as records to every rank (NVLink stores) and reports to a per-(receiver, parity, sender) arrival counter; every
 // block sums the records of the senders that are complete into the GLOBAL cells (mgr_collect), P2 runs over those.  The
 // decisions are replicated: U bounds and site counts are sums over the ranks, capacities minima (headers of the messages).
+// The header, its fold, the waits on the peers' flags and the tie-break are mg_kernels.cuh's, shared with k_merge_loop_mg.
 //
 // Exactness argument for the order inside a batch (SURVEY.md A.2, core.ts:294-305): counts of existing pairs never grow
 // under merging, so an old pair that ranked below m_j at the decision still does; born pairs are bounded by U; m_j's own
-// count is unchanged; equal keys never enter a batch (position tie-breaks run alone, through the path k_merge_loop uses).
+// count is unchanged; equal keys never enter a batch (position tie-breaks run alone: phase_tie, as in k_merge_loop, or
+// mg_tie_winner on a sharded corpus).
 #pragma once
 #include "train_kernels.cuh"
 #include "mg_kernels.cuh"
@@ -411,7 +413,7 @@ __device__ __forceinline__ void round_flush_stage(const RoundArgs& R, RoundSm& S
 
 // ---- sharded corpus: the message of a round ----
 // u64 words of one (parity, sender) area of an inbox: MGR_HDR words of header, then the records.
-//   [0..5]   the twelve u32 of mg_kernels' header (H_N records, H_ERR, capacities)
+//   [0..5]   the twelve u32 of mg_store_header (H_N records, H_ERR, capacities)
 //   [8 + j]  U bounds of merge j on the sender (left | right << 32)       [24 + j]  sites of merge j on the sender
 //   [40]     merges the sender tried (its batch; every rank commits at most the smallest)
 // record: ((merge * 2 + side) << 16 | token) << 42 | counted occurrences << 21 | decrements    (one per warp and distinct
@@ -499,23 +501,8 @@ __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, 
   const unsigned long long ub_lane = ((uint32_t)q < k) ? ld_cg(&R.rs->ub[par][q].v) : 0ull;
   const uint32_t ns_lane = ((uint32_t)q < k) ? ld_cg(&R.rs->n_sites[par][q].v) : 0u;
   if (q < M.world) {
-    const unsigned long long cur = ld_cg(&st->pool_cursor);
-    uint32_t h[12];
-#pragma unroll
-    for (int i = 0; i < 12; i++) h[i] = 0;
-    h[H_N] = min(ld_cg(&st->n_out), M.inbox_stride - MGR_HDR);
-    h[H_ERR] = ld_cg(&st->err);
-    h[H_POOL_FREE] = (uint32_t)min(L.pool_cap > cur ? L.pool_cap - cur : 0ull, 0xFFFFFFFFull);  // (only gates the next batch)
-    h[H_SITES_CAP] = L.A.sites_cap;
-    h[H_NEW_CAP] = 0xFFFFFFFFu;
-    h[H_HOT_CAP] = min(L.hot_cap, L.hot_limit);
-    h[H_LEN16_CAP] = L.len16_cap;
-    h[H_TBL_CAP] = L.tbl_cap;
-    h[H_CAND_CAP] = min(L.cand_cap, M.tie_cap);
     unsigned long long* dst = mg_area(M, q, epar, M.rank);
-    uint4* d4 = reinterpret_cast<uint4*>(dst);
-#pragma unroll
-    for (int i = 0; i < 3; i++) d4[i] = make_uint4(h[4 * i], h[4 * i + 1], h[4 * i + 2], h[4 * i + 3]);
+    mg_store_header(L, M, dst, min(ld_cg(&st->n_out), M.inbox_stride - MGR_HDR), 0xFFFFFFFFu);
     dst[40] = k;
   }
   for (uint32_t j = 0; j < RB; j++) {  // (every lane takes part in the shuffles; the lanes that talk to a rank store)
@@ -533,40 +520,18 @@ __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, 
   if (with_flag && q < M.world) st_release_sys(M.flag_data[q] + 16 * M.rank, epoch);  // (own rank included: every block of every rank polls all flags)
 }
 
-// fold the headers of all senders (their messages are complete): OR of the error flags, minima of the capacities
-// (st->g_vals, as mg_kernels.cuh), sums of the per-merge bounds and site counts, the smallest batch
+// fold the headers of all senders (their messages are complete): st->g_vals (mg_fold_headers_warp), sums of the per-merge
+// bounds and site counts, the smallest batch
 __device__ __forceinline__ void mgr_fold_warp(const RoundArgs& R, uint32_t epar) {
   const MgArgs& M = R.mg;
-  DevState* st = R.L.A.st;
   RoundState* rs = R.rs;
   const int q = (int)lane_id();
-  uint32_t w[12];
+  uint32_t kq = (q < M.world) ? (uint32_t)ld_cg(mg_area(M, M.rank, epar, q) + 40) : 0xFFFFFFFFu;
+  const uint32_t n = mg_fold_headers_warp(M, R.L.A.st, epar);
+  if (q < M.world) rs->mg_n[q] = n;
 #pragma unroll
-  for (int i = 0; i < 12; i++) w[i] = (i == H_ERR) ? 0u : 0xFFFFFFFFu;
-  uint32_t kq = 0xFFFFFFFFu;
-  if (q < M.world) {
-    const unsigned long long* hq = mg_area(M, M.rank, epar, q);
-    const uint4* h4 = reinterpret_cast<const uint4*>(hq);
-    const uint4 v0 = ld_cg4(h4), v1 = ld_cg4(h4 + 1), v2 = ld_cg4(h4 + 2);
-    w[0] = v0.x; w[1] = v0.y; w[2] = v0.z; w[3] = v0.w; w[4] = v1.x; w[5] = v1.y; w[6] = v1.z; w[7] = v1.w; w[8] = v2.x; w[9] = v2.y; w[10] = v2.z; w[11] = v2.w;
-    rs->mg_n[q] = w[H_N];
-    kq = (uint32_t)ld_cg(hq + 40);
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-    for (int i = H_ERR; i <= H_CAND_CAP; i++) {
-      const uint32_t other = __shfl_xor_sync(0xFFFFFFFFu, w[i], o);
-      w[i] = (i == H_ERR) ? (w[i] | other) : min(w[i], other);
-    }
-    kq = min(kq, __shfl_xor_sync(0xFFFFFFFFu, kq, o));
-  }
-  if (q == 0) {
-    uint4* g = reinterpret_cast<uint4*>(st->g_vals);
-    g[0] = make_uint4(w[H_ERR], w[H_POOL_FREE], w[H_SITES_CAP], w[H_NEW_CAP]);
-    g[1] = make_uint4(w[H_HOT_CAP], w[H_LEN16_CAP], w[H_TBL_CAP], w[H_CAND_CAP]);
-    rs->mg_k = kq;
-  }
+  for (int o = 16; o > 0; o >>= 1) kq = min(kq, __shfl_xor_sync(0xFFFFFFFFu, kq, o));
+  if (q == 0) rs->mg_k = kq;
   if (q < RB) {  // lane j sums merge j's bounds and sites over the senders
     unsigned long long ul = 0, ur = 0;
     uint32_t nsum = 0;
@@ -585,29 +550,6 @@ __device__ __forceinline__ void mgr_fold_warp(const RoundArgs& R, uint32_t epar)
   }
 }
 
-
-// the hello exchange at the start of a launch: wait for every peer's flag, then fold the headers
-__device__ __forceinline__ void mgr_wait_fold_warp(const RoundArgs& R, uint32_t epar, unsigned long long epoch) {
-  const MgArgs& M = R.mg;
-  DevState* st = R.L.A.st;
-  const int q = (int)lane_id();
-  if (q < M.world) {  // (warp 0 of EVERY block)
-    const unsigned long long* f = M.flag_data[M.rank] + 16 * q;
-    const unsigned long long t0 = now_ns();
-    uint32_t ns = 16;
-    while (ld_acquire_sys(f) < epoch) {
-      __nanosleep(ns);
-      if (ns < 128) ns <<= 1;
-      if (now_ns() - t0 > MG_TIMEOUT_NS) {
-        atomicOr(&st->err, ERR_PEER_TIMEOUT);
-        st->mg_abort = 1;
-        break;
-      }
-    }
-  }
-  __syncwarp();
-  mgr_fold_warp(R, epar);
-}
 
 // X2 of a round: the messages are summed as they complete.  Warp 0 of the block watches the arrival counters of all senders;
 // whenever some are complete (every block of the sender has reported) the whole block adds ITS share of those senders'
@@ -1018,7 +960,11 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
     // hello exchange: headers only (capacities, errors), so that the first decision is taken on global minima
     if (lead) st->mg_abort = 0;
     if (bid == 0 && warp == 0) mgr_send_warp(R, 0, (uint32_t)((mg_epoch + 1) & 1u), 0, mg_epoch + 1, true);
-    if (warp == 0) mgr_wait_fold_warp(R, (uint32_t)((mg_epoch + 1) & 1u), mg_epoch + 1);
+    if (warp == 0) {  // (in EVERY block: wait for every rank's flag, own included, then fold the headers)
+      if (lane < (uint32_t)R.mg.world) mg_wait_flag(R.mg.flag_data[R.mg.rank] + 16 * lane, mg_epoch + 1, now_ns(), 16, 128, st);
+      __syncwarp();
+      mgr_fold_warp(R, (uint32_t)((mg_epoch + 1) & 1u));
+    }
     mg_epoch++;
   }
   RBARRIER();
@@ -1231,77 +1177,17 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       }
       phase_collect(t, A.len16, L.max_length, 1, L.hot, hot_pre, S.cp[0], L.cands, L.cand_cap, st, bid, nblk);
       RBARRIER();
-      unsigned long long tp;
-      uint32_t tie_slot = NOSLOT;
+      uint32_t tie_slot;
       if (!R.mg_on) {
         phase_tie(A.slots, A.n, t, A.pool, L.cands, ld_cg(&st->n_cand), st, S.s_max, bid, nblk);
         RBARRIER();
-        tp = ld_cg(&st->tie_pos);
-        tie_slot = (uint32_t)(tp & 0xFFFFFFFFu);
+        const unsigned long long tp = ld_cg(&st->tie_pos);
+        tie_slot = (tp == ~0ull) ? NOSLOT : (uint32_t)(tp & 0xFFFFFFFFu);
       } else {
-        // sharded: last counted occurrence in GLOBAL scan order = (rank, local position); the candidates go in canonical
-        // (pair key) order so that every rank talks about the same one, and each rank tells every other where ITS last
-        // counted occurrence of each candidate is (mg_kernels.cuh)
-        const MgArgs& M = R.mg;
-        const uint32_t tpar = (uint32_t)((tie_epoch + 1) & 1u);
-        const uint32_t nc = ld_cg(&st->n_cand);  // == mult0 on every rank
-        for (uint32_t i = gt; i < nc; i += gn) {
-          const uint32_t si = ld_cg(&L.cands[i]);
-          const uint32_t ki = t.keys[si];
-          uint32_t r = 0;
-          for (uint32_t j2 = 0; j2 < nc; j2++) r += t.keys[ld_cg(&L.cands[j2])] < ki;
-          M.tie_sorted[r] = si;
-        }
-        RBARRIER();
-        for (uint32_t cnd = bid; cnd < nc; cnd += nblk) {  // one block per candidate
-          const uint32_t sc = ld_cg(&M.tie_sorted[cnd]);
-          const uint32_t key = t.keys[sc];
-          const uint32_t ca = key >> 16, cb = key & 0xFFFFu;
-          const unsigned long long start = t.occ_start.get(sc);
-          const uint32_t len = t.occ_len[sc];
-          uint32_t vmax = 0;
-          for (uint32_t i = tid; i < len; i += blockDim.x) {
-            const uint32_t pp = A.pool[start + i];
-            if (counted_occurrence(A.slots, A.n, pp, ca, cb)) vmax = max(vmax, pp + 1);
-          }
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) vmax = max(vmax, __shfl_xor_sync(0xFFFFFFFFu, vmax, o));
-          __syncthreads();
-          if (lane == 0) S.s_max[warp] = vmax;
-          __syncthreads();
-          if (tid == 0) {
-            uint32_t m = 0;
-            for (uint32_t i = 0; i < (blockDim.x >> 5); i++) m = max(m, S.s_max[i]);
-            for (int q = 0; q < M.world; q++) M.tiebox[q][((size_t)tpar * M.world + M.rank) * M.tie_cap + cnd] = m;
-            __threadfence_system();
-          }
-        }
-        RBARRIER();
-        if (lead) {
-          st->tie_pos = ~0ull;
-          mg_signal_and_wait(M, M.flag_tie, tie_epoch + 1, st);
-        }
-        tie_epoch++;
-        RBARRIER();
-        if (bid == 0) {
-          const uint32_t* box = M.tiebox[M.rank] + (size_t)tpar * M.world * M.tie_cap;
-          for (uint32_t i = tid; i < nc; i += blockDim.x) {
-            for (int q = M.world - 1; q >= 0; q--) {  // the highest rank holding the pair owns its last occurrence
-              const uint32_t vq = ld_cg(box + (size_t)q * M.tie_cap + i);
-              if (vq) {
-                atomicMin(&st->tie_pos, ((((unsigned long long)q << 32) | (vq - 1)) << 16) | i);
-                break;
-              }
-            }
-          }
-        }
-        RBARRIER();
-        tp = ld_cg(&st->tie_pos);
-        if (ld_cg(&st->mg_abort)) tp = ~0ull;
-        if (tp != ~0ull) tie_slot = ld_cg(&M.tie_sorted[(uint32_t)(tp & 0xFFFFu)]);
+        tie_slot = mg_tie_winner(L, R.mg, S.s_max, tie_epoch, [&] { RBARRIER(); });  // (rank, local position) decides
       }
       __syncthreads();
-      if (tp == ~0ull) {
+      if (tie_slot == NOSLOT) {
         status = LOOP_ERROR;
       } else if (tid == 0) {
         const uint32_t s = tie_slot;

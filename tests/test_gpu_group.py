@@ -11,6 +11,17 @@ import pytest
 from bpe_tokenizer_b200 import _abi
 
 SIZES = pytest.mark.parametrize("members", ["2", "up to 4"])
+# every size with the default loop, and again with BPE_LOOP_ROUNDS=0: then k_merge_loop_mg runs every merge, where by default
+# it only takes those above 2^20 global sites, which these corpora never reach
+_LOOPS = [("2", None), ("up to 4", None), ("2", "0"), ("up to 4", "0")]
+SIZES_LOOPS = pytest.mark.parametrize("members,loop_rounds", _LOOPS, ids=[m if r is None else m + "-rounds0" for m, r in _LOOPS])
+
+
+def _set_loop(monkeypatch, loop_rounds):
+    if loop_rounds is None:
+        monkeypatch.delenv("BPE_LOOP_ROUNDS", raising=False)
+    else:
+        monkeypatch.setenv("BPE_LOOP_ROUNDS", loop_rounds)
 
 
 def _devices(members):
@@ -66,17 +77,19 @@ def test_create_group_without_a_device_is_a_cuda_error():
 
 
 @pytest.mark.gpu
-@SIZES
-def test_fuzz_against_literal(members):
+@SIZES_LOOPS
+def test_fuzz_against_literal(members, loop_rounds, monkeypatch):
     """Small alphabets, runs, empty documents, option mixes; every other case adds documents after a mergeUntil (they go to the
-    last member) and merges again."""
+    last member) and merges again.  The small alphabets make position tie-breaks, which each loop kernel must settle."""
     devs = _devices(members)
+    _set_loop(monkeypatch, loop_rounds)
     from bpe_tokenizer_b200 import BPETokenizer
     from oracle import LiteralTokenizer
 
     def docs_of(rng, alphabet):
         return ["".join(rng.choice(alphabet) for _ in range(rng.randint(0, rng.choice([0, 20, 100, 400])))) for _ in range(rng.randint(1, 12))]
 
+    tie_breaks = 0
     for case in range(10):
         rng = random.Random(7100 + case)
         alphabet = "ab" if case % 3 == 0 else "abcde "
@@ -109,7 +122,9 @@ def test_fuzz_against_literal(members):
                 continue
             assert grp.encodeToVector(d) == want
             assert grp.decodeVector(want) == lit.decodeVector(want)
+        tie_breaks += grp.stats()["tie_breaks"]
         grp.close()
+    assert tie_breaks > 0
 
 
 def _zipf_tokenizers(devs, n_bytes):
@@ -136,9 +151,10 @@ def _zipf_tokenizers(devs, n_bytes):
 
 
 @pytest.mark.gpu
-@SIZES
-def test_zipf_1mb_500_merges(members):
+@SIZES_LOOPS
+def test_zipf_1mb_500_merges(members, loop_rounds, monkeypatch):
     devs = _devices(members)
+    _set_loop(monkeypatch, loop_rounds)
     grp, one, orc = _zipf_tokenizers(devs, 1_000_000)
     assert [t.mergeUntil({"max_iterations": 500}) for t in (grp, one, orc)] == [500] * 3
     assert _merges(grp) == _merges(orc) == _merges(one)
