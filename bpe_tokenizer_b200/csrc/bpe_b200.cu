@@ -1407,7 +1407,7 @@ int mg_alloc_mailbox(bpe_engine* e, int rank, int world) {
   e->mg_rank = rank;
   e->mg_world = world;
   // records one rank can send per exchange (k_merge_rounds: the cells of up to 16 merges a round; k_merge_loop_mg: of one merge)
-  e->mg_inbox_stride = 1u << 20;
+  e->mg_inbox_stride = MG_INBOX_STRIDE;
   e->mg_tie_cap = 4096;
   size_t bytes = (size_t)2 * MG_MAX_WORLD * 128 + (size_t)2 * world * e->mg_inbox_stride * 8 + (size_t)2 * world * e->mg_tie_cap * 4;
   CK(cudaMalloc(&e->mg_mailbox, bytes));

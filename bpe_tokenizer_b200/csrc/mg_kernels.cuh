@@ -31,6 +31,10 @@ constexpr uint32_t MG_HDR = 16;  // u64 words of header in front of the records 
 enum { H_N = 0, H_ERR, H_POOL_FREE, H_SITES_CAP, H_NEW_CAP, H_HOT_CAP, H_LEN16_CAP, H_TBL_CAP, H_CAND_CAP, H_STATUS };
 constexpr unsigned long long MG_TIMEOUT_NS = 8000000000ull;
 constexpr uint32_t MG_DIRECT_MAX = 8192;  // merges with at most this many (global) occurrences push their deltas unstaged
+// u64 words of one (parity, sender) message area of an inbox, header included.  k_merge_loop_mg sends at most 2 (c + 1) born-pair
+// records and one per touched pair (< 4 BPE_MAX_TOKENS) per merge; k_merge_rounds bounds the records of a batch when it builds it.
+constexpr uint32_t MG_INBOX_STRIDE = 1u << 20;
+static_assert(2u * ND_STRIDE + 4u * BPE_MAX_TOKENS + 64u + MG_HDR <= MG_INBOX_STRIDE, "one merge of k_merge_loop_mg must fit a message");
 
 struct MgArgs {
   int rank, world;

@@ -85,6 +85,7 @@ __host__ __device__ __forceinline__ uint32_t cell_dec(unsigned long long v) { re
 __host__ __device__ __forceinline__ uint32_t cell_len(unsigned long long v) { return (uint32_t)((v >> R_FIELD) & R_FMASK); }
 __host__ __device__ __forceinline__ uint32_t cell_cnt(unsigned long long v) { return (uint32_t)((v >> (2 * R_FIELD)) & R_FMASK); }
 constexpr uint32_t MGR_HDR = 64;          // sharded: u64 words of header in front of the records of a round's message
+static_assert(2u * ND_STRIDE <= MG_INBOX_STRIDE - MGR_HDR, "the records of a round's first merge always fit a message");
 constexpr uint32_t LOOP_NEED_LEGACY = 7;  // the winner is too big for the packed cells: k_merge_loop takes the merges above R_HUGE
 constexpr uint32_t R_QCAP = 512;         // per-block partial entries a decision can fold (RT x blocks)
 
@@ -1088,6 +1089,9 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           else if (j == 0 && wj > S.gv[2]) cap_fail = LOOP_NEED_HOST;
           else if ((unsigned long long)hot_pre + keys_incl > S.gv[4]) cap_fail = LOOP_NEED_REBUILD;
           else if (cj + 1 > S.gv[5]) cap_fail = LOOP_NEED_HOST;
+          // a rank sends one record per touched cell, at most 2 min(w_i, c_i + 1) per merge: new_keys less 2, so the batch's
+          // records are at most keys_incl - 2 (j + 1), and they must fit this rank's message area in every peer's inbox
+          else if (pj && keys_incl - 2ull * (j + 1u) > (unsigned long long)(R.mg.inbox_stride - MGR_HDR)) cap_fail = LOOP_NEED_HOST;
         } else
         if ((unsigned long long)n_keys + keys_incl > (unsigned long long)(L.tbl_cap >> 1)) cap_fail = LOOP_NEED_HOST;
         else if (pool_cursor + 2ull * w_incl + (unsigned long long)nblk * R_POOL_CHUNK > L.pool_cap) cap_fail = LOOP_NEED_HOST;
