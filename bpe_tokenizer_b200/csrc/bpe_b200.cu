@@ -590,9 +590,6 @@ ApplyArgs apply_args(bpe_engine* e) {
   A.dlt = nullptr;
   A.touched = nullptr;
   A.touched_cap = 0;
-  for (int q = 0; q < 8; q++) A.push[q] = nullptr;
-  A.push_world = 0;
-  A.push_cap = 0;
   return A;
 }
 

@@ -19,7 +19,8 @@
 // BPE_LOOP_ROUNDS=0.  Their record formats differ; the steps every rank must run identically live here once, for both: the
 // header of a message (mg_store_header) and its fold (mg_fold_headers_warp), the wait on a peer's flag (mg_wait_flag) and the
 // tie-break.  Every decision that ends or interrupts the loop is taken from replicated values (or minima over ranks carried in
-// the message headers), so all ranks leave the kernel at the same merge with the same status.  Waits on peers are bounded
+// the message headers: loop_caps_folded), with the stop chain and capacity test every loop kernel shares (loop_stop,
+// loop_cap_status in train_kernels.cuh), so all ranks leave the kernel at the same merge with the same status.  Waits on peers are bounded
 // (MG_TIMEOUT_NS) and abort the loop.
 #pragma once
 #include "train_kernels.cuh"
@@ -30,7 +31,6 @@ constexpr int MG_MAX_WORLD = 8;
 constexpr uint32_t MG_HDR = 16;  // u64 words of header in front of the records of one message
 enum { H_N = 0, H_ERR, H_POOL_FREE, H_SITES_CAP, H_NEW_CAP, H_HOT_CAP, H_LEN16_CAP, H_TBL_CAP, H_CAND_CAP, H_STATUS };
 constexpr unsigned long long MG_TIMEOUT_NS = 8000000000ull;
-constexpr uint32_t MG_DIRECT_MAX = 8192;  // merges with at most this many (global) occurrences push their deltas unstaged
 // u64 words of one (parity, sender) message area of an inbox, header included.  k_merge_loop_mg sends at most 2 (c + 1) born-pair
 // records and one per touched pair (< 4 BPE_MAX_TOKENS) per merge; k_merge_rounds bounds the records of a batch when it builds it.
 constexpr uint32_t MG_INBOX_STRIDE = 1u << 20;
@@ -128,30 +128,31 @@ __device__ __forceinline__ unsigned long long* mg_area(const MgArgs& M, int dst,
 }
 
 // header of a message: 16 u32 (H_* indices) in the first 64 bytes of the area, moved with 128-bit accesses.  This rank's
-// record count, error flags and capacities (H_N .. H_CAND_CAP) into the header at `dst`; the pool figure only gates the next
-// decision.
+// record count, error flags and capacities (its LoopCaps, H_N .. H_CAND_CAP, the pool figure clamped to 32 bits) into the header
+// at `dst`; the pool figure only gates the next decision.
 __device__ __forceinline__ void mg_store_header(const LoopArgs& L, const MgArgs& M, unsigned long long* dst, uint32_t n_rec, uint32_t new_cap) {
   DevState* st = L.A.st;
-  const unsigned long long cur = ld_cg(&st->pool_cursor);
+  const LoopCaps g = loop_caps(L, ld_cg(&st->pool_cursor));
   uint32_t h[12];
 #pragma unroll
   for (int i = 0; i < 12; i++) h[i] = 0;
   h[H_N] = n_rec;
   h[H_ERR] = ld_cg(&st->err);
-  h[H_POOL_FREE] = (uint32_t)min(L.pool_cap > cur ? L.pool_cap - cur : 0ull, 0xFFFFFFFFull);
-  h[H_SITES_CAP] = L.A.sites_cap;
+  h[H_POOL_FREE] = (uint32_t)min(max(g.pool_free, 0ll), 0xFFFFFFFFll);
+  h[H_SITES_CAP] = g.sites_cap;
   h[H_NEW_CAP] = new_cap;
-  h[H_HOT_CAP] = min(L.hot_cap, L.hot_limit);
-  h[H_LEN16_CAP] = L.len16_cap;
-  h[H_TBL_CAP] = L.tbl_cap;
-  h[H_CAND_CAP] = min(L.cand_cap, M.tie_cap);
+  h[H_HOT_CAP] = g.hot_cap;
+  h[H_LEN16_CAP] = g.len16_cap;
+  h[H_TBL_CAP] = g.tbl_cap;
+  h[H_CAND_CAP] = min(g.cand_cap, M.tie_cap);
   uint4* d4 = reinterpret_cast<uint4*>(dst);
 #pragma unroll
   for (int i = 0; i < 3; i++) d4[i] = make_uint4(h[4 * i], h[4 * i + 1], h[4 * i + 2], h[4 * i + 3]);
 }
 
 // One warp, lane q reads sender q's header in this rank's area `par` (the messages are complete): the G headers fold into
-// st->g_vals (OR of the error flags, minima of the capacities), the same values on every rank.  Returns sender q's H_N.
+// st->g_vals (OR of the error flags, minima of the capacities; loop_caps_folded reads them), the same values on every rank.
+// Returns sender q's H_N.
 __device__ __forceinline__ uint32_t mg_fold_headers_warp(const MgArgs& M, DevState* st, uint32_t par) {
   const int q = (int)lane_id();
   uint32_t w[12];
@@ -330,7 +331,6 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
       w = best_merge(w, pb);
     }
     w = best_block_reduce(w, s_best);
-    uint32_t status = LOOP_RUNNING;
     uint32_t wa = 0, wb = 0, wcnt = 0;
     if (w.primary) {
       uint32_t key = t.keys[w.slot];
@@ -339,26 +339,15 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
       wcnt = (uint32_t)(w.primary >> 20);
     }
     const uint32_t c = n_tokens0 + it;
-    const uint4 g0 = ld_cg4(reinterpret_cast<const uint4*>(st->g_vals)), g1 = ld_cg4(reinterpret_cast<const uint4*>(st->g_vals) + 1);
-    const uint32_t g_err = g0.x, g_pool_free = g0.y, g_sites_cap = g0.z, g_new_cap = g0.w, g_hot_cap = g1.x, g_len16_cap = g1.y,
-                   g_tbl_cap = g1.z, g_cand_cap = g1.w;
-    const uint32_t snap_n_keys = ld_cg(&st->snap_n_keys), snap_hot_n = ld_cg(&st->snap_hot_n), aborted = ld_cg(&st->mg_abort);
-    if (aborted || g_err) status = LOOP_ERROR;
-    else if (!w.primary) status = (thresh <= 1) ? LOOP_EMPTY : LOOP_NEED_REBUILD;
-    else if (wcnt < thresh) status = LOOP_NEED_REBUILD;
-    else if (wcnt < L.min_weight) status = LOOP_DONE;  // core.ts:313
-    else if (it >= L.log_cap) status = LOOP_LIMIT;
-    else if (c >= L.max_tokens) status = LOOP_NEED_HOST;
+    const LoopCaps g = loop_caps_folded(st);
+    uint32_t status = loop_stop(L, ld_cg(&st->mg_abort) || g.err, w.primary, wcnt, thresh, it, c);
     if (status == LOOP_RUNNING) {
-      unsigned long long new_keys = min(2ull * wcnt + 2ull, 2ull * (c + 1ull) + 2ull);
-      unsigned long long pool_free = g_pool_free;
-      pool_free = pool_free > 2ull * wcnt_prev ? pool_free - 2ull * wcnt_prev : 0;  // headers are one merge old
-      if ((unsigned long long)snap_n_keys + new_keys > (unsigned long long)(g_tbl_cap >> 1)) status = LOOP_NEED_HOST;
-      else if (2ull * wcnt > pool_free) status = LOOP_NEED_HOST;
-      else if (wcnt > g_sites_cap || new_keys > g_new_cap) status = LOOP_NEED_HOST;
-      else if ((unsigned long long)snap_hot_n + newk_prev + new_keys > g_hot_cap) status = LOOP_NEED_REBUILD;
-      else if (c + 1 > g_len16_cap) status = LOOP_NEED_HOST;
-      else if (w.mult > 1 && w.mult > g_cand_cap) status = LOOP_NEED_HOST;
+      // the headers are one merge old: the pool cells and hot-list entries the previous merge may have taken count against them
+      // (2 wcnt >= 2 min_weight > 0, so this is 2 wcnt tested against the cells left after the previous merge, saturated at 0)
+      const unsigned long long new_keys = min(2ull * wcnt + 2ull, 2ull * (c + 1ull) + 2ull);
+      status = loop_cap_status(g, ld_cg(&st->snap_n_keys), new_keys, 2ull * wcnt + 2ull * wcnt_prev, wcnt,
+                               ld_cg(&st->snap_hot_n) + newk_prev + new_keys, c);
+      if (status == LOOP_RUNNING && w.mult > 1 && w.mult > g.cand_cap) status = LOOP_NEED_HOST;
     }
     MGPROF(0)
     if (status == LOOP_RUNNING && w.mult > 1) {
@@ -376,16 +365,7 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
     }
     MGPROF(11)
     if (status != LOOP_RUNNING) {
-      if (lead) {
-        st->status = status;
-        st->iters_done = it;
-        st->n_tokens = n_tokens0 + it;
-        publish_best(t, st, w);
-        st->n_cand = 0;
-        st->tie_pos = ~0ull;
-        st->mg_epoch = epoch;
-        st->mg_tie_epoch = tie_epoch;
-      }
+      if (lead) loop_exit(t, st, status, it, c, &w, true, epoch, tie_epoch);
       return;
     }
     // ---- P1: local sites, staged count deltas ----
@@ -405,25 +385,13 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
       if (w.mult > 1) st->tie_breaks++;
     }
     const uint32_t epar = (uint32_t)((epoch + 1) & 1u);
-    // small merges: every warp-aggregated delta goes straight into all inboxes (no staging pass, one barrier less);
-    // big merges stage per pair first (a handful of pairs get millions of deltas)
-    const bool direct = wcnt <= MG_DIRECT_MAX;
-    {
-      ApplyArgs Ad = A;
-      if (direct) {
-        for (int q = 0; q < M.world; q++) Ad.push[q] = mg_area(M, q, epar, M.rank) + MG_HDR;
-        Ad.push_world = M.world;
-        Ad.push_cap = M.inbox_stride - MG_HDR;
-      }
-      phase_sites(Ad, wa, wb, c, par, w.slot, bid * blockDim.x + threadIdx.x, nblk * blockDim.x);
-      if (direct) __threadfence_system();
-    }
+    phase_sites(A, wa, wb, c, par, w.slot, gtid, gthreads);
     MGPROF(1)
     GRID_BARRIER();
     MGPROF(2)
-    // ---- M1 (staged mode; small merges pushed everything during P1): the counts of the pairs born by this merge (dense
-    // rows, one record per pair) and one (pair, delta) record per touched pair -- stored into every rank's inbox ----
-    if (!direct) {
+    // ---- M1: the counts of the pairs born by this merge (dense rows, one record per pair) and one (pair, delta) record per
+    // touched pair -- stored into every rank's inbox ----
+    {
       const uint32_t lane = lane_id();
       const uint32_t per_side = c + 1u, total2 = 2u * per_side;
       for (uint32_t i = gtid; i < ((total2 + 31u) & ~31u); i += gthreads) {
@@ -450,7 +418,7 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
         }
       }
     }
-    if (!direct) {
+    {
       const uint32_t nt = min(ld_cg(&st->n_touched[par]), A.touched_cap);
       for (uint32_t i = gtid; i < nt; i += gthreads) {
         uint32_t s = ld_cg(&A.touched[i]);
@@ -465,12 +433,10 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
         for (int q = 0; q < M.world; q++) mg_area(M, q, epar, M.rank)[MG_HDR + k] = rec;
       }
     }
-    if (!direct) {
-      __threadfence_system();
-      MGPROF(3)
-      GRID_BARRIER();
-      MGPROF(4)
-    }
+    __threadfence_system();
+    MGPROF(3)
+    GRID_BARRIER();
+    MGPROF(4)
     // ---- send, then do the LOCAL half of P2 while the peers' messages travel: the pairs born on this shard enter the table
     // (their counts come with the records), the shard is rewritten.  The wait for the peers sits behind that work. ----
     if (bid == 0 && threadIdx.x < 32) mg_send_warp(P, epar, min(ld_cg(&st->n_out), M.inbox_stride - MG_HDR), epoch + 1, M.flag_data);
@@ -491,13 +457,8 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop_mg(Loo
     MGPROF(6)
     GRID_BARRIER();
     if (ld_cg(&st->mg_abort)) {
-      if (lead) {
-        st->status = LOOP_ERROR;
-        st->iters_done = it + 1;  // the local shard was already rewritten for this merge; the engine is unusable after an abort
-        st->n_tokens = n_tokens0 + it + 1;
-        st->mg_epoch = epoch;
-        st->mg_tie_epoch = tie_epoch;
-      }
+      // the local shard was already rewritten for this merge; the engine is unusable after an abort
+      if (lead) loop_exit(t, st, LOOP_ERROR, it + 1, c + 1, nullptr, true, epoch, tie_epoch);
       return;
     }
     // ---- P2 (second half): apply the deltas of all ranks to the replicated counts; the lists of the pairs born on this

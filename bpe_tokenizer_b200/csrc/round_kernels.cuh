@@ -86,7 +86,6 @@ __host__ __device__ __forceinline__ uint32_t cell_len(unsigned long long v) { re
 __host__ __device__ __forceinline__ uint32_t cell_cnt(unsigned long long v) { return (uint32_t)((v >> (2 * R_FIELD)) & R_FMASK); }
 constexpr uint32_t MGR_HDR = 64;          // sharded: u64 words of header in front of the records of a round's message
 static_assert(2u * ND_STRIDE <= MG_INBOX_STRIDE - MGR_HDR, "the records of a round's first merge always fit a message");
-constexpr uint32_t LOOP_NEED_LEGACY = 7;  // the winner is too big for the packed cells: k_merge_loop takes the merges above R_HUGE
 constexpr uint32_t R_QCAP = 512;         // per-block partial entries a decision can fold (RT x blocks)
 
 constexpr uint32_t ERR_ROUND_MISMATCH = 2048u;  // a merge of a round found a different number of sites than its count
@@ -281,9 +280,8 @@ struct RoundSm {
   unsigned long long cp[RB];
   uint32_t cs[RB], cm[RB], ck[RB], cll[RB], clen[RB];
   unsigned long long cls[RB];
-  unsigned long long g_pool_cursor;
+  LoopCaps caps;  // this GPU's, or sharded: the minima over the ranks (loop_caps_folded)
   uint32_t g_n_keys, g_snap_err, g_abort;
-  uint32_t gv[8];  // sharded: the folded header values (OR of the ranks' error flags, minima of their capacities)
   uint32_t ncell[2];  // cells this block touched first in the round of either parity (entries of its list)
   uint32_t nstage;    // staged cells this block touched in the current P1 (entries of r_stage_list)
   uint32_t gncell[2]; // sharded: global cells this block touched first while summing the ranks' records
@@ -1006,10 +1004,12 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       }
       if (tid == 1) S.ncell[par] = 0;  // (the cells the round before last listed were cleared next to the last P1)
       if (tid == 320) S.g_n_keys = ld_cg(&st->n_keys);  // (stable here: they only change in P2)
-      if (tid == 321) S.g_pool_cursor = ld_cg(&st->pool_cursor);
+      if (tid == 321) {
+        S.caps = R.mg_on ? loop_caps_folded(st) : loop_caps(L, ld_cg(&st->pool_cursor));
+        S.caps.new_cap = 0xFFFFFFFFu;  // the rounds keep no list of born pairs (their message headers carry the same)
+      }
       if (tid == 322) S.g_snap_err = ld_cg(&st->snap_err);
       if (tid == 323) S.g_abort = R.mg_on ? ld_cg(&st->mg_abort) : 0u;
-      if (tid >= 324 && tid < 332) S.gv[tid - 324] = R.mg_on ? ld_cg(&st->g_vals[tid - 324]) : 0u;
       if (tid == 2) S.gncell[par] = 0;
       // the list of candidates is exact down to the largest LAST (RT-th best) primary any block published
       const unsigned long long Lcut = block_max_u64((tid % RT == RT - 1) ? myp : 0ull, S.red);  // (syncs inside: qn / cp are visible)
@@ -1055,16 +1055,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         const uint32_t j = lane;
         const unsigned long long p0 = S.cp[0];
         const uint32_t w0 = (uint32_t)(p0 >> 20);
-        const uint32_t n_keys = S.g_n_keys;
-        const unsigned long long pool_cursor = S.g_pool_cursor;
-        uint32_t status = LOOP_RUNNING;
-        if (S.g_snap_err || (R.mg_on && (S.g_abort || S.gv[0]))) status = LOOP_ERROR;
-        else if (!p0) status = (thresh <= 1) ? LOOP_EMPTY : LOOP_NEED_REBUILD;
-        else if (w0 < thresh) status = LOOP_NEED_REBUILD;
-        else if (w0 < L.min_weight) status = LOOP_DONE;  // core.ts:313
-        else if (it >= L.log_cap) status = LOOP_LIMIT;
-        else if (c_first >= L.max_tokens) status = LOOP_NEED_HOST;
-        else if (w0 > R_HUGE) status = LOOP_NEED_LEGACY;
+        uint32_t status = loop_stop(L, S.g_snap_err || S.g_abort || S.caps.err, p0, w0, thresh, it, c_first);
+        if (status == LOOP_RUNNING && w0 > R_HUGE) status = LOOP_NEED_LEGACY;
         const unsigned long long pj = (j < RB) ? S.cp[j] : 0ull;
         const uint32_t wj = (uint32_t)(pj >> 20), key = (j < RB) ? S.ck[j] : 0u;
         const uint32_t aj = key >> 16, bj = key & 0xFFFFu, cj = c_first + j;
@@ -1078,31 +1070,19 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
             w_incl += y;
           }
         }
-        // capacity the host guarantees (k_merge_loop's checks, cumulative over the batch)
-        uint32_t cap_fail = 0;  // 0 fine, else the status it would mean for candidate 0
-        if (R.mg_on) {
-          // sharded: the minima over the ranks that the last exchange carried (so that every rank takes the same decision);
-          // the pool figure is one round old
-          const unsigned long long pool_free = S.gv[1] > mg_prev_alloc ? S.gv[1] - mg_prev_alloc : 0ull;
-          if ((unsigned long long)n_keys + keys_incl > (unsigned long long)(S.gv[6] >> 1)) cap_fail = LOOP_NEED_HOST;
-          else if (2ull * w_incl + (unsigned long long)nblk * R_POOL_CHUNK > pool_free) cap_fail = LOOP_NEED_HOST;
-          else if (j == 0 && wj > S.gv[2]) cap_fail = LOOP_NEED_HOST;
-          else if ((unsigned long long)hot_pre + keys_incl > S.gv[4]) cap_fail = LOOP_NEED_REBUILD;
-          else if (cj + 1 > S.gv[5]) cap_fail = LOOP_NEED_HOST;
-          // a rank sends one record per touched cell, at most 2 min(w_i, c_i + 1) per merge: new_keys less 2, so the batch's
-          // records are at most keys_incl - 2 (j + 1), and they must fit this rank's message area in every peer's inbox
-          else if (pj && keys_incl - 2ull * (j + 1u) > (unsigned long long)(R.mg.inbox_stride - MGR_HDR)) cap_fail = LOOP_NEED_HOST;
-        } else
-        if ((unsigned long long)n_keys + keys_incl > (unsigned long long)(L.tbl_cap >> 1)) cap_fail = LOOP_NEED_HOST;
-        else if (pool_cursor + 2ull * w_incl + (unsigned long long)nblk * R_POOL_CHUNK > L.pool_cap) cap_fail = LOOP_NEED_HOST;
-        else if (j == 0 && wj > A.sites_cap) cap_fail = LOOP_NEED_HOST;
-        else if ((unsigned long long)hot_pre + keys_incl > min(L.hot_cap, L.hot_limit)) cap_fail = LOOP_NEED_REBUILD;
-        else if (cj + 1 > L.len16_cap) cap_fail = LOOP_NEED_HOST;
+        // capacity the host guarantees, cumulative over the batch: 0 (LOOP_RUNNING) fine, else the status it would mean for
+        // candidate 0.  Every block takes each round's list space from the pool in chunks.  Sharded: the headers' pool figure is
+        // one round old, so what the previous round may have taken counts against it (mg_prev_alloc; this need is never 0).
+        uint32_t cap_fail = loop_cap_status(S.caps, S.g_n_keys, keys_incl, 2ull * w_incl + (unsigned long long)nblk * R_POOL_CHUNK + mg_prev_alloc,
+                                            j == 0 ? wj : 0u, (unsigned long long)hot_pre + keys_incl, cj);
+        // sharded: a rank sends one record per touched cell, at most 2 min(w_i, c_i + 1) per merge: new_keys less 2, so the batch's
+        // records are at most keys_incl - 2 (j + 1), and they must fit this rank's message area in every peer's inbox
+        if (!cap_fail && R.mg_on && pj && keys_incl - 2ull * (j + 1u) > (unsigned long long)(R.mg.inbox_stride - MGR_HDR)) cap_fail = LOOP_NEED_HOST;
         const uint32_t mult0 = S.cm[0];
         if (status == LOOP_RUNNING) {
           const uint32_t cf0 = __shfl_sync(0xFFFFFFFFu, cap_fail, 0);
           if (cf0) status = cf0;
-          else if (mult0 > 1 && mult0 > (R.mg_on ? S.gv[7] : L.cand_cap)) status = LOOP_NEED_HOST;
+          else if (mult0 > 1 && mult0 > S.caps.cand_cap) status = LOOP_NEED_HOST;
         }
         // why candidate j >= 1 cannot join (0: it can); same codes as RoundState::stop_reason
         uint32_t stop = 0;
@@ -1215,17 +1195,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       round_fill_all(R, S, F, gt, gn);
       if (F.k) round_clear_cells(R, S, F, tid, blockDim.x, gt, gn);
       if (lead) {
-        st->status = status;
-        st->iters_done = it;
-        st->n_tokens = n_tokens0 + it;
-        if (R.mg_on) {
-          st->mg_epoch = mg_epoch;
-          st->mg_tie_epoch = tie_epoch;
-        }
-        Best wb{S.cp[0], S.cp[0] ? S.cs[0] : NOSLOT, S.cm[0]};
-        publish_best(t, st, wb);
-        st->n_cand = 0;
-        st->tie_pos = ~0ull;
+        const Best wb{S.cp[0], S.cp[0] ? S.cs[0] : NOSLOT, S.cm[0]};
+        loop_exit(t, st, status, it, c_first, &wb, R.mg_on, mg_epoch, tie_epoch);
       }
       return;
     }
@@ -1317,13 +1288,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       XPROF(1)
       mg_epoch++;
       if (ld_cg(&st->mg_abort)) {  // a peer did not answer: every block of every rank that still runs leaves
-        if (lead) {
-          st->status = LOOP_ERROR;
-          st->iters_done = it;
-          st->n_tokens = n_tokens0 + it;
-          st->mg_epoch = mg_epoch;
-          st->mg_tie_epoch = tie_epoch;
-        }
+        if (lead) loop_exit(t, st, LOOP_ERROR, it, c_first, nullptr, true, mg_epoch, tie_epoch);
         return;
       }
       RBARRIER();

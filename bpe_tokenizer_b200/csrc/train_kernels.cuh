@@ -70,8 +70,9 @@ struct DevState {
   unsigned long long bucket_ns[32][4];  // BPE_FINE_PROF: per log2(weight) bucket: P1, P2, P3 work (block 0), merges
 };
 
+// LOOP_NEED_LEGACY: the winner is too big for the packed cells of k_merge_rounds, k_merge_loop takes the merges above R_HUGE
 constexpr uint32_t LOOP_RUNNING = 0, LOOP_DONE = 1, LOOP_NEED_REBUILD = 2, LOOP_NEED_HOST = 3, LOOP_EMPTY = 4,
-                   LOOP_ERROR = 5, LOOP_LIMIT = 6;
+                   LOOP_ERROR = 5, LOOP_LIMIT = 6, LOOP_NEED_LEGACY = 7;
 
 struct SiteRec {
   uint32_t p;      // position of the `a` being merged
@@ -696,10 +697,6 @@ struct ApplyArgs {
   // pair is listed by whoever inserts its key -- phase_new_pairs for pairs born on this shard, the record pass otherwise
   uint32_t* newpair;
   uint32_t newpair_cap;
-  // sharded training, small merges: every (pair, delta) goes straight into the record area of each rank's inbox
-  unsigned long long* push[8];
-  int push_world;  // 0: staged mode (or single GPU)
-  uint32_t push_cap;
 };
 
 constexpr uint32_t ND_STRIDE = 56320;  // >= BPE_MAX_TOKENS + 1
@@ -735,27 +732,10 @@ __device__ __forceinline__ void prefetch_pair(const PairTable& t, uint32_t key) 
 }
 
 // Count deltas, warp-collective (all 32 lanes call; `has` lanes carry one delta of pair slot s): applied to the table
-// (single GPU), pushed into every rank's inbox (sharded, small merges) or staged per pair (sharded, big merges).
-// Counters shared by the whole grid (n_out, n_touched) get ONE atomic per warp.
-__device__ __forceinline__ void cnt_delta_warp(const ApplyArgs& A, bool has, uint32_t s, uint32_t key, int32_t d, uint32_t par) {
+// (single GPU) or staged per pair (sharded).  The grid-wide n_touched counter gets ONE atomic per warp.
+__device__ __forceinline__ void cnt_delta_warp(const ApplyArgs& A, bool has, uint32_t s, int32_t d, uint32_t par) {
   const uint32_t lane = lane_id();
-  if (A.push_world) {
-    uint32_t m = __ballot_sync(0xFFFFFFFFu, has);
-    if (!m) return;
-    uint32_t base = 0;
-    int src = __ffs(m) - 1;
-    if ((int)lane == src) base = atomicAdd(&A.st->n_out, (uint32_t)__popc(m));
-    base = __shfl_sync(0xFFFFFFFFu, base, src);
-    if (has) {
-      uint32_t k = base + __popc(m & ((1u << lane) - 1u));
-      if (k < A.push_cap) {
-        unsigned long long rec = ((unsigned long long)key << 32) | (uint32_t)d;
-        for (int q = 0; q < A.push_world; q++) A.push[q][k] = rec;
-      } else {
-        atomicOr(&A.st->err, ERR_INBOX_OVERFLOW);
-      }
-    }
-  } else if (A.dlt) {
+  if (A.dlt) {
     bool first = has && atomicAdd(A.dlt + s, d) == 0;  // first delta of this pair in this merge (deltas of a pair share a sign)
     uint32_t m = __ballot_sync(0xFFFFFFFFu, first);
     if (!m) return;
@@ -785,7 +765,7 @@ __device__ __forceinline__ void agg_dec(const ApplyArgs& A, uint32_t key, bool h
     s = tbl_find(t, key);
     if (s == NOSLOT) atomicOr(&A.st->err, ERR_MISSING_KEY);
   }
-  cnt_delta_warp(A, leader && s != NOSLOT, s, key, -(int32_t)__popc(peers), par);
+  cnt_delta_warp(A, leader && s != NOSLOT, s, -(int32_t)__popc(peers), par);
 }
 
 // Two decrements at once: both first probes are issued before either is consumed (one DRAM round trip instead of two).
@@ -822,15 +802,15 @@ __device__ __forceinline__ void agg_dec2(const ApplyArgs& A, uint32_t key1, bool
     s2 = (k2 == key2) ? h2 : (k2 == EMPTY_KEY ? NOSLOT : tbl_find(t, key2));
     if (s2 == NOSLOT) atomicOr(&A.st->err, ERR_MISSING_KEY);
   }
-  cnt_delta_warp(A, lead1 && s1 != NOSLOT, s1, key1, -(int32_t)__popc(peers1), par);
-  cnt_delta_warp(A, lead2 && s2 != NOSLOT, s2, key2, -(int32_t)__popc(peers2), par);
+  cnt_delta_warp(A, lead1 && s1 != NOSLOT, s1, -(int32_t)__popc(peers1), par);
+  cnt_delta_warp(A, lead2 && s2 != NOSLOT, s2, -(int32_t)__popc(peers2), par);
 }
 
 // One adjacency of a pair BORN by this merge -- (tok, c) for side 0, (c, tok) for side 1 -- per `has` lane: occurrences
 // and counted occurrences go to the dense rows with fire-and-forget atomics (one per distinct token per warp), or, with
 // `stage` and tok below R_STAGE_T, to the block's staged copy of those rows (single GPU only: see phase_sites).
-__device__ __forceinline__ void agg_new_dense(const ApplyArgs& A, uint32_t side, uint32_t tok, uint32_t c, bool has, bool counted,
-                                              uint32_t par, uint32_t* stage = nullptr) {
+__device__ __forceinline__ void agg_new_dense(const ApplyArgs& A, uint32_t side, uint32_t tok, bool has, bool counted,
+                                              uint32_t* stage = nullptr) {
   uint32_t lane = lane_id();
   uint32_t k = has ? tok : (0xFFFFFF00u + lane);
   uint32_t peers = __match_any_sync(0xFFFFFFFFu, k);
@@ -846,18 +826,16 @@ __device__ __forceinline__ void agg_new_dense(const ApplyArgs& A, uint32_t side,
     } else {
       uint32_t* row = A.nd + (size_t)(side ? ND_R_LEN : ND_L_LEN) * ND_STRIDE;
       atomicAdd(row + tok, (uint32_t)__popc(peers));
-      if (nc && !A.push_world) atomicAdd(row + ND_STRIDE + tok, nc);
+      if (nc) atomicAdd(row + ND_STRIDE + tok, nc);
     }
   }
-  // sharded, small merges: the count goes straight to every rank's inbox (partial counts per warp add up on arrival)
-  if (A.push_world) cnt_delta_warp(A, nc != 0, NOSLOT, side ? pair_key(c, tok) : pair_key(tok, c), (int32_t)nc, par);
 }
 
 // vt / nvt: virtual thread id and count (whole warps), so that a loop kernel can give the phase a subset of its warps;
 // site_buf: where the site records go (the loop kernel alternates between two buffers), A.sites when null.
 // stage: the block's staged rows ([LS_ROWS][R_STAGE_T] u32 in shared memory, zero) when every thread of the block runs the phase
-// and the merge stages; loop_flush_stage must then follow, with every thread of the block.  Single GPU only (A.push_world == 0,
-// A.dlt == nullptr, as in k_merge_loop): the staged words go to nd and the table counts, not to an inbox or the touched list.
+// and the merge stages; loop_flush_stage must then follow, with every thread of the block.  Single GPU only (A.dlt == nullptr,
+// as in k_merge_loop): the staged words go to nd and the table counts, not to the touched list.
 __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint32_t b, uint32_t c, uint32_t par,
                                             uint32_t pair_slot, uint32_t vt, uint32_t nvt, SiteRec* site_buf = nullptr,
                                             uint32_t* stage = nullptr) {
@@ -963,7 +941,7 @@ __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint
     }
     FINE(2, (uint32_t)dec1_key + new1_tok)
     FINE(3, 0)
-    agg_new_dense(A, 0, new1_tok, c, new1, new1_counted, par, stage);
+    agg_new_dense(A, 0, new1_tok, new1, new1_counted, stage);
     rec.lslot = new1 ? new1_tok : NOTOKV;  // resolved to the pair's table slot by phase_apply (ND_L_SLOT)
     FINE(4, rec.lslot)
 
@@ -996,7 +974,7 @@ __device__ __forceinline__ void phase_sites(const ApplyArgs& A, uint32_t a, uint
     FINE(5, (uint32_t)dec2_key + new2_tok)
     agg_dec2(A, dec1_key, dec1, dec2_key, dec2, par, stage);
     FINE(6, 0)
-    agg_new_dense(A, 1, new2_tok, c, new2, true, par, stage);
+    agg_new_dense(A, 1, new2_tok, new2, true, stage);
     rec.rslot = new2 ? new2_tok : NOTOKV;
     FINE(7, rec.rslot)
 
@@ -1312,6 +1290,68 @@ struct LoopArgs {
                        // k_merge_loop and k_merge_rounds, BPE_BLOCK_CELLS_MIN_SITES
 };
 
+// The capacities the host guarantees a launch, in the order of a message header's H_ERR .. H_CAND_CAP (mg_kernels.cuh) and of
+// DevState::g_vals: one GPU's own (loop_caps) or, on a sharded corpus, the minima over the ranks that the last exchange carried
+// (loop_caps_folded), so that every rank takes the same decision.  loop_cap_status tests a merge against them.
+struct LoopCaps {
+  uint32_t err;        // error flags: OR over the ranks (loop_caps leaves 0; the header writer adds this GPU's)
+  long long pool_free; // occurrence-pool cells left; negative once a failed allocation has moved the cursor past the pool
+  uint32_t sites_cap, new_cap, hot_cap, len16_cap, tbl_cap, cand_cap;
+};
+
+__device__ __forceinline__ LoopCaps loop_caps(const LoopArgs& L, unsigned long long pool_cursor) {
+  return LoopCaps{0u, (long long)L.pool_cap - (long long)pool_cursor, L.A.sites_cap, L.A.new_cap, min(L.hot_cap, L.hot_limit),
+                  L.len16_cap, L.tbl_cap, L.cand_cap};
+}
+
+__device__ __forceinline__ LoopCaps loop_caps_folded(const DevState* st) {
+  const uint4 g0 = ld_cg4(reinterpret_cast<const uint4*>(st->g_vals)), g1 = ld_cg4(reinterpret_cast<const uint4*>(st->g_vals) + 1);
+  return LoopCaps{g0.x, (long long)g0.y, g0.z, g0.w, g1.x, g1.y, g1.z, g1.w};
+}
+
+// The stop chain every decision starts with: an error, no pair left, the winner (count w) below the hot-list threshold, below
+// min_weight, the launch's log full, the token table full.  `primary` is the winner's, 0 for none.
+__device__ __forceinline__ uint32_t loop_stop(const LoopArgs& L, bool err, unsigned long long primary, uint32_t w, uint32_t thresh,
+                                              uint32_t it, uint32_t c) {
+  if (err) return LOOP_ERROR;
+  if (!primary) return (thresh <= 1) ? LOOP_EMPTY : LOOP_NEED_REBUILD;
+  if (w < thresh) return LOOP_NEED_REBUILD;
+  if (w < L.min_weight) return LOOP_DONE;  // core.ts:313
+  if (it >= L.log_cap) return LOOP_LIMIT;
+  if (c >= L.max_tokens) return LOOP_NEED_HOST;
+  return LOOP_RUNNING;
+}
+
+// The capacity the host guarantees (grow_merge_buffers makes room for what fails here), for a merge (or a batch of merges)
+// creating token c: new pairs are (x,c) or (c,y), so at most 2*(c+1) of them and at most 2 per site (new_keys); new list cells
+// <= 2 per site.  The caller's own figures: pool_need cells of the pool, `sites` into the site buffer, hot_need hot-list
+// entries once the new pairs have joined (0: the merge does not feed the hot list).  The first failing status, or LOOP_RUNNING.
+__device__ __forceinline__ uint32_t loop_cap_status(const LoopCaps& g, uint32_t n_keys, unsigned long long new_keys,
+                                                    unsigned long long pool_need, uint32_t sites, unsigned long long hot_need, uint32_t c) {
+  if ((unsigned long long)n_keys + new_keys > (unsigned long long)(g.tbl_cap >> 1)) return LOOP_NEED_HOST;
+  if ((long long)pool_need > g.pool_free) return LOOP_NEED_HOST;
+  if (sites > g.sites_cap || new_keys > g.new_cap) return LOOP_NEED_HOST;
+  if (hot_need > g.hot_cap) return LOOP_NEED_REBUILD;
+  if (c + 1 > g.len16_cap) return LOOP_NEED_HOST;
+  return LOOP_RUNNING;
+}
+
+// Thread 0 of block 0, leaving the loop: the exit record the host reads.  w: the winner the loop stopped at (grow_merge_buffers
+// sizes for it), nullptr when the caller publishes none.  A sharded loop also leaves the exchange epochs the next launch continues from.
+__device__ __forceinline__ void loop_exit(const PairTable& t, DevState* st, uint32_t status, uint32_t iters, uint32_t n_tokens,
+                                          const Best* w, bool mg = false, unsigned long long epoch = 0, unsigned long long tie_epoch = 0) {
+  st->status = status;
+  st->iters_done = iters;
+  st->n_tokens = n_tokens;
+  if (w) publish_best(t, st, *w);
+  st->n_cand = 0;
+  st->tie_pos = ~0ull;
+  if (mg) {
+    st->mg_epoch = epoch;
+    st->mg_tie_epoch = tie_epoch;
+  }
+}
+
 // Grid barrier for the co-resident (cooperative) launch.  The arrival counter lives in its own 128-byte line, away
 // from the DevState counters the phases hit with atomics, and pollers back off so that they do not saturate the
 // L2 slice that owns it.
@@ -1469,13 +1509,9 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopAr
         wcnt = (uint32_t)(w.primary >> 20);
       }
     }
-    if (ld_cg(&st->snap_err)) status = LOOP_ERROR;
-    else if (replay) status = (it >= L.log_cap) ? LOOP_LIMIT : (c >= L.max_tokens ? LOOP_NEED_HOST : LOOP_RUNNING);
-    else if (!w.primary) status = (thresh <= 1) ? LOOP_EMPTY : LOOP_NEED_REBUILD;
-    else if (wcnt < thresh) status = LOOP_NEED_REBUILD;
-    else if (wcnt < L.min_weight) status = LOOP_DONE;  // core.ts:313
-    else if (it >= L.log_cap) status = LOOP_LIMIT;
-    else if (c >= L.max_tokens) status = LOOP_NEED_HOST;
+    if (!replay) status = loop_stop(L, ld_cg(&st->snap_err) != 0, w.primary, wcnt, thresh, it, c);
+    else if (ld_cg(&st->snap_err)) status = LOOP_ERROR;
+    else status = (it >= L.log_cap) ? LOOP_LIMIT : (c >= L.max_tokens ? LOOP_NEED_HOST : LOOP_RUNNING);
     PROF(0)
     if (status == LOOP_RUNNING && w.mult > 1) {
       // tie on (weight, a.index+b.index): the pair whose last counted occurrence comes first wins (core.ts:294-305)
@@ -1503,30 +1539,19 @@ __global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopAr
     }
     PROF(7)
     if (status == LOOP_RUNNING) {
-      // capacity the host guarantees: sites = wcnt; new pairs are (x,c) or (c,y), so at most 2*(c+1) of them and
-      // at most 2 per site; new list cells <= 2 per site
-      unsigned long long new_keys = min(2ull * wcnt + 2ull, 2ull * (c + 1ull) + 2ull);
-      if ((unsigned long long)ld_cg(&st->n_keys) + new_keys > (unsigned long long)(L.tbl_cap >> 1)) status = LOOP_NEED_HOST;
-      else if ((unsigned long long)ld_cg(&st->pool_cursor) + 2ull * wcnt > L.pool_cap) status = LOOP_NEED_HOST;
-      else if (wcnt > A.sites_cap || new_keys > A.new_cap) status = LOOP_NEED_HOST;
-      else if (!replay && (unsigned long long)hot_pre + new_keys > min(L.hot_cap, L.hot_limit)) status = LOOP_NEED_REBUILD;
-      else if (c + 1 > L.len16_cap) status = LOOP_NEED_HOST;
+      const unsigned long long new_keys = min(2ull * wcnt + 2ull, 2ull * (c + 1ull) + 2ull);
+      status = loop_cap_status(loop_caps(L, ld_cg(&st->pool_cursor)), ld_cg(&st->n_keys), new_keys, 2ull * wcnt, wcnt,
+                               replay ? 0ull : hot_pre + new_keys, c);  // (replayed merges do not feed the hot list)
     }
     if (status != LOOP_RUNNING) {
       if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);  // the kernel leaves every list complete
       if (bid == 0 && threadIdx.x == 0) {
-        st->status = status;
-        st->iters_done = it;
-        st->n_tokens = n_tokens0 + it;
+        loop_exit(t, st, status, it, c, replay ? nullptr : &w);
         if (replay) {
           st->best_primary = 0;
           st->best_cnt = wcnt;  // what the host must make room for
           st->best_mult = 1;
-        } else {
-          publish_best(t, st, w);
         }
-        st->n_cand = 0;
-        st->tie_pos = ~0ull;
       }
       return;
     }
