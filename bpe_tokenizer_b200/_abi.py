@@ -75,6 +75,8 @@ SYMBOLS = {
     "bpe_debug_lane_table": (C.c_int, [i32p, C.c_int64, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, C.c_int64, i64p]),
     "bpe_debug_plan_chunks": (C.c_int, [i64p, C.c_int64, C.c_int64, i64p, C.c_int64, i64p, i64p]),
     "bpe_encode_text_batch": (C.c_int, [vp, u8p, i64p, C.c_int64, i32p, C.c_int32, i32p, C.c_int64, i64p, i64p, i64p, i64p, i32p]),
+    "bpe_encode_text_batch_dev": (C.c_int, [vp, vp, C.c_int64, vp, C.c_int64, vp, C.c_int32, vp, vp, vp, i64p, i64p, i32p]),
+    "bpe_pad_batch_dev": (C.c_int, [vp, vp, vp, C.c_int64, C.c_int64, C.c_int32, vp, vp]),
     "bpe_mg_init": (C.c_int, [vp, C.c_int, C.c_int, vp]),
     "bpe_mg_connect": (C.c_int, [vp, C.c_char_p]),
     "bpe_mg_state": (C.c_int, [vp, C.POINTER(C.c_int)]),

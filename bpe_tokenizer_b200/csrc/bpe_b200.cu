@@ -3014,6 +3014,73 @@ int bpe_encode_text_batch(bpe_engine* e, const uint8_t* utf8, const int64_t* doc
                      unknown_code_point);
 }
 
+int bpe_encode_text_batch_dev(bpe_engine* e, const uint8_t* dev_utf8, int64_t n_bytes, const int64_t* dev_doc_byte_offsets, int64_t n_docs,
+                              const int32_t* dev_to_vector_index, int32_t n_tvi, int32_t* dev_out, int64_t* dev_out_offsets, int64_t* dev_first_bad,
+                              int64_t* n_out, int64_t* unknown_pos, int32_t* unknown_code_point) {
+  if (!e || !n_out || n_docs < 0 || n_bytes < 0 || !dev_doc_byte_offsets || !dev_out_offsets || (n_bytes > 0 && (!dev_utf8 || !dev_out)) ||
+      (dev_to_vector_index && n_tvi < 0))
+    return fail(e, BPE_E_INVALID, "bad encode arguments");
+  *n_out = 0;
+  if (unknown_pos) *unknown_pos = -1;
+  GROUP_REFUSES(e, "bpe_encode_text_batch_dev (device pointers belong to one device)");
+  CK(cudaSetDevice(e->device));
+  e->txt_staged = false;  // x_ids is about to be reused
+  TRY(ensure_cpmap(e));
+  CK(e->x_flag.reserve(8));
+  // the offsets live in the caller's device memory: check them there, before any kernel reads the text through them
+  unsigned long long chk[3] = {0, 0, 0};
+  CK(cudaMemsetAsync(e->x_flag.p + 6, 0, 8, e->stream));
+  k_check_byte_offsets<<<(int)std::min<int64_t>((n_docs + 256) / 256, (int64_t)e->grid(4)), 256, 0, e->stream>>>(dev_doc_byte_offsets, n_docs, n_bytes,
+                                                                                                                 e->x_flag.p + 4);
+  CKL();
+  CK(cudaMemcpyAsync(chk, e->x_flag.p + 4, sizeof chk, cudaMemcpyDeviceToHost, e->stream));
+  CK(cudaStreamSynchronize(e->stream));
+  if (chk[2]) return fail(e, BPE_E_INVALID, "document offsets must be non-decreasing and lie inside the text (0 .. %lld)", (long long)n_bytes);
+  const int64_t base = (int64_t)chk[0], nbytes = (int64_t)chk[1] - base;
+  if ((uint64_t)nbytes >= 0xFFFFFFF0ull) return fail(e, BPE_E_DOMAIN, "text batch too large for one call");
+  if (n_docs == 0) {
+    CK(cudaMemsetAsync(dev_out_offsets, 0, 8, e->stream));
+    return BPE_OK;
+  }
+  const int64_t* d_byte_off = dev_doc_byte_offsets;  // text_decode_dev wants offsets relative to the first document
+  if (base) {
+    CK(e->x_ooff.reserve((size_t)n_docs + 1));
+    CK(cudaMemcpyAsync(e->x_ooff.p, dev_doc_byte_offsets, (size_t)(n_docs + 1) * 8, cudaMemcpyDeviceToDevice, e->stream));
+    k_shift_i64<<<(int)std::min<int64_t>((n_docs + 256) / 256, (int64_t)e->grid(4)), 256, 0, e->stream>>>(e->x_ooff.p, n_docs + 1, -base);
+    CKL();
+    d_byte_off = e->x_ooff.p;
+  }
+  CK(e->x_ids.reserve((size_t)std::max<int64_t>(nbytes, 1)));  // at most one code point per byte
+  CK(e->x_off.reserve((size_t)n_docs + 1));
+  TRY(text_decode_dev(e, dev_utf8 + base, nbytes, d_byte_off, n_docs, e->x_ids.p, e->x_off.p, false, e->x_flag.p));
+  // the lane width of encode_dev depends on the longest document, so the decode's flags come back before the encode starts
+  unsigned long long fl[3];
+  CK(cudaMemcpyAsync(fl, e->x_flag.p, sizeof fl, cudaMemcpyDeviceToHost, e->stream));
+  CK(cudaStreamSynchronize(e->stream));
+  if (fl[0] != ~0ull) {  // encodeToCode throws at the first unknown character (core.ts:398-400)
+    const int64_t pos = (int64_t)(fl[0] >> 32);
+    if (unknown_pos) *unknown_pos = pos;
+    if (unknown_code_point) *unknown_code_point = (int32_t)(fl[0] & 0xFFFFFFFFu);
+    return fail(e, BPE_E_INVALID, "unknown token, char: U+%04X at code point %lld", (unsigned)(fl[0] & 0xFFFFFFFFu), (long long)pos);
+  }
+  return encode_dev(e, e->x_scratch, e->x_ids.p, e->x_off.p, n_docs, (int64_t)fl[2], (int64_t)fl[1], dev_to_vector_index, n_tvi, dev_out, dev_out_offsets,
+                    dev_first_bad, n_out);
+}
+
+int bpe_pad_batch_dev(bpe_engine* e, const int32_t* dev_values, const int64_t* dev_offsets, int64_t n_docs, int64_t width, int32_t pad_value,
+                      int32_t* dev_out, int64_t* dev_lengths) {
+  if (!e || n_docs < 0 || width < 0 || (n_docs > 0 && (!dev_offsets || (width > 0 && (!dev_values || !dev_out)))))
+    return fail(e, BPE_E_INVALID, "bad pad arguments");
+  if (n_docs > 0 && width > INT64_MAX / n_docs) return fail(e, BPE_E_DOMAIN, "%lld rows of %lld values overflow", (long long)n_docs, (long long)width);
+  GROUP_REFUSES(e, "bpe_pad_batch_dev (device pointers belong to one device)");
+  CK(cudaSetDevice(e->device));
+  if (n_docs == 0) return BPE_OK;
+  k_pad_rows<<<(int)std::min<int64_t>((n_docs + 7) / 8, (int64_t)e->grid(16)), 256, 0, e->stream>>>(dev_values, dev_offsets, n_docs, width, pad_value, dev_out,
+                                                                                                      dev_lengths);
+  CKL();
+  return BPE_OK;
+}
+
 int bpe_debug_lane_table(const int32_t* abc, int64_t n_merges, int32_t n_tokens, int32_t* a, int32_t* b, int32_t* rank, int32_t* c,
                          int32_t* right_spine_bound, int32_t* left_spine_bound, int64_t cap, int64_t* n) {
   if (n_merges < 0 || (n_merges > 0 && !abc) || !n) return BPE_E_INVALID;

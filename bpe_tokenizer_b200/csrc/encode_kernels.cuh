@@ -252,6 +252,23 @@ __global__ void __launch_bounds__(128) k_gather_map(const int32_t* __restrict__ 
   }
 }
 
+// Ragged -> dense (bpe_pad_batch_dev): row d of out[n_docs x width] = the first min(len_d, width) values of document d, then
+// `pad`.  One warp per row: the warp's loads and stores are 32 consecutive values, and the pad tail goes out in the same pass.
+__global__ void __launch_bounds__(256) k_pad_rows(const int32_t* __restrict__ values, const int64_t* __restrict__ off, int64_t n_docs,
+                                                  int64_t width, int32_t pad, int32_t* __restrict__ out, int64_t* __restrict__ lengths) {
+  const uint32_t lane = threadIdx.x & 31;
+  const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t d = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; d < n_docs; d += nw) {
+    const int64_t s = off[d];
+    const int64_t len = max((int64_t)0, min(off[d + 1] - s, width));
+    const int32_t* src = values + s;
+    int32_t* dst = out + d * width;
+#pragma unroll 4
+    for (int64_t j = lane; j < width; j += 32) dst[j] = (j < len) ? __ldg(src + j) : pad;
+    if (lengths && lane == 0) lengths[d] = len;
+  }
+}
+
 // ---- exclusive scan of the per-document token counts (u32 -> u64 offsets), three launches: tile sums, scan of the
 // tile sums (k_scan_counts, one block), tile-local scan + tile offset ----
 constexpr int SC_THREADS = 256, SC_ITEMS = 16, SC_TILE = SC_THREADS * SC_ITEMS;

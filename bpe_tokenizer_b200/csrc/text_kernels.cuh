@@ -118,6 +118,19 @@ __global__ void k_shift_i64(int64_t* __restrict__ p, int64_t n, int64_t delta) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) p[i] += delta;
 }
 
+// The caller's device offsets of bpe_encode_text_batch_dev, checked before anything reads through them: res[0] = off[0],
+// res[1] = off[n_docs], res[2] != 0 when an offset lies outside [0, n_bytes] or one decreases (res[2] is zeroed before; every
+// offender stores the same value, so no atomic is needed)
+__global__ void k_check_byte_offsets(const int64_t* __restrict__ off, int64_t n_docs, int64_t n_bytes, unsigned long long* __restrict__ res) {
+  int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i <= n_docs; i += stride) {
+    const int64_t v = off[i];
+    if (v < 0 || v > n_bytes || (i < n_docs && off[i + 1] < v)) res[2] = 1;
+    if (i == 0) res[0] = (unsigned long long)v;
+    if (i == n_docs) res[1] = (unsigned long long)v;
+  }
+}
+
 // *out = max(*out, max of in[0..n))
 __global__ void k_max_u32(const uint32_t* __restrict__ in, int64_t n, unsigned long long* __restrict__ out) {
   uint32_t m = 0;

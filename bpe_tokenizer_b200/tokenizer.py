@@ -25,6 +25,8 @@ EOF = chr(4)
 LF = "\n"
 CR = "\r"
 
+_CUDA_STREAM_LEGACY = 1  # cudaStreamLegacy: the legacy default stream, which torch's default stream is (handle 0)
+
 _JS_WS = (
     "\t\n\x0b\x0c\r \xa0\u1680\u2000\u2001\u2002\u2003\u2004\u2005\u2006\u2007\u2008\u2009\u200a"
     "\u2028\u2029\u202f\u205f\u3000\ufeff"
@@ -130,6 +132,7 @@ class BPETokenizer:
             raise BpeError(rc, "cannot create the CUDA engine (no usable device, or GPUs without peer access? there is no CPU fallback)")
         self._h = h
         self._device = device
+        self._stream = 0  # the stream set_stream gave the engine (0: its own); the C ABI has no getter
         self._reset_host()
 
     # ---- plumbing -------------------------------------------------------------------------
@@ -143,6 +146,7 @@ class BPETokenizer:
         self.from_vector_index: Optional[Dict[int, int]] = None  # core.ts:103
         self._pending: List[np.ndarray] = []  # documents added on the host, not yet uploaded
         self._tvi_dev: Optional[np.ndarray] = None
+        self._tvi_cuda = None  # _tvi_dev as a CUDA tensor on the engine's device (encodeTextTensor)
         self._chars_synced = -1  # entries of char_to_token the engine's character table holds (-1: never pushed)
 
     def __del__(self):
@@ -192,6 +196,7 @@ class BPETokenizer:
     def set_stream(self, cuda_stream: int) -> None:
         """Run the engine on an existing CUDA stream (e.g. ``torch.cuda.current_stream().cuda_stream``)."""
         self._check(self._lib.bpe_set_stream(self._h, C.c_void_p(cuda_stream)))
+        self._stream = cuda_stream or 0
 
     def stats(self) -> dict:
         s = bpe_stats()
@@ -242,6 +247,7 @@ class BPETokenizer:
         self.to_vector_index = None
         self.from_vector_index = None
         self._tvi_dev = None
+        self._tvi_cuda = None
 
     # ---- corpus -----------------------------------------------------------------------------
     def _char_ids(self, content: str, create: bool) -> np.ndarray:
@@ -357,6 +363,97 @@ class BPETokenizer:
         self._check(rc)
         return out[: n.value], out_off, bad[:n_docs]
 
+    def encodeTextTensor(self, texts, doc_byte_offsets=None, *, vector: bool = True, pad_to=None, pad_value: int = -1):
+        """encodeTextBatch into CUDA tensors on the engine's device, for a model that consumes the vectors there.
+        `texts`: a sequence of str (UTF-8 with lone surrogates as 'surrogatepass' writes them), bytes with host offsets, or a
+        torch.uint8 CUDA tensor with an int64 CUDA offsets tensor (both on the engine's device; they are read in place).
+        -> (values int32[N], offsets int64[B+1]) when pad_to is None, else (ids int32[B, L], lengths int64[B]) with
+        L = pad_to, or the longest document for pad_to="longest"; longer documents are cut on the right and the rest of a
+        row holds pad_value.  Raises as encodeTextBatch (unknown character) and, with vector=True, as encodeToVector at the
+        first hole in document order.  The work runs on torch.cuda.current_stream() of the engine's device and is complete
+        when the call returns; the engine's own stream setting is restored afterwards."""
+        import torch
+
+        self._flush()
+        self._sync_chars()
+        dev = torch.device("cuda", self._device)
+        if pad_to is not None and not (isinstance(pad_to, str) and pad_to == "longest"):
+            if isinstance(pad_to, (bool, str, float)) or not hasattr(pad_to, "__index__") or pad_to.__index__() < 0:
+                raise ValueError('pad_to must be None, "longest" or an int >= 0, got %r' % (pad_to,))
+            pad_to = pad_to.__index__()
+        if isinstance(texts, str):
+            raise ValueError("texts must be a sequence of str (one per document), not one str")
+        if isinstance(texts, torch.Tensor):
+            if not isinstance(doc_byte_offsets, torch.Tensor):
+                raise ValueError("a text tensor takes its document offsets as an int64 tensor on the same device")
+            if texts.device != dev or doc_byte_offsets.device != dev:
+                raise ValueError("text and offsets must be on %s, the engine's device (got %s and %s)" % (dev, texts.device, doc_byte_offsets.device))
+            if texts.dtype != torch.uint8 or texts.dim() != 1 or doc_byte_offsets.dtype != torch.int64 or doc_byte_offsets.dim() != 1:
+                raise ValueError("text must be a 1-D uint8 tensor and offsets a 1-D int64 tensor")
+            text_d, off_d = texts.contiguous(), doc_byte_offsets.contiguous()
+        else:
+            if isinstance(texts, (bytes, bytearray, memoryview)):
+                if doc_byte_offsets is None:
+                    raise ValueError("bytes need doc_byte_offsets")
+                data, off = bytes(texts), np.ascontiguousarray(doc_byte_offsets, dtype=np.int64)
+            else:
+                if doc_byte_offsets is not None:
+                    raise ValueError("a sequence of str carries its own document boundaries")
+                chunks = [s.encode("utf-8", "surrogatepass") for s in texts]
+                off = np.zeros(len(chunks) + 1, dtype=np.int64)
+                np.cumsum([len(c) for c in chunks], out=off[1:])
+                data = b"".join(chunks)
+            with torch.cuda.device(dev):  # the copies go out on the current stream of the engine's device
+                if data:
+                    import warnings
+
+                    with warnings.catch_warnings():  # (the tensor only reads the bytes: that they are immutable does not matter)
+                        warnings.simplefilter("ignore", UserWarning)
+                        text_d = torch.frombuffer(data, dtype=torch.uint8).to(dev)
+                else:
+                    text_d = torch.empty(0, dtype=torch.uint8, device=dev)
+                off_d = torch.from_numpy(off).to(dev)
+        if off_d.numel() < 1:
+            raise BpeError(_abi.BPE_E_INVALID, "doc_byte_offsets must hold n_docs + 1 entries")
+        n_docs, n_bytes = off_d.numel() - 1, text_d.numel()
+        tvi = None
+        if vector:
+            if self.to_vector_index is None:
+                self.compactVectorIndex()
+            if self._tvi_cuda is None:
+                self._tvi_cuda = torch.from_numpy(self._tvi_array()).to(dev)
+            tvi = self._tvi_cuda
+        out = torch.empty(max(n_bytes, 1), dtype=torch.int32, device=dev)
+        out_off = torch.empty(n_docs + 1, dtype=torch.int64, device=dev)
+        bad = torch.empty(max(n_docs, 1), dtype=torch.int64, device=dev) if vector else None
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None  # noqa: E731
+        n, upos, ucp = C.c_int64(), C.c_int64(-1), C.c_int32()
+        # torch's default stream has the handle 0, which bpe_set_stream reads as the engine's own (non-blocking) stream: that
+        # stream is not ordered after the work torch queued on the legacy default stream, so name that stream explicitly
+        self._check(self._lib.bpe_set_stream(self._h, C.c_void_p(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)))
+        try:
+            rc = self._lib.bpe_encode_text_batch_dev(self._h, ptr(text_d), n_bytes, ptr(off_d), n_docs, ptr(tvi), tvi.numel() if vector else 0,
+                                                     ptr(out), ptr(out_off), ptr(bad), C.byref(n), C.byref(upos), C.byref(ucp))
+            if rc == _abi.BPE_E_INVALID and upos.value >= 0:
+                raise ValueError("unknown token, char: " + _js_stringify(chr(ucp.value)))  # core.ts:399
+            self._check(rc)
+            values = out[: n.value]
+            if vector:
+                holes = torch.nonzero(bad[:n_docs] >= 0)
+                if holes.numel():  # encodeToVector throws at its document's first hole (core.ts:437-441)
+                    d = int(holes[0, 0])
+                    raise ValueError("unknown token index: %d" % (-int(values[int(out_off[d]) + int(bad[d])]) - 1))
+            if pad_to is None:  # (a copy of the N values: `out` holds 4 B per byte of input, a multiple of what they need)
+                return values.clone(), out_off
+            width = pad_to if pad_to != "longest" else (int((out_off[1:] - out_off[:-1]).max()) if n_docs else 0)
+            ids = torch.empty((n_docs, width), dtype=torch.int32, device=dev)
+            lengths = torch.empty(n_docs, dtype=torch.int64, device=dev)
+            self._check(self._lib.bpe_pad_batch_dev(self._h, ptr(out), ptr(out_off), n_docs, width, int(pad_value), ptr(ids), ptr(lengths)))
+            return ids, lengths
+        finally:
+            # bpe_set_stream waits for the stream it leaves: the pad kernel is done when this returns
+            self._check(self._lib.bpe_set_stream(self._h, C.c_void_p(self._stream)))
+
     def restoreToCorpus(self, content: str) -> None:  # core.ts:213-216
         ids = self._char_ids(content, create=False)
         self._flush()
@@ -414,6 +511,7 @@ class BPETokenizer:
                 vector_index += 1
         self.to_vector_index, self.from_vector_index = to_vi, from_vi
         self._tvi_dev = None
+        self._tvi_cuda = None
 
     def _tvi_array(self) -> np.ndarray:
         if self._tvi_dev is None:
@@ -602,6 +700,34 @@ class BPETokenizer:
                                                len(fvi) if fvi is not None else 0, arena.ctypes.data_as(_abi.u8p), p64(tok_off), len(chunks),
                                                out.ctypes.data_as(_abi.u8p), out.size, p64(out_off), p64(bad), C.byref(n)))
         return out[: n.value].tobytes(), out_off, bad[:n_docs]
+
+    def decodeTensor(self, values, offsets=None, *, lengths=None, vector: bool = True) -> List[str]:
+        """decodeVector (core.ts:455-471) per document for vectors held in tensors, e.g. a model's output on the GPU: ragged
+        (values, offsets) or dense (ids[B, L], lengths=[B]) as encodeTextTensor returns them.  The values come to the host once
+        and are decoded in one bpe_decode_batch call.  With vector=False they are raw token indices."""
+        if values.dim() == 2:
+            if lengths is None or offsets is not None:
+                raise ValueError("dense ids take their row lengths as lengths=, and no offsets")
+            ids, lens = values.cpu().numpy(), lengths.cpu().numpy().astype(np.int64)
+            if lens.shape != (ids.shape[0],) or bool(np.any(lens < 0)) or bool(np.any(lens > ids.shape[1])):
+                raise ValueError("lengths must hold one value in [0, %d] per row" % ids.shape[1])
+            vals = ids[np.arange(ids.shape[1])[None, :] < lens[:, None]]
+            off = np.zeros(len(lens) + 1, dtype=np.int64)
+            np.cumsum(lens, out=off[1:])
+        elif values.dim() == 1:
+            if offsets is None or lengths is not None:
+                raise ValueError("ragged values take their document offsets, and no lengths")
+            vals = values.cpu().numpy()
+            off = np.ascontiguousarray(offsets.cpu().numpy() if hasattr(offsets, "cpu") else offsets, dtype=np.int64)
+        else:
+            raise ValueError("values must be 1-D (with offsets) or 2-D (with lengths)")
+        utf8, out_off, bad = self.decodeBatch(vals, off, vector=vector)
+        holes = np.flatnonzero(bad >= 0)
+        if holes.size:
+            d = int(holes[0])
+            v = int(vals[int(off[d]) + int(bad[d])])
+            raise ValueError(("unknown vector index: %s" if vector else "unknown token index: %s") % (v,))  # core.ts:467
+        return [utf8[out_off[d]:out_off[d + 1]].decode("utf-8", "surrogatepass") for d in range(len(off) - 1)]
 
     def decodeTokens(self, tokens: Iterable[Token]) -> str:  # core.ts:447-453
         return "".join(t.chars for t in tokens)

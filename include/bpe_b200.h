@@ -192,7 +192,7 @@ int bpe_pair_counts(bpe_engine* e, int32_t* a, int32_t* b, int64_t* count, int64
  *     every other field (the times included) is member 0's.
  *   - BPE_E_INVALID, as on a sharded engine: bpe_find_next_merge, bpe_apply_merge and bpe_apply_merges on a non-empty corpus
  *     (on an empty one they grow the vocabulary of every member), bpe_set_stream, bpe_add_documents_dev,
- *     bpe_encode_batch_dev, bpe_add_text_stage / _commit and bpe_mg_*.
+ *     bpe_encode_batch_dev, bpe_encode_text_batch_dev, bpe_pad_batch_dev, bpe_add_text_stage / _commit and bpe_mg_*.
  * With BPE_GROUP_SHARE_DEVICE=1 in the environment, devices may repeat: the members on one device share its SMs.  It lets the
  * group run on a host with fewer GPUs than members (tests); it gives no speed-up. */
 int bpe_create_group(const int* devices, int n, bpe_engine** out);
@@ -295,6 +295,29 @@ int bpe_encode_text_batch(bpe_engine* e, const uint8_t* utf8, const int64_t* doc
                           const int32_t* to_vector_index, int32_t n_tvi, int32_t* out, int64_t out_cap,
                           int64_t* out_offsets, int64_t* first_bad, int64_t* n_out, int64_t* unknown_pos,
                           int32_t* unknown_code_point);
+/* bpe_encode_text_batch with every buffer on the engine's device, ordered on the engine's stream: text that is already on
+ * the GPU (a dataloader's output, another kernel's result) is encoded without a trip through the host.
+ *   dev_utf8[0..n_bytes)         the text; dev_doc_byte_offsets[n_docs+1] index into it.  They are checked on the device:
+ *                                non-decreasing and inside [0, n_bytes].  Otherwise BPE_E_INVALID, and nothing is written.
+ *                                offsets[0] need not be 0; bytes after offsets[n_docs] are not read.
+ *   dev_to_vector_index / n_tvi  device, as bpe_encode_batch_dev (NULL: raw token indices)
+ *   dev_out                      room for at least as many values as the batch has code points (n_bytes always suffices)
+ *   dev_out_offsets[n_docs+1]    from 0; dev_first_bad[n_docs] optional, as bpe_encode_batch_dev
+ *   n_out, unknown_pos, unknown_code_point   host, as bpe_encode_text_batch (same BPE_E_INVALID, same position)
+ * A batch of 2^32 - 16 bytes or more: BPE_E_DOMAIN.  Discards a staged text batch, as every encode does.
+ * Staging: the engine's grow-only buffers hold the decoded characters (4 B per byte of the batch) and the encode's scratch
+ * (4 B per code point), as bpe_encode_text_batch's do.  The call waits for the stream a fixed number of times (offsets check,
+ * decode flags, encode), whatever the batch size; when it returns BPE_OK, dev_out and dev_out_offsets are complete. */
+int bpe_encode_text_batch_dev(bpe_engine* e, const uint8_t* dev_utf8, int64_t n_bytes, const int64_t* dev_doc_byte_offsets,
+                              int64_t n_docs, const int32_t* dev_to_vector_index, int32_t n_tvi, int32_t* dev_out,
+                              int64_t* dev_out_offsets, int64_t* dev_first_bad, int64_t* n_out, int64_t* unknown_pos,
+                              int32_t* unknown_code_point);
+/* Ragged -> dense on the device, ordered on the engine's stream (no wait).  Row d of dev_out[n_docs x width] holds the first
+ * min(len_d, width) values of document d (dev_values[dev_offsets[d] .. dev_offsets[d+1])), then pad_value.
+ * dev_lengths[d] (optional) = min(len_d, width).  Works on the output of either _dev encode; dev_offsets must be
+ * non-decreasing and index dev_values (they are not checked). */
+int bpe_pad_batch_dev(bpe_engine* e, const int32_t* dev_values, const int64_t* dev_offsets, int64_t n_docs, int64_t width,
+                      int32_t pad_value, int32_t* dev_out, int64_t* dev_lengths);
 
 /* ---- synthetic corpus (bench / tests; SURVEY.md section 8(d), spec in synth.py) ------------ */
 /* Fills `text` (may be NULL to size) with documents until target_bytes is reached. */
