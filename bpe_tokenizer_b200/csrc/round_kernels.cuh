@@ -8,8 +8,9 @@
 //
 //   decide      every block folds the per-block top-2 partials into the exact, strictly ordered list of the best pairs
 //               (exact down to the largest "second best" any block published) and builds the same batch m_0 .. m_{k-1}:
-//               strictly decreasing (count, -(a+b)) keys, no tie inside the batch, pairwise disjoint tokens, no token born in
-//               the previous round (its occurrence lists are still being written), capacities.
+//               strictly decreasing (count, -(a+b)) keys, no tie inside the batch, pairwise disjoint tokens, capacities.
+//               A pair with a token born in the previous round has its occurrence list still being written; its site pass
+//               walks the site records of the merge of that round whose row holds the pair instead (RoundSm::src).
 //   P1          site passes of all k merges over the corpus as it was at the decision.  A merge changes counts only of
 //               pairs that contain a, b or c, so ALL its count deltas live in dense per-token rows (no hashing in P1): one
 //               packed 64-bit cell per (merge, side, other token x) = decrements of the old pair (x,a) / (b,x) | occurrences
@@ -113,7 +114,7 @@ struct RoundState {
   uint32_t mg_pad;
   unsigned long long rounds, round_merges, rounds_cut_born, rounds_single, tried;
   unsigned long long stop_reason[8];
-  unsigned long long iters_small, iters_big, cells_small, cells_big, sites_small, sites_big;  // P1 warp-iterations, touched cells, sites  // why a batch was not extended: 0 cap, 1 no exact candidate, 2 tie, 3 big, 4 token, 5 fresh token, 6 limits
+  unsigned long long iters_small, iters_big, cells_small, cells_big, sites_small, sites_big;  // P1 warp-iterations, touched cells, sites  // why a batch was not extended: 0 cap, 1 no exact candidate, 2 tie, 3 big, 4 token, 5 (none: fresh tokens join), 6 limits
 };
 
 struct RoundArgs {
@@ -160,6 +161,7 @@ __device__ __forceinline__ uint32_t round_dec_of(const RoundArgs& R, uint32_t pa
 // z = left token | right token << 16 of the born pairs (R_NOTOK: none), w = what the rewrite needs without walking the corpus
 // again: DOCSTART of p << 31 | overflow << 30 | (q - p) << 15 | (e - p)   (q = start of b, e = last slot of b).
 constexpr uint32_t R_NOTOK = 0xFFFFu;
+constexpr uint32_t R_SRC_LIST = 0xFFFFFFFFu;  // RoundSm::src: the merge's sites are in its occurrence list
 __device__ __forceinline__ uint32_t round_pack_span(uint32_t w, uint32_t p, uint32_t q, uint32_t e) {
   const uint32_t dq = q - p, de = e - p;
   const uint32_t doc = (w & DOCSTART) ? 0x80000000u : 0u;
@@ -271,6 +273,7 @@ struct RoundSm {
   uint32_t k, status, mult0, pad0;
   uint32_t a[RB], b[RB], w[RB], slot[RB], llen[RB], lenc[RB];
   unsigned long long lstart[RB];  // where each merge's occurrence list starts in the pool
+  uint32_t src[RB];        // where P1 finds each merge's sites: R_SRC_LIST, or merge i of the previous round << 1 | side of its row
   uint32_t iter0[RB + 1];  // warp-iterations of P1: merge j owns [iter0[j], iter0[j+1])
   uint32_t fill_n[RB];     // sites of the previous round's merges whose born adjacencies are not in their lists yet
   // decision scratch
@@ -630,10 +633,22 @@ __device__ __forceinline__ void mgr_collect(const RoundArgs& R, RoundSm& S, uint
   if (warp == 0) mgr_fold_warp(R, epar);
 }
 
-// One warp-iteration of the site pass of merge j of the round: 32 entries of its occurrence list.
+__device__ __forceinline__ SiteRec* round_sites_buf(const RoundArgs& R, uint32_t par, uint32_t j) {
+  if (j == 0) return par ? R.L.sites2 : R.L.A.sites;
+  return R.bsites + ((size_t)par * RB + j) * R_SMALL;
+}
+
+// What a site record of merge i gives the pair merge i created on `side` (0: (tok, c_i), 1: (c_i, tok)): tok (R_NOTOK: none),
+// and the entry of that pair's occurrence list -- the position of its left token.  The list fill of the following round and
+// its site passes of pairs that contain c_i share this definition.
+__device__ __forceinline__ uint32_t round_rec_tok(const uint4& rv, uint32_t side) { return side ? rv.z >> 16 : rv.z & 0xFFFFu; }
+__device__ __forceinline__ uint32_t round_rec_pos(const uint4& rv, uint32_t side) { return side ? rv.x : rv.y; }
+
+// One warp-iteration of the site pass of merge j of the round: 32 entries of its occurrence list, or -- when the pair contains
+// a token the previous round created (S.src[j]) -- 32 site records of that round's merge whose row holds the pair.
 // The logic of the neighbourhoods is phase_sites' (train_kernels.cuh); what differs is where the deltas go (the merge's
 // dense rows) and the virtual neighbours c_i of the earlier merges of the batch.
-__device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t j, uint32_t c_first,
+__device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t fpar, uint32_t j, uint32_t c_first,
                                                  uint32_t i, SiteRec* site_out, uint32_t sites_cap) {
   const ApplyArgs& A = R.L.A;
   const uint32_t* slots = A.slots;
@@ -647,8 +662,19 @@ __device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S,
   unsigned long long* const cells_r = round_cells(R, par, j, 1);
   bool site = false;
   uint32_t p = 0, w = 0, q = 0, koff = 0;
-  if (i < total) {
-    p = A.pool[S.lstart[j] + i];
+  bool has = i < total;
+  if (has) {
+    const uint32_t src = S.src[j];
+    if (src == R_SRC_LIST) {
+      p = A.pool[S.lstart[j] + i];
+    } else {  // record i of merge src >> 1 of the previous round: an entry of this pair's list iff its token on that side matches
+      const uint4 rv = ld_cg4(reinterpret_cast<const uint4*>(round_sites_buf(R, fpar, src >> 1)) + i);
+      const uint32_t side = src & 1u;
+      has = round_rec_tok(rv, side) == (side ? b : a);
+      p = round_rec_pos(rv, side);
+    }
+  }
+  if (has) {
     w = ld_slot(slots + p);
     if (slot_is_id(w) && slot_val(w) == a && right_token(slots, n, p, &q) == (int)b) {
       site = true;
@@ -805,11 +831,6 @@ __device__ __forceinline__ void round_sites_iter(const RoundArgs& R, RoundSm& S,
   }
 }
 
-__device__ __forceinline__ SiteRec* round_sites_buf(const RoundArgs& R, uint32_t par, uint32_t j) {
-  if (j == 0) return par ? R.L.sites2 : R.L.A.sites;
-  return R.bsites + ((size_t)par * RB + j) * R_SMALL;
-}
-
 struct RoundFill {  // what the previous round left to do
   uint32_t v, par, k, c_first;  // merges committed / row parity / merges tried (rows to clear) / first token it created
   uint32_t overflow;            // a list of touched cells overflowed in that round: clear by scanning
@@ -832,15 +853,15 @@ __device__ __forceinline__ void round_fill_all(const RoundArgs& R, const RoundSm
     }
     const bool has = off < S.fill_n[j];
     const uint4 rv = has ? ld_cg4(reinterpret_cast<const uint4*>(round_sites_buf(R, F.par, j)) + off) : make_uint4(0, NOPOS, R_NOTOK | (R_NOTOK << 16), 0);
-    const uint32_t ltok = rv.z & 0xFFFFu, rtok = rv.z >> 16;
+    const uint32_t ltok = round_rec_tok(rv, 0), rtok = round_rec_tok(rv, 1);
     const uint32_t lslot = (has && ltok != R_NOTOK) ? ld_cg(round_slotrow(R, F.par, j, 0) + ltok) : NOSLOT;
     const uint32_t rslot = (has && rtok != R_NOTOK) ? ld_cg(round_slotrow(R, F.par, j, 1) + rtok) : NOSLOT;
     const bool hl = has && lslot != NOSLOT && t.occ_len[lslot];
     const bool hr = has && rslot != NOSLOT && t.occ_len[rslot];
     const unsigned long long il = agg_cursor(t, lslot, hl);
     const unsigned long long ir = agg_cursor(t, rslot, hr);
-    if (hl) A.pool[il] = rv.y;
-    if (hr) A.pool[ir] = rv.x;
+    if (hl) A.pool[il] = round_rec_pos(rv, 0);
+    if (hr) A.pool[ir] = round_rec_pos(rv, 1);
   }
 }
 
@@ -1060,14 +1081,25 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         const unsigned long long pj = (j < RB) ? S.cp[j] : 0ull;
         const uint32_t wj = (uint32_t)(pj >> 20), key = (j < RB) ? S.ck[j] : 0u;
         const uint32_t aj = key >> 16, bj = key & 0xFFFFu, cj = c_first + j;
+        // A pair with a token the previous round created is still having its list written (helper warps of this P1), but all
+        // its occurrences are among that round's site records (double-buffered: intact), in exactly one row: (c_i, y) in merge
+        // i's right row, (x, c_m) in merge m's left row, (c_i, c_m) in the row of the later merge (for i > m merge i's site
+        // pass saw c_m as its virtual right neighbour; for i <= m merge m's saw c_i on its left).
+        const bool fa = pj && F.v && aj >= F.c_first, fb = pj && F.v && bj >= F.c_first;
+        const uint32_t src = (fa && (!fb || aj > bj)) ? (((aj - F.c_first) << 1) | 1u) : fb ? ((bj - F.c_first) << 1) : R_SRC_LIST;
+        const uint32_t slen = (src != R_SRC_LIST) ? S.fill_n[src >> 1] : (j < RB ? S.cll[j] : 0u);  // entries P1 walks
         const unsigned long long new_keys = pj ? min(2ull * wj + 2ull, 2ull * (cj + 1ull) + 2ull) : 0ull;
-        unsigned long long keys_incl = new_keys, w_incl = pj ? wj : 0u;  // cumulative over candidates 0..j (the batch is a prefix)
+        // cumulative over candidates 0..j (the batch is a prefix): new keys, counts, and the counts again with a pair's site
+        // records in place of its count where P1 walks those (the batch limit: what a dropped tail's site pass costs)
+        unsigned long long keys_incl = new_keys, w_incl = pj ? wj : 0u, s_incl = pj ? (src == R_SRC_LIST ? wj : slen) : 0u;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-          const unsigned long long x = __shfl_up_sync(0xFFFFFFFFu, keys_incl, o), y = __shfl_up_sync(0xFFFFFFFFu, w_incl, o);
+          const unsigned long long x = __shfl_up_sync(0xFFFFFFFFu, keys_incl, o), y = __shfl_up_sync(0xFFFFFFFFu, w_incl, o),
+                                   z = __shfl_up_sync(0xFFFFFFFFu, s_incl, o);
           if ((int)lane >= o) {
             keys_incl += x;
             w_incl += y;
+            s_incl += z;
           }
         }
         // capacity the host guarantees, cumulative over the batch: 0 (LOOP_RUNNING) fine, else the status it would mean for
@@ -1090,10 +1122,9 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         else if (!pj) stop = 1;
         else if (cap_fail) stop = 6;
         else if (mult0 > 1 || S.cm[j] > 1) stop = 2;                                   // position tie-breaks run alone
-        else if (w0 > R_SMALL || w_incl > R_BATCH_SITES) stop = 3;                     // a big merge keeps the whole grid
+        else if (w0 > R_SMALL || s_incl > R_BATCH_SITES) stop = 3;                     // a big merge keeps the whole grid
         else if (wj < thresh || wj < L.min_weight) stop = 6;                           // the next decision handles the status
         else if (it + j >= L.log_cap || cj >= L.max_tokens) stop = 6;
-        else if (F.v && (aj >= F.c_first || bj >= F.c_first)) stop = 5;                // its list is still being written
         else {
           for (uint32_t i2 = 0; i2 < j; i2++) {  // shares a token with an earlier candidate
             const uint32_t k2 = S.ck[i2], a2 = k2 >> 16, b2 = k2 & 0xFFFFu;
@@ -1115,10 +1146,11 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
           S.w[j] = wj;
           S.slot[j] = S.cs[j];
           S.lstart[j] = S.cls[j];
-          S.llen[j] = S.cll[j];
+          S.src[j] = src;
+          S.llen[j] = slen;
           S.lenc[j] = S.clen[j];
         }
-        uint32_t it_incl = (j < k) ? ((S.cll[j] + 31u) >> 5) : 0u;
+        uint32_t it_incl = (j < k) ? ((slen + 31u) >> 5) : 0u;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
           const uint32_t x = __shfl_up_sync(0xFFFFFFFFu, it_incl, o);
@@ -1183,6 +1215,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         S.filt_a[((key >> 16) >> 5) & 7u] = 1u << ((key >> 16) & 31u);
         S.filt_b[((key & 0xFFFFu) >> 5) & 7u] = 1u << (key & 31u);
         S.lstart[0] = t.occ_start.get(s);
+        S.src[0] = R_SRC_LIST;  // (the lists of the last round are complete: filled above)
         S.llen[0] = t.occ_len[s];
         S.lenc[0] = A.len16[key >> 16] + A.len16[key & 0xFFFFu];
         S.iter0[1] = (S.llen[0] + 31u) >> 5;
@@ -1199,14 +1232,6 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         loop_exit(t, st, status, it, c_first, &wb, R.mg_on, mg_epoch, tie_epoch);
       }
       return;
-    }
-    if (F.v && (S.a[0] >= F.c_first || S.b[0] >= F.c_first)) {
-      // the winner contains a token the previous round created: its list is what fill still has to write
-      round_fill_all(R, S, F, gt, gn);
-      __syncthreads();
-      if (tid < RB) S.fill_n[tid] = 0;
-      F.v = 0;
-      RBARRIER();
     }
     // ================= P1: the site passes of the batch, next to the list filling of the previous round =================
     if (bid == 0 && warp == 0) {
@@ -1230,7 +1255,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         for (uint32_t wi = bid * ws + warp; wi < iters; wi += nblk * ws) {
           uint32_t j = 0;
           while (j + 1 < k && wi >= S.iter0[j + 1]) j++;
-          round_sites_iter(R, S, par, j, c_first, (wi - S.iter0[j]) * 32u + lane, round_sites_buf(R, par, j), j == 0 ? A.sites_cap : R_SMALL);
+          round_sites_iter(R, S, par, F.par, j, c_first, (wi - S.iter0[j]) * 32u + lane, round_sites_buf(R, par, j), j == 0 ? A.sites_cap : R_SMALL);
         }
         if (!split) {
           if (F.v) round_fill_all(R, S, F, gt, gn);
