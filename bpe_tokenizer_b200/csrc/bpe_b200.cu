@@ -1341,6 +1341,10 @@ int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t m
       const auto tg = std::chrono::steady_clock::now();
       if ((rc = grow_merge_buffers(e, mg, use_rounds, trace)) != BPE_OK) break;
       host_ms[1] += ms_since(tg);
+      // A rank whose pair table grew must rebuild its hot list (new slot numbers), and the rebuild sets a new hot_thresh.  The
+      // ranks decide every merge, and when to leave the kernel (w < hot_thresh), on their own lists and thresholds, so they all
+      // rebuild: table sizes follow the shard sizes, and on uneven shards only some ranks grow.
+      if (mg) e->hot_valid = false;
       continue;
     }
     rc = fail(e, BPE_E_INTERNAL, "merge loop returned status %u", status);

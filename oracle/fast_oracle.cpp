@@ -38,6 +38,7 @@ struct Fast {
   std::vector<int32_t> tok;      // token at a position; -1: the position no longer starts a token
   std::vector<uint32_t> nxt, prv;
   std::vector<uint8_t> first;    // the position starts a document (no pair reaches across, core.ts:265-267)
+  std::vector<uint32_t> doc_start;  // first position of every document, empty ones included (they hold no position)
   std::vector<int32_t> len16;    // UTF-16 length of token.chars (the max_length test, core.ts:270-273)
   std::unordered_map<uint64_t, PairInfo> pairs;
   typedef std::tuple<int64_t, int64_t, uint64_t> Entry;  // count, -(a + b), key
@@ -212,6 +213,7 @@ int fast_add_documents(void* h, const int32_t* ids, const int64_t* off, int64_t 
   F.prv.reserve(want);
   F.nxt.reserve(want);
   for (int64_t d = 0; d < n_docs; d++) {
+    F.doc_start.push_back((uint32_t)F.tok.size());
     for (int64_t i = off[d]; i < off[d + 1]; i++) {
       uint32_t p = (uint32_t)F.tok.size();
       F.tok.push_back(ids[i]);
@@ -240,6 +242,20 @@ void fast_get_corpus(void* h, int32_t* out) {
   for (uint32_t p = 0; p != NONE; p = F.nxt[p]) out[k++] = F.tok[p];
 }
 
+int64_t fast_num_documents(void* h) { return (int64_t) static_cast<Fast*>(h)->doc_start.size(); }
+
+// current number of tokens of every document, in addition order (out holds fast_num_documents values)
+void fast_document_lengths(void* h, int64_t* out) {
+  Fast& F = *static_cast<Fast*>(h);
+  const size_t nd = F.doc_start.size();
+  for (size_t d = 0; d < nd; d++) {
+    const uint32_t end = d + 1 < nd ? F.doc_start[d + 1] : (uint32_t)F.tok.size();
+    int64_t n = 0;
+    for (uint32_t p = F.doc_start[d]; p < end; p++) n += F.tok[p] >= 0;
+    out[d] = n;
+  }
+}
+
 // mergeUntil (core.ts:365-383): falsy options mean the defaults (min_weight 2, no max_length, no iteration limit).
 // Token c of merge i is first_new_index + i.  Returns the number of merges; la/lb/lw receive pair and weight.
 int64_t fast_merge_until(void* h, int64_t min_weight, int32_t max_length, int64_t max_iterations, int32_t first_new_index, int32_t* la,
@@ -248,6 +264,8 @@ int64_t fast_merge_until(void* h, int64_t min_weight, int32_t max_length, int64_
   if (!F.built) build(F);
   if (min_weight <= 0) min_weight = 2;
   int64_t done = 0;
+  // entries of pairs that this call's max_length excludes: set aside, not dropped, because a later call may allow them
+  std::vector<Fast::Entry> too_long_kept;
   while (done < cap && (max_iterations <= 0 || done < max_iterations)) {
     // ---- findNextMerge (core.ts:247-326) ----
     std::vector<Fast::Entry> tied;
@@ -260,7 +278,11 @@ int64_t fast_merge_until(void* h, int64_t min_weight, int32_t max_length, int64_
       bool too_long = max_length > 0 && F.len16[a] + F.len16[b] > max_length;  // core.ts:270-273: never eligible
       if (!tied.empty() && !(std::get<0>(e) == std::get<0>(tied[0]) && std::get<1>(e) == std::get<1>(tied[0]))) break;
       F.heap.pop();
-      if (stale || too_long) continue;
+      if (stale) continue;
+      if (too_long) {
+        too_long_kept.push_back(e);
+        continue;
+      }
       bool dup = false;
       for (const Fast::Entry& t : tied) dup = dup || std::get<2>(t) == key;
       if (!dup) tied.push_back(e);
@@ -300,6 +322,7 @@ int64_t fast_merge_until(void* h, int64_t min_weight, int32_t max_length, int64_
     F.merge_no++;
     done++;
   }
+  for (const Fast::Entry& e : too_long_kept) F.heap.push(e);
   return done;
 }
 

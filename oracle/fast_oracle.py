@@ -34,6 +34,9 @@ def lib():
         L.fast_total_tokens.argtypes = [C.c_void_p]
         L.fast_total_tokens.restype = C.c_int64
         L.fast_get_corpus.argtypes = [C.c_void_p, i32p]
+        L.fast_num_documents.argtypes = [C.c_void_p]
+        L.fast_num_documents.restype = C.c_int64
+        L.fast_document_lengths.argtypes = [C.c_void_p, i64p]
         L.fast_merge_until.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int32, i32p, i32p, i64p, C.c_int64]
         L.fast_merge_until.restype = C.c_int64
         _lib = L
@@ -79,3 +82,10 @@ class FastOracle:
         out = np.zeros(max(self.L.fast_total_tokens(self.h), 1), dtype=np.int32)
         self.L.fast_get_corpus(self.h, _p32(out))
         return out[: self.L.fast_total_tokens(self.h)]
+
+    def document_lengths(self) -> np.ndarray:
+        """Current number of tokens of every document, empty documents included (corpus() holds them back to back)."""
+        out = np.zeros(self.L.fast_num_documents(self.h), dtype=np.int64)
+        if out.size:
+            self.L.fast_document_lengths(self.h, _p64(out))
+        return out

@@ -10,6 +10,7 @@ import pytest
 import kat_suite
 from oracle import LiteralTokenizer, compact_merge
 from oracle.int_oracle import IntOracleTokenizer
+from pair_counts import device_counts, loop_counts, recount
 
 pytestmark = pytest.mark.gpu
 
@@ -87,6 +88,8 @@ def test_fuzz_step_by_step_against_literal(seed, scan_mode):
         lit.applyMerge(m1)
         gpu.applyMerge(m2)
         assert gpu.corpus_in_code == lit.corpus_in_code, step
+        toks = [[ord(ch) - 1 for ch in doc] for doc in lit.corpus_in_code]
+        assert device_counts(gpu) == recount([x for d in toks for x in d], [len(d) for d in toks]), step
     assert gpu.toJSON() == lit.toJSON()
     for d in docs + _random_docs(rng, alphabet, 3, 60):
         try:
@@ -158,20 +161,7 @@ def test_pair_histogram_matches_oracle_counts():
     n = C.c_int64()
     gpu._check(gpu._lib.bpe_pair_counts(gpu._h, _abi.p32(a), _abi.p32(b), _abi.p64(c), cap, C.byref(n)))
     got = {(int(a[i]), int(b[i])): int(c[i]) for i in range(n.value)}
-    want = {}
-    for doc in lit.corpus_in_code:
-        toks = [ord(ch) - 1 for ch in doc]
-        run = 0
-        for i in range(1, len(toks)):
-            x, y = toks[i - 1], toks[i]
-            if x == y:
-                run = run + 1 if (i >= 2 and toks[i - 2] == x) else 1
-                if run % 2 == 0:
-                    continue
-            else:
-                run = 0
-            want[(x, y)] = want.get((x, y), 0) + 1
-    assert got == want
+    assert got == loop_counts([[ord(ch) - 1 for ch in doc] for doc in lit.corpus_in_code])
 
 
 def _zipf_pair(n_bytes, seed=43):

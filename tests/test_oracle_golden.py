@@ -223,6 +223,64 @@ def test_fast_oracle_equals_literal_oracle_on_zipf_text():
     assert _int_vs_fast(docs, len(alphabet), 2, 6, 200, cap=200) == 200
 
 
+def _int_vs_fast_calls(docs, nsym, calls):
+    """One corpus trained through a sequence of merge_until calls (min_weight, max_length, max_iterations) on both oracles: the
+    logs of every call, the corpus and the document lengths after every call must be equal.  -> merges done"""
+    from oracle.fast_oracle import FastOracle
+    from oracle.int_oracle import IntOracle
+
+    ids = np.array([t for d in docs for t in d], dtype=np.int32)
+    off = np.zeros(len(docs) + 1, dtype=np.int64)
+    off[1:] = np.cumsum([len(d) for d in docs])
+    lit, fast = IntOracle(), FastOracle()
+    for o in (lit, fast):
+        o.set_len16(np.ones(nsym, dtype=np.int32))
+        o.add_documents(ids, off)
+    done = 0
+    for i, (mw, ml, mi) in enumerate(calls):
+        cap = mi if mi > 0 else 1000
+        want, got = lit.merge_until(mw, ml, mi, nsym + done, cap), fast.merge_until(mw, ml, mi, nsym + done, cap)
+        assert all(np.array_equal(x, y) for x, y in zip(want, got)), (i, [x[:12].tolist() for x in want], [x[:12].tolist() for x in got])
+        done += len(want[0])
+        assert np.array_equal(fast.document_lengths(), [lit.document(d).size for d in range(lit.num_documents())]), i
+        corpus = np.concatenate([lit.document(d) for d in range(lit.num_documents())]) if docs else np.zeros(0, np.int32)
+        assert np.array_equal(corpus, fast.corpus()), i
+    return done
+
+
+def test_fast_oracle_keeps_pairs_a_max_length_excluded():
+    """(3, 2) -- the token of the first merge, then 2 -- is too long under max_length 2 and is the next merge once the limit is gone:
+    a call that skips a pair for its length must leave it to later calls."""
+    docs = [[0, 1, 2]] * 10 + [[0, 1]] * 2 + [[2, 2]] * 3
+    assert _int_vs_fast_calls(docs, 3, [(2, 2, 5), (2, 0, 5)]) == 3
+    assert _int_vs_fast_calls(docs + [[]], 3, [(2, 2, 1), (2, 2, 1), (2, 0, 1), (2, 2, 1), (2, 0, 5)]) == 3
+
+
+@pytest.mark.parametrize("chunk", range(4))
+def test_fast_oracle_equals_literal_oracle_across_calls(chunk):
+    """sequences of calls whose max_length and min_weight change between calls, and cuts at max_iterations, on the corpora of
+    the fuzz test above: empty and one-token documents, runs, ties"""
+    total = 0
+    for seed in range(chunk * 60, (chunk + 1) * 60):
+        rng = random.Random(50000 + seed)
+        nsym = rng.choice([1, 2, 3, 3, 5, 8])
+        docs = [[rng.randrange(nsym) for _ in range(rng.choice([0, 1, 2, 5, 20, 60, 200]))] for _ in range(rng.randint(1, 6))]
+        calls = [(rng.choice([1, 2, 2, 3, 5]), rng.choice([0, 0, 2, 3, 4, 8]), rng.choice([1, 2, 3, 5, 40])) for _ in range(rng.randint(2, 6))]
+        total += _int_vs_fast_calls(docs, nsym, calls)
+    assert total > 300
+
+
+def test_fast_oracle_equals_literal_oracle_across_calls_on_zipf_text():
+    """the option sequences the GPU state tests train through (tests/test_gpu_merge_state.py), at 100 kB"""
+    from bpe_tokenizer_b200.synth import first_appearance_ids, synth_corpus
+
+    text, off = synth_corpus(100_000, seed=43)
+    ids, alphabet = first_appearance_ids(text)
+    docs = [ids[off[d]:off[d + 1]].tolist() for d in range(len(off) - 1)]
+    for calls in ([(2, 4, 40), (2, 0, 40), (2, 6, 40)], [(150, 0, 60), (2, 0, 40)], [(3, 9, 60), (2, 0, 40)]):
+        assert _int_vs_fast_calls(docs, len(alphabet), calls) > 60
+
+
 def test_fast_oracle_reproduces_the_cfg2_golden_log():
     """10 MB, 4 000 merges: the incremental oracle (seconds) gives the SHA-1 the literal restatement needed 34 minutes for
     (tests/golden/cfg2_merge_log.json) -- and the GPU gives (test_gpu_parity.py)"""
