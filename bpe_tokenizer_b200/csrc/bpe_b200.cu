@@ -235,7 +235,6 @@ struct bpe_engine {
   uint32_t mg_inbox_stride = 0, mg_tie_cap = 0;
   DevBuf<int32_t> mg_dlt;
   DevBuf<uint32_t> mg_mark, mg_touched, mg_tie_sorted, mg_export_n, mg_newpair;
-  int mg_loop_blocks = 0;
   unsigned long long mg_epoch = 0, mg_tie_epoch = 0;
   bool mg_timed_out = false;             // the last sharded mergeUntil stopped because a peer did not answer
   LaunchGate* mg_gate = nullptr;         // group member inside the group's bpe_merge_until: the members' launch rendezvous
@@ -1003,7 +1002,6 @@ RoundArgs round_args(bpe_engine* e, const LoopArgs& L, int round_k) {
   RA.kmax = (uint32_t)round_k;
   RA.bar_mode = 1;
   if (const char* v = getenv("BPE_LOOP_BAR")) RA.bar_mode = atoi(v) ? 1 : 0;
-  RA.mg_on = 0;
   RA.gcells = e->r_gcells.p;
   RA.glists = e->r_glists.p;
   return RA;
@@ -1037,8 +1035,6 @@ MgArgs mg_args(bpe_engine* e) {
     M.tiebox[q] = reinterpret_cast<uint32_t*>(base + 2 * flags_bytes + inbox_bytes);
   }
   M.tie_sorted = e->mg_tie_sorted.p;
-  M.newpair = e->mg_newpair.p;
-  M.newpair_cap = (uint32_t)e->mg_newpair.cap;
   return M;
 }
 
@@ -1046,11 +1042,14 @@ double ms_since(std::chrono::steady_clock::time_point t) {
   return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count();
 }
 
-// the arguments of one launch; a sharded engine stages its count deltas (dlt, touched) and lists the pairs born on any rank
+// the arguments of one launch; a sharded engine stages its count deltas (dlt, touched), lists the pairs born on any rank and
+// talks to its peers through the mailboxes
 LoopArgs loop_args(bpe_engine* e, bool mg, bool use_rounds, uint32_t chunk, uint32_t ml, int64_t mw) {
   LoopArgs L{};
   L.A = apply_args(e);
   if (mg) {
+    L.mg_on = 1;
+    L.mg = mg_args(e);
     L.A.newpair = e->mg_newpair.p;
     L.A.newpair_cap = (uint32_t)e->mg_newpair.cap;
     L.A.dlt = e->mg_dlt.p;
@@ -1096,33 +1095,25 @@ LoopArgs loop_args(bpe_engine* e, bool mg, bool use_rounds, uint32_t chunk, uint
   return L;
 }
 
-// one launch: k_merge_rounds, or the one-merge kernel (k_merge_loop, k_merge_loop_mg).  `above`: the winner has more sites than the
+// one launch: k_merge_rounds, or the one-merge kernel k_merge_loop.  `above`: the winner has more sites than the
 // packed delta cells of a round can count, so the one-merge kernel takes the merges above R_HUGE -- it stops, "done", at the first
 // winner at or below it -- and the rounds continue from there
 cudaError_t launch_merge_loop(bpe_engine* e, bool mg, LoopArgs L, bool rounds, bool above, int64_t mw, int round_k) {
-  if (!mg || rounds) {  // the second site buffer, which k_merge_loop_mg does not use
+  if (!mg || rounds) {  // the second site buffer, which k_merge_loop does not use on a sharded corpus
     L.sites2 = e->sites2.p;
     L.A.sites_cap = (uint32_t)std::min<size_t>(L.A.sites_cap, e->sites2.cap);
   }
   if (rounds) {
     RoundArgs RA = round_args(e, L, round_k);
-    if (mg) {
-      RA.mg_on = 1;
-      RA.mg = mg_args(e);
-    }
     k_rounds_prepare<<<1, 32, 0, e->stream>>>(e->r_state.p);
     e->stats.kernel_launches++;
     void* args[] = {&RA};
     return cudaLaunchCooperativeKernel((void*)k_merge_rounds, dim3(e->round_blocks), dim3(RD_THREADS), args, R_STAGE_BYTES, e->stream);
   }
   if (above) L.min_weight = (uint32_t)std::max<int64_t>(mw, (int64_t)R_HUGE + 1);
-  if (mg) {
-    LoopArgsMg P{L, mg_args(e)};
-    void* args[] = {&P};
-    return cudaLaunchCooperativeKernel((void*)k_merge_loop_mg, dim3(e->mg_loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
-  }
   void* args[] = {&L};
-  return cudaLaunchCooperativeKernel((void*)k_merge_loop, dim3(e->loop_blocks), dim3(ML_THREADS), args, 0, e->stream);
+  return cudaLaunchCooperativeKernel(mg ? (void*)k_merge_loop<true> : (void*)k_merge_loop<false>, dim3(e->loop_blocks), dim3(ML_THREADS), args, 0,
+                                     e->stream);
 }
 
 // appends the `iters` merges of the last launch to the caller's log and to the host's token lengths and merge list
@@ -1212,17 +1203,17 @@ int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t m
     return fail(e, BPE_E_INVALID, "sharded engine: exchange the pair counts first (bpe_mg_export_counts / bpe_mg_import_counts)");
   const uint32_t ml = max_length > 0 ? (uint32_t)max_length : 0;
   const int64_t mw = min_weight > 0 ? min_weight : 2;
-  int& loop_blocks = mg ? e->mg_loop_blocks : e->loop_blocks;
+  int& loop_blocks = e->loop_blocks;
   if (!loop_blocks) {
     int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mg ? (const void*)k_merge_loop_mg : (const void*)k_merge_loop, ML_THREADS, 0));
-    if (per_sm < 1) return fail(e, BPE_E_CUDA, "%s does not fit on an SM", mg ? "k_merge_loop_mg" : "k_merge_loop");
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mg ? (const void*)k_merge_loop<true> : (const void*)k_merge_loop<false>, ML_THREADS, 0));
+    if (per_sm < 1) return fail(e, BPE_E_CUDA, "k_merge_loop does not fit on an SM");
     // one 512-thread block per SM: measured best on cfg3 (1.28 s vs 1.41 s with two per SM, 1.33 s with half an SM count,
     // 1.55 s with 1024-thread blocks) -- a merge is latency bound, fewer arrivals per grid barrier and fewer partials win
     int want = 1;
     if (const char* v = getenv("BPE_LOOP_PER_SM")) want = std::max(1, atoi(v));  // tuning knob: co-resident blocks per SM
     loop_blocks = e->sm_count * std::min(per_sm, want);
-    const char* v = getenv("BPE_LOOP_BLOCKS");  // (a single-GPU knob: it has never sized k_merge_loop_mg's grid)
+    const char* v = getenv("BPE_LOOP_BLOCKS");  // (a single-GPU knob: it does not size a sharded rank's grid)
     if (v && !mg) loop_blocks = std::max(1, std::min(atoi(v), e->sm_count * per_sm));
   }
   // several exact merges per barrier round (round_kernels.cuh; on a sharded corpus ONE exchange per round) unless a merge list is
@@ -1233,8 +1224,9 @@ int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t m
   if (const char* v = getenv("BPE_LOOP_K")) round_k = std::max(1, std::min(atoi(v), (int)RB));
   if (use_rounds) TRY(ensure_round_buffers(e));
   CK(e->partials.reserve((size_t)std::max(loop_blocks, e->grid(8))));
+  CK(e->partial_keys.reserve((size_t)std::max(loop_blocks, e->grid(8))));
   CK(e->sites.reserve(1u << 16, 0, e->stream, 1.0));
-  if (!mg || use_rounds) CK(e->sites2.reserve(std::max<size_t>(e->sites.cap, 1u << 16), 0, e->stream, 1.0));  // (not read by k_merge_loop_mg)
+  if (!mg || use_rounds) CK(e->sites2.reserve(std::max<size_t>(e->sites.cap, 1u << 16), 0, e->stream, 1.0));  // (not read by a sharded k_merge_loop)
   CK(e->newslots.reserve(mg ? 1u << 17 : 1u << 16, 0, e->stream, 1.0));
   CK(e->cands.reserve(4096, 0, e->stream, 1.0));
   CK(e->barrier.reserve(64));
@@ -1242,8 +1234,6 @@ int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t m
     CK(e->mg_touched.reserve((size_t)4 * BPE_MAX_TOKENS + 64));
     CK(e->mg_tie_sorted.reserve(e->mg_tie_cap));
     CK(e->mg_newpair.reserve((size_t)2 * BPE_MAX_TOKENS + 64));
-  } else {
-    CK(e->partial_keys.reserve((size_t)std::max(loop_blocks, e->grid(8))));  // (read by k_merge_loop only)
   }
   static const bool trace = getenv("BPE_TRACE") != nullptr;
   cudaEvent_t t0, t1;
@@ -1303,7 +1293,7 @@ int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t m
       fprintf(stderr, "[bpe] k_merge_loop: %u merges in %.2f ms, status %u, best_cnt %u, hot_n %u thresh %u, keys %u/%u\n", iters, ms_since(tw0),
               e->h_st->status, e->h_st->best_cnt, e->h_st->hot_n, e->h_st->hot_thresh, e->h_st->n_keys, e->tbl_cap);
     if (trace && mg)
-      fprintf(stderr, "[bpe r%d] k_merge_loop_mg: %u merges in %.2f ms, status %u, best_cnt %u, hot_n %u thresh %u, keys %u/%u err 0x%x gerr 0x%x\n",
+      fprintf(stderr, "[bpe r%d] k_merge_loop: %u merges in %.2f ms, status %u, best_cnt %u, hot_n %u thresh %u, keys %u/%u err 0x%x gerr 0x%x\n",
               e->mg_rank, iters, ms_since(tw0), e->h_st->status, e->h_st->best_cnt, e->h_st->hot_n, e->h_st->hot_thresh, e->h_st->n_keys, e->tbl_cap,
               e->h_st->err, e->h_st->g_vals[0]);
     const auto tl = std::chrono::steady_clock::now();
@@ -1407,7 +1397,7 @@ int merge_until(bpe_engine* e, int64_t min_weight, int32_t max_length, int64_t m
 int mg_alloc_mailbox(bpe_engine* e, int rank, int world) {
   e->mg_rank = rank;
   e->mg_world = world;
-  // records one rank can send per exchange (k_merge_rounds: the cells of up to 16 merges a round; k_merge_loop_mg: of one merge)
+  // records one rank can send per exchange (k_merge_rounds: the cells of up to 16 merges a round; k_merge_loop: of one merge)
   e->mg_inbox_stride = MG_INBOX_STRIDE;
   e->mg_tie_cap = 4096;
   size_t bytes = (size_t)2 * MG_MAX_WORLD * 128 + (size_t)2 * world * e->mg_inbox_stride * 8 + (size_t)2 * world * e->mg_tie_cap * 4;

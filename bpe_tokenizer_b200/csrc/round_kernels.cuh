@@ -39,7 +39,7 @@
 // listed as records to every rank (NVLink stores) and reports to a per-(receiver, parity, sender) arrival counter; every
 // block sums the records of the senders that are complete into the GLOBAL cells (mgr_collect), P2 runs over those.  The
 // decisions are replicated: U bounds and site counts are sums over the ranks, capacities minima (headers of the messages).
-// The header, its fold, the waits on the peers' flags and the tie-break are mg_kernels.cuh's, shared with k_merge_loop_mg.
+// The header, its fold, the waits on the peers' flags and the tie-break are mg_kernels.cuh's, shared with k_merge_loop.
 //
 // Exactness argument for the order inside a batch (SURVEY.md A.2, core.ts:294-305): counts of existing pairs never grow
 // under merging, so an old pair that ranked below m_j at the decision still does; born pairs are bounded by U; m_j's own
@@ -128,11 +128,9 @@ struct RoundArgs {
   uint32_t* gk;      // [RT * blocks] ... and the pair key of that slot
   RoundState* rs;
   uint32_t kmax;     // merges per round (1 .. RB)
-  // corpus sharded by document over several GPUs (mg_kernels.cuh): the counts of the pair table are global and replicated, the
-  // cells above hold THIS shard's deltas; once per round every rank stores its non-empty cells as records into every rank's
-  // inbox over NVLink, and every rank sums all records into gcells -- the global deltas P2 then works from
-  int mg_on;
-  MgArgs mg;
+  // corpus sharded by document over several GPUs (L.mg_on, mg_kernels.cuh): the counts of the pair table are global and
+  // replicated, the cells above hold THIS shard's deltas; once per round every rank stores its non-empty cells as records into
+  // every rank's inbox over NVLink, and every rank sums all records into gcells -- the global deltas P2 then works from
   unsigned long long* gcells;  // [2][RB][2][ND_STRIDE]: decrements | counted occurrences << 21, summed over the ranks
   uint32_t* glists;            // [2][blocks][R_LISTCAP]: global cells each block touched first while summing
 };
@@ -154,7 +152,7 @@ __device__ __forceinline__ uint32_t* round_glist(const RoundArgs& R, uint32_t pa
   return R.glists + ((size_t)par * gridDim.x + blockIdx.x) * R_LISTCAP;
 }
 __device__ __forceinline__ uint32_t round_dec_of(const RoundArgs& R, uint32_t par, uint32_t j, uint32_t side, uint32_t tok) {
-  return cell_dec(ld_cg((R.mg_on ? round_gcells(R, par, j, side) : round_cells(R, par, j, side)) + tok));  // (both layouts keep it in the low bits)
+  return cell_dec(ld_cg((R.L.mg_on ? round_gcells(R, par, j, side) : round_cells(R, par, j, side)) + tok));  // (both layouts keep it in the low bits)
 }
 
 // Site record of a round: x = p, y = position of the left token of the born left adjacency (NOPOS: none),
@@ -434,7 +432,7 @@ __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, 
 // coalesced NVLink stores.  (Records written while the passes run -- one per warp and neighbour -- were measured: the
 // frequent neighbours then receive hundreds of records each and the summing on the other side queues on those cells.)
 __device__ __forceinline__ void round_emit_records(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t epar, uint32_t k, uint32_t c_hi, unsigned long long epoch) {
-  const MgArgs& M = R.mg;
+  const MgArgs& M = R.L.mg;
   DevState* st = R.L.A.st;
   const uint32_t cap = M.inbox_stride - MGR_HDR;
   // (block 0: its last warp -- the records of a round keep the first warps busy, not that one -- also writes this rank's header)
@@ -495,7 +493,7 @@ __device__ __forceinline__ void round_emit_records(const RoundArgs& R, RoundSm& 
 
 // warp 0 of block 0, lane q talks to rank q: header of this rank's message, then the flag
 __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, uint32_t epar, uint32_t k, unsigned long long epoch, bool with_flag) {
-  const MgArgs& M = R.mg;
+  const MgArgs& M = R.L.mg;
   const LoopArgs& L = R.L;
   DevState* st = L.A.st;
   const int q = (int)lane_id();
@@ -504,7 +502,7 @@ __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, 
   const uint32_t ns_lane = ((uint32_t)q < k) ? ld_cg(&R.rs->n_sites[par][q].v) : 0u;
   if (q < M.world) {
     unsigned long long* dst = mg_area(M, q, epar, M.rank);
-    mg_store_header(L, M, dst, min(ld_cg(&st->n_out), M.inbox_stride - MGR_HDR), 0xFFFFFFFFu);
+    mg_store_header(L, dst, min(ld_cg(&st->n_out), M.inbox_stride - MGR_HDR), 0xFFFFFFFFu);
     dst[40] = k;
   }
   for (uint32_t j = 0; j < RB; j++) {  // (every lane takes part in the shuffles; the lanes that talk to a rank store)
@@ -525,7 +523,7 @@ __device__ __forceinline__ void mgr_send_warp(const RoundArgs& R, uint32_t par, 
 // fold the headers of all senders (their messages are complete): st->g_vals (mg_fold_headers_warp), sums of the per-merge
 // bounds and site counts, the smallest batch
 __device__ __forceinline__ void mgr_fold_warp(const RoundArgs& R, uint32_t epar) {
-  const MgArgs& M = R.mg;
+  const MgArgs& M = R.L.mg;
   RoundState* rs = R.rs;
   const int q = (int)lane_id();
   uint32_t kq = (q < M.world) ? (uint32_t)ld_cg(mg_area(M, M.rank, epar, q) + 40) : 0xFFFFFFFFu;
@@ -559,7 +557,7 @@ __device__ __forceinline__ void mgr_fold_warp(const RoundArgs& R, uint32_t epar)
 // that finds a cell empty lists it.  Sender q's records start at thread q * (threads / world) of the grid: a round's few
 // thousand records per sender spread over all blocks instead of queueing on the first ones.
 __device__ __forceinline__ void mgr_collect(const RoundArgs& R, RoundSm& S, uint32_t par, uint32_t epar) {
-  const MgArgs& M = R.mg;
+  const MgArgs& M = R.L.mg;
   DevState* st = R.L.A.st;
   RoundState* rs = R.rs;
   const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
@@ -883,7 +881,7 @@ __device__ __forceinline__ void round_clear_cells(const RoundArgs& R, const Roun
       round_cells(R, F.par, js >> 1, js & 1u)[tok] = 0ull;
     }
   }
-  if (!R.mg_on) return;
+  if (!R.L.mg_on) return;
   if (!F.goverflow) {  // sharded: the global cells this block listed while summing
     const uint32_t n = min(S.gncell[F.par], R_LISTCAP);
     const uint32_t* list = round_glist(R, F.par);
@@ -974,14 +972,14 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
   }
   // sharded: exchanges completed so far (the peers' flags keep counting across launches), what the previous round may have
   // taken from the pool since the headers were written
-  unsigned long long mg_epoch = R.mg_on ? ld_cg(&st->mg_epoch) : 0ull, tie_epoch = R.mg_on ? ld_cg(&st->mg_tie_epoch) : 0ull;
+  unsigned long long mg_epoch = R.L.mg_on ? ld_cg(&st->mg_epoch) : 0ull, tie_epoch = R.L.mg_on ? ld_cg(&st->mg_tie_epoch) : 0ull;
   unsigned long long mg_prev_alloc = 0;
-  if (R.mg_on) {
+  if (R.L.mg_on) {
     // hello exchange: headers only (capacities, errors), so that the first decision is taken on global minima
     if (lead) st->mg_abort = 0;
     if (bid == 0 && warp == 0) mgr_send_warp(R, 0, (uint32_t)((mg_epoch + 1) & 1u), 0, mg_epoch + 1, true);
     if (warp == 0) {  // (in EVERY block: wait for every rank's flag, own included, then fold the headers)
-      if (lane < (uint32_t)R.mg.world) mg_wait_flag(R.mg.flag_data[R.mg.rank] + 16 * lane, mg_epoch + 1, now_ns(), 16, 128, st);
+      if (lane < (uint32_t)R.L.mg.world) mg_wait_flag(R.L.mg.flag_data[R.L.mg.rank] + 16 * lane, mg_epoch + 1, now_ns(), 16, 128, st);
       __syncwarp();
       mgr_fold_warp(R, (uint32_t)((mg_epoch + 1) & 1u));
     }
@@ -1026,11 +1024,11 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       if (tid == 1) S.ncell[par] = 0;  // (the cells the round before last listed were cleared next to the last P1)
       if (tid == 320) S.g_n_keys = ld_cg(&st->n_keys);  // (stable here: they only change in P2)
       if (tid == 321) {
-        S.caps = R.mg_on ? loop_caps_folded(st) : loop_caps(L, ld_cg(&st->pool_cursor));
+        S.caps = R.L.mg_on ? loop_caps_folded(st) : loop_caps(L, ld_cg(&st->pool_cursor));
         S.caps.new_cap = 0xFFFFFFFFu;  // the rounds keep no list of born pairs (their message headers carry the same)
       }
       if (tid == 322) S.g_snap_err = ld_cg(&st->snap_err);
-      if (tid == 323) S.g_abort = R.mg_on ? ld_cg(&st->mg_abort) : 0u;
+      if (tid == 323) S.g_abort = R.L.mg_on ? ld_cg(&st->mg_abort) : 0u;
       if (tid == 2) S.gncell[par] = 0;
       // the list of candidates is exact down to the largest LAST (RT-th best) primary any block published
       const unsigned long long Lcut = block_max_u64((tid % RT == RT - 1) ? myp : 0ull, S.red);  // (syncs inside: qn / cp are visible)
@@ -1109,7 +1107,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
                                             j == 0 ? wj : 0u, (unsigned long long)hot_pre + keys_incl, cj);
         // sharded: a rank sends one record per touched cell, at most 2 min(w_i, c_i + 1) per merge: new_keys less 2, so the batch's
         // records are at most keys_incl - 2 (j + 1), and they must fit this rank's message area in every peer's inbox
-        if (!cap_fail && R.mg_on && pj && keys_incl - 2ull * (j + 1u) > (unsigned long long)(R.mg.inbox_stride - MGR_HDR)) cap_fail = LOOP_NEED_HOST;
+        if (!cap_fail && R.L.mg_on && pj && keys_incl - 2ull * (j + 1u) > (unsigned long long)(R.L.mg.inbox_stride - MGR_HDR)) cap_fail = LOOP_NEED_HOST;
         const uint32_t mult0 = S.cm[0];
         if (status == LOOP_RUNNING) {
           const uint32_t cf0 = __shfl_sync(0xFFFFFFFFu, cap_fail, 0);
@@ -1194,13 +1192,13 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       phase_collect(t, A.len16, L.max_length, 1, L.hot, hot_pre, S.cp[0], L.cands, L.cand_cap, st, bid, nblk);
       RBARRIER();
       uint32_t tie_slot;
-      if (!R.mg_on) {
+      if (!R.L.mg_on) {
         phase_tie(A.slots, A.n, t, A.pool, L.cands, ld_cg(&st->n_cand), st, S.s_max, bid, nblk);
         RBARRIER();
         const unsigned long long tp = ld_cg(&st->tie_pos);
         tie_slot = (tp == ~0ull) ? NOSLOT : (uint32_t)(tp & 0xFFFFFFFFu);
       } else {
-        tie_slot = mg_tie_winner(L, R.mg, S.s_max, tie_epoch, [&] { RBARRIER(); });  // (rank, local position) decides
+        tie_slot = mg_tie_winner(L, S.s_max, tie_epoch, [&] { RBARRIER(); });  // (rank, local position) decides
       }
       __syncthreads();
       if (tie_slot == NOSLOT) {
@@ -1229,7 +1227,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
       if (F.k) round_clear_cells(R, S, F, tid, blockDim.x, gt, gn);
       if (lead) {
         const Best wb{S.cp[0], S.cp[0] ? S.cs[0] : NOSLOT, S.cm[0]};
-        loop_exit(t, st, status, it, c_first, &wb, R.mg_on, mg_epoch, tie_epoch);
+        loop_exit(t, st, status, it, c_first, &wb, R.L.mg_on, mg_epoch, tie_epoch);
       }
       return;
     }
@@ -1294,7 +1292,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
     RBARRIER();
     if (tid == 0) S.nstage = 0;  // (every thread of the block has read it: RBARRIER ends with __syncthreads)
     RPROF(2)
-    if (R.mg_on) {
+    if (R.L.mg_on) {
       // ================= sharded: one exchange per round =================
       // block 0 writes this rank's header (bounds, site counts, capacities, batch) into every rank's inbox, every block the
       // cells it listed as records; each block then reports to every rank's arrival counter.  No grid barrier on the way out:
@@ -1317,8 +1315,8 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         return;
       }
       RBARRIER();
-      if (bid == 0 && tid < (uint32_t)R.mg.world) {  // (used again two rounds on; the next round's records are reserved after more barriers)
-        *mgr_counter(R.mg, R.mg.rank, epar, (int)tid) = 0ull;
+      if (bid == 0 && tid < (uint32_t)R.L.mg.world) {  // (used again two rounds on; the next round's records are reserved after more barriers)
+        *mgr_counter(R.L.mg, R.L.mg.rank, epar, (int)tid) = 0ull;
         if (tid == 0) st->n_out = 0;
       }
       XPROF(2)
@@ -1328,14 +1326,14 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
     // ================= P2 =================
     // valid prefix: no pair born by an earlier merge of the batch may reach the count of a later one
     // (sharded: every rank commits at most the smallest batch any rank tried, bounds and site counts are sums over the ranks)
-    const uint32_t k_all = R.mg_on ? min(k, ld_cg(&rs->mg_k)) : k;
+    const uint32_t k_all = R.L.mg_on ? min(k, ld_cg(&rs->mg_k)) : k;
     uint32_t v = k_all;
     const uint32_t ns_all = (lane < k) ? ld_cg(&rs->n_sites[par][lane].v) : 0u;  // (requested together with the bounds and the flag)
-    const uint32_t ns_glob = R.mg_on ? ((lane < k_all) ? ld_cg(&rs->mg_ns[lane]) : 0u) : ns_all;
+    const uint32_t ns_glob = R.L.mg_on ? ((lane < k_all) ? ld_cg(&rs->mg_ns[lane]) : 0u) : ns_all;
     const uint32_t overflow = ld_cg(&rs->overflow[par]);                         // (set during P1 only)
-    const uint32_t goverflow = R.mg_on ? ld_cg(&rs->goverflow[par]) : 0u;
+    const uint32_t goverflow = R.L.mg_on ? ld_cg(&rs->goverflow[par]) : 0u;
     {
-      const unsigned long long ub2 = (lane < k_all) ? (R.mg_on ? ld_cg(&rs->mg_ub[lane]) : ld_cg(&rs->ub[par][lane].v)) : 0ull;
+      const unsigned long long ub2 = (lane < k_all) ? (R.L.mg_on ? ld_cg(&rs->mg_ub[lane]) : ld_cg(&rs->ub[par][lane].v)) : 0ull;
       const uint32_t ubv = max((uint32_t)ub2, (uint32_t)(ub2 >> 32));  // lane j: the larger of merge j's two bounds
       uint32_t run = 0;
       for (uint32_t j = 0; j + 1 < k_all; j++) {
@@ -1549,13 +1547,13 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
         // sharded: the global cell (decrements, counted occurrences: sums over the ranks) and this shard's (occurrences: its
         // list space) of one (merge, side, token), in the layout `process` reads
         auto cell_of = [&](uint32_t jj, uint32_t side, uint32_t tok) -> unsigned long long {
-          if (!R.mg_on) return ld_cg(round_cells(R, par, jj, side) + tok);
+          if (!R.L.mg_on) return ld_cg(round_cells(R, par, jj, side) + tok);
           const unsigned long long g = ld_cg(round_gcells(R, par, jj, side) + tok), l = ld_cg(round_cells(R, par, jj, side) + tok);
           return (g & R_FMASK) | ((unsigned long long)cell_len(l) << R_FIELD) | (((g >> R_FIELD) & R_FMASK) << (2 * R_FIELD));
         };
-        if (!(R.mg_on ? goverflow : overflow)) {
-          const uint32_t ncell = R.mg_on ? S.gncell[par] : S.ncell[par];
-          const uint32_t* list = R.mg_on ? round_glist(R, par) : round_list(R, par);
+        if (!(R.L.mg_on ? goverflow : overflow)) {
+          const uint32_t ncell = R.L.mg_on ? S.gncell[par] : S.ncell[par];
+          const uint32_t* list = R.L.mg_on ? round_glist(R, par) : round_list(R, par);
           if (lt == 0 && ncell) atomicAdd(S.w[0] > R_LAT ? &rs->cells_big : &rs->cells_small, (unsigned long long)ncell);
           for (uint32_t base = 0; base < ncell; base += n1t) {
             const uint32_t idx = base + lt;
@@ -1668,7 +1666,7 @@ __global__ void __launch_bounds__(RD_THREADS, 1) k_merge_rounds(RoundArgs R) {
     F.overflow = overflow;
     F.goverflow = goverflow;
     if (lead) rs->overflow[par ^ 1u] = rs->goverflow[par ^ 1u] = 0;  // (read by nobody before the next round's P2, set by nobody before its P1)
-    if (R.mg_on) {  // what this round's P2 may take from the pool on any rank: the headers of the next exchange are written before
+    if (R.L.mg_on) {  // what this round's P2 may take from the pool on any rank: the headers of the next exchange are written before
       unsigned long long wsum = 0;
       for (uint32_t j = 0; j < v; j++) wsum += S.w[j];
       mg_prev_alloc = 2ull * wsum + (unsigned long long)nblk * R_POOL_CHUNK;

@@ -1,6 +1,7 @@
 // train_kernels.cuh -- K1 (pair histogram + occurrence lists), K2 (arg-max with the reference's exact
-// tie-break) and K3 (apply merge in place with count deltas) for sm_100a, plus the persistent
-// cooperative kernel that runs the whole mergeUntil loop on the device.
+// tie-break) and K3 (apply merge in place with count deltas) for sm_100a, plus the arguments, stop chain and
+// exit record of the persistent cooperative kernel that runs the whole mergeUntil loop on the device (k_merge_loop,
+// defined after the sharded helpers at the end of mg_kernels.cuh).
 //
 // Reference semantics restated (SURVEY.md Appendix A; all citations are /root/reference/core.ts):
 //   counting  :265-310  every adjacent pair inside a document; for a == b only every other pair of a
@@ -1257,6 +1258,20 @@ __global__ void __launch_bounds__(256) k_apply(ApplyArgs A, uint32_t a, uint32_t
 constexpr int ML_THREADS = BPE_ML_THREADS;
 constexpr int ML_MIN_BLOCKS = ML_THREADS >= 1024 ? 1 : 2;
 
+// corpus sharded by document over several GPUs (mg_kernels.cuh): this rank's place and the mailboxes of the exchange
+constexpr int MG_MAX_WORLD = 8;
+struct MgArgs {
+  int rank, world;
+  uint32_t inbox_stride;  // u64 words per (parity, sender) message area, header included
+  uint32_t tie_cap;       // candidates per tie message
+  // mailboxes, indexed by rank; [rank] is this GPU's own (peers store into it), the others are peer-mapped
+  unsigned long long* flag_data[MG_MAX_WORLD];  // [world] one 128-byte line per sender
+  unsigned long long* flag_tie[MG_MAX_WORLD];
+  unsigned long long* inbox[MG_MAX_WORLD];      // [2][world][inbox_stride]
+  uint32_t* tiebox[MG_MAX_WORLD];               // [2][world][tie_cap]
+  uint32_t* tie_sorted;    // local scratch: candidates (table slots) in canonical key order
+};
+
 struct LoopArgs {
   ApplyArgs A;
   unsigned long long pool_cap;  // cells of the occurrence pool
@@ -1288,6 +1303,8 @@ struct LoopArgs {
   int prefetch;  // speculative L2 prefetch of the sites of this many runner-ups (prefetch_runner_up); BPE_LOOP_PREFETCH=0..2
   uint32_t stage_min;  // a merge whose occurrence list is longer stages its frequent neighbours' deltas per block (R_STAGE_T);
                        // k_merge_loop and k_merge_rounds, BPE_BLOCK_CELLS_MIN_SITES
+  int mg_on;           // the corpus is sharded over several GPUs: `mg` holds the exchange (zero on one GPU)
+  MgArgs mg;
 };
 
 // The capacities the host guarantees a launch, in the order of a message header's H_ERR .. H_CAND_CAP (mg_kernels.cuh) and of
@@ -1421,238 +1438,6 @@ __global__ void k_loop_prepare(DevState* st, uint32_t n_tokens, unsigned long lo
     st->n_out = 0;
     st->mg_abort = 0;
   }
-}
-
-__global__ void __launch_bounds__(ML_THREADS, ML_MIN_BLOCKS) k_merge_loop(LoopArgs L) {
-  __shared__ Best s_best[ML_THREADS / 32];
-  __shared__ uint32_t s_max[32];
-  __shared__ __align__(8) uint32_t s_stage[LS_ROWS * R_STAGE_T];  // loop_flush_stage leaves it zero (phase_fill: u64 rows)
-  for (uint32_t i = threadIdx.x; i < LS_ROWS * R_STAGE_T; i += blockDim.x) s_stage[i] = 0;
-  const ApplyArgs& A = L.A;
-  DevState* st = A.st;
-  const PairTable& t = A.t;
-  const uint32_t bid = blockIdx.x, nblk = gridDim.x;
-  unsigned long long epoch = 0;
-  const uint32_t n_tokens0 = ld_cg(&st->n_tokens);
-  const uint32_t thresh = ld_cg(&st->hot_thresh);
-
-  const bool replay = L.replay != nullptr;
-  __shared__ uint32_t s_rslot, s_wkey;
-
-  // first arg-max partials
-  if (bid == 0 && threadIdx.x == 0) st->snap_err = st->err;
-  if (!replay) {
-    Best v = best_block_reduce(argmax_stripe(t, A.len16, L.max_length, 1, L.hot, ld_cg(&st->hot_n), bid, nblk), s_best);
-    if (threadIdx.x == 0) {
-      L.partials[bid] = v;
-      L.partial_keys[bid] = v.primary ? t.keys[v.slot] : 0u;
-    }
-  }
-  grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-
-  const bool prof = (bid == 0 && threadIdx.x == 0);
-  unsigned long long tp0 = prof ? now_ns() : 0, tp1;
-#define PROF(i)                      \
-  if (prof) {                        \
-    tp1 = now_ns();                  \
-    st->prof_ns[i] += tp1 - tp0;     \
-    tp0 = tp1;                       \
-  }
-  const uint32_t gt = bid * blockDim.x + threadIdx.x, gn = nblk * blockDim.x;
-  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
-  // deferred phase_fill: the sites of the previous merge whose new adjacencies are not in their lists yet
-  uint32_t fill_n = 0;
-  const SiteRec* fill_sites = nullptr;
-  for (uint32_t it = 0;; it++) {
-    const uint32_t par = it & 1u;
-    SiteRec* const my_sites = par ? L.sites2 : A.sites;
-    // ---- every block folds the partials and takes the same decision ----
-    // n_keys, pool_cursor and hot_n only change in P2, err is snapshot by block 0 in P2: all stable here
-    Best w{0ull, NOSLOT, 0};
-    uint32_t status = LOOP_RUNNING;
-    uint32_t wa = 0, wb = 0, wcnt = 0;
-    const uint32_t c = n_tokens0 + it;
-    const uint32_t hot_pre = ld_cg(&st->hot_n);  // entries before this merge's pairs join
-    if (replay) {
-      // the logged pair; it may not occur at all (a merge whose pair is absent still appends its token, core.ts:350-354)
-      if (it < L.log_cap) {
-        wa = (uint32_t)L.replay[2 * it];
-        wb = (uint32_t)L.replay[2 * it + 1];
-        __syncthreads();
-        if (threadIdx.x == 0) s_rslot = tbl_find(t, pair_key(wa, wb));
-        __syncthreads();
-        w.slot = s_rslot;
-        w.mult = 1;
-        w.primary = 1;
-        if (w.slot != NOSLOT) wcnt = max(t.cnt[w.slot], t.occ_len[w.slot]);  // bound on the sites (the list may hold stale entries)
-      }
-    } else {
-      uint32_t my_key = 0;
-      for (uint32_t i = threadIdx.x; i < nblk; i += blockDim.x) {
-        Best pb;
-        pb.primary = ld_cg(&L.partials[i].primary);
-        pb.slot = ld_cg(&L.partials[i].slot);
-        pb.mult = ld_cg(&L.partials[i].mult);
-        const uint32_t pk = ld_cg(&L.partial_keys[i]);
-        const uint32_t before = w.slot;
-        w = best_merge(w, pb);
-        if (w.slot != before) my_key = pk;
-      }
-      const Best mine_w = w;
-      w = best_block_reduce(w, s_best);
-      if (w.primary) {  // block-uniform: the thread that holds the winning partial hands out its key
-        if (mine_w.primary == w.primary && mine_w.slot == w.slot) s_wkey = my_key;
-        __syncthreads();
-        const uint32_t key = s_wkey;
-        wa = key >> 16;
-        wb = key & 0xFFFFu;
-        wcnt = (uint32_t)(w.primary >> 20);
-      }
-    }
-    if (!replay) status = loop_stop(L, ld_cg(&st->snap_err) != 0, w.primary, wcnt, thresh, it, c);
-    else if (ld_cg(&st->snap_err)) status = LOOP_ERROR;
-    else status = (it >= L.log_cap) ? LOOP_LIMIT : (c >= L.max_tokens ? LOOP_NEED_HOST : LOOP_RUNNING);
-    PROF(0)
-    if (status == LOOP_RUNNING && w.mult > 1) {
-      // tie on (weight, a.index+b.index): the pair whose last counted occurrence comes first wins (core.ts:294-305)
-      if (w.mult > L.cand_cap) status = LOOP_NEED_HOST;
-      else {
-        if (fill_n) {  // the tie-break reads occurrence lists: those of the last merge must be complete
-          phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);
-          fill_n = 0;
-          grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-        }
-        phase_collect(t, A.len16, L.max_length, 1, L.hot, hot_pre, w.primary, L.cands, L.cand_cap, st, bid, nblk);
-        grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-        phase_tie(A.slots, A.n, t, A.pool, L.cands, ld_cg(&st->n_cand), st, s_max, bid, nblk);
-        grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-        unsigned long long tp = ld_cg(&st->tie_pos);
-        if (tp == ~0ull) status = LOOP_ERROR;
-        else {
-          uint32_t s = (uint32_t)(tp & 0xFFFFFFFFu);
-          uint32_t key = t.keys[s];
-          w.slot = s;
-          wa = key >> 16;
-          wb = key & 0xFFFFu;
-        }
-      }
-    }
-    PROF(7)
-    if (status == LOOP_RUNNING) {
-      const unsigned long long new_keys = min(2ull * wcnt + 2ull, 2ull * (c + 1ull) + 2ull);
-      status = loop_cap_status(loop_caps(L, ld_cg(&st->pool_cursor)), ld_cg(&st->n_keys), new_keys, 2ull * wcnt, wcnt,
-                               replay ? 0ull : hot_pre + new_keys, c);  // (replayed merges do not feed the hot list)
-    }
-    if (status != LOOP_RUNNING) {
-      if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);  // the kernel leaves every list complete
-      if (bid == 0 && threadIdx.x == 0) {
-        loop_exit(t, st, status, it, c, replay ? nullptr : &w);
-        if (replay) {
-          st->best_primary = 0;
-          st->best_cnt = wcnt;  // what the host must make room for
-          st->best_mult = 1;
-        }
-      }
-      return;
-    }
-    if (fill_n && it && (wa == c - 1u || wb == c - 1u)) {
-      // the winner was born by the previous merge: its list is exactly what fill(t-1) still has to write
-      phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);
-      fill_n = 0;
-      grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-    }
-    // ---- P1: sites + deltas, next to the list filling of the previous merge ----
-    if (bid == 0 && threadIdx.x == 0) {
-      A.len16[c] = A.len16[wa] + A.len16[wb];  // chars = a.chars + b.chars (:318)
-      MergeRec r;
-      r.a = (int32_t)wa;
-      r.b = (int32_t)wb;
-      r.c = (int32_t)c;
-      r.reserved = 0;
-      r.weight = (long long)wcnt;
-      L.log[it] = r;
-      st->n_sites[par ^ 1u] = 0;
-      st->n_new[par ^ 1u] = 0;
-      if (w.mult > 1) st->tie_breaks++;
-    }
-    if (fill_n <= 8192u && wcnt <= 16384u && blockDim.x == 512u) {
-      // latency bound: 12 warps of every block walk the sites, 4 fill the lists of the last merge and then warm the L2
-      // for the next one
-      const uint32_t ws = L.p1_sites, wh = 16u - ws;
-      if (warp < ws) {
-        phase_sites(A, wa, wb, c, par, w.slot, (bid * ws + warp) * 32 + lane, nblk * ws * 32, my_sites);
-      } else {
-        if (fill_n) phase_fill(A, fill_n, (bid * wh + warp - ws) * 32 + lane, nblk * wh * 32, fill_sites);
-        if (L.prefetch && !replay) prefetch_runner_up(L, w.slot, nblk, (bid * wh + warp - ws) * 32 + lane, nblk * wh * 32);
-      }
-    } else {
-      // (the list length is block-uniform: nothing writes occ_len between P2's barrier and the next P2)
-      const bool staged = w.slot != NOSLOT && t.occ_len[w.slot] > L.stage_min;
-      if (fill_n) phase_fill(A, fill_n, gt, gn, fill_sites, fill_n > L.stage_min ? s_stage : nullptr);
-      phase_sites(A, wa, wb, c, par, w.slot, gt, gn, my_sites, staged ? s_stage : nullptr);
-      if (staged) loop_flush_stage(A, s_stage, wa, wb);
-    }
-    fill_n = 0;
-#ifdef BPE_FINE_PROF
-    const int bkt = 31 - __clz(wcnt | 1u);
-    if (prof) {
-      st->bucket_ns[bkt][0] += now_ns() - tp0;
-      st->bucket_ns[bkt][3] += 1;
-    }
-#endif
-    PROF(1)
-    grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-    PROF(2)
-    // ---- P2: the born pairs (table, list space, hot list, arg-max), the corpus rewrite, the arg-max over the old hot pairs ----
-    if (bid == 0 && threadIdx.x == 0) {
-      st->n_cand = 0;
-      st->tie_pos = ~0ull;
-      st->snap_err = st->err;  // what every block will act on at the next decision (errors of this phase: one merge later)
-      if (w.slot != NOSLOT) t.cnt[w.slot] = 0;  // every counted occurrence of the winner is being replaced (no delta of P1
-                                                // touches the winner's own pair); the arg-max below skips the slot
-      if (replay) L.log[it].weight = (long long)st->n_sites[par];  // replacements performed (bpe_apply_merge's n_replaced)
-    }
-    const uint32_t n_sites_now = ld_cg(&st->n_sites[par]);
-    Best mine{0ull, NOSLOT, 0};
-    uint32_t mine_key = 0;
-    {
-      // Three independent jobs.  Small merges are latency bound, so the warps of every block split up (p2_new / p2_rw / rest) and the
-      // three dependency chains run side by side; big merges keep every thread on every job.
-      const bool split = n_sites_now <= 16384u && blockDim.x == 512u;
-      const uint32_t wn = L.p2_new, wr = L.p2_rw, wm = 16u - wn - wr;
-      if (!split || warp < wn)
-        phase_new_pairs(A, c, A.len16, L.max_length, replay ? 0 : 1, L.hot, L.hot_cap, L.pool_cap, false,
-                        split ? (bid * wn + warp) * 32 + lane : gt, split ? nblk * wn * 32 : gn, &mine, &mine_key);
-      if (!split || (warp >= wn && warp < wn + wr))
-        phase_rewrite(A, c, n_sites_now, split ? (bid * wr + warp - wn) * 32 + lane : gt, split ? nblk * wr * 32 : gn, my_sites);
-      if (!replay && (!split || warp >= wn + wr)) {
-        for (uint32_t i = split ? (bid * wm + warp - wn - wr) * 32 + lane : gt; i < hot_pre; i += split ? nblk * wm * 32 : gn) {
-          uint32_t hs = L.hot[i], hk;
-          if (hs == w.slot) continue;  // the winner's count is being zeroed
-          unsigned long long pr = slot_primary_k(t, A.len16, hs, L.max_length, &hk);
-          if (pr) {
-            const uint32_t before = mine.slot;
-            mine = best_merge(mine, Best{pr, hs, 1});
-            if (mine.slot != before) mine_key = hk;
-          }
-        }
-      }
-    }
-    if (!replay) {
-      Best v = best_block_reduce(mine, s_best);
-      if (threadIdx.x == 0) L.partials[bid] = v;
-      if (mine.primary == v.primary && mine.slot == v.slot) L.partial_keys[bid] = mine_key;  // the owner of the block's best
-    }
-    fill_n = n_sites_now;
-    fill_sites = my_sites;
-#ifdef BPE_FINE_PROF
-    if (prof) st->bucket_ns[bkt][1] += now_ns() - tp0;
-#endif
-    PROF(3)
-    grid_barrier(L.barrier, ++epoch * nblk, L.bar_ns);
-    PROF(4)
-  }
-#undef PROF
 }
 
 // ------------------------------------------------------------------------------------------------

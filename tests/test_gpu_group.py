@@ -11,7 +11,7 @@ import pytest
 from bpe_tokenizer_b200 import _abi
 
 SIZES = pytest.mark.parametrize("members", ["2", "up to 4"])
-# every size with the default loop, and again with BPE_LOOP_ROUNDS=0: then k_merge_loop_mg runs every merge, where by default
+# every size with the default loop, and again with BPE_LOOP_ROUNDS=0: then the sharded k_merge_loop runs every merge, where by default
 # it only takes those above 2^20 global sites, which these corpora never reach
 _LOOPS = [("2", None), ("up to 4", None), ("2", "0"), ("up to 4", "0")]
 SIZES_LOOPS = pytest.mark.parametrize("members,loop_rounds", _LOOPS, ids=[m if r is None else m + "-rounds0" for m, r in _LOOPS])

@@ -1,4 +1,4 @@
-"""GPU: the sharded merge kernels (k_merge_rounds with mg_on, k_merge_loop_mg) at the limits test_gpu_block_cells and
+"""GPU: the sharded merge kernels (k_merge_rounds and k_merge_loop with mg_on) at the limits test_gpu_block_cells and
 test_gpu_loop_stage pin for one GPU: staged cells and their exchange, a full list of touched cells (locally, or only once the
 ranks' records are summed), the records of a round against the inbox, position tie-breaks across ranks, the tie mailbox, the
 hand-off of merges above R_HUGE global sites, the born-pair cut and the last token indices.  A device group (bpe_create_group)
@@ -301,7 +301,7 @@ def test_group_tie_mailbox(monkeypatch):
     grp.close()
 
 
-# ---- merges above R_HUGE global sites: the decision on global counts, k_merge_loop_mg, and back ----
+# ---- merges above R_HUGE global sites: the decision on global counts, the sharded k_merge_loop, and back ----
 def test_group_giant_merge_on_global_counts(monkeypatch):
     """1.1 M sites of (0, 1) split over two members: neither holds more than R_HUGE, the corpus does."""
     devs = _devices(2, monkeypatch)

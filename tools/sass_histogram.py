@@ -46,7 +46,7 @@ for k, c in kernels.items():
         row.append(str(sum(v for op, v in c.items() if re.search(pat, op))))
     print("| `%s` | %d | %s |" % (k, total, " | ".join(row)))
 print("\n## Full opcode lists of the hot kernels\n")
-for k in ("k_merge_rounds", "k_merge_loop", "k_merge_loop_mg", "k_encode_lanes<20, 16>", "k_hist", "k_scatter"):
+for k in ("k_merge_rounds", "k_merge_loop", "k_encode_lanes<20, 16>", "k_hist", "k_scatter"):
     for name, c in kernels.items():
         if name.startswith(k.split("<")[0]) and (k == name or "<" not in k):
             print("**`%s`**: " % name + ", ".join("%s x%d" % (op, v) for op, v in c.most_common(40)) + "\n")
